@@ -2,6 +2,7 @@
 """bench.py -- throughput of the MALVA genotyping hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload wg|wg3|small]
+                    [--dump-outputs DIR]
 
 Metric (BASELINE.json): sample k-mers/sec through the Bloom-filter + signature count (headline `value`),
 with variants genotyped/sec reported beside it.  One "step" = one pass of the call-side hot path over one
@@ -270,6 +271,30 @@ def profile_json(name):
         return json.load(open(os.path.join(ROOT, "profiles", name)))
     except Exception:
         return {}
+
+
+DUMP_MAX_VARIANTS = 1 << 19   # ~40 MB of float64 with their alleles: under 64 MB at every workload
+
+
+def dump_outputs(out_dir, d, vao):
+    """What the last timed step returned to its caller (per-allele coverage, per-variant n_gts / status / GT / GQ) as
+    float64 .npy files, so that two builds can be compared output for output.  Above DUMP_MAX_VARIANTS variants a
+    fixed, seeded sample of them is written (with all their alleles); variant_index / allele_index name the rows."""
+    nv = len(vao) - 1
+    if nv > DUMP_MAX_VARIANTS:
+        vi = np.sort(np.random.default_rng(SEED + 1000).choice(nv, DUMP_MAX_VARIANTS, replace=False))
+    else:
+        vi = np.arange(nv)
+    lo = vao[vi].astype(np.int64)
+    n = vao[vi + 1].astype(np.int64) - lo
+    ai = np.arange(int(n.sum())) - np.repeat(np.cumsum(n) - n, n) + np.repeat(lo, n)
+    out = {"variant_index": vi, "allele_index": ai, "cov": d["cov"].cpu().numpy()[ai]}
+    for name in ("n_gts", "status", "best_gt", "gq"):
+        out[name] = d[name].cpu().numpy()[vi]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
+    log(f"outputs of the last timed step ({len(vi)} of {nv} variants, {len(ai)} alleles) written to {out_dir}")
 
 
 def bind_to_gpu_numa(local_rank):
@@ -698,6 +723,8 @@ def run_ours(args, wl, rank, local_rank, world):
     clocks = sampler.stop()
     launches = g.launch_count() - launches0
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, d, vb["vao"])
     scan_ms = [g.event_elapsed_ms(10 + 2 * j, 11 + 2 * j) for j in range(min(8, args.steps))]
     geno_ms = g.genotype_kernel_ms() if rank == 0 else None
     tm = torch.tensor([region_ms], dtype=torch.float64, device=dev)
@@ -774,7 +801,7 @@ def run_ours(args, wl, rank, local_rank, world):
         del src, dst
 
         def e2e_leg(scan):
-            steps = max(3, min(args.steps, 6))
+            steps = args.steps
             scan()
             g.genotype_packed_host(h_ptrs, nv, 0, ERR, MAX_COV, False)
             if world > 1:
@@ -929,7 +956,14 @@ def main():
     ap.add_argument("--verify", action="store_true",
                     help="N > 1: every rank scans the same batches; checks that the NCCL-reduced counters are exactly "
                          "N x one rank's (replicas are identical, the reduce is exact)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (coverages, GT, GQ; a seeded sample of the variants "
+                         "at large workloads) as DIR/<name>.npy, float64")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm times the sample scan alone, which returns nothing to its caller")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -1,6 +1,7 @@
 """TEST INFRASTRUCTURE ONLY -- ctypes loaders for the parity checkers.
 
 ``oracle()``  -> oracle/liboracle.so        (plain-C restatement, malva_oracle.c)
+``kmc_shim()`` -> oracle/libkmc_shim.so     (the stand-in CKMCFile, kmc_shim_hooks.cpp)
 ``ref()``     -> oracle/_ref/libmalva_ref.so (the reference's own classes, hooks in
                                             ref_hooks.cpp; built only where
                                             /root/reference exists, shipped prebuilt)
@@ -16,6 +17,7 @@ import subprocess
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ORACLE_SO = os.path.join(HERE, "liboracle.so")
+KMC_SHIM_SO = os.path.join(HERE, "libkmc_shim.so")
 REF_SO = os.path.join(HERE, "_ref", "libmalva_ref.so")
 REF_BIN = os.path.join(HERE, "_ref", "malva-geno-ref")
 
@@ -28,10 +30,11 @@ _intp = C.POINTER(C.c_int)
 
 
 def build(force: bool = False) -> None:
-    """Compile liboracle.so (and _ref/ when /root/reference is present)."""
+    """Compile liboracle.so, libkmc_shim.so (and _ref/ where the reference's sources are present: Makefile REF)."""
     if force or not os.path.exists(ORACLE_SO) or \
             os.path.getmtime(ORACLE_SO) < os.path.getmtime(os.path.join(HERE, "malva_oracle.c")):
         subprocess.check_call(["make", "-C", HERE, "liboracle.so"], stdout=subprocess.DEVNULL)
+    subprocess.check_call(["make", "-C", HERE, "libkmc_shim.so"], stdout=subprocess.DEVNULL)
     subprocess.check_call(["make", "-C", HERE, "ref"], stdout=subprocess.DEVNULL)
 
 
@@ -87,6 +90,13 @@ def oracle() -> C.CDLL:
     return L
 
 
+def kmc_shim() -> C.CDLL:
+    L = C.CDLL(KMC_SHIM_SO)
+    L.shim_kmc_list.restype = C.c_long
+    L.shim_kmc_list.argtypes = [C.c_char_p, _u64p, C.c_char_p, C.c_long]
+    return L
+
+
 def have_ref() -> bool:
     return os.path.exists(REF_SO) and os.path.exists(REF_BIN)
 
@@ -119,8 +129,6 @@ def ref() -> C.CDLL:
     L.ref_add_packed.argtypes = [C.c_void_p, C.c_void_p, _u64p, _u8p, C.c_uint64, C.c_int]
     L.ref_scan_packed.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, _u64p, _u32p, C.c_uint64, C.c_int, C.c_int]
     L.ref_reference_pass.argtypes = [C.c_void_p, C.c_void_p, C.c_char_p, C.c_int, C.c_int]
-    L.ref_kmc_list.restype = C.c_long
-    L.ref_kmc_list.argtypes = [C.c_char_p, _u64p, C.c_char_p, C.c_long]
     L.ref_get_counts_packed.argtypes = [C.c_void_p, C.c_void_p, _u64p, _u8p, C.c_uint64, C.c_int, C.POINTER(C.c_int32)]
     L.ref_genotype_batch.restype = C.c_uint64
     L.ref_genotype_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, _u32p, _u32p, _u32p, _u64p, _f32p, C.c_int,

@@ -171,36 +171,6 @@ uint64_t ref_genotype_batch(void *bf_, void *ref_bf_, uint64_t n_variants, const
   return sum;
 }
 
-// ---- KMC listing as call_main drives it (main.cpp:444-449, 482-490), through the stand-in CKMCFile -------------
-// Writes "KMER\tCOUNT\n" lines; returns the text length (negative: buffer too small), -1 if the database cannot
-// be opened.  info[0..7] = kmer_length, mode, counter_size, lut_prefix_length, signature_len, min_count, max_count,
-// total_kmers as CKMCFile::Info reports them.
-long ref_kmc_list(const char *prefix, uint64_t *info, char *out, long out_cap) {
-  CKMCFile db;
-  if (!db.OpenForListing(prefix)) return -1;
-  uint32 klen, mode, csz, lpl, sl, minc;
-  uint64 maxc, total;
-  db.Info(klen, mode, csz, lpl, sl, minc, maxc, total);
-  if (info) {
-    info[0] = klen, info[1] = mode, info[2] = csz, info[3] = lpl, info[4] = sl, info[5] = minc, info[6] = maxc,
-    info[7] = total;
-  }
-  CKmerAPI kmer_obj(klen);
-  std::string res;
-  uint32 counter;
-  std::vector<char> context(klen + 1);
-  while (db.ReadNextKmer(kmer_obj, counter)) {
-    kmer_obj.to_string(context.data());
-    res.append(context.data(), klen);
-    res += '\t';
-    res += std::to_string(counter);
-    res += '\n';
-  }
-  if ((long)res.size() + 1 > out_cap) return -(long)res.size() - 2;
-  memcpy(out, res.c_str(), res.size() + 1);
-  return (long)res.size();
-}
-
 // ---- reference rolling pass over one contig (main.cpp:385-400) ---------------
 void ref_reference_pass(void *bf_, void *context_bf_, const char *seq, int k_, int ref_k_) {
   BF &bf = *(BF *)bf_;

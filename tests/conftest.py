@@ -23,13 +23,13 @@ def oracle_lib():
 
 
 @pytest.fixture(scope="session")
-def ref_lib():
+def ref_or_none():
+    """the reference's own classes (oracle/_ref) where they are built, else None: tests that take this fixture then
+    check against data stored under tests/golden"""
     from oracle import pyoracle
 
     pyoracle.build()
-    if not pyoracle.have_ref():
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
-    return pyoracle.ref()
+    return pyoracle.ref() if pyoracle.have_ref() else None
 
 
 @pytest.fixture(scope="session", autouse=True)

@@ -3,6 +3,9 @@ model (oracle/liboracle.so) of one malva-geno run that mirrors MalvaGpu call for
 from __future__ import annotations
 
 import ctypes as C
+import hashlib
+import json
+import os
 import random
 from typing import List, Sequence
 
@@ -16,6 +19,54 @@ u32p = C.POINTER(C.c_uint32)
 u8p = C.POINTER(C.c_uint8)
 f32p = C.POINTER(C.c_float)
 f64p = C.POINTER(C.c_double)
+
+
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+
+
+def check_digest(name: str, key: str, digest: str, live: bool, what: str = "") -> None:
+    """Results that are compared with the reference's own code (oracle/_ref) where it is built are also pinned by
+    their SHA-256, stored under `key` in tests/golden/<name>.json: checked here when the live comparison cannot run
+    (live False).  MALVA_RECORD_DIGESTS=1 stores the digest instead."""
+    path = os.path.join(GOLDEN, name + ".json")
+    digests = json.load(open(path)) if os.path.exists(path) else {}
+    if os.environ.get("MALVA_RECORD_DIGESTS"):
+        digests[key] = digest
+        with open(path, "w") as fh:
+            json.dump(digests, fh, indent=0, sort_keys=True)
+    elif not live:
+        assert key in digests, f"no stored digest for {key} in {path}"
+        assert digest == digests[key], f"{key}: results differ from the stored ones {what}"
+
+
+class NoRef:
+    """Stands in for oracle/_ref where it is not built: every hook does nothing and returns None."""
+
+    def __getattr__(self, name):
+        return lambda *a: None
+
+
+class Agree:
+    """oracle value == the reference's value, live where oracle/_ref is built (ref_lib not None); the oracle's values
+    are hashed in order either way and done() checks the digest with check_digest (file oracle_vs_reference)."""
+
+    def __init__(self, key: str, ref_lib):
+        self.key, self.live = key, ref_lib is not None
+        self.L = ref_lib if self.live else NoRef()
+        self.h, self.n = hashlib.sha256(), 0
+
+    def record(self, *values) -> None:
+        for v in values:
+            self.h.update(v.tobytes() if isinstance(v, np.ndarray) else repr(v).encode())
+        self.n += 1
+
+    def eq(self, mine, theirs, msg=None) -> None:
+        if self.live:
+            assert mine == theirs, msg
+        self.record(mine)
+
+    def done(self) -> None:
+        check_digest("oracle_vs_reference", self.key, self.h.hexdigest(), self.live, f"({self.n} checks)")
 
 
 def rand_seq(rng: random.Random, n: int, alpha: str = "ACGT") -> str:

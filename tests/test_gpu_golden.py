@@ -3,8 +3,8 @@
 Inputs/outputs are the committed fixtures of tests/golden/haploid (made by tests/golden/make_golden.py):
 the GPU index + scan + genotype must reproduce COVS, GT, GQ and the printed GTS of every record of the
 verbose golden (produced by the shim-built reference; its GT:GQ equal example/haploid.malva.vcf).
-Signatures are enumerated by the reference's own VB::extract_kmers (oracle/_ref hook), so this pins
-kernels K1-K5 and the C ABI, not the (host-kept) enumeration."""
+Signatures are enumerated by the reference's own VB::extract_kmers (oracle/_ref hook) where it is built, so this
+pins kernels K1-K5 and the C ABI, not the (host-kept) enumeration; elsewhere by `malva-geno signatures`."""
 import pytest
 
 import golden_flow
@@ -13,7 +13,7 @@ from malva_b200 import MalvaGpu
 pytestmark = pytest.mark.gpu
 
 
-def test_haploid_example_golden_on_gpu(ref_lib):
+def test_haploid_example_golden_on_gpu(ref_or_none):
     g = MalvaGpu(k=35, ref_k=43, bf_bits=1 << 33)  # -b 1, as in the README command
 
     def genotype(batch):
@@ -25,7 +25,7 @@ def test_haploid_example_golden_on_gpu(ref_lib):
         return r.cov, out
 
     try:
-        lines = golden_flow.run_haploid_example(g, ref_lib, genotype)
+        lines = golden_flow.run_haploid_example(g, ref_or_none, genotype)
         assert g.popcount(0) == 422 and g.kmap_size() == 679  # SURVEY 8: bundled example sizes
     finally:
         g.close()

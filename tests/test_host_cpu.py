@@ -1,6 +1,7 @@
 """Host logic of the malva-geno CLI (malva_b200/csrc/host), checked on CPU against the reference's own
 VB::extract_kmers (oracle/_ref hook) and block grouping rules: `malva-geno signatures` prints what the CLI would
 send to the device for every var_block.  No GPU involved (the signatures sub-command never touches CUDA)."""
+import hashlib
 import os
 import re
 import subprocess
@@ -10,6 +11,7 @@ import pytest
 import synth
 import vcf_blocks
 from malva_b200 import build as mbuild
+from parity_util import check_digest
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "haploid")
 
@@ -63,17 +65,38 @@ def expected_signatures(ref_lib, fa, vcf, k, haploid, freq_key, uniform, index_m
     return blocks, used
 
 
-def test_signatures_haploid_example(cli, ref_lib):
+def signatures_digest(blocks, used):
+    h = hashlib.sha256()
+    for b in sorted(blocks):
+        for key in sorted(blocks[b]):
+            h.update(repr((b, key, sorted(blocks[b][key]))).encode())
+    h.update(repr(used).encode())
+    return h.hexdigest()
+
+
+def assert_reference_enumeration(ref_lib, key, got, used, *args, **kw):
+    """`malva-geno signatures` (got, used) against the reference's VB::extract_kmers on the same files: live through
+    oracle/_ref where it is built, else against the digest stored under `key` in tests/golden/signatures.json"""
+    if ref_lib is not None:
+        exp, exp_used = expected_signatures(ref_lib, *args, **kw)
+        assert set(got) == set(exp), f"{key}: different set of blocks with signatures"
+        for b in exp:
+            assert got[b] == exp[b], f"{key}: block {b} differs"
+        assert used == exp_used, key
+    n = sum(len(v) for blk in got.values() for v in blk.values())
+    check_digest("signatures", key, signatures_digest(got, used), ref_lib is not None, f"({n} signatures, {len(got)} blocks)")
+
+
+def test_signatures_haploid_example(cli, ref_or_none):
     fa, vcf = os.path.join(GOLD, "haploid.fa"), os.path.join(GOLD, "haploid.vcf.gz")
     for index_mode in (True, False):
         got, used = cli_signatures(cli, fa, vcf, ["-1"], index_mode)
-        exp, exp_used = expected_signatures(ref_lib, fa, vcf, 35, True, "AF", False, index_mode)
-        assert got == exp
-        assert used == exp_used
+        assert_reference_enumeration(ref_or_none, f"haploid_example/index_mode={index_mode}", got, used,
+                                     fa, vcf, 35, True, "AF", False, index_mode)
 
 
 @pytest.mark.parametrize("case", synth.CASES, ids=[c.name for c in synth.CASES])
-def test_signatures_synthetic(cli, ref_lib, case, tmp_path):
+def test_signatures_synthetic(cli, ref_or_none, case, tmp_path):
     fa, vcf, _, _ = synth.build_case(case, str(tmp_path))
     uniform = "-u" in case.flags
     if case.sample_subset:
@@ -87,9 +110,9 @@ def test_signatures_synthetic(cli, ref_lib, case, tmp_path):
         # ... and against VB::extract_kmers fed with the kept columns (header order, whatever the order of the list)
         for index_mode in (True, False):
             got, used = cli_signatures(cli, fa, vcf, ["-u", "-s", lst], index_mode)
-            exp, exp_used = expected_signatures(ref_lib, fa, vcf, case.k, case.haploid, case.freq_key, True, index_mode,
-                                                strip_chr=case.chr_prefix, sample_cols=sorted(case.sample_subset))
-            assert got == exp and used == exp_used
+            assert_reference_enumeration(ref_or_none, f"synthetic/{case.name}/index_mode={index_mode}", got, used,
+                                         fa, vcf, case.k, case.haploid, case.freq_key, True, index_mode,
+                                         strip_chr=case.chr_prefix, sample_cols=sorted(case.sample_subset))
         return
     sig_flags = [f for f in case.flags]
     # only the flags the enumeration depends on
@@ -103,13 +126,10 @@ def test_signatures_synthetic(cli, ref_lib, case, tmp_path):
             keep.append(f)
     for index_mode in (True, False):
         got, used = cli_signatures(cli, fa, vcf, keep, index_mode)
-        exp, exp_used = expected_signatures(ref_lib, fa, vcf, case.k, case.haploid, case.freq_key, uniform, index_mode,
-                                            strip_chr=case.chr_prefix)
-        assert set(got) == set(exp), "different set of blocks with signatures"
-        for b in exp:
-            assert got[b] == exp[b], f"block {b} differs"
-        assert used == exp_used
-        assert sum(len(v) for v in exp.values()) > 100
+        assert_reference_enumeration(ref_or_none, f"synthetic/{case.name}/index_mode={index_mode}", got, used,
+                                     fa, vcf, case.k, case.haploid, case.freq_key, uniform, index_mode,
+                                     strip_chr=case.chr_prefix)
+        assert sum(len(v) for v in got.values()) > 100
 
 
 def test_cli_usage_errors(cli):
@@ -187,7 +207,7 @@ def test_kmc_dump_lists_what_the_python_reader_lists(cli, tmp_path):
     assert r.returncode == 1 and "cannot open" in r.stderr
 
 
-def test_signatures_fuzz_small_blocks(cli, ref_lib, tmp_path):
+def test_signatures_fuzz_small_blocks(cli, ref_or_none, tmp_path):
     """many small random VCFs (dense clusters, 20 % multi-allelic, symbolic and long alleles, 1-9 samples, haploid and
     diploid, k from 15 to 35): enumeration == VB::extract_kmers in both grouping modes"""
     import random
@@ -206,8 +226,8 @@ def test_signatures_fuzz_small_blocks(cli, ref_lib, tmp_path):
         flags = (["-1"] if haploid else []) + ["-k", str(k)]
         for index_mode in (True, False):
             got, used = cli_signatures(cli, fa, vcf, flags, index_mode)
-            exp, exp_used = expected_signatures(ref_lib, fa, vcf, k, haploid, "AF", False, index_mode)
-            assert got == exp and used == exp_used, f"seed {seed} index_mode {index_mode}"
+            assert_reference_enumeration(ref_or_none, f"fuzz_small_blocks/seed={seed}/index_mode={index_mode}", got, used,
+                                         fa, vcf, k, haploid, "AF", False, index_mode)
 
 
 def test_index_file_roundtrip(tmp_path):
@@ -322,7 +342,7 @@ def test_sample_list_errors_and_subset(cli, tmp_path):
 
 
 @pytest.mark.parametrize("haploid", [False, True])
-def test_signatures_many_samples(cli, ref_lib, tmp_path, haploid):
+def test_signatures_many_samples(cli, ref_or_none, tmp_path, haploid):
     """400 panel samples (hundreds of distinct genotype patterns per block: the sample-class hash set grows), dense
     variants, unphased and missing genotypes"""
     import random
@@ -358,9 +378,9 @@ def test_signatures_many_samples(cli, ref_lib, tmp_path, haploid):
     flags = ["-1"] if haploid else []
     for index_mode in (True, False):
         got, used = cli_signatures(cli, fa, vcf, flags, index_mode)
-        exp, exp_used = expected_signatures(ref_lib, fa, vcf, 35, haploid, "AF", False, index_mode)
-        assert got == exp and used == exp_used
-        assert sum(len(v) for b in exp.values() for v in b.values()) > 2000
+        assert_reference_enumeration(ref_or_none, f"many_samples/haploid={haploid}/index_mode={index_mode}", got, used,
+                                     fa, vcf, 35, haploid, "AF", False, index_mode)
+        assert sum(len(v) for b in got.values() for v in b.values()) > 2000
 
 
 # ---- short cuts of the VCF reader (block-parallel BGZF inflate, fixed-stride GT columns) against its general paths --------
@@ -435,7 +455,7 @@ def test_bgzf_reader_equals_gzip_reader(cli, tmp_path):
 
 @pytest.mark.parametrize("haploid", [False, True])
 @pytest.mark.parametrize("n_samples", [1, 2, 3, 5, 17, 64, 131])
-def test_fixed_stride_gt_columns_equal_general_decode(cli, ref_lib, tmp_path, haploid, n_samples):
+def test_fixed_stride_gt_columns_equal_general_decode(cli, ref_or_none, tmp_path, haploid, n_samples):
     """FORMAT = GT with one-symbol alleles takes the fixed-stride decode (vcf_io.hpp fast_gt_columns); the result is
     what the general decode gives and what the reference's Variant / VB::extract_kmers give (variant.hpp:158-211),
     for every mix the short cut has to get right or hand back: phased / unphased / mostly-unphased rows, missing
@@ -491,15 +511,15 @@ def test_fixed_stride_gt_columns_equal_general_decode(cli, ref_lib, tmp_path, ha
             assert a.stdout == b.stdout, (name, fl)
         if name in ("half", "but_first"):   # and what the reference's own enumeration gives for the kept columns
             got, used = cli_signatures(cli, fa, vcf, flags + ["-s", str(lst)], False)
-            exp, exp_used = expected_signatures(ref_lib, fa, vcf, 35, haploid, "AF", False, False, sample_cols=cols)
-            assert got == exp and used == exp_used, name
+            assert_reference_enumeration(ref_or_none, f"fixed_stride/haploid={haploid}/n_samples={n_samples}/{name}",
+                                         got, used, fa, vcf, 35, haploid, "AF", False, False, sample_cols=cols)
     tr = subprocess.run([cli, "signatures", "--trace"] + flags + [fa, vcf], capture_output=True, text=True, check=True).stderr
     took, rows = map(int, re.search(r"fixed-stride GT decode: (\d+) of (\d+) rows", tr).groups())
     assert 0.8 * len(recs) <= rows <= len(recs) and took < rows
     assert n_samples < 5 or took >= rows // 3             # both ways are exercised by the file
     got, used = cli_signatures(cli, fa, vcf, flags, False)
-    exp, exp_used = expected_signatures(ref_lib, fa, vcf, 35, haploid, "AF", False, False)
-    assert got == exp and used == exp_used
+    assert_reference_enumeration(ref_or_none, f"fixed_stride/haploid={haploid}/n_samples={n_samples}/all", got, used,
+                                 fa, vcf, 35, haploid, "AF", False, False)
 
 
 def test_sars_cov2_panel_fast_and_general_decode_agree(cli):
@@ -527,7 +547,7 @@ def test_small_containers_equal_std_vector(cli):
     assert r.returncode == 0 and " 0 differ" in r.stdout, r.stdout + r.stderr
 
 
-def test_sars_cov2_panel_against_the_reference_enumeration(cli, ref_lib, tmp_path):
+def test_sars_cov2_panel_against_the_reference_enumeration(cli, ref_or_none, tmp_path):
     """BASELINE config 1's real VCF -- 15,154 records in ONE var_block (every other base of the genome has a variant:
     chains of ~19 members) -- with 400 of its 27,934 haploid samples (the reference's own enumeration needs ~12 s for
     these; 5 minutes for all): malva-geno signatures == VB::extract_kmers, block by block, allele by allele"""
@@ -543,9 +563,9 @@ def test_sars_cov2_panel_against_the_reference_enumeration(cli, ref_lib, tmp_pat
     lst = tmp_path / "kept.txt"
     lst.write_text("".join(names[i] + "\n" for i in cols))
     got, used = cli_signatures(cli, fa, vcf, ["-1", "-s", str(lst)], False)
-    exp, exp_used = expected_signatures(ref_lib, fa, vcf, 35, True, "AF", False, False, sample_cols=cols)
-    assert got == exp and used == exp_used
-    assert sum(len(v) for b in exp.values() for v in b.values()) > 30_000
+    assert_reference_enumeration(ref_or_none, "sars_cov2_panel_400", got, used, fa, vcf, 35, True, "AF", False, False,
+                                 sample_cols=cols)
+    assert sum(len(v) for b in got.values() for v in b.values()) > 30_000
 
 
 def test_error_in_a_later_batch_ends_the_pipeline(cli, tmp_path):

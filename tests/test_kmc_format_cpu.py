@@ -3,7 +3,7 @@
 No `kmc` binary and no KMC-written database exist in the build image, so what is checked here is that the THREE
 independent readers of this repository -- the Python reader (malva_b200/kmc.py), the C++ host reader
 (csrc/host/kmc_db.hpp, through `malva-geno kmc-dump`) and the stand-in CKMCFile the reference's own main.cpp is
-compiled against (oracle/shim/kmc_file.h, through the ref_kmc_list hook, driven exactly like main.cpp:482-490) --
+compiled against (oracle/shim/kmc_file.h, through the shim_kmc_list hook, driven exactly like main.cpp:482-490) --
 agree with each other and with the semantics the KMC API documents, over every header variant the format allows:
 counter_size 1-4, both_strands stored inverted, lut_prefix_len 1-9, KMC1 ("version 0") and KMC2/3 (0x200) headers,
 one and several bins, min_count / max_count filtering in ReadNextKmer (a 64-bit max_count split over two header
@@ -41,11 +41,11 @@ def _dump_cli(cli, prefix):
     return [(l.split("\t")[0], int(l.split("\t")[1])) for l in out.splitlines()]
 
 
-def _dump_shim(ref_lib, prefix):
+def _dump_shim(shim, prefix):
     cap = 1 << 24
     buf = C.create_string_buffer(cap)
     info = (C.c_uint64 * 8)()
-    n = ref_lib.ref_kmc_list(prefix.encode(), info, buf, cap)
+    n = shim.shim_kmc_list(prefix.encode(), info, buf, cap)
     assert n >= 0, n
     lines = buf.value.decode().splitlines()
     return [(l.split("\t")[0], int(l.split("\t")[1])) for l in lines], list(info)
@@ -75,8 +75,16 @@ def cli():
     return mbuild.CLI
 
 
+@pytest.fixture(scope="module")
+def shim():
+    from oracle import pyoracle
+
+    pyoracle.build()
+    return pyoracle.kmc_shim()
+
+
 @pytest.mark.parametrize("k,p,version,csz,both,minc,maxc", CASES)
-def test_three_readers_agree(cli, ref_lib, tmp_path, k, p, version, csz, both, minc, maxc):
+def test_three_readers_agree(cli, shim, tmp_path, k, p, version, csz, both, minc, maxc):
     rng = random.Random(k * 1000 + p * 10 + csz)
     packed, counts = _records(rng, k, 600, csz)
     prefix = str(tmp_path / "db")
@@ -89,7 +97,7 @@ def test_three_readers_agree(cli, ref_lib, tmp_path, k, p, version, csz, both, m
     assert k_py == k
     assert list(zip(kmc.packed_to_strings(got_py, k), [int(c) for c in cts_py])) == exp
     assert _dump_cli(cli, prefix) == exp
-    got_shim, info = _dump_shim(ref_lib, prefix)
+    got_shim, info = _dump_shim(shim, prefix)
     assert got_shim == exp
     # CKMCFile::Info as main.cpp:446-449 reads it
     assert info[0] == k and info[2] == csz and info[3] == p and info[5] == minc and info[6] == maxc
@@ -116,7 +124,7 @@ def test_inverted_both_strands_byte_and_header_words(tmp_path):
         assert version == 0x200 and pre[:4] == b"KMCP" and pre[-4:] == b"KMCP"
 
 
-def test_lut_without_guard_entry_and_several_bins(cli, ref_lib, tmp_path):
+def test_lut_without_guard_entry_and_several_bins(cli, shim, tmp_path):
     """real KMC2 files hold n_bins x 4^p LUT entries and no guard; the writer here appends one.  Both must list alike."""
     rng = random.Random(5)
     k, p = 43, 3
@@ -130,7 +138,7 @@ def test_lut_without_guard_entry_and_several_bins(cli, ref_lib, tmp_path):
     os.link(a + ".kmc_suf", b + ".kmc_suf")
     la, lb = _dump_cli(cli, a), _dump_cli(cli, b)
     assert la == lb and len(la) == sum(1 for c in counts if 2 <= c <= 255)
-    assert _dump_shim(ref_lib, a)[0] == la and _dump_shim(ref_lib, b)[0] == la
+    assert _dump_shim(shim, a)[0] == la and _dump_shim(shim, b)[0] == la
     pa, ca, _ = kmc.read_kmc_db(a)
     pb, cb, _ = kmc.read_kmc_db(b)
     assert list(zip(kmc.packed_to_strings(pa, k), ca.tolist())) == la == list(zip(kmc.packed_to_strings(pb, k), cb.tolist()))

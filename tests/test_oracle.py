@@ -1,7 +1,9 @@
 """Pins the CPU oracle (oracle/malva_oracle.c) before anything trusts it.
 
 Anchors: XXH3 known answers (SURVEY 8c), python-xxhash, the reference's own
-classes through oracle/_ref/libmalva_ref.so, and glibc's logf.
+classes through oracle/_ref/libmalva_ref.so, and glibc's logf.  Where oracle/_ref
+is not built, the oracle's side of each comparison with the reference is checked
+against its digest in tests/golden/oracle_vs_reference.json (parity_util.Agree).
 """
 import ctypes as C
 import random
@@ -9,10 +11,17 @@ import random
 import numpy as np
 import pytest
 
+from parity_util import Agree
+
 KATS = [
     (b"ACGT" * 8 + b"ACG", 0x6AE639F026113AEA),
     (b"ACGT" * 10 + b"ACG", 0x1E2873EC7681F59A),
 ]
+
+
+@pytest.fixture
+def agree(request, ref_or_none):
+    return Agree(request.node.name, ref_or_none)
 
 
 def rand_kmer(rng, k, alphabet="ACGT"):
@@ -33,11 +42,12 @@ def test_xxh3_against_python_xxhash_all_lengths(oracle_lib):
             assert oracle_lib.mo_xxh3_64(s, n) == xxhash.xxh3_64_intdigest(s), n
 
 
-def test_xxh3_against_reference_build(oracle_lib, ref_lib):
+def test_xxh3_against_reference_build(oracle_lib, agree):
     rng = random.Random(2)
     for n in list(range(0, 130)) + [200, 240]:
         s = bytes(rng.randrange(256) for _ in range(n))
-        assert oracle_lib.mo_xxh3_64(s, n) == ref_lib.ref_xxh3(s, n)
+        agree.eq(oracle_lib.mo_xxh3_64(s, n), agree.L.ref_xxh3(s, n))
+    agree.done()
 
 
 def test_logf_restatement_matches_libm(oracle_lib):
@@ -57,7 +67,8 @@ def test_logf_restatement_matches_libm(oracle_lib):
 
 
 @pytest.mark.parametrize("k", [35, 43, 16, 31, 64])
-def test_bf_matches_reference_class(oracle_lib, ref_lib, k):
+def test_bf_matches_reference_class(oracle_lib, agree, k):
+    ref_lib = agree.L
     rng = random.Random(10 + k)
     size = 5003 if k != 35 else 4096  # non power of two and power of two
     ob = oracle_lib.mo_bf_new(size)
@@ -68,9 +79,11 @@ def test_bf_matches_reference_class(oracle_lib, ref_lib, k):
         oracle_lib.mo_bf_add_key(ob, s)
         ref_lib.ref_bf_add_key(rb, s)
     for s in keys:
-        assert oracle_lib.mo_bf_test_key(ob, s) == ref_lib.ref_bf_test_key(rb, s)
+        agree.eq(oracle_lib.mo_bf_test_key(ob, s), ref_lib.ref_bf_test_key(rb, s))
     # increments before switch_mode are no-ops in both
-    assert oracle_lib.mo_bf_increment(ob, keys[0], 5) == ref_lib.ref_bf_increment(rb, keys[0], 5) == 0
+    inc = oracle_lib.mo_bf_increment(ob, keys[0], 5)
+    agree.eq(inc, ref_lib.ref_bf_increment(rb, keys[0], 5))
+    assert inc == 0
     oracle_lib.mo_bf_switch_mode(ob)
     ref_lib.ref_bf_switch_mode(rb)
     for s in keys:
@@ -78,12 +91,14 @@ def test_bf_matches_reference_class(oracle_lib, ref_lib, k):
         oracle_lib.mo_bf_increment(ob, s, c)
         ref_lib.ref_bf_increment(rb, s, c)
     for s in keys:
-        assert oracle_lib.mo_bf_get_count(ob, s) == ref_lib.ref_bf_get_count(rb, s)
+        agree.eq(oracle_lib.mo_bf_get_count(ob, s), ref_lib.ref_bf_get_count(rb, s))
     oracle_lib.mo_bf_free(ob)
     ref_lib.ref_bf_free(rb)
+    agree.done()
 
 
-def test_kmap_matches_reference_class(oracle_lib, ref_lib):
+def test_kmap_matches_reference_class(oracle_lib, agree):
+    ref_lib = agree.L
     rng = random.Random(20)
     om = oracle_lib.mo_kmap_new()
     rm = ref_lib.ref_kmap_new()
@@ -91,7 +106,7 @@ def test_kmap_matches_reference_class(oracle_lib, ref_lib):
     for s in keys[:1500]:
         oracle_lib.mo_kmap_add_key(om, s)
         ref_lib.ref_kmap_add_key(rm, s)
-    assert oracle_lib.mo_kmap_size(om) == ref_lib.ref_kmap_size(rm)
+    agree.eq(oracle_lib.mo_kmap_size(om), ref_lib.ref_kmap_size(rm))
     for s in keys:
         c = rng.choice([1, 7, 255, 2 ** 31 - 1])
         oracle_lib.mo_kmap_increment(om, s, c)
@@ -100,17 +115,19 @@ def test_kmap_matches_reference_class(oracle_lib, ref_lib):
     oracle_lib.mo_kmap_add_key(om, keys[0])
     ref_lib.ref_kmap_add_key(rm, keys[0])
     for s in keys:
-        assert oracle_lib.mo_kmap_test_key(om, s) == ref_lib.ref_kmap_test_key(rm, s)
-        assert oracle_lib.mo_kmap_get_count(om, s) == ref_lib.ref_kmap_get_count(rm, s)
+        agree.eq(oracle_lib.mo_kmap_test_key(om, s), ref_lib.ref_kmap_test_key(rm, s))
+        agree.eq(oracle_lib.mo_kmap_get_count(om, s), ref_lib.ref_kmap_get_count(rm, s))
     oracle_lib.mo_kmap_free(om)
     ref_lib.ref_kmap_free(rm)
+    agree.done()
 
 
 def _u32(a):
     return a.ctypes.data_as(C.POINTER(C.c_uint32))
 
 
-def test_scan_and_reference_pass_match_reference_loops(oracle_lib, ref_lib):
+def test_scan_and_reference_pass_match_reference_loops(oracle_lib, agree):
+    ref_lib = agree.L
     rng = random.Random(30)
     k, ref_k, size = 35, 43, 1 << 16
     genome = "".join(rng.choice("ACGT") for _ in range(6000))
@@ -152,13 +169,13 @@ def test_scan_and_reference_pass_match_reference_loops(oracle_lib, ref_lib):
     for p in range(0, len(genome) - ref_k):
         w43 = genome[p:p + ref_k].encode()
         w35 = genome[p + 4:p + 4 + k].encode()
-        assert oracle_lib.mo_bf_test_key(oc, w43) == ref_lib.ref_bf_test_key(rc, w43)
-        a, b = oracle_lib.mo_bf_get_count(ob, w35), ref_lib.ref_bf_get_count(rb, w35)
-        assert a == b
-        a, b = oracle_lib.mo_kmap_get_count(om, w35), ref_lib.ref_kmap_get_count(rm, w35)
-        assert a == b
+        agree.eq(oracle_lib.mo_bf_test_key(oc, w43), ref_lib.ref_bf_test_key(rc, w43))
+        agree.eq(oracle_lib.mo_bf_get_count(ob, w35), ref_lib.ref_bf_get_count(rb, w35))
+        a = oracle_lib.mo_kmap_get_count(om, w35)
+        agree.eq(a, ref_lib.ref_kmap_get_count(rm, w35))
         nonzero += a > 0
     assert nonzero > 50
+    agree.done()
 
 
 def test_scan_packed_equals_scan_ascii(oracle_lib):
@@ -212,7 +229,7 @@ def _genotype_ref(L, cov, freq, err, max_cov, haploid):
     return probs[:ng].copy(), line.value.decode()
 
 
-def test_genotype_bit_exact_against_reference(oracle_lib, ref_lib):
+def test_genotype_bit_exact_against_reference(oracle_lib, agree):
     rng = np.random.default_rng(40)
     checked = 0
     for it in range(4000):
@@ -232,23 +249,27 @@ def test_genotype_bit_exact_against_reference(oracle_lib, ref_lib):
         f0 = np.float32(1.0 - float(np.sum(af.astype(np.float64))))
         freq = np.concatenate([[max(f0, np.float32(0))], af]).astype(np.float32)
         po, status, bi, gq = _genotype_oracle(oracle_lib, cov, freq, err, 200, haploid)
-        pr, line = _genotype_ref(ref_lib, cov, freq, err, 200, haploid)
-        assert len(po) == len(pr)
-        assert np.array_equal(po.view(np.uint64), pr.view(np.uint64)), (cov, freq, po, pr)
-        # GT and GQ as printed by the reference's output_variants
-        gtgq = line.rstrip("\n").split("\t")[-1]
         names = [str(g) for g in range(n)] if haploid else [f"{a}/{b}" for a in range(n) for b in range(a, n)]
         exp_gt = ("0" if haploid else "0/0") if status != 0 else names[bi]
-        assert gtgq == f"{exp_gt}:{gq}", (line, status, bi, gq)
+        if agree.live:
+            pr, line = _genotype_ref(agree.L, cov, freq, err, 200, haploid)
+            assert len(po) == len(pr)
+            assert np.array_equal(po.view(np.uint64), pr.view(np.uint64)), (cov, freq, po, pr)
+            # GT and GQ as printed by the reference's output_variants
+            gtgq = line.rstrip("\n").split("\t")[-1]
+            assert gtgq == f"{exp_gt}:{gq}", (line, status, bi, gq)
+        agree.record(po.view(np.uint64), f"{exp_gt}:{gq}")
         checked += 1
     assert checked == 4000
+    agree.done()
 
 
 @pytest.mark.parametrize("k,ref_k", [(35, 43), (36, 43), (31, 40), (20, 21), (43, 43), (15, 21)])
 @pytest.mark.parametrize("glen", [12, 30, 43, 44, 100, 1500])
-def test_reference_pass_matches_reference_loop_all_shapes(oracle_lib, ref_lib, k, ref_k, glen):
+def test_reference_pass_matches_reference_loop_all_shapes(oracle_lib, agree, k, ref_k, glen):
     """Odd (ref_k - k) makes the reference's k-mer window non-contiguous for its first k-1 slides
     (main.cpp:395-397); contigs shorter than ref_k hash truncated substr() results."""
+    ref_lib = agree.L
     rng = random.Random(1000 * k + ref_k + glen)
     d = (ref_k - k) // 2
     if glen < d:
@@ -275,21 +296,24 @@ def test_reference_pass_matches_reference_loop_all_shapes(oracle_lib, ref_lib, k
     for p in range(0, max(1, glen - ref_k + 1)):
         probes.add(genome[p:p + ref_k])
     probes.add(genome[:ref_k])
-    for w in probes:
-        assert oracle_lib.mo_bf_test_key(oc, w.encode()) == ref_lib.ref_bf_test_key(rc, w.encode()), w
-    hits = sum(ref_lib.ref_bf_test_key(rc, w.encode()) for w in probes)
-    assert int(np.unpackbits(a.view(np.uint8)).sum()) == len(_distinct_bits(ref_lib, rc, probes, size, oracle_lib))
+    present = []
+    for w in sorted(probes):
+        hit = oracle_lib.mo_bf_test_key(oc, w.encode())
+        agree.eq(hit, ref_lib.ref_bf_test_key(rc, w.encode()), w)
+        if hit:
+            present.append(w)
+    assert int(np.unpackbits(a.view(np.uint8)).sum()) == len(_distinct_bits(present, size, oracle_lib))
     if glen >= 100:
-        assert hits > 5
+        assert len(present) > 5
+    agree.done()
 
 
-def _distinct_bits(ref_lib, rc, probes, size, oracle_lib):
-    """bit indices of the probes the reference reports as present."""
+def _distinct_bits(present, size, oracle_lib):
+    """bit indices of the probes reported as present (by both filters: checked k-mer by k-mer)."""
     import ctypes as C
     out = set()
-    for w in probes:
-        if ref_lib.ref_bf_test_key(rc, w.encode()):
-            buf = C.create_string_buffer(len(w) + 1)
-            oracle_lib.mo_canonical(w.encode(), len(w), buf)
-            out.add(oracle_lib.mo_xxh3_64(buf.raw[:len(w)], len(w)) % size)
+    for w in present:
+        buf = C.create_string_buffer(len(w) + 1)
+        oracle_lib.mo_canonical(w.encode(), len(w), buf)
+        out.add(oracle_lib.mo_xxh3_64(buf.raw[:len(w)], len(w)) % size)
     return out

@@ -4,7 +4,7 @@ import golden_flow
 from parity_util import OracleRun
 
 
-def test_oracle_reproduces_haploid_golden(oracle_lib, ref_lib):
+def test_oracle_reproduces_haploid_golden(oracle_lib, ref_or_none):
     o = OracleRun(oracle_lib, 35, 43, 1 << 26)
 
     def genotype(batch):
@@ -12,7 +12,7 @@ def test_oracle_reproduces_haploid_golden(oracle_lib, ref_lib):
         return cov, [(e["status"], e["best"], e["gq"], e["probs"]) for e in res]
 
     try:
-        lines = golden_flow.run_haploid_example(o, ref_lib, genotype)
+        lines = golden_flow.run_haploid_example(o, ref_or_none, genotype)
         assert oracle_lib.mo_bf_popcount(o.bf) == 422 and o.kmap_size() == 679
     finally:
         o.close()
