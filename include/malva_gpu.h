@@ -94,6 +94,8 @@ typedef struct {
   const float *freq;              /* [n_alleles]    a-priori allele frequencies (Variant::frequencies) */
 } mg_variant_batch;
 
+/* A variant with no allele slot (var_allele_off[v+1] == var_allele_off[v]) has no genotype: it reserves no
+ * likelihood slot, none is written for it, and it reports n_gts 0, status 2, best_gt 0, gq 0. */
 typedef struct {
   uint32_t *cov;           /* [n_alleles]   Variant::coverages                               */
   int32_t *n_gts;          /* [n_variants]  number of computed_gts entries                   */

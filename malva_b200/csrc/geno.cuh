@@ -161,11 +161,21 @@ MG_HD float glibc_logf(float x) {
   return (float)y;
 }
 
-MG_HD double log_binomial(int n, int k) {  // var_block.hpp:792-797
+// log((double)i) for 0 < i < LOG_TABLE_N as the host's libm computes it (built at mg_create).  CUDA's fp64 log is
+// within 1 ulp, glibc's is correctly rounded nearly everywhere, and one ulp of log_binomial decides GT wherever two
+// genotypes are mathematically tied (uniform priors, coverages like 2,12,2): with the table the device's log-posterior
+// is the reference's bit for bit for every tot < 2^16.  Larger arguments (and the host self-test path, table NULL)
+// use the libm at hand.
+constexpr int LOG_TABLE_N = 1 << 16;
+MG_HD double log_int(int x, const double *log_table) {
+  return (log_table && x > 0 && x < LOG_TABLE_N) ? log_table[x] : log((double)x);
+}
+
+MG_HD double log_binomial(int n, int k, const double *log_table) {  // var_block.hpp:792-797
   if (n == 0 || n == k || k == 0) return 0.0;
-  double a = f64_mul((double)n, log((double)n));
-  double b = f64_mul((double)k, log((double)k));
-  double c = f64_mul((double)(n - k), log((double)(n - k)));
+  double a = f64_mul((double)n, log_int(n, log_table));
+  double b = f64_mul((double)k, log_int(k, log_table));
+  double c = f64_mul((double)(n - k), log_int(n - k, log_table));
   return f64_sub(f64_sub(a, b), c);
 }
 
@@ -184,23 +194,33 @@ MG_HD GenoConsts geno_consts(float e, int n) {
 
 MG_HD double prob_from_log(double log_prior, double log_post) {
   double lp = f64_add(log_prior, log_post);
-  return isinf(lp) ? 0.0 : exp(lp);
+  if (isinf(lp)) return 0.0;
+#if defined(__CUDA_ARCH__)
+  // results below DBL_MIN: CUDA's exp does not return glibc's subnormals there, and when every likelihood of a variant
+  // is that small the one glibc keeps decides GT.  exp(lp + 64 ln2_hi) * exp(64 (ln2 - ln2_hi)) * 2^-64 instead:
+  // lp + 64 ln2_hi is exact (ln2_hi has 32 significant bits), the factor is a constant, and the scaling rounds into
+  // the subnormal range once -- within ~1 ulp of the normal-range result, so 1-ulp-of-lp ties keep glibc's order
+  // almost always.
+  if (lp < -708.0) return __dmul_rn(__dmul_rn(exp(__dadd_rn(lp, 64.0 * 0x1.62e42feep-1)), 0x1.0000003473de7p+0), 0x1p-64);
+#endif
+  return exp(lp);
 }
 
 // homozygous / haploid genotype g (var_block.hpp:272-285, 296-304)
-MG_HD double geno_hom(uint32_t t, uint32_t tot, float f, const GenoConsts &c) {
+MG_HD double geno_hom(uint32_t t, uint32_t tot, float f, const GenoConsts &c, const double *log_table) {
   uint32_t er = tot - t;
   double log_prior = (double)f32_mul(2.0f, glibc_logf(f));
-  double lb = log_binomial((int)(t + er), (int)t);
+  double lb = log_binomial((int)(t + er), (int)t, log_table);
   double log_post = f64_add(f64_add(lb, (double)f32_mul((float)t, c.c1)), (double)f32_mul((float)er, c.c2));
   return prob_from_log(log_prior, log_post);
 }
 // heterozygous genotype g1<g2 (var_block.hpp:306-318)
-MG_HD double geno_het(uint32_t t1, uint32_t t2, uint32_t tot, float f1, float f2, int n, const GenoConsts &c) {
+MG_HD double geno_het(uint32_t t1, uint32_t t2, uint32_t tot, float f1, float f2, int n, const GenoConsts &c,
+                      const double *log_table) {
   uint32_t er = tot - t1 - t2;
   double log_prior = (double)glibc_logf(f32_mul(f32_mul(2.0f, f1), f2));
-  double lb1 = log_binomial((int)(t1 + t2 + er), (int)(t1 + t2));
-  double lb2 = log_binomial((int)(t1 + t2), (int)t1);
+  double lb1 = log_binomial((int)(t1 + t2 + er), (int)(t1 + t2), log_table);
+  double lb2 = log_binomial((int)(t1 + t2), (int)t1, log_table);
   double log_post = f64_add(f64_add(f64_add(lb1, lb2), (double)f32_mul((float)t1, c.c3)),
                             (double)f32_mul((float)t2, c.c3));
   if (n > 2) log_post = f64_add(log_post, (double)f32_mul((float)er, c.c4));

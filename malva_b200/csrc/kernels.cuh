@@ -1290,8 +1290,15 @@ __global__ void __launch_bounds__(128) k_coverage(const int32_t *__restrict__ w,
 // ---------------------------------------------------------------------------
 // K5: genotype likelihoods + posterior arg-max (var_block.hpp:224-330, 367-394)
 // ---------------------------------------------------------------------------
+// log_table: glibc's log of small integers (geno.cuh log_int); NULL on the host self-test path
 MG_HD int genotype_one(const uint32_t *cov, const float *freq, int n, float err, int max_cov, bool haploid,
-                       double *lik, int *status, int *best_gt, int *gq) {
+                       const double *log_table, double *lik, int *status, int *best_gt, int *gq) {
+  if (n == 0) {  // a variant without alleles has no genotype and no likelihood slot (include/malva_gpu.h)
+    *status = 2;
+    *best_gt = 0;
+    *gq = 0;
+    return 0;
+  }
   int ng = 0;
   for (int i = 0; i < n; ++i)
     if ((int)cov[i] > max_cov) lik[ng++] = 0.0;  // one {best,0} per offending allele
@@ -1322,8 +1329,8 @@ MG_HD int genotype_one(const uint32_t *cov, const float *freq, int n, float err,
   for (int g1 = 0; g1 < n; ++g1) {
     for (int g2 = g1; g2 < n; ++g2) {
       if (haploid && g2 != g1) break;
-      double p = (g1 == g2) ? geno_hom(cov[g1], tot, freq[g1], c)
-                            : geno_het(cov[g1], cov[g2], tot, freq[g1], freq[g2], n, c);
+      double p = (g1 == g2) ? geno_hom(cov[g1], tot, freq[g1], c, log_table)
+                            : geno_het(cov[g1], cov[g2], tot, freq[g1], freq[g2], n, c, log_table);
       lik[ng++] = p;
       total = f64_add(total, p);
     }
@@ -1350,6 +1357,7 @@ __global__ void __launch_bounds__(128) k_genotype(const uint32_t *__restrict__ c
                                                  const OFF *__restrict__ var_allele_off,
                                                  const uint64_t *__restrict__ lik_off, unsigned long long *cursor,
                                                  uint64_t n_variants, float err, int max_cov, int haploid,
+                                                 const double *__restrict__ log_table,
                                                  double *__restrict__ lik, int32_t *__restrict__ n_gts,
                                                  int32_t *__restrict__ status, int32_t *__restrict__ best_gt,
                                                  int32_t *__restrict__ gq) {
@@ -1378,7 +1386,7 @@ __global__ void __launch_bounds__(128) k_genotype(const uint32_t *__restrict__ c
   }
   if (!live) return;
   int st, bg, q;
-  int ng = genotype_one(cov + a0, freq + a0, n, err, max_cov, haploid != 0, lik + lo, &st, &bg, &q);
+  int ng = genotype_one(cov + a0, freq + a0, n, err, max_cov, haploid != 0, log_table, lik + lo, &st, &bg, &q);
   n_gts[vi] = ng;
   status[vi] = st;
   best_gt[vi] = bg;

@@ -118,6 +118,7 @@ struct mg_ctx {
   void *geno_scratch = nullptr;  // per-k-mer weights + ref flags of mg_genotype
   uint64_t geno_scratch_bytes = 0;
   void *geno_arena = nullptr;  // device image of the last mg_genotype batch (grow-only)
+  double *log_table = nullptr;  // the host libm's log((double)i), i < mg::LOG_TABLE_N (geno.cuh log_int)
   uint64_t geno_arena_bytes = 0;
   cudaEvent_t evs[64] = {};
 
@@ -250,6 +251,12 @@ static int ctx_init(mg_ctx *c) {
       CU(cudaMemsetAsync(c->occ, 0, c->n_occ_words * 4, c->stream[0]));
     }
   }
+  {  // log_binomial's logs of small integers from the reference's libm: GT of exact ties comes from their last bits
+    std::vector<double> tab(mg::LOG_TABLE_N, 0.0);
+    for (int i = 1; i < mg::LOG_TABLE_N; ++i) tab[i] = log((double)i);
+    CU(cudaMalloc(&c->log_table, tab.size() * sizeof(double)));
+    CU(cudaMemcpy(c->log_table, tab.data(), tab.size() * sizeof(double), cudaMemcpyHostToDevice));
+  }
   CU(cudaMalloc(&c->d_scalars, 8 * sizeof(unsigned long long)));
   CU(cudaMemsetAsync(c->d_scalars, 0, 8 * sizeof(unsigned long long), c->stream[0]));
   c->ovf_log2 = 10;
@@ -283,6 +290,7 @@ extern "C" void mg_destroy(mg_ctx *c) {
   cudaFree(c->d_scalars);
   cudaFree(c->geno_scratch);
   cudaFree(c->geno_arena);
+  cudaFree(c->log_table);
   cudaFree(c->kmc_lut);
   for (int i = 0; i < 2; ++i) {
     cudaFree(c->hit_buf[i]);
@@ -1143,7 +1151,8 @@ static int genotype_on_device(mg_ctx *c, const mg_variant_batch *in, const mg_ge
   CU(cudaEventRecord(c->ge[2], st));
   c->launches++;
   mg::k_genotype<uint64_t><<<grid_for(nv, 128), 128, 0, st>>>(out->cov, in->freq, in->var_allele_off, out->lik_off, nullptr,
-                                                              nv, error_rate, max_coverage, haploid, out->lik, out->n_gts,
+                                                              nv, error_rate, max_coverage, haploid, c->log_table,
+                                                              out->lik, out->n_gts,
                                                               out->status, out->best_gt, out->gq);
   CU(cudaGetLastError());
   CU(cudaEventRecord(c->ge[3], st));
@@ -1278,7 +1287,8 @@ static int genotype_from_weights(mg_ctx *c, const mg_packed_batch *in, const mg_
   c->launches++;
   mg::k_genotype<uint32_t><<<grid_for(nv, 128), 128, 0, st>>>(out->cov, in->freq, in->var_allele_off,
                                                               own_lik ? nullptr : out->lik_off, c->d_scalars + 5, nv,
-                                                              error_rate, max_coverage, haploid, d_lik, out->n_gts,
+                                                              error_rate, max_coverage, haploid, c->log_table, d_lik,
+                                                              out->n_gts,
                                                               out->status, out->best_gt, out->gq);
   CU(cudaGetLastError());
   CU(cudaEventRecord(c->ge[3], st));
@@ -2079,5 +2089,5 @@ extern "C" int mg_selftest_pack35(const char *s35, uint64_t *lo, uint64_t *hi) {
 extern "C" float mg_selftest_logf(float x) { return mg::glibc_logf(x); }
 extern "C" int mg_selftest_genotype(const uint32_t *cov, const float *freq, int n_alleles, float error_rate,
                                     int max_cov, int haploid, double *lik, int *status, int *best_gt, int *gq) {
-  return mg::genotype_one(cov, freq, n_alleles, error_rate, max_cov, haploid != 0, lik, status, best_gt, gq);
+  return mg::genotype_one(cov, freq, n_alleles, error_rate, max_cov, haploid != 0, nullptr, lik, status, best_gt, gq);
 }

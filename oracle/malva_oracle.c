@@ -565,3 +565,22 @@ void mo_call(const double *probs, int n_gts, int *best_idx, int *gq) { /* var_bl
   *best_idx = bi;
   *gq = (int)round(best * 100);
 }
+
+void mo_genotype_batch(const uint32_t *cov, const float *freq, const uint64_t *var_allele_off, uint64_t n_variants,
+                       float error_rate, int max_cov, int haploid, double *lik, const uint64_t *lik_off,
+                       int32_t *n_gts, int32_t *status, int32_t *best, int32_t *gq) {
+  uint64_t v;
+  for (v = 0; v < n_variants; ++v) {
+    const uint64_t a0 = var_allele_off[v];
+    const int n = (int)(var_allele_off[v + 1] - a0);
+    int st = 2, bi = 0, q = 0, ng = 0;
+    if (n > 0) { /* a variant without alleles reserves no slot: nothing is written for it */
+      ng = mo_genotype(cov + a0, freq + a0, n, error_rate, max_cov, haploid, lik + lik_off[v], &st);
+      mo_call(lik + lik_off[v], ng, &bi, &q);
+    }
+    n_gts[v] = ng;
+    status[v] = st;
+    best[v] = bi;
+    gq[v] = q;
+  }
+}

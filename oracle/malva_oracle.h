@@ -80,6 +80,13 @@ int mo_genotype(const uint32_t *cov, const float *freq, int n_alleles, float err
                 int haploid, double *probs, int *status);
 /* var_block.hpp:367-394: total, normalise, first strict maximum, GQ */
 void mo_call(const double *probs, int n_gts, int *best_idx, int *gq);
+/* mo_genotype + mo_call over a batch (CSR: alleles of variant v are var_allele_off[v] .. var_allele_off[v+1]).
+ * The likelihoods of variant v go to lik[lik_off[v] ..], which must hold max(n, n(n+1)/2) slots (n for haploid).
+ * A variant with no allele writes no likelihood and reports n_gts 0, status 2, best 0, gq 0 (the GPU's contract,
+ * include/malva_gpu.h). */
+void mo_genotype_batch(const uint32_t *cov, const float *freq, const uint64_t *var_allele_off, uint64_t n_variants,
+                       float error_rate, int max_cov, int haploid, double *lik, const uint64_t *lik_off,
+                       int32_t *n_gts, int32_t *status, int32_t *best, int32_t *gq);
 /* glibc 2.39 logf restated (verified exhaustively against libm in tests) */
 float mo_logf(float x);
 

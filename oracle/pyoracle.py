@@ -84,6 +84,9 @@ def oracle() -> C.CDLL:
     L.mo_coverages.argtypes = [C.c_void_p, C.c_void_p, C.c_char_p, _u64p, _u64p, _u64p, _u8p, C.c_uint64, _u32p]
     L.mo_genotype.argtypes = [_u32p, _f32p, C.c_int, C.c_float, C.c_int, C.c_int, _f64p, _intp]
     L.mo_call.argtypes = [_f64p, C.c_int, _intp, _intp]
+    _i32p = C.POINTER(C.c_int32)
+    L.mo_genotype_batch.argtypes = [_u32p, _f32p, _u64p, C.c_uint64, C.c_float, C.c_int, C.c_int, _f64p, _u64p,
+                                    _i32p, _i32p, _i32p, _i32p]
     L.mo_logf.restype = C.c_float
     L.mo_logf.argtypes = [C.c_float]
     _oracle = L

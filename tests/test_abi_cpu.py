@@ -124,9 +124,20 @@ def test_genotype_host_path_matches_oracle(L, oracle_lib):
         obi, ogq = C.c_int(), C.c_int()
         oracle_lib.mo_call(lb.ctypes.data_as(f64p), nb, C.byref(obi), C.byref(ogq))
         assert na == nb and st_a.value == st_b.value
-        # same libm on the host -> bit identical here; on the device the bound is 1e-9 relative
+        # same libm on the host -> bit identical here; the device is held to tests/geno_util.lik_bound
         assert np.array_equal(la[:na].view(np.uint64), lb[:nb].view(np.uint64)), (cov, freq)
         assert (bg.value, gq.value) == (obi.value, ogq.value)
+
+
+def test_genotype_zero_alleles_writes_nothing(L):
+    """a variant without alleles reserves no likelihood slot (include/malva_gpu.h): genotype_one writes none"""
+    lik = np.full(4, 7.0)
+    st, bg, gq = C.c_int(-1), C.c_int(-1), C.c_int(-1)
+    ng = L.mg_selftest_genotype(np.zeros(1, np.uint32).ctypes.data_as(C.POINTER(C.c_uint32)),
+                                np.zeros(1, np.float32).ctypes.data_as(C.POINTER(C.c_float)), 0, C.c_float(0.001), 200, 0,
+                                lik.ctypes.data_as(C.POINTER(C.c_double)), C.byref(st), C.byref(bg), C.byref(gq))
+    assert (ng, st.value, bg.value, gq.value) == (0, 2, 0, 0)
+    assert (lik == 7.0).all()
 
 
 def test_wordwise_packer_of_the_lookup_kernel(L):
