@@ -67,6 +67,8 @@ extern "C" int mg_warmup(int device) {
 // ---------------------------------------------------------------------------
 // context
 // ---------------------------------------------------------------------------
+// k-mers (KMC records) per staging chunk of the host-buffer scans; tests/test_gpu_scale.py sizes its inputs to cross
+// these chunks on both streams and fails if this changes
 constexpr uint64_t STAGE_KMERS = 1ull << 22;
 
 struct mg_ctx {
@@ -690,6 +692,7 @@ static cudaError_t launch_refpass(mg_ctx *c, const uint8_t *d_chunk, uint64_t ch
 // the H2D copy of chunk i+1 (stream 1) overlaps the kernel of chunk i (stream 0).  A caller buffer in pinned memory
 // (mg_host_alloc) is copied from directly; pageable memory goes through two pinned staging buffers, filled by
 // several host threads (one thread moves ~8 GB/s, the link takes ~50).
+// (tests/test_gpu_scale.py plants input at the seams of this size and fails if it changes)
 constexpr uint64_t REF_CHUNK = 32ull << 20;  // window end positions per chunk (a multiple of RP_TILE)
 
 static void parallel_memcpy(void *dst, const void *src, size_t n) {

@@ -195,6 +195,23 @@ void mo_bf_add_key(mo_bf *b, const char *kmer) {
   b->w[i >> 6] |= 1ULL << (i & 63);
 }
 int mo_bf_test_key(const mo_bf *b, const char *kmer) { return bf_bit(b, kmer_hash(kmer) % b->size); }
+uint64_t mo_find_kmers_at(const char *seed, int k, uint64_t size, uint64_t lo, uint64_t first, uint64_t n_trials,
+                          char *out, uint64_t max_out) {
+  /* k-mers whose filter index kmer_hash % size is >= lo: trial t is the seed with t written in base 4 into its
+   * symbols 1..31; k(+NUL)-byte results go to out.  The seed starts and ends with 'A', so every trial is its own
+   * canonical form (its reverse complement starts with 'T') and is hashed as it is. */
+  char s[512];
+  uint64_t t, found = 0;
+  int j, w = k - 2 < 31 ? k - 2 : 31;
+  if (k < 3 || k >= (int)sizeof(s) || seed[0] != 'A' || seed[k - 1] != 'A') return 0;
+  memcpy(s, seed, (size_t)k);
+  s[k] = '\0';
+  for (t = first; t < first + n_trials && found < max_out; ++t) {
+    for (j = 0; j < w; ++j) s[1 + j] = "ACGT"[(t >> (2 * j)) & 3];
+    if (mo_xxh3_64(s, (size_t)k) % size >= lo) memcpy(out + (k + 1) * found++, s, (size_t)k + 1);
+  }
+  return found;
+}
 void mo_bf_switch_mode(mo_bf *b) {
   uint64_t nb = b->nwords / 8 + 2, acc = 0, wi;
   b->mode = 1;

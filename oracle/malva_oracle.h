@@ -39,6 +39,10 @@ uint64_t mo_bf_size(const mo_bf *b);
 uint64_t mo_bf_popcount(const mo_bf *b);
 const uint64_t *mo_bf_words(const mo_bf *b);   /* bit i = (words[i>>6] >> (i&63)) & 1 */
 const uint16_t *mo_bf_counts(const mo_bf *b);  /* rank-indexed, valid after switch_mode */
+/* up to max_out k-mers (k bytes + NUL each, into out), variants first .. first+n_trials-1 of seed (which must start
+ * and end with 'A'), whose index in a filter of `size` bits is >= lo; returns how many it found */
+uint64_t mo_find_kmers_at(const char *seed, int k, uint64_t size, uint64_t lo, uint64_t first, uint64_t n_trials,
+                          char *out, uint64_t max_out);
 
 /* ---- KMAP (kmap.hpp:46-132) ---- */
 typedef struct mo_kmap mo_kmap;

@@ -69,6 +69,9 @@ def oracle() -> C.CDLL:
     L.mo_bf_words.argtypes = [C.c_void_p]
     L.mo_bf_counts.restype = C.POINTER(C.c_uint16)
     L.mo_bf_counts.argtypes = [C.c_void_p]
+    L.mo_find_kmers_at.restype = C.c_uint64
+    L.mo_find_kmers_at.argtypes = [C.c_char_p, C.c_int, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint64, C.c_char_p,
+                                   C.c_uint64]
     L.mo_kmap_new.restype = C.c_void_p
     L.mo_kmap_free.argtypes = [C.c_void_p]
     L.mo_kmap_add_key.argtypes = [C.c_void_p, C.c_char_p]
