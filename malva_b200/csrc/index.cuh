@@ -97,11 +97,10 @@ __device__ __forceinline__ uint2 ldg_na(const uint2 *p) {
   asm volatile("ld.global.nc.L1::no_allocate.v2.u32 {%0, %1}, [%2];" : "=r"(r.x), "=r"(r.y) : "l"(p));
   return r;
 }
-template <bool NA = false>
 __device__ __forceinline__ bool occ_test(const DevView &v, uint64_t idx) {
   if (!v.occ) return true;
   uint64_t o = idx >> v.occ_shift;
-  const uint32_t w = NA ? ldg_na(v.occ + (o >> 5)) : __ldg(v.occ + (o >> 5));
+  const uint32_t w = __ldg(v.occ + (o >> 5));
   return (w >> (o & 31)) & 1u;
 }
 __device__ __forceinline__ void occ_set(const DevView &v, uint32_t *occ_rw, uint64_t idx) {

@@ -423,12 +423,13 @@ __global__ void k_refpass_short(const uint8_t *seq, uint64_t len, DevView v, uin
 // K1: sample k-mer scan (main.cpp:487-500)
 //   ref_bf.increment(kmer, c);  if (!context_bf.test_key(context)) bf.increment(kmer, c);
 //
-// A warp owns 32 (x ILP) k-mers per iteration: lane i hashes k-mer i (coalesced loads, canonical form, XXH3) and
-// tests the L2-resident occupancy pre-filter (default build: its 16-byte piece arrives in shared memory by cp.async).  Only about a third of the k-mers of a whole-genome workload need their
-// probe line at all, so probing lane by lane would leave two thirds of the lanes idle through the whole probe
-// sequence (the kernel is bound by instruction issue, profiles/round1_k1_v5.md).  The k-mers that need a line are
-// therefore COMPACTED: they go into a ring in shared memory ({canonical k-mer | line, index, count, bit}; 64-128 entries),
-// and whenever the ring holds 32 entries the warp runs one FULL probe round:
+// A warp owns 32 k-mers per iteration (packed input: 64, two per lane): lane i hashes k-mer i (coalesced loads,
+// canonical form, XXH3) and tests the L2-resident occupancy pre-filter (its 16-byte piece arrives in shared memory by
+// cp.async).  Only about a third of the k-mers of a whole-genome workload need their probe line at all, so probing
+// lane by lane would leave two thirds of the lanes idle through the whole probe sequence (the kernel is bound by
+// instruction issue, profiles/round1_k1_v5.md).  The k-mers that need a line are therefore COMPACTED: they go into a
+// ring in shared memory ({canonical k-mer | line, index, count, bit}; 64-128 entries), and whenever the ring holds 32
+// entries the warp runs one FULL probe round:
 //   * the 32 probe lines are copied into the warp's 4 KB tile with cp.async (LDGSTS, no register staging): eight
 //     unrolled rounds, in each the four 8-lane groups move one line each, lane j of a group moving uint4 j -- a line
 //     costs exactly one fully coalesced 128-byte request and all 32 are in flight together.  The tile is XOR-swizzled
@@ -477,31 +478,24 @@ __device__ __forceinline__ u128 canon_only(u128 x, int k) {
   return less128(x, rc) ? x : rc;
 }
 
-// ring entries per warp: [a round in flight (32) +] the entries that pile up until the next turn (< 64; < 32 + 32 ILP
-// when all ILP k-mers of a lane are pushed in one go: the cp.async build, which has the shared memory to spare)
-__host__ __device__ constexpr bool scan_push_all(bool async, int ilp, int ld) { return async && ilp >= 2 && ld == 2; }
-__host__ __device__ constexpr int scan_q(bool async, int ilp = 1, int ld = 0) {
-  return async ? (scan_push_all(async, ilp, ld) ? 64 + 32 * ilp : 96) : 64;
-}
-// per warp: 4 KB tile + ring keys + ring meta (uint4 units)
-// LD == 2 needs one 16-byte landing slot per k-mer of a batch for the pre-filter pieces: its own, except with
-// synchronous rounds and two k-mers per lane, where the (then idle) tile takes them
-__host__ __device__ constexpr bool scan_occs(int ld, bool async, int ilp) { return ld == 2 && (async || ilp == 1); }
-__host__ __device__ constexpr bool scan_dense(int ld, bool async, int ilp) { return ld == 2 && !async && ilp == 2; }
-// (+ with `occs`, those slots)
-__host__ __device__ constexpr int scan_warp_u4(bool async, int ilp = 1, bool occs = false) {
-  return 256 + 2 * scan_q(async, ilp, occs ? 2 : 0) + (occs ? 32 * ilp : 0);
-}
-// + the 1 KB expansion table and a deferred-hit counter per warp
-__host__ __device__ constexpr int scan_smem(int threads, bool async, int ilp = 1, bool occs = false) {
-  return (threads / 32) * scan_warp_u4(async, ilp, occs) * 16 + 256 * 4 + (threads / 32) * 4;
-}
-// CTAs per SM that fit the shared memory (227 KB usable, 1 KB reserved per CTA), capped at 1024 threads (64 registers
-// each) -- 768 threads (85 registers) for the two-chain variant
-__host__ __device__ constexpr int scan_min_ctas(int threads, bool async, int ilp = 1, bool occs = false, bool dense = false) {
-  const int by_smem = (227 * 1024) / (scan_smem(threads, async, ilp, occs) + 1024),
-            by_threads = (ilp >= 4 ? 512 : ilp == 3 ? 640 : ilp == 2 && !dense ? 768 : 1024) / threads;
-  return by_smem < by_threads ? by_smem : by_threads;
+// The shape of the scan for input MODE (see k_scan), in 256-thread CTAs.
+//   ilp:      k-mers per lane and batch: 2 for packed k-mers, 1 for KMC records
+//   q:        ring entries per warp: the round in flight (32; MODE 0 only) + the entries that pile up until the next
+//             turn (fewer than 32 + 32 * ilp)
+//   warp_u4:  shared memory per warp in uint4: the 4 KB tile, the ring keys, the ring meta and a 16-byte landing slot
+//             per k-mer of a batch for the pre-filter pieces
+//   smem:     bytes per CTA: the warps + the 1 KB expansion table and a deferred-hit counter per warp
+//   min_ctas: CTAs per SM that fit the shared memory (227 KB usable, 1 KB reserved per CTA), capped at 1024 threads
+//             (64 registers each) -- 768 threads (85 registers) for the two chains of MODE 0
+constexpr int SCAN_THREADS = 256;
+struct ScanShape {
+  int ilp, q, warp_u4, smem, min_ctas;
+};
+__host__ __device__ constexpr ScanShape scan_shape(int mode) {
+  const int ilp = mode == 0 ? 2 : 1, q = mode == 0 ? 128 : 64, warp_u4 = 256 + 2 * q + 32 * ilp;
+  const int warps = SCAN_THREADS / 32, smem = warps * warp_u4 * 16 + 256 * 4 + warps * 4;
+  const int by_smem = (227 * 1024) / (smem + 1024), by_threads = (mode == 0 ? 768 : 1024) / SCAN_THREADS;
+  return {ilp, q, warp_u4, smem, by_smem < by_threads ? by_smem : by_threads};
 }
 
 // Where the sample k-mers come from.  MODE 0: packed {lo,hi} words + u32 counts.  MODE 1: raw records of a
@@ -539,47 +533,47 @@ __device__ __forceinline__ uint32_t lut_bucket(const uint64_t *lut, uint32_t n_l
   return lo;
 }
 
-// THREADS: CTA size (the per-warp state is private, the CTA only shares the expansion table).
-// RING = false probes after every batch of 32 k-mers, with whatever lanes need a line (the round-1 scheme), for
-// comparison.  ASYNC: the k-mers of batch i+1 are loaded into registers while batch i is hashed, and the gather of a
-// round is only STARTED when the ring holds 32 entries: the warp goes on hashing and finishes the round (wait,
-// compare, count) at the next turn, a batch or more later.  (Also tried, profiles/round2_k1.md: parking a hashed
-// batch in shared memory until its pre-filter word arrives -- the extra shared-memory traffic cost more than the
-// hidden L2 latency.)  The raw-record mode stages records in the tile and stays synchronous.
-// ILP = 2..4 (packed input): every lane hashes ILP k-mers per iteration, written as straight-line code over all of
-// them so that the dependent chains (canonical form -> table look-ups -> four 128-bit products) interleave: with ~30
-// resident warps per SM the single chain left the issue slots half empty (~11 cycles between two instructions of a
-// warp, ncu).  Two is the default; three and four (sweep builds) cost warps for registers and are no faster.
-// LD: how the scan reads global memory.  0: ld.global.nc through L1.  1: the k-mer, count and pre-filter loads do
-// not allocate in L1 (ld.global.nc.L1::no_allocate).  2 (the default build): as 1, and the 16-byte piece of the
-// pre-filter that holds a k-mer's bit is copied to a shared-memory slot with cp.async.cg (LDGSTS.BYPASS: nothing of
-// it passes through L1) and read from there.  Why: the 32 random pre-filter words of a warp each hold an L1 line
-// while in flight; with shared memory carved out for three CTAs the remaining L1 (28-60 KB) capped the loads in
-// flight per SM, and the kernel ran 25 % slower at the 228 KB carve-out than at 196 KB (profiles/round2_k1_final.md).
-// Through cp.async the kernel no longer cares, takes the whole carve-out, and has room for a ring deep enough to
-// push all k-mers of a lane at once (one ballot / prefix / turn check per batch instead of one per k-mer).
-template <int K, int REFK, int MODE, int THREADS, bool RING, bool ASYNC, int ILP = 1, int LD = 0>
-__global__ void __launch_bounds__(THREADS, scan_min_ctas(THREADS, ASYNC, ILP, scan_occs(LD, ASYNC, ILP), scan_dense(LD, ASYNC, ILP)))
-    k_scan(ScanSrc src, uint64_t n, DevView v) {
-  static_assert(!ASYNC || (RING && MODE == 0), "the asynchronous round needs the ring and leaves the tile alone");
-  static_assert(ILP == 1 || (ILP >= 2 && ILP <= 4 && RING && MODE == 0), "several k-mers per lane: ring, packed input");
-  static_assert(ILP <= 2 || scan_push_all(ASYNC, ILP, LD), "more than two k-mers per lane: the cp.async build only");
+// K, REFK: the (k, ref_k) the hashes are specialised for; 0 takes them from the view at run time.  The per-warp state
+// is private, the CTA only shares the expansion table.
+// MODE 0 (packed k-mers) runs ASYNCHRONOUS rounds: the k-mers of batch i+1 are loaded into registers while batch i
+// is hashed, and the gather of a round is only STARTED when the ring holds 32 entries: the warp goes on hashing and
+// finishes the round (wait, compare, count) at the next turn, a batch or more later.  Every lane hashes two k-mers
+// per batch, written as straight-line code over both so that the two dependent chains (canonical form -> table
+// look-ups -> four 128-bit products) interleave: with ~30 resident warps per SM a single chain left the issue slots
+// half empty (~11 cycles between two instructions of a warp, ncu).  Both k-mers of every lane go into the ring in one
+// go: one ballot / prefix / turn check per batch instead of one per k-mer.
+// MODE 1 (KMC records) stages the records of a batch in the tile, one per lane, and runs SYNCHRONOUS rounds: the tile
+// is busy with the records until the batch is hashed, so a round starts and finishes before the next batch.
+// MODE 0 reads the counts and short context k-mers with ld.global.nc.L1::no_allocate.  Both modes copy the 16-byte
+// piece of the pre-filter that holds a k-mer's bit to a shared-memory slot with cp.async.cg (LDGSTS.BYPASS: nothing
+// of it passes through L1) and read it from there.  Why: the 32 random pre-filter words of a warp each hold an L1 line
+// while in flight; with shared memory carved out for three CTAs the remaining L1 (28-60 KB) capped the loads in flight
+// per SM, and the kernel ran 25 % slower at the 228 KB carve-out than at 196 KB (profiles/round2_k1_final.md).  Through
+// cp.async the kernel no longer cares, takes the whole carve-out, and has room for a ring deep enough for MODE 0's
+// whole batch.
+// The schemes measured against this one are in profiles/round2_k1*.md: probing after every batch, one, three or four
+// k-mers per lane, synchronous rounds for packed input, 128-thread CTAs, loads through L1, and parking a hashed batch
+// in shared memory until its pre-filter word arrives (the extra shared-memory traffic cost more than the hidden L2
+// latency).
+template <int K, int REFK, int MODE>
+__global__ void __launch_bounds__(SCAN_THREADS, scan_shape(MODE).min_ctas) k_scan(ScanSrc src, uint64_t n, DevView v) {
   extern __shared__ uint4 scan_sm[];
-  constexpr int SCAN_WARPS = THREADS / 32, SCAN_Q = scan_q(ASYNC, ILP, LD), SCAN_WARP_U4 = scan_warp_u4(ASYNC, ILP, scan_occs(LD, ASYNC, ILP));
+  constexpr ScanShape S = scan_shape(MODE);
+  constexpr int SCAN_WARPS = SCAN_THREADS / 32, SCAN_Q = S.q, SCAN_WARP_U4 = S.warp_u4;
   const int k = K > 0 ? K : v.k, ref_k = REFK > 0 ? REFK : v.ref_k;
   const int tail = ref_k - k - (ref_k - k) / 2;  // bases of the context after the k-mer (main.cpp:493)
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, sub = lane & 7, grp = lane >> 3;
   uint4 *tile = scan_sm + wid * SCAN_WARP_U4;  // 32 rows x 8 uint4
   uint4 *qkey = tile + 256, *qmeta = qkey + SCAN_Q;
-  // LD == 2: this lane's landing slots (one per k-mer of a batch, 32 apart)
-  const uint4 *oslot = (scan_dense(LD, ASYNC, ILP) ? tile : qmeta + SCAN_Q) + lane;
+  // this lane's pre-filter landing slots (one per k-mer of a batch, 32 apart)
+  const uint4 *oslot = qmeta + SCAN_Q + lane;
   const uint32_t oslot_addr = (uint32_t)__cvta_generic_to_shared(oslot);
   const uint32_t tile_addr = (uint32_t)__cvta_generic_to_shared(tile);
   uint32_t *tab = reinterpret_cast<uint32_t *>(scan_sm + SCAN_WARPS * SCAN_WARP_U4);
   uint32_t *hitc = tab + 256 + wid;  // this warp's deferred-hit counter
   if (lane == 0) *hitc = 0;
   if constexpr (K > 0) {
-    for (int t = threadIdx.x; t < 256; t += THREADS) tab[t] = expand4((uint32_t)t);
+    for (int t = threadIdx.x; t < 256; t += SCAN_THREADS) tab[t] = expand4((uint32_t)t);
     __syncthreads();
   } else {
     __syncwarp();
@@ -595,7 +589,7 @@ __global__ void __launch_bounds__(THREADS, scan_min_ctas(THREADS, ASYNC, ILP, sc
   const uint32_t d_even = tile_addr + (uint32_t)(grp * 128 + ((sub ^ grp) * 16));
   const uint32_t d_odd = tile_addr + (uint32_t)(grp * 128 + ((sub ^ (grp + 4)) * 16));
   const char *line_src = reinterpret_cast<const char *>(v.lines) + sub * 16;
-  // ring state (warp-uniform): fl_n entries from fl_pos on are the round in flight (ASYNC), the pd_n entries after
+  // ring state (warp-uniform): fl_n entries from fl_pos on are the round in flight (MODE 0), the pd_n entries after
   // them wait for the next round; fl_pos stays a multiple of 32 (only the very last round is partial)
   uint32_t fl_pos = 0, fl_n = 0, pd_n = 0;
   bool more = true;
@@ -691,23 +685,21 @@ __global__ void __launch_bounds__(THREADS, scan_min_ctas(THREADS, ASYNC, ILP, sc
     fl_pos = wrap(fl_pos + fl_n);
     fl_n = 0;
   };
-  // A context k-mer of up to 48 bases never uses the top word of its 16 bytes: it is not loaded at all.  (Loaded
-  // and unused, its register gets recycled as a temporary while the 16-byte load is still in flight, and that
-  // write-after-write wait exposes the whole load latency -- ncu, profiles/round2_k1.md.)
-  constexpr bool SHORT_CTX = REFK > 0 && REFK <= 48;
-  auto load_kmer = [&](uint32_t i) {
-    if constexpr (SHORT_CTX && LD != 0) {
-      const uint2 lo = ldg_na(reinterpret_cast<const uint2 *>(src.kmers + i));
-      return make_uint4(lo.x, lo.y, ldg_na(reinterpret_cast<const uint32_t *>(src.kmers + i) + 2), 0u);
-    } else if constexpr (SHORT_CTX) {
-      const uint2 lo = __ldg(reinterpret_cast<const uint2 *>(src.kmers + i));
-      return make_uint4(lo.x, lo.y, __ldg(reinterpret_cast<const uint32_t *>(src.kmers + i) + 2), 0u);
-    } else {
-      return __ldg(src.kmers + i);
-    }
-  };
-  if constexpr (ASYNC) {
-    constexpr uint32_t W = 32u * ILP;  // k-mers per warp and iteration: ILP per lane
+  if constexpr (MODE == 0) {  // asynchronous rounds, two k-mers per lane
+    // A context k-mer of up to 48 bases never uses the top word of its 16 bytes: it is not loaded at all.  (Loaded
+    // and unused, its register gets recycled as a temporary while the 16-byte load is still in flight, and that
+    // write-after-write wait exposes the whole load latency -- ncu, profiles/round2_k1.md.)
+    constexpr bool SHORT_CTX = REFK > 0 && REFK <= 48;
+    auto load_kmer = [&](uint32_t i) {
+      if constexpr (SHORT_CTX) {
+        const uint2 lo = ldg_na(reinterpret_cast<const uint2 *>(src.kmers + i));
+        return make_uint4(lo.x, lo.y, ldg_na(reinterpret_cast<const uint32_t *>(src.kmers + i) + 2), 0u);
+      } else {
+        return __ldg(src.kmers + i);
+      }
+    };
+    constexpr int ILP = S.ilp;
+    constexpr uint32_t W = 32u * ILP;  // k-mers per warp and iteration
     uint32_t base = warp_id * W;
     uint4 q_cur[ILP];
     uint32_t c_cur[ILP];
@@ -715,7 +707,7 @@ __global__ void __launch_bounds__(THREADS, scan_min_ctas(THREADS, ASYNC, ILP, sc
     for (int u = 0; u < ILP; ++u) {
       const uint32_t i = base + 32u * u + lane;
       q_cur[u] = i < n32 ? load_kmer(i) : make_uint4(0, 0, 0, 0);
-      c_cur[u] = i < n32 ? (LD ? ldg_na(src.counts + i) : __ldg(src.counts + i)) : 0u;
+      c_cur[u] = i < n32 ? ldg_na(src.counts + i) : 0u;
     }
     for (;; base += step * ILP) {
       more = more && base < n32;
@@ -735,7 +727,7 @@ __global__ void __launch_bounds__(THREADS, scan_min_ctas(THREADS, ASYNC, ILP, sc
           for (int u = 0; u < ILP; ++u) {
             const uint32_t i = nb + 32u * u + lane;
             q_cur[u] = i < n32 ? load_kmer(i) : make_uint4(0, 0, 0, 0);
-            c_cur[u] = i < n32 ? (LD ? ldg_na(src.counts + i) : __ldg(src.counts + i)) : 0u;
+            c_cur[u] = i < n32 ? ldg_na(src.counts + i) : 0u;
           }
           if (lane < 5 * ILP && nb + step * ILP < n32) {  // and the batch after that into L2 (k-mers, then counts)
             const char *pf = lane < 4 * ILP
@@ -746,7 +738,7 @@ __global__ void __launch_bounds__(THREADS, scan_min_ctas(THREADS, ASYNC, ILP, sc
         }
         uint64_t idx[ILP];
 #pragma unroll
-        for (int u = 0; u < ILP; ++u) {  // (straight-line code over the ILP independent chains: they interleave)
+        for (int u = 0; u < ILP; ++u) {  // (straight-line code over the independent chains: they interleave)
           const u128 x35 = mask128(shr128(x43[u], 2 * tail), 2 * k);
           uint64_t h;
           if constexpr (K > 0)
@@ -755,76 +747,47 @@ __global__ void __launch_bounds__(THREADS, scan_min_ctas(THREADS, ASYNC, ILP, sc
             h = canon_hash_rt(x35, k, &canon[u]);
           idx[u] = bf_index(v, h);
         }
-        if constexpr (LD == 2) {
-          uint32_t ob[ILP];  // bit inside the 16-byte piece
-          if (v.occ) {
-#pragma unroll
-            for (int u = 0; u < ILP; ++u) {
-              const uint64_t o = idx[u] >> v.occ_shift;
-              ob[u] = (uint32_t)o & 127u;
-              cp_async16(oslot_addr + (uint32_t)(u * 512), reinterpret_cast<const char *>(v.occ) + ((o >> 7) << 4));
-            }
-            asm volatile("cp.async.commit_group;\n" ::: "memory");
-            asm volatile("cp.async.wait_group 0;\n" ::: "memory");
-          }
+        // occupancy pre-filter (L2): most probe lines hold nothing for a given k-mer; those are never fetched
+        uint32_t ob[ILP];  // bit inside the 16-byte piece
+        if (v.occ) {
 #pragma unroll
           for (int u = 0; u < ILP; ++u) {
-            bool hit = true;
-            if (v.occ) hit = (reinterpret_cast<const uint32_t *>(oslot + u * 32)[ob[u] >> 5] >> (ob[u] & 31u)) & 1u;
-            need[u] = base + 32u * u + lane < n32 && hit;
-            idx_hi[u] = (uint32_t)(idx[u] >> 8);
-            bit[u] = (uint32_t)(idx[u] & 255);
+            const uint64_t o = idx[u] >> v.occ_shift;
+            ob[u] = (uint32_t)o & 127u;
+            cp_async16(oslot_addr + (uint32_t)(u * 512), reinterpret_cast<const char *>(v.occ) + ((o >> 7) << 4));
           }
-        } else {
+          asm volatile("cp.async.commit_group;\n" ::: "memory");
+          asm volatile("cp.async.wait_group 0;\n" ::: "memory");
+        }
 #pragma unroll
-        for (int u = 0; u < ILP; ++u) {  // occupancy pre-filter (L2), all words in flight together
-          need[u] = base + 32u * u + lane < n32 && occ_test<LD != 0>(v, idx[u]);
+        for (int u = 0; u < ILP; ++u) {
+          bool hit = true;
+          if (v.occ) hit = (reinterpret_cast<const uint32_t *>(oslot + u * 32)[ob[u] >> 5] >> (ob[u] & 31u)) & 1u;
+          need[u] = base + 32u * u + lane < n32 && hit;
           idx_hi[u] = (uint32_t)(idx[u] >> 8);  // n_lines < 2^32 (bf_bits < 2^40)
           bit[u] = (uint32_t)(idx[u] & 255);
         }
+        // all k-mers of the lane go into the ring in one go
+        const uint32_t lt = (1u << lane) - 1u, at = fl_pos + fl_n + pd_n;
+        uint32_t m[ILP], off = 0;
+#pragma unroll
+        for (int u = 0; u < ILP; ++u) m[u] = __ballot_sync(0xffffffffu, need[u]);
+#pragma unroll
+        for (int u = 0; u < ILP; ++u) {
+          if (need[u]) {
+            const uint32_t e = wrap(at + off + (uint32_t)__popc(m[u] & lt));
+            qkey[e] = uint4_of(canon[u]);
+            qmeta[e] = make_uint4(idx_hi[u], base + 32u * u + lane, cnt[u], bit[u]);
+          }
+          off += (uint32_t)__popc(m[u]);
         }
-        if constexpr (scan_push_all(ASYNC, ILP, LD)) {  // all k-mers of the lane go into the ring in one go
-          const uint32_t lt = (1u << lane) - 1u, at = fl_pos + fl_n + pd_n;
-          uint32_t m[ILP], off = 0;
-#pragma unroll
-          for (int u = 0; u < ILP; ++u) m[u] = __ballot_sync(0xffffffffu, need[u]);
-#pragma unroll
-          for (int u = 0; u < ILP; ++u) {
-            if (need[u]) {
-              const uint32_t e = wrap(at + off + (uint32_t)__popc(m[u] & lt));
-              qkey[e] = uint4_of(canon[u]);
-              qmeta[e] = make_uint4(idx_hi[u], base + 32u * u + lane, cnt[u], bit[u]);
-            }
-            off += (uint32_t)__popc(m[u]);
-          }
-          pd_n += off;
-          // a full ring turns: the round in flight is finished (started a batch or more ago: its lines have landed),
-          // the next one started (again when the batches passed the pre-filter almost whole)
+        pd_n += off;
+        // a full ring turns: the round in flight is finished (started a batch or more ago: its lines have landed),
+        // the next one started (again when the batches passed the pre-filter almost whole)
 #pragma unroll 1
-          while (pd_n >= 32) {
-            if (fl_n) complete_round();
-            start_round();
-          }
-        } else {
-#pragma unroll 1
-          for (int u = 0; u < ILP; ++u) {
-            const bool hi = ILP == 2 && u == 1;
-            const bool nd = hi ? need[ILP - 1] : need[0];
-            const uint32_t need_mask = __ballot_sync(0xffffffffu, nd);
-            if (nd) {
-              const uint32_t e = wrap(fl_pos + fl_n + pd_n + (uint32_t)__popc(need_mask & ((1u << lane) - 1u)));
-              qkey[e] = uint4_of(hi ? canon[ILP - 1] : canon[0]);
-              qmeta[e] = make_uint4(hi ? idx_hi[ILP - 1] : idx_hi[0], base + 32u * u + lane, hi ? cnt[ILP - 1] : cnt[0],
-                                    hi ? bit[ILP - 1] : bit[0]);
-            }
-            pd_n += (uint32_t)__popc(need_mask);
-            // a full ring turns: the round in flight is finished (started a batch or more ago: its lines have landed),
-            // the next one started
-            if (pd_n >= 32) {
-              if (fl_n) complete_round();
-              start_round();
-            }
-          }
+        while (pd_n >= 32) {
+          if (fl_n) complete_round();
+          start_round();
         }
       } else {  // the tail: nothing more to hash
         if (fl_n) complete_round();
@@ -832,104 +795,13 @@ __global__ void __launch_bounds__(THREADS, scan_min_ctas(THREADS, ASYNC, ILP, sc
         if (pd_n == 0 && fl_n == 0) break;
       }
     }
-  } else if constexpr (ILP == 2) {  // synchronous rounds, two k-mers per lane
-    for (uint32_t base = warp_id * 64;; base += 2 * step) {
+  } else {  // synchronous rounds, one KMC record per lane
+    for (uint32_t base = warp_id * 32;; base += step) {
       more = more && base < n32;
       if (more) {
-        uint4 q[2];
-        uint32_t cnt[2], idx_lo[2], bit[2];
-        bool need[2];
-        u128 canon[2];
-#pragma unroll
-        for (int u = 0; u < 2; ++u) {
-          const uint32_t i = base + 32u * u + lane;
-          q[u] = i < n32 ? load_kmer(i) : make_uint4(0, 0, 0, 0);
-          cnt[u] = i < n32 ? (LD ? ldg_na(src.counts + i) : __ldg(src.counts + i)) : 0u;
-        }
-        // the warp's next 64 k-mers (1 KB + 256 B of counts) into L2 while these are hashed
-        if (lane < 10 && base + 2 * step < n32) {
-          const char *pf = lane < 8 ? reinterpret_cast<const char *>(src.kmers + base + 2 * step) + lane * 128
-                                    : reinterpret_cast<const char *>(src.counts + base + 2 * step) + (lane - 8) * 128;
-          asm volatile("prefetch.global.L2 [%0];" ::"l"(pf));
-        }
-        uint64_t idx[2];
-#pragma unroll
-        for (int u = 0; u < 2; ++u) {
-          const u128 x35 = mask128(shr128(u128_of(q[u]), 2 * tail), 2 * k);
-          uint64_t h;
-          if constexpr (K > 0)
-            h = canon_hash_lut<K>(x35, &canon[u], tab);
-          else
-            h = canon_hash_rt(x35, k, &canon[u]);
-          idx[u] = bf_index(v, h);
-        }
-        if constexpr (LD == 2) {  // the pieces land in the tile: no round is in flight here
-          uint32_t ob[2];
-          if (v.occ) {
-#pragma unroll
-            for (int u = 0; u < 2; ++u) {
-              const uint64_t o = idx[u] >> v.occ_shift;
-              ob[u] = (uint32_t)o & 127u;
-              cp_async16(oslot_addr + (uint32_t)(u * 512), reinterpret_cast<const char *>(v.occ) + ((o >> 7) << 4));
-            }
-            asm volatile("cp.async.commit_group;\n" ::: "memory");
-            asm volatile("cp.async.wait_group 0;\n" ::: "memory");
-          }
-#pragma unroll
-          for (int u = 0; u < 2; ++u) {
-            bool hit = true;
-            if (v.occ) hit = (reinterpret_cast<const uint32_t *>(oslot + u * 32)[ob[u] >> 5] >> (ob[u] & 31u)) & 1u;
-            need[u] = base + 32u * u + lane < n32 && hit;
-            idx_lo[u] = (uint32_t)(idx[u] >> 8);
-            bit[u] = (uint32_t)(idx[u] & 255);
-          }
-        } else {
-#pragma unroll
-        for (int u = 0; u < 2; ++u) {  // (both pre-filter words are in flight together)
-          need[u] = base + 32u * u + lane < n32 && occ_test<LD != 0>(v, idx[u]);
-          idx_lo[u] = (uint32_t)(idx[u] >> 8);
-          bit[u] = (uint32_t)(idx[u] & 255);
-        }
-        }
-#pragma unroll 1
-        for (int u = 0; u < 2; ++u) {
-          const bool nd = u ? need[1] : need[0];
-          const uint32_t need_mask = __ballot_sync(0xffffffffu, nd);
-          if (nd) {
-            const uint32_t e = wrap(fl_pos + fl_n + pd_n + (uint32_t)__popc(need_mask & ((1u << lane) - 1u)));
-            qkey[e] = uint4_of(u ? canon[1] : canon[0]);
-            qmeta[e] = make_uint4(u ? idx_lo[1] : idx_lo[0], base + 32u * u + lane, u ? cnt[1] : cnt[0], u ? bit[1] : bit[0]);
-          }
-          pd_n += (uint32_t)__popc(need_mask);
-          if (pd_n >= 32) {
-            start_round();
-            complete_round();
-          }
-        }
-      } else if (pd_n) {
-        start_round();
-        complete_round();
-      }
-      if (!more && pd_n == 0) break;
-    }
-  } else {
-  for (uint32_t base = warp_id * 32;; base += step) {
-    more = more && base < n32;
-    if (more) {
-      const uint32_t i = base + lane;
-      bool live = i < n32;
-      uint32_t cnt;
-      u128 x43, canon;
-      if constexpr (MODE == 0) {
-        x43 = u128_of(live ? load_kmer(i) : make_uint4(0, 0, 0, 0));
-        cnt = live ? (LD ? ldg_na(src.counts + i) : __ldg(src.counts + i)) : 0u;
-        // the warp's next batch (512 B of k-mers + 128 B of counts) into L2 while this one is hashed
-        if (lane < 5 && base + step < n32) {
-          const char *pf = lane < 4 ? reinterpret_cast<const char *>(src.kmers + base + step) + lane * 128
-                                    : reinterpret_cast<const char *>(src.counts + base + step);
-          asm volatile("prefetch.global.L2 [%0];" ::"l"(pf));
-        }
-      } else {
+        const uint32_t i = base + lane;
+        bool live = i < n32;
+        u128 x43, canon;
         // stage the warp's 32 records (contiguous bytes) in its shared-memory tile, then decode one per lane
         const int rec = src.suf_bytes + src.counter_size;
         const uint64_t byte0 = (uint64_t)base * (uint64_t)rec, start = byte0 & ~3ull;
@@ -966,18 +838,16 @@ __global__ void __launch_bounds__(THREADS, scan_min_ctas(THREADS, ASYNC, ILP, sc
         x43.hi = pre.hi | suf.hi;
         // CKMCFile::ReadNextKmer skips records whose count is outside [min_count, max_count]
         if (c64 < src.min_count || c64 > src.max_count) live = false;
-        cnt = (uint32_t)c64;
-      }
-      u128 x35 = mask128(shr128(x43, 2 * tail), 2 * k);
-      uint64_t h;
-      if constexpr (K > 0)
-        h = canon_hash_lut<K>(x35, &canon, tab);
-      else
-        h = canon_hash_rt(x35, k, &canon);
-      const uint64_t idx = bf_index(v, h);
-      // occupancy pre-filter (L2): most probe lines hold nothing for a given k-mer; those are never fetched
-      bool need = live;
-      if constexpr (LD == 2) {
+        const uint32_t cnt = (uint32_t)c64;
+        u128 x35 = mask128(shr128(x43, 2 * tail), 2 * k);
+        uint64_t h;
+        if constexpr (K > 0)
+          h = canon_hash_lut<K>(x35, &canon, tab);
+        else
+          h = canon_hash_rt(x35, k, &canon);
+        const uint64_t idx = bf_index(v, h);
+        // occupancy pre-filter (L2): most probe lines hold nothing for a given k-mer; those are never fetched
+        bool need = live;
         if (v.occ) {
           const uint64_t o = idx >> v.occ_shift;
           cp_async16(oslot_addr, reinterpret_cast<const char *>(v.occ) + ((o >> 7) << 4));
@@ -985,24 +855,21 @@ __global__ void __launch_bounds__(THREADS, scan_min_ctas(THREADS, ASYNC, ILP, sc
           asm volatile("cp.async.wait_group 0;\n" ::: "memory");
           need = live && ((reinterpret_cast<const uint32_t *>(oslot)[((uint32_t)o & 127u) >> 5] >> ((uint32_t)o & 31u)) & 1u);
         }
-      } else {
-        need = live && occ_test<LD != 0>(v, idx);
+        const uint32_t need_mask = __ballot_sync(0xffffffffu, need);
+        if (need) {
+          const uint32_t e = (fl_pos + fl_n + pd_n + (uint32_t)__popc(need_mask & ((1u << lane) - 1u))) & (SCAN_Q - 1);
+          qkey[e] = uint4_of(x43);  // (complete_round derives the canonical k-mer from the record's context k-mer)
+          qmeta[e] = make_uint4((uint32_t)(idx >> 8), i, cnt, (uint32_t)(idx & 255));  // n_lines < 2^32 (bf_bits < 2^40)
+        }
+        pd_n += (uint32_t)__popc(need_mask);
       }
-      const uint32_t need_mask = __ballot_sync(0xffffffffu, need);
-      if (need) {
-        const uint32_t e = (fl_pos + fl_n + pd_n + (uint32_t)__popc(need_mask & ((1u << lane) - 1u))) & (SCAN_Q - 1);
-        qkey[e] = uint4_of(MODE == 0 ? canon : x43);
-        qmeta[e] = make_uint4((uint32_t)(idx >> 8), i, cnt, (uint32_t)(idx & 255));  // n_lines < 2^32 (bf_bits < 2^40)
+      if (pd_n >= 32 || (!more && pd_n)) {
+        start_round();
+        complete_round();
       }
-      pd_n += (uint32_t)__popc(need_mask);
+      if (!more && pd_n == 0) break;
     }
-    if (pd_n >= 32 || (!RING && pd_n) || (!more && pd_n)) {
-      start_round();
-      complete_round();
-    }
-    if (!more && pd_n == 0) break;
   }
-  }  // !ASYNC
   if (src.hit_buf) {
     __syncwarp();
     if (lane == 0) src.hit_counts[warp_id] = *hitc < src.seg_cap ? *hitc : src.seg_cap;

@@ -109,7 +109,6 @@ struct mg_ctx {
   uint32_t *hit_counts[2] = {nullptr, nullptr};
   uint64_t hit_entries[2] = {0, 0}, hit_warps[2] = {0, 0};
   bool defer_hits = true;
-  int scan_ctas_per_sm = 64;  // grid cap of the scan kernel, in 256-thread CTAs per SM (measured optimum 32..128, profiles/)
   uint64_t *kmc_lut = nullptr;  // device copy of the KMC prefix LUT (+ guard)
   uint32_t kmc_n_lut = 0, kmc_min = 0;
   uint64_t kmc_max = 0;
@@ -225,7 +224,6 @@ static int ctx_init(mg_ctx *c) {
   cudaDeviceProp prop;
   CU(cudaGetDeviceProperties(&prop, device));
   c->sms = prop.multiProcessorCount;
-  if (const char *e = getenv("MG_SCAN_CTAS_PER_SM")) c->scan_ctas_per_sm = atoi(e) > 0 ? atoi(e) : 64;
   if (const char *e = getenv("MG_SCAN_DEFER_HITS")) c->defer_hits = atoi(e) != 0;
   for (int i = 0; i < 2; ++i) CU(cudaStreamCreateWithFlags(&c->stream[i], cudaStreamNonBlocking));
   CU(cudaMalloc(&c->lines, c->n_lines * 128));
@@ -794,13 +792,13 @@ extern "C" int mg_finalize_context(mg_ctx *c) {
   return MG_OK;
 }
 
-template <int K, int REFK, int MODE, int THREADS, bool RING, bool ASYNC, int ILP = 1, int LD = 0>
+template <int K, int REFK, int MODE>
 static cudaError_t launch_scan(mg_ctx *c, const mg::ScanSrc &src_in, uint64_t n, cudaStream_t st) {
-  constexpr int WARPS = THREADS / 32;
-  uint64_t want = (n + THREADS * ILP - 1) / (THREADS * ILP);  // one warp per 32 (64) k-mers
-  int per_sm = c->scan_ctas_per_sm;
-  if (const char *ev = getenv("MG_SCAN_CTAS_PER_SM")) per_sm = atoi(ev) > 0 ? atoi(ev) : per_sm;  // (sweeps: read per launch)
-  uint64_t cap = (uint64_t)c->sms * (uint64_t)per_sm * (256 / THREADS);
+  constexpr mg::ScanShape S = mg::scan_shape(MODE);
+  constexpr int WARPS = mg::SCAN_THREADS / 32;
+  constexpr int CTAS_PER_SM = 64;  // grid cap (measured optimum 32..128, profiles/): past it, every warp takes more batches
+  uint64_t want = (n + mg::SCAN_THREADS * S.ilp - 1) / (mg::SCAN_THREADS * S.ilp);  // one warp per 32 (64) k-mers
+  uint64_t cap = (uint64_t)c->sms * CTAS_PER_SM;
   int grid = (int)(want < cap ? want : cap);
   if (grid < 1) grid = 1;
   mg::ScanSrc src = src_in;
@@ -831,32 +829,15 @@ static cudaError_t launch_scan(mg_ctx *c, const mg::ScanSrc &src_in, uint64_t n,
     src.hit_counts = c->hit_counts[si];
     src.seg_cap = (uint32_t)seg;
   }
-  constexpr int SMEM = mg::scan_smem(THREADS, ASYNC, ILP, mg::scan_occs(LD, ASYNC, ILP));
-  if (SMEM > 48 * 1024) {  // more than 48 KB of dynamic shared memory needs the opt-in (per device; cheap enough to repeat)
-    cudaError_t e = cudaFuncSetAttribute(mg::k_scan<K, REFK, MODE, THREADS, RING, ASYNC, ILP, LD>,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM);
-    if (e != cudaSuccess) return e;
-  }
-  if (LD == 2 && !getenv("MG_SCAN_CARVEOUT")) {  // nothing of this build's traffic needs L1: all of it to shared memory
-    cudaError_t e = cudaFuncSetAttribute(mg::k_scan<K, REFK, MODE, THREADS, RING, ASYNC, ILP, LD>,
-                                         cudaFuncAttributePreferredSharedMemoryCarveout, 100);
-    if (e != cudaSuccess) return e;
-  }
-  if (const char *ev = getenv("MG_SCAN_CARVEOUT")) {  // (sweeps) shared-memory share of the unified L1, percent
-    cudaError_t e = cudaFuncSetAttribute(mg::k_scan<K, REFK, MODE, THREADS, RING, ASYNC, ILP, LD>,
-                                         cudaFuncAttributePreferredSharedMemoryCarveout, atoi(ev));
-    if (e != cudaSuccess) return e;
-    int nb = 0;
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, mg::k_scan<K, REFK, MODE, THREADS, RING, ASYNC, ILP, LD>, THREADS, SMEM);
-    static int said = -1;
-    if (said != atoi(ev) * 1000 + THREADS) {
-      said = atoi(ev) * 1000 + THREADS;
-      fprintf(stderr, "[k_scan] carveout %d %%: %d CTAs of %d threads per SM, %d B of shared memory each\n", atoi(ev), nb, THREADS, SMEM);
-    }
-  }
+  // both modes take more than 48 KB of dynamic shared memory: the opt-in (per device; cheap enough to repeat).  Nothing
+  // of the scan's traffic needs L1 (the pre-filter pieces come through cp.async): all of it to shared memory.
+  const auto kernel = mg::k_scan<K, REFK, MODE>;
+  cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, S.smem);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+  if (e != cudaSuccess) return e;
   c->launches++;
-  mg::k_scan<K, REFK, MODE, THREADS, RING, ASYNC, ILP, LD><<<grid, THREADS, SMEM, st>>>(src, n, c->view());
-  cudaError_t e = cudaGetLastError();
+  kernel<<<grid, mg::SCAN_THREADS, S.smem, st>>>(src, n, c->view());
+  e = cudaGetLastError();
   if (e != cudaSuccess || !src.hit_buf) return e;
   const uint64_t threads = n_warps * src.seg_cap;
   c->launches++;
@@ -865,54 +846,14 @@ static cudaError_t launch_scan(mg_ctx *c, const mg::ScanSrc &src_in, uint64_t n,
   return cudaGetLastError();
 }
 
+// the scan kernel for the context's (k, ref_k): specialised hashes for (35, 43), run-time ones for any other
 template <int MODE>
 static int scan_src(mg_ctx *c, const mg::ScanSrc &src, uint64_t n, cudaStream_t st) {
   cudaError_t e;
-  if (c->k == 35 && c->ref_k == 43) {
-    // MG_SCAN_VARIANT (tuning sweeps, profiles/sweep_k1_r2.py): the schemes tried for the packed-input scan.
-    // Default = 0: two k-mers per lane, asynchronous probe rounds, 256-thread CTAs, pre-filter pieces through
-    // cp.async (profiles/round2_k1.md).
-    int variant = 0;
-    if (MODE == 0)
-      if (const char *ev = getenv("MG_SCAN_VARIANT")) variant = atoi(ev);
-    if (MODE == 0 && variant == 1)
-      e = launch_scan<35, 43, 0, 256, true, false>(c, src, n, st);     // one k-mer per lane, synchronous rounds
-    else if (MODE == 0 && variant == 2)
-      e = launch_scan<35, 43, 0, 256, false, false>(c, src, n, st);    // probe after every batch (the round-1 scheme)
-    else if (MODE == 0 && variant == 3)
-      e = launch_scan<35, 43, 0, 256, true, true>(c, src, n, st);      // one k-mer per lane, asynchronous rounds
-    else if (MODE == 0 && variant == 4)
-      e = launch_scan<35, 43, 0, 256, true, false, 2>(c, src, n, st);  // two k-mers per lane, synchronous rounds
-    else if (MODE == 0 && variant == 5)
-      e = launch_scan<35, 43, 0, 128, true, false, 2>(c, src, n, st);
-    else if (MODE == 0 && variant == 6)
-      e = launch_scan<35, 43, 0, 128, true, true, 2>(c, src, n, st);   // two k-mers per lane, asynchronous rounds, 128
-    else if (MODE == 0 && variant == 7)
-      e = launch_scan<35, 43, 0, 256, true, true, 2>(c, src, n, st);     // the default, all loads through L1
-    else if (MODE == 0 && variant == 8)
-      e = launch_scan<35, 43, 0, 256, true, true, 2, 1>(c, src, n, st);  // the default, loads that do not allocate in L1
-    else if (MODE == 0 && variant == 9)
-      e = launch_scan<35, 43, 0, 128, true, true, 2, 2>(c, src, n, st);  // the default with 128-thread CTAs
-    else if (MODE == 0 && variant == 10)
-      e = launch_scan<35, 43, 0, 256, true, false, 1, 2>(c, src, n, st);  // one k-mer per lane, 4 CTAs (32 warps) per SM
-    else if (MODE == 0 && variant == 11)
-      e = launch_scan<35, 43, 0, 256, true, false, 2, 2>(c, src, n, st);  // two per lane, synchronous, 4 CTAs per SM
-    else if (MODE == 0 && variant == 12)
-      e = launch_scan<35, 43, 0, 128, true, true, 3, 2>(c, src, n, st);   // three k-mers per lane, 5 CTAs of 128
-    else if (MODE == 0 && variant == 13)
-      e = launch_scan<35, 43, 0, 128, true, true, 4, 2>(c, src, n, st);   // four k-mers per lane, 4 CTAs of 128
-    else if (MODE == 0 && variant == 14)
-      e = launch_scan<35, 43, 0, 256, true, true, 3, 2>(c, src, n, st);   // three k-mers per lane, 2 CTAs of 256
-    else if (MODE == 0)
-      e = launch_scan<35, 43, 0, 256, true, true, 2, 2>(c, src, n, st);
-    else
-      e = launch_scan<35, 43, MODE, 256, true, false, 1, 2>(c, src, n, st);
-  } else {
-    if (MODE == 0)
-      e = launch_scan<0, 0, 0, 256, true, true, 2, 2>(c, src, n, st);
-    else
-      e = launch_scan<0, 0, MODE, 256, true, false, 1, 2>(c, src, n, st);
-  }
+  if (c->k == 35 && c->ref_k == 43)
+    e = launch_scan<35, 43, MODE>(c, src, n, st);
+  else
+    e = launch_scan<0, 0, MODE>(c, src, n, st);
   if (e != cudaSuccess) return set_err(MG_ERR_CUDA, "k_scan launch -> %s", cudaGetErrorString(e));
   return MG_OK;
 }

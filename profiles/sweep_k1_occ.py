@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""K1 sweep on the bench workload: occupancy pre-filter size (MG_OCC_LOG2_BITS, 0 = off) x L2 persistence x CTAs/SM.
+"""K1 sweep on the bench workload: occupancy pre-filter size (MG_OCC_LOG2_BITS, 0 = off) x L2 persistence x deferred hits.
 Run on a GPU box:  python profiles/sweep_k1_occ.py [wg|small] > gpurun_out/sweep_k1_occ.txt"""
 import os
 import sys
@@ -27,14 +27,13 @@ del alt, ref
 p = torch.cuda.get_device_properties(0)
 print("L2", p.L2_cache_size, flush=True)
 
-configs = [(29, 1, 128, 1), (29, 1, 128, 0)]
+configs = [(29, 1, 1), (29, 1, 0)]
 for sig_frac in (1.0, 0.1):
     n_sig = int(len(alt_h) * sig_frac)
-    for occ, persist, ctas, defer in configs:
+    for occ, persist, defer in configs:
         os.environ["MG_SCAN_DEFER_HITS"] = str(defer)
         os.environ["MG_OCC_LOG2_BITS"] = str(occ)
         os.environ["MG_L2_PERSIST"] = str(persist)
-        os.environ["MG_SCAN_CTAS_PER_SM"] = str(ctas)
         g = MalvaGpu(k=bench.K, ref_k=bench.REF_K, bf_bits=wl["bf_bits"])
         chunk = 1 << 24
         for arr, flag in ((alt_h[:n_sig], 0), (ref_h[:n_sig], 1)):
@@ -51,6 +50,6 @@ for sig_frac in (1.0, 0.1):
             g.scan_sample_kmers_ptr(batches[i & 1][0].data_ptr(), batches[i & 1][1].data_ptr(), B, device=True)
         g.event_record(1)
         ms = g.event_elapsed_ms(0, 1) / n
-        print(f"signatures={2 * n_sig:.1e} occ_log2={occ} persist={persist} ctas_per_sm={ctas} defer_hits={defer}: {ms:.3f} ms/scan  "
+        print(f"signatures={2 * n_sig:.1e} occ_log2={occ} persist={persist} defer_hits={defer}: {ms:.3f} ms/scan  "
               f"{B / ms / 1e6:.2f} G k-mers/s  {B * 84 / ms / 1e6:.0f} GB/s algorithmic", flush=True)
         g.close()

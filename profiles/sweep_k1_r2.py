@@ -1,14 +1,9 @@
 #!/usr/bin/env python
-"""Round-2 sweep of the sample-scan kernel (K1) on the bench workload: probe scheme x CTA size x grid cap
-(MG_SCAN_VARIANT: 0 = two k-mers per lane, asynchronous rounds, 256-thread CTAs, pre-filter pieces through cp.async
-(default); 1 = one k-mer per lane, synchronous rounds; 2 = probe after every batch of 32 k-mers as in round 1; 3 = one
-k-mer per lane, asynchronous rounds; 4 / 5 = two k-mers per lane, synchronous rounds, 256 / 128 threads; 6 = as 7 with
-128 threads; 7 = as 0 with every load through L1; 8 = as 7 with loads that do not allocate in L1; 9 = as 0 with
-128 threads; 10 / 11 = one / two k-mers per lane, synchronous rounds, cp.async pre-filter, 4 CTAs per SM; 12 / 13 = three /
-four k-mers per lane in 128-thread CTAs; 14 = three per lane in 256-thread CTAs;
-MG_SCAN_CTAS_PER_SM: grid cap in 256-thread units; MG_SCAN_CARVEOUT: shared-memory carve-out in percent).
-The index is built once; the variant is read at every launch.
-    python profiles/sweep_k1_r2.py [--workload wg] [--variants 0,1,2,3] [--reps 10] > gpurun_out/r2_sweep_k1.txt"""
+"""Times the sample-scan kernel (K1, k_scan + k_scan_hits) on a bench workload: the index is built once, then
+--reps scans of 2^27 packed k-mers run back to back between two CUDA events.  `--workload l2` keeps every probe line
+L2-resident, which gives the kernel's arithmetic floor.  The schemes the round-2 sweeps compared (probe scheme, CTA
+size, grid cap, carve-out) are recorded in profiles/round2_sweep_k1_*.txt.
+    python profiles/sweep_k1_r2.py [--workload wg] [--reps 10]"""
 import argparse
 import os
 import sys
@@ -24,9 +19,7 @@ from malva_b200.kmc import KMER_DTYPE  # noqa: E402
 
 ap = argparse.ArgumentParser()
 ap.add_argument("--workload", default="wg")
-ap.add_argument("--variants", default="0,1,2,3")
 ap.add_argument("--reps", type=int, default=10)
-ap.add_argument("--ctas", default="128")
 args = ap.parse_args()
 wl = bench.WORKLOADS[args.workload]
 dev = torch.device("cuda", 0)
@@ -46,17 +39,14 @@ g.finalize_context()
 batches = [bench.make_sample_batch(torch, B, alt, ref, gen, dev)[:2] for _ in range(2)]
 del alt, ref
 torch.cuda.synchronize()
-for v, ctas in [(int(x), int(y)) for x in args.variants.split(",") for y in args.ctas.split(",")]:
-    os.environ["MG_SCAN_VARIANT"] = str(v)
-    os.environ["MG_SCAN_CTAS_PER_SM"] = str(ctas)
-    for i in range(3):
-        g.scan_sample_kmers_ptr(batches[i & 1][0].data_ptr(), batches[i & 1][1].data_ptr(), B, device=True)
-    g.sync()
-    g.event_record(0)
-    for i in range(args.reps):
-        g.scan_sample_kmers_ptr(batches[i & 1][0].data_ptr(), batches[i & 1][1].data_ptr(), B, device=True)
-    g.event_record(1)
-    ms = g.event_elapsed_ms(0, 1) / args.reps
-    print(f"variant={v} ctas_per_sm={ctas}: {ms:.3f} ms/scan  {B / ms / 1e6:.2f} G k-mers/s  {B * 84 / ms / 1e6:.0f} GB/s algorithmic "
-          f"(frac {B * 84 / ms / 1e6 / 6551.4:.3f})", flush=True)
+for i in range(3):
+    g.scan_sample_kmers_ptr(batches[i & 1][0].data_ptr(), batches[i & 1][1].data_ptr(), B, device=True)
+g.sync()
+g.event_record(0)
+for i in range(args.reps):
+    g.scan_sample_kmers_ptr(batches[i & 1][0].data_ptr(), batches[i & 1][1].data_ptr(), B, device=True)
+g.event_record(1)
+ms = g.event_elapsed_ms(0, 1) / args.reps
+print(f"workload={args.workload}: {ms:.3f} ms/scan  {B / ms / 1e6:.2f} G k-mers/s  {B * 84 / ms / 1e6:.0f} GB/s algorithmic "
+      f"(frac {B * 84 / ms / 1e6 / 6551.4:.3f})", flush=True)
 g.close()

@@ -77,12 +77,9 @@ def test_index_scan_state_bit_exact(oracle_lib, k, ref_k, bf_bits):
         o.close()
 
 
-@pytest.mark.parametrize("variant", list(range(1, 15)))
-def test_every_scan_build_is_bit_exact(oracle_lib, monkeypatch, variant):
-    """the other builds of the (35, 43) scan kernel that the sweeps select with MG_SCAN_VARIANT (csrc/malva_gpu.cu:
-    probe after every batch, ring with synchronous / asynchronous rounds, one or two k-mers per lane, 128-thread CTAs,
-    loads through L1, four CTAs per SM, three and four k-mers per lane) leave exactly the oracle's counters -- dense filter, counts past 2^16"""
-    monkeypatch.setenv("MG_SCAN_VARIANT", str(variant))       # (read at every launch)
+def test_scan_dense_filter_big_counts_bit_exact(oracle_lib):
+    """the (35, 43) packed-input scan leaves exactly the oracle's counters on a dense non-power-of-two filter with
+    counts past 2^16"""
     g, o, genome, nested, freqs, ks, fl, words = _run_pair(oracle_lib, 35, 43, 3 * (1 << 18) + 5, seed=4242, n_var=400,
                                                            n_sample=9000, big_counts=True)
     try:
