@@ -106,15 +106,11 @@ typedef struct {
   double *lik;             /* un-normalised probabilities, emission order (may be NULL)      */
 } mg_genotype_out;
 
+/* The reference-shaped form: the library packs the batch on the host into the mg_packed_batch form below and runs
+ * mg_genotype_packed on it; out->lik == NULL: likelihoods are not returned.  Allele slots, signatures and k-mers
+ * of one batch must each number less than 2^32 (MG_ERR_ARG otherwise). */
 int mg_genotype(mg_ctx *ctx, const mg_variant_batch *in, const mg_genotype_out *out, float error_rate,
                 int max_coverage, int haploid);
-/* same with every array of in/out DEVICE-resident (enqueued on the context's stream; mg_sync completes it) */
-typedef struct {
-  uint64_t n_variants, n_alleles, n_sigs, n_kmers;
-  uint64_t pool_bytes; /* readable bytes at in->pool (>= kmer_off[n_kmers]); 0 = unknown (slower byte-wise reads) */
-} mg_batch_dims;
-int mg_genotype_device(mg_ctx *ctx, const mg_variant_batch *in, const mg_genotype_out *out, const mg_batch_dims *dims,
-                       float error_rate, int max_coverage, int haploid);
 
 /* The same step for signature k-mers the host already packed -- what the C++ host (csrc/host/) sends: 16 B per
  * k-mer instead of k ASCII bytes + an 8-byte offset, u32 offsets, no likelihood traffic unless asked for.
@@ -260,8 +256,6 @@ uint64_t mg_selftest_hash_packed(uint64_t lo, uint64_t hi, int k, uint64_t *cano
 uint64_t mg_selftest_hash_packed_k35(uint64_t lo, uint64_t hi);
 uint64_t mg_selftest_hash_packed_k43(uint64_t lo, uint64_t hi);
 uint64_t mg_selftest_hash_ascii(const char *s, int len);
-/* the word-wise ASCII -> 2-bit packer of the signature look-up kernel: 1 = 35 symbols of ACGT (packed word returned) */
-int mg_selftest_pack35(const char *s35, uint64_t *lo, uint64_t *hi);
 float mg_selftest_logf(float x);
 int mg_selftest_genotype(const uint32_t *cov, const float *freq, int n_alleles, float error_rate, int max_cov,
                          int haploid, double *lik, int *status, int *best_gt, int *gq);

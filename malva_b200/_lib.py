@@ -49,11 +49,6 @@ class GenotypeOut(C.Structure):
     ]
 
 
-class BatchDims(C.Structure):
-    _fields_ = [("n_variants", C.c_uint64), ("n_alleles", C.c_uint64), ("n_sigs", C.c_uint64),
-                ("n_kmers", C.c_uint64), ("pool_bytes", C.c_uint64)]
-
-
 class PackedBatch(C.Structure):
     _fields_ = [
         ("n_variants", C.c_uint64),
@@ -95,8 +90,6 @@ SYMBOLS = {
     "mg_sync": (C.c_int, [C.c_void_p]),
     "mg_genotype": (C.c_int, [C.c_void_p, C.POINTER(VariantBatch), C.POINTER(GenotypeOut), C.c_float, C.c_int,
                               C.c_int]),
-    "mg_genotype_device": (C.c_int, [C.c_void_p, C.POINTER(VariantBatch), C.POINTER(GenotypeOut),
-                                     C.POINTER(BatchDims), C.c_float, C.c_int, C.c_int]),
     "mg_genotype_packed": (C.c_int, [C.c_void_p, C.POINTER(PackedBatch), C.POINTER(GenotypeOut), C.c_float, C.c_int,
                                      C.c_int]),
     "mg_genotype_packed_device": (C.c_int, [C.c_void_p, C.POINTER(PackedBatch), C.POINTER(GenotypeOut),
@@ -141,7 +134,6 @@ SYMBOLS = {
     "mg_selftest_hash_packed_k35": (C.c_uint64, [C.c_uint64, C.c_uint64]),
     "mg_selftest_hash_packed_k43": (C.c_uint64, [C.c_uint64, C.c_uint64]),
     "mg_selftest_hash_ascii": (C.c_uint64, [C.c_char_p, C.c_int]),
-    "mg_selftest_pack35": (C.c_int, [C.c_char_p, u64p, u64p]),
     "mg_selftest_logf": (C.c_float, [C.c_float]),
     "mg_selftest_genotype": (C.c_int, [u32p, f32p, C.c_int, C.c_float, C.c_int, C.c_int, f64p, C.POINTER(C.c_int),
                                        C.POINTER(C.c_int), C.POINTER(C.c_int)]),

@@ -346,19 +346,6 @@ class MalvaGpu:
         check(self._L.mg_event_elapsed_ms(self._h, a, b, C.byref(ms)))
         return ms.value
 
-    def genotype_host(self, ptrs: dict, n_variants: int, error_rate: float, max_coverage: int, haploid: bool) -> None:
-        """mg_genotype on caller-owned HOST buffers given by address (e.g. pinned memory), keyed like the fields of
-        mg_variant_batch / mg_genotype_out.  Results are in the output buffers when this returns."""
-        c = lambda name, typ: C.cast(C.c_void_p(ptrs[name]), typ)
-        vb = _lib.VariantBatch(n_variants, c("var_allele_off", _lib.u64p), c("allele_sig_off", _lib.u64p),
-                               c("sig_kmer_off", _lib.u64p), c("kmer_off", _lib.u64p), C.c_void_p(ptrs["pool"]),
-                               c("freq", _lib.f32p))
-        out = _lib.GenotypeOut(c("cov", _lib.u32p), c("n_gts", _lib.i32p), c("status", _lib.i32p),
-                               c("best_gt", _lib.i32p), c("gq", _lib.i32p), c("lik_off", _lib.u64p),
-                               c("lik", _lib.f64p))
-        check(self._L.mg_genotype(self._h, C.byref(vb), C.byref(out), C.c_float(error_rate), int(max_coverage),
-                                  int(bool(haploid))))
-
     def genotype_packed(self, batch: "PackedSignatureBatch", error_rate: float = 0.001, max_coverage: int = 200,
                         haploid: bool = False, want_lik: bool = True) -> GenotypeResult:
         """mg_genotype_packed: the batch form the C++ host sends (2-bit k-mer words, u32 offsets)."""
@@ -444,20 +431,6 @@ class MalvaGpu:
                                c("best_gt", _lib.i32p), c("gq", _lib.i32p), c("lik_off", _lib.u64p), c("lik", _lib.f64p))
         check(self._L.mg_genotype_packed(self._h, C.byref(pb), C.byref(out), C.c_float(error_rate), int(max_coverage),
                                          int(bool(haploid))))
-
-    def genotype_device(self, ptrs: dict, dims: tuple, error_rate: float, max_coverage: int, haploid: bool) -> None:
-        """ptrs: device addresses keyed like mg_variant_batch / mg_genotype_out fields; dims = (nv, na, ns, nk)
-        or (nv, na, ns, nk, pool_bytes)."""
-        c = lambda name, typ: C.cast(C.c_void_p(ptrs[name]), typ)
-        vb = _lib.VariantBatch(dims[0], c("var_allele_off", _lib.u64p), c("allele_sig_off", _lib.u64p),
-                               c("sig_kmer_off", _lib.u64p), c("kmer_off", _lib.u64p), C.c_void_p(ptrs["pool"]),
-                               c("freq", _lib.f32p))
-        out = _lib.GenotypeOut(c("cov", _lib.u32p), c("n_gts", _lib.i32p), c("status", _lib.i32p),
-                               c("best_gt", _lib.i32p), c("gq", _lib.i32p), c("lik_off", _lib.u64p),
-                               c("lik", _lib.f64p))
-        dm = _lib.BatchDims(*(tuple(dims) + (0,) * (5 - len(dims))))
-        check(self._L.mg_genotype_device(self._h, C.byref(vb), C.byref(out), C.byref(dm), C.c_float(error_rate),
-                                         int(max_coverage), int(bool(haploid))))
 
     def scan_counted(self, counter: "KmerCounter") -> None:
         """the counted k-mers of a finished KmerCounter straight into the sample scan (no database file)"""

@@ -17,7 +17,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libmalva_gpu.so")
 CLI = os.path.join(HERE, "malva-geno")
 SOURCES = ["malva_gpu.cu"]
-HEADERS = ["xxh3.cuh", "geno.cuh", "index.cuh", "kernels.cuh", "count.cuh",
+HEADERS = ["xxh3.cuh", "geno.cuh", "index.cuh", "kernels.cuh", "count.cuh", os.path.join("host", "signatures.hpp"),
            os.path.join("..", "..", "include", "malva_gpu.h")]
 HOST_DIR = os.path.join(CSRC, "host")
 HOST_SOURCES = ["malva_geno.cpp"]

@@ -2,7 +2,7 @@
 //   K3  k_add_signatures / k_add_packed / k_add_spill / k_line_popc    index-time inserts + switch_mode
 //   K2  k_refpass / k_refpass_short                                    reference rolling pass
 //   K1  k_scan / k_scan_hits                                           sample k-mer scan
-//   K4  k_lookup_packed / k_lookup_fast / k_lookup / k_coverage        coverage read-back
+//   K4  k_lookup_packed / k_lookup / k_coverage                        coverage read-back
 //   K5  k_genotype                                                     likelihoods + posterior arg-max
 //       k_counters_xfer / k_sum_peers                                  dense counter image for the multi-GPU reduce
 #pragma once
@@ -935,19 +935,6 @@ __device__ __forceinline__ int32_t ref_get_count(const DevView &v, uint64_t idx,
   return slot < 0 ? 0 : (int32_t)__ldg(v.ovf_counts + slot);
 }
 
-// flags the k-mers of allele slot 0 of every variant (they are looked up in ref_bf, main.cpp:167-170)
-__global__ void __launch_bounds__(256) k_mark_ref(const uint64_t *__restrict__ var_allele_off,
-                                                 const uint64_t *__restrict__ allele_sig_off,
-                                                 const uint64_t *__restrict__ sig_kmer_off, uint64_t n_variants,
-                                                 uint8_t *__restrict__ flags) {
-  uint64_t vi = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (vi >= n_variants) return;
-  uint64_t a0 = var_allele_off[vi];
-  if (var_allele_off[vi + 1] == a0) return;
-  for (uint64_t s = allele_sig_off[a0]; s < allele_sig_off[a0 + 1]; ++s)
-    for (uint64_t q = sig_kmer_off[s]; q < sig_kmer_off[s + 1]; ++q) flags[q] = 1;
-}
-
 // mode 0: get_count  (is_ref selects KMAP/BF, out = int32 count)
 // mode 1: test_key on filter/table `which` (0 bf, 1 context_bf, 2 ref_bf; out = 0/1, -1 = irregular KMAP key)
 // out_pos != nullptr: k-mer i is written to out[out_pos[i]] and its is_ref flag is bit 62 of packed[out_pos[i]].hi
@@ -955,12 +942,10 @@ __global__ void __launch_bounds__(256) k_mark_ref(const uint64_t *__restrict__ v
 __global__ void __launch_bounds__(128) k_lookup(const uint8_t *__restrict__ pool, const uint64_t *__restrict__ off,
                                                const uint8_t *__restrict__ is_ref, uint64_t n, DevView v, int mode,
                                                int which, int32_t *__restrict__ out, unsigned long long *scalars,
-                                               const uint8_t *__restrict__ only_flagged,
                                                const uint32_t *__restrict__ out_pos, const uint4 *__restrict__ packed,
                                                bool raw = false) {
   uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  if (only_flagged && !only_flagged[i]) return;  // second pass after k_lookup_fast: the k-mers it deferred
   const uint64_t o = out_pos ? (uint64_t)out_pos[i] : i;
   uint64_t b = off[i], e = off[i + 1];
   int len = (int)(e - b);
@@ -995,43 +980,6 @@ __global__ void __launch_bounds__(128) k_lookup(const uint8_t *__restrict__ pool
     out[o] = which == 1 ? ctx_test(v, idx) : bf_test(v, idx);
   else
     out[o] = alt_get_count(v, idx, raw);
-}
-
-// Fast path of mode 0 for the compiled k: signature k-mers that are exactly K bytes long are read as aligned
-// 32-bit words, packed to 2-bit codes four bases at a time and validated by re-expanding the codes to ASCII
-// (pack_words, xxh3.cuh); anything that is not K symbols of ACGT, and the few k-mers at the very end of the
-// pool, take the generic byte path above.  ~10x fewer instructions per k-mer than the generic kernel.
-template <int K>
-__global__ void __launch_bounds__(128) k_lookup_fast(const uint8_t *__restrict__ pool, uint64_t pool_bytes,
-                                                    const uint64_t *__restrict__ off,
-                                                    const uint8_t *__restrict__ is_ref, uint64_t n, DevView v,
-                                                    int32_t *__restrict__ out, uint8_t *__restrict__ slow_flag) {
-  uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  constexpr int NW = (K + 3) / 4;  // 4-base groups
-  const uint64_t b = off[i], e = off[i + 1];
-  const uint64_t a0 = b & ~3ull;
-  if (e - b != (uint64_t)K || a0 + 4ull * (NW + 1) > pool_bytes) {
-    slow_flag[i] = 1;
-    return;
-  }
-  const uint32_t *wp = reinterpret_cast<const uint32_t *>(pool + a0);
-  const uint32_t sh = (uint32_t)(b & 3) * 8;
-  uint32_t raw[NW + 1], t[NW];
-#pragma unroll
-  for (int j = 0; j <= NW; ++j) raw[j] = __ldg(wp + j);
-#pragma unroll
-  for (int j = 0; j < NW; ++j) t[j] = __funnelshift_r(raw[j], raw[j + 1], sh);  // bases 4j..4j+3, first base low
-  u128 x;
-  const uint32_t bad = pack_words<K>(t, &x);
-  if (bad) {
-    slow_flag[i] = 1;
-    return;
-  }
-  u128 canon;
-  uint64_t h = canon_hash<K>(x, &canon);
-  uint64_t idx = bf_index(v, h);
-  out[i] = is_ref[i] ? ref_get_count(v, idx, canon) : alt_get_count(v, idx);
 }
 
 // Packed signature k-mers (exactly k symbols of ACGT, the form the host enumerator emits): {lo, hi} words;
@@ -1132,9 +1080,8 @@ __global__ void __launch_bounds__(256) k_mask_alt(const uint4 *__restrict__ kmer
 
 // set_coverages (main.cpp:157-182): per allele slot, max over signatures of the order-dependent integer
 // running mean of the non-zero k-mer weights
-template <typename OFF>
-__global__ void __launch_bounds__(128) k_coverage(const int32_t *__restrict__ w, const OFF *__restrict__ sig_kmer_off,
-                                                 const OFF *__restrict__ allele_sig_off, uint64_t n_alleles,
+__global__ void __launch_bounds__(128) k_coverage(const int32_t *__restrict__ w, const uint32_t *__restrict__ sig_kmer_off,
+                                                 const uint32_t *__restrict__ allele_sig_off, uint64_t n_alleles,
                                                  uint32_t *__restrict__ cov) {
   uint64_t a = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (a >= n_alleles) return;
@@ -1219,9 +1166,8 @@ MG_HD int genotype_one(const uint32_t *cov, const float *freq, int n, float err,
 
 // lik_off != nullptr: the likelihoods of variant vi go to lik[lik_off[vi] ..] (the caller reads them back);
 // lik_off == nullptr: nobody reads them, the slots are bump-allocated from `cursor` (scratch)
-template <typename OFF>
 __global__ void __launch_bounds__(128) k_genotype(const uint32_t *__restrict__ cov, const float *__restrict__ freq,
-                                                 const OFF *__restrict__ var_allele_off,
+                                                 const uint32_t *__restrict__ var_allele_off,
                                                  const uint64_t *__restrict__ lik_off, unsigned long long *cursor,
                                                  uint64_t n_variants, float err, int max_cov, int haploid,
                                                  const double *__restrict__ log_table,

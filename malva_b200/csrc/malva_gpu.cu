@@ -21,6 +21,7 @@
 
 #include "../../include/malva_gpu.h"
 #include "count.cuh"
+#include "host/signatures.hpp"
 #include "kernels.cuh"
 
 using mg::DevView;
@@ -45,7 +46,7 @@ static int set_err(int code, const char *fmt, ...) {
   } while (0)
 
 extern "C" const char *mg_last_error(void) { return g_err; }
-extern "C" int mg_version(void) { return 200; }
+extern "C" int mg_version(void) { return 201; }
 extern "C" int mg_device_count(void) {
   int n = 0;
   cudaError_t e = cudaGetDeviceCount(&n);
@@ -116,11 +117,12 @@ struct mg_ctx {
   uint64_t launches = 0;  // kernels launched by this context (bench.py's gpu_launches)
   cudaEvent_t tj = nullptr;
   cudaEvent_t ge[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};  // look-up [0,1], coverage [4,2], genotype [2,3]
-  void *geno_scratch = nullptr;  // per-k-mer weights + ref flags of mg_genotype
+  void *geno_scratch = nullptr;  // per-k-mer weights (+ likelihood slots nobody reads) of the genotyping calls
   uint64_t geno_scratch_bytes = 0;
-  void *geno_arena = nullptr;  // device image of the last mg_genotype batch (grow-only)
+  void *geno_arena = nullptr;  // device image of the last mg_genotype_packed batch (grow-only)
   double *log_table = nullptr;  // the host libm's log((double)i), i < mg::LOG_TABLE_N (geno.cuh log_int)
   uint64_t geno_arena_bytes = 0;
+  mh::SignatureCsr ascii_batch;  // mg_genotype's batch packed on the host (grow-only)
   cudaEvent_t evs[64] = {};
 
   DevView view() const {
@@ -993,7 +995,7 @@ static int lookup_common(mg_ctx *c, const char *pool, const uint64_t *off, const
   CU(cudaMalloc(&d_out.p, (n ? n : 1) * 4));
   c->launches++;
   mg::k_lookup<<<grid_for(n, 128), 128, 0, c->stream[0]>>>(b.pool, b.off, b.flags, n, c->view(), mode, which,
-                                                           (int32_t *)d_out.p, c->d_scalars, nullptr, nullptr, nullptr);
+                                                           (int32_t *)d_out.p, c->d_scalars, nullptr, nullptr);
   CU(cudaGetLastError());
   CU(cudaMemcpyAsync(out_host, d_out.p, n * 4, cudaMemcpyDeviceToHost, c->stream[0]));
   CU(cudaStreamSynchronize(c->stream[0]));
@@ -1026,7 +1028,7 @@ extern "C" int mg_get_counts(mg_ctx *c, const char *pool, const uint64_t *off, c
   return lookup_common(c, pool, off, is_ref, n, 0, 0, out);
 }
 
-// library-owned scratch of the genotyping calls: per-k-mer weights (+ flags), and the likelihood slots nobody reads
+// library-owned scratch of the genotyping calls: per-k-mer weights, and the likelihood slots nobody reads
 static int geno_scratch(mg_ctx *c, uint64_t need) {
   if (c->geno_scratch_bytes < need) {
     CU(cudaStreamSynchronize(c->stream[0]));
@@ -1046,147 +1048,13 @@ static int join_streams(mg_ctx *c) {
   return MG_OK;
 }
 
-// all pointers of in/out are DEVICE pointers here; scratch (k-mer flags + weights) is library-owned
-static int genotype_on_device(mg_ctx *c, const mg_variant_batch *in, const mg_genotype_out *out,
-                              const mg_batch_dims *dm, float error_rate, int max_coverage, int haploid) {
-  cudaStream_t st = c->stream[0];
-  uint64_t nv = dm->n_variants, na = dm->n_alleles, nk = dm->n_kmers;
-  int rc = geno_scratch(c, (nk ? nk : 1) * 6);  // i32 weight + ref flag + deferred flag per k-mer
-  if (rc) return rc;
-  rc = join_streams(c);
-  if (rc) return rc;
-  int32_t *d_w = reinterpret_cast<int32_t *>(c->geno_scratch);
-  uint8_t *d_flags = reinterpret_cast<uint8_t *>(c->geno_scratch) + (nk ? nk : 1) * 4;
+// ---- the genotyping step on PACKED signature k-mers (2-bit words, u32 offsets): what the C++ host sends ----
+// the look-up, coverage and likelihood events that mg_genotype_kernel_ms reads
+static int geno_events(mg_ctx *c) {
   for (int i = 0; i < 5; ++i)
     if (!c->ge[i]) CU(cudaEventCreate(&c->ge[i]));
-  CU(cudaEventRecord(c->ge[0], st));
-  if (nk) {
-    CU(cudaMemsetAsync(d_flags, 0, nk, st));
-    c->launches++;
-    mg::k_mark_ref<<<grid_for(nv, 256), 256, 0, st>>>(in->var_allele_off, in->allele_sig_off, in->sig_kmer_off, nv,
-                                                      d_flags);
-    CU(cudaGetLastError());
-    const uint8_t *d_pool = reinterpret_cast<const uint8_t *>(in->pool);
-    if (c->k == 35 && dm->pool_bytes && (reinterpret_cast<uintptr_t>(d_pool) & 3) == 0) {
-      // fast path for well-formed 35-mers; whatever it defers (odd lengths, non-ACGT, pool tail) goes through
-      // the generic kernel, which is skipped when nothing was deferred
-      uint8_t *d_slow = d_flags + nk;
-      CU(cudaMemsetAsync(d_slow, 0, nk, st));
-      c->launches++;
-      mg::k_lookup_fast<35><<<grid_for(nk, 128), 128, 0, st>>>(d_pool, dm->pool_bytes, in->kmer_off, d_flags, nk,
-                                                               c->view(), d_w, d_slow);
-      CU(cudaGetLastError());
-      c->launches++;
-      mg::k_lookup<<<grid_for(nk, 128), 128, 0, st>>>(d_pool, in->kmer_off, d_flags, nk, c->view(), 0, 0, d_w,
-                                                      c->d_scalars, d_slow, nullptr, nullptr);
-      CU(cudaGetLastError());
-    } else {
-      c->launches++;
-      mg::k_lookup<<<grid_for(nk, 128), 128, 0, st>>>(d_pool, in->kmer_off, d_flags, nk, c->view(), 0, 0, d_w,
-                                                      c->d_scalars, nullptr, nullptr, nullptr);
-      CU(cudaGetLastError());
-    }
-  }
-  CU(cudaEventRecord(c->ge[1], st));
-  CU(cudaEventRecord(c->ge[4], st));
-  c->launches++;
-  mg::k_coverage<uint64_t><<<grid_for(na, 128), 128, 0, st>>>(d_w, in->sig_kmer_off, in->allele_sig_off, na, out->cov);
-  CU(cudaGetLastError());
-  CU(cudaEventRecord(c->ge[2], st));
-  c->launches++;
-  mg::k_genotype<uint64_t><<<grid_for(nv, 128), 128, 0, st>>>(out->cov, in->freq, in->var_allele_off, out->lik_off, nullptr,
-                                                              nv, error_rate, max_coverage, haploid, c->log_table,
-                                                              out->lik, out->n_gts,
-                                                              out->status, out->best_gt, out->gq);
-  CU(cudaGetLastError());
-  CU(cudaEventRecord(c->ge[3], st));
   return MG_OK;
 }
-
-extern "C" int mg_genotype_device(mg_ctx *c, const mg_variant_batch *in, const mg_genotype_out *out,
-                                  const mg_batch_dims *dims, float error_rate, int max_coverage, int haploid) {
-  if (!c || !in || !out || !dims) return set_err(MG_ERR_ARG, "NULL argument");
-  if (!c->alt_final) return set_err(MG_ERR_STATE, "mg_genotype_device before mg_finalize_alt");
-  if (dims->n_variants == 0) return MG_OK;
-  if (!in->var_allele_off || !in->allele_sig_off || !in->sig_kmer_off || !in->kmer_off || !in->freq || !out->cov ||
-      !out->n_gts || !out->status || !out->best_gt || !out->gq || !out->lik_off || !out->lik)
-    return set_err(MG_ERR_ARG, "NULL array in batch");
-  CU(cudaSetDevice(c->device));
-  return genotype_on_device(c, in, out, dims, error_rate, max_coverage, haploid);
-}
-
-extern "C" int mg_genotype(mg_ctx *c, const mg_variant_batch *in, const mg_genotype_out *out, float error_rate,
-                           int max_coverage, int haploid) {
-  if (!c || !in || !out) return set_err(MG_ERR_ARG, "NULL argument");
-  if (!c->alt_final) return set_err(MG_ERR_STATE, "mg_genotype before mg_finalize_alt");
-  uint64_t nv = in->n_variants;
-  if (nv == 0) return MG_OK;
-  if (!in->var_allele_off || !in->allele_sig_off || !in->sig_kmer_off || !in->kmer_off || !in->freq || !out->cov ||
-      !out->n_gts || !out->status || !out->best_gt || !out->gq || !out->lik_off)
-    return set_err(MG_ERR_ARG, "NULL array in batch");
-  CU(cudaSetDevice(c->device));
-  int rc = mg_sync(c);
-  if (rc) return rc;
-  mg_batch_dims dm;
-  dm.n_variants = nv;
-  dm.n_alleles = in->var_allele_off[nv];
-  dm.n_sigs = in->allele_sig_off[dm.n_alleles];
-  dm.n_kmers = in->sig_kmer_off[dm.n_sigs];
-  dm.pool_bytes = in->kmer_off[dm.n_kmers];
-  uint64_t na = dm.n_alleles, ns = dm.n_sigs, nk = dm.n_kmers, nl = out->lik_off[nv];
-  uint64_t pool_bytes = in->kmer_off[nk];
-  cudaStream_t st = c->stream[0];
-  // one device arena for the whole batch
-  auto al = [](uint64_t x) { return (x + 255) & ~255ull; };
-  uint64_t o_vao = 0, o_aso = o_vao + al((nv + 1) * 8), o_sko = o_aso + al((na + 1) * 8),
-           o_ko = o_sko + al((ns + 1) * 8), o_lo = o_ko + al((nk + 1) * 8), o_freq = o_lo + al((nv + 1) * 8),
-           o_pool = o_freq + al(na * 4), o_cov = o_pool + al(pool_bytes), o_i32 = o_cov + al(na * 4),
-           o_lik = o_i32 + al(nv * 16), total = o_lik + al(nl * 8) + 256;
-  if (c->geno_arena_bytes < total) {  // grow-only device arena, reused across calls
-    cudaFree(c->geno_arena);
-    c->geno_arena = nullptr;
-    c->geno_arena_bytes = 0;
-    CU(cudaMalloc(&c->geno_arena, total + total / 4));
-    c->geno_arena_bytes = total + total / 4;
-  }
-  uint8_t *d = (uint8_t *)c->geno_arena;
-  CU(cudaMemcpyAsync(d + o_vao, in->var_allele_off, (nv + 1) * 8, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d + o_aso, in->allele_sig_off, (na + 1) * 8, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d + o_sko, in->sig_kmer_off, (ns + 1) * 8, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d + o_ko, in->kmer_off, (nk + 1) * 8, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d + o_lo, out->lik_off, (nv + 1) * 8, cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(d + o_freq, in->freq, na * 4, cudaMemcpyHostToDevice, st));
-  if (pool_bytes) CU(cudaMemcpyAsync(d + o_pool, in->pool, pool_bytes, cudaMemcpyHostToDevice, st));
-  mg_variant_batch din;
-  din.n_variants = nv;
-  din.var_allele_off = reinterpret_cast<uint64_t *>(d + o_vao);
-  din.allele_sig_off = reinterpret_cast<uint64_t *>(d + o_aso);
-  din.sig_kmer_off = reinterpret_cast<uint64_t *>(d + o_sko);
-  din.kmer_off = reinterpret_cast<uint64_t *>(d + o_ko);
-  din.pool = reinterpret_cast<const char *>(d + o_pool);
-  din.freq = reinterpret_cast<float *>(d + o_freq);
-  mg_genotype_out dout;
-  int32_t *i32 = reinterpret_cast<int32_t *>(d + o_i32);
-  dout.cov = reinterpret_cast<uint32_t *>(d + o_cov);
-  dout.n_gts = i32;
-  dout.status = i32 + nv;
-  dout.best_gt = i32 + 2 * nv;
-  dout.gq = i32 + 3 * nv;
-  dout.lik_off = reinterpret_cast<uint64_t *>(d + o_lo);
-  dout.lik = reinterpret_cast<double *>(d + o_lik);
-  rc = genotype_on_device(c, &din, &dout, &dm, error_rate, max_coverage, haploid);
-  if (rc) return rc;
-  CU(cudaMemcpyAsync(out->cov, dout.cov, na * 4, cudaMemcpyDeviceToHost, st));
-  CU(cudaMemcpyAsync(out->n_gts, dout.n_gts, nv * 4, cudaMemcpyDeviceToHost, st));
-  CU(cudaMemcpyAsync(out->status, dout.status, nv * 4, cudaMemcpyDeviceToHost, st));
-  CU(cudaMemcpyAsync(out->best_gt, dout.best_gt, nv * 4, cudaMemcpyDeviceToHost, st));
-  CU(cudaMemcpyAsync(out->gq, dout.gq, nv * 4, cudaMemcpyDeviceToHost, st));
-  if (out->lik && nl) CU(cudaMemcpyAsync(out->lik, dout.lik, nl * 8, cudaMemcpyDeviceToHost, st));
-  CU(cudaStreamSynchronize(st));
-  return check_too_long(c);
-}
-
-// ---- the same step for PACKED signature k-mers (2-bit words, u32 offsets): what the C++ host sends ----
 // all pointers of in/out are DEVICE pointers
 // K4 alone: the count of every signature k-mer of the batch into d_w (raw: bf counters unmasked)
 static int lookup_packed_on_device(mg_ctx *c, const mg_packed_batch *in, const mg_packed_dims *dm, int32_t *d_w, bool raw) {
@@ -1211,7 +1079,7 @@ static int lookup_packed_on_device(mg_ctx *c, const mg_packed_batch *in, const m
   if (in->n_irregular) {  // not k symbols of ACGT: the byte-exact path, written to their places in the weight array
     c->launches++;
     mg::k_lookup<<<grid_for(in->n_irregular, 128), 128, 0, st>>>(
-        (const uint8_t *)in->irr_pool, in->irr_off, nullptr, in->n_irregular, c->view(), 0, 0, d_w, c->d_scalars, nullptr,
+        (const uint8_t *)in->irr_pool, in->irr_off, nullptr, in->n_irregular, c->view(), 0, 0, d_w, c->d_scalars,
         in->irr_kmer, (const uint4 *)in->kmers, raw);
     CU(cudaGetLastError());
   }
@@ -1224,16 +1092,14 @@ static int genotype_from_weights(mg_ctx *c, const mg_packed_batch *in, const mg_
   const uint64_t nv = dm->n_variants, na = dm->n_alleles;
   const bool own_lik = out->lik == nullptr;
   c->launches++;
-  mg::k_coverage<uint32_t><<<grid_for(na, 128), 128, 0, st>>>(d_w, in->sig_kmer_off, in->allele_sig_off, na, out->cov);
+  mg::k_coverage<<<grid_for(na, 128), 128, 0, st>>>(d_w, in->sig_kmer_off, in->allele_sig_off, na, out->cov);
   CU(cudaGetLastError());
   CU(cudaEventRecord(c->ge[2], st));
   if (own_lik) CU(cudaMemsetAsync(c->d_scalars + 5, 0, 8, st));
   c->launches++;
-  mg::k_genotype<uint32_t><<<grid_for(nv, 128), 128, 0, st>>>(out->cov, in->freq, in->var_allele_off,
-                                                              own_lik ? nullptr : out->lik_off, c->d_scalars + 5, nv,
-                                                              error_rate, max_coverage, haploid, c->log_table, d_lik,
-                                                              out->n_gts,
-                                                              out->status, out->best_gt, out->gq);
+  mg::k_genotype<<<grid_for(nv, 128), 128, 0, st>>>(out->cov, in->freq, in->var_allele_off, own_lik ? nullptr : out->lik_off,
+                                                    c->d_scalars + 5, nv, error_rate, max_coverage, haploid, c->log_table,
+                                                    d_lik, out->n_gts, out->status, out->best_gt, out->gq);
   CU(cudaGetLastError());
   CU(cudaEventRecord(c->ge[3], st));
   return MG_OK;
@@ -1250,8 +1116,8 @@ static int genotype_packed_on_device(mg_ctx *c, const mg_packed_batch *in, const
   if (rc) return rc;
   int32_t *d_w = reinterpret_cast<int32_t *>(c->geno_scratch);
   double *d_lik = own_lik ? reinterpret_cast<double *>(reinterpret_cast<uint8_t *>(c->geno_scratch) + w_bytes) : out->lik;
-  for (int i = 0; i < 5; ++i)
-    if (!c->ge[i]) CU(cudaEventCreate(&c->ge[i]));
+  rc = geno_events(c);
+  if (rc) return rc;
   CU(cudaEventRecord(c->ge[0], st));
   rc = lookup_packed_on_device(c, in, dm, d_w, false);
   if (rc) return rc;
@@ -1273,8 +1139,8 @@ extern "C" int mg_lookup_packed_device(mg_ctx *c, const mg_packed_batch *in, con
   CU(cudaSetDevice(c->device));
   int rc = join_streams(c);
   if (rc) return rc;
-  for (int i = 0; i < 5; ++i)
-    if (!c->ge[i]) CU(cudaEventCreate(&c->ge[i]));
+  rc = geno_events(c);
+  if (rc) return rc;
   CU(cudaEventRecord(c->ge[0], c->stream[0]));
   rc = lookup_packed_on_device(c, in, dims, reinterpret_cast<int32_t *>(d_weights), true);
   if (rc) return rc;
@@ -1293,8 +1159,8 @@ extern "C" int mg_genotype_weights_device(mg_ctx *c, const mg_packed_batch *in, 
   const bool own_lik = out->lik == nullptr;
   int rc = geno_scratch(c, own_lik ? dims->lik_slots * 8 + 256 : 256);
   if (rc) return rc;
-  for (int i = 0; i < 5; ++i)
-    if (!c->ge[i]) CU(cudaEventCreate(&c->ge[i]));
+  rc = geno_events(c);
+  if (rc) return rc;
   CU(cudaEventRecord(c->ge[4], c->stream[0]));
   if (dims->n_kmers) {  // BF::get_count returns uint16_t: the wrap-around of the summed bf counters
     c->launches++;
@@ -1418,6 +1284,41 @@ extern "C" int mg_genotype_packed(mg_ctx *c, const mg_packed_batch *in, const mg
   if (nl) CU(cudaMemcpyAsync(out->lik, dout.lik, nl * 8, cudaMemcpyDeviceToHost, st));
   CU(cudaStreamSynchronize(st));
   return check_too_long(c);
+}
+
+// The reference-shaped batch (ASCII k-mers, u64 offsets), packed on the host into the batch of mg_genotype_packed by
+// the packer of malva-geno (SignatureCsr::add_kmer): a k-mer is regular iff it is exactly k symbols of ACGT, the rule of
+// pack_ascii; every other k-mer goes to the side pool, where k_lookup hashes its bytes as BF::_get_hash would.  The
+// k-mers of allele slot 0 are looked up in ref_bf.
+extern "C" int mg_genotype(mg_ctx *c, const mg_variant_batch *in, const mg_genotype_out *out, float error_rate,
+                           int max_coverage, int haploid) {
+  if (!c || !in || !out) return set_err(MG_ERR_ARG, "NULL argument");
+  if (!c->alt_final) return set_err(MG_ERR_STATE, "mg_genotype before mg_finalize_alt");
+  const uint64_t nv = in->n_variants;
+  if (nv == 0) return MG_OK;
+  if (!in->var_allele_off || !in->allele_sig_off || !in->sig_kmer_off || !in->kmer_off || !in->freq || !out->cov ||
+      !out->n_gts || !out->status || !out->best_gt || !out->gq || !out->lik_off)
+    return set_err(MG_ERR_ARG, "NULL array in batch");
+  const uint64_t na = in->var_allele_off[nv], ns = in->allele_sig_off[na], nk = in->sig_kmer_off[ns];
+  if (!in->pool && in->kmer_off[nk]) return set_err(MG_ERR_ARG, "NULL array in batch");
+  if (na > 0xFFFFFFFFull || ns > 0xFFFFFFFFull || nk > 0xFFFFFFFFull)
+    return set_err(MG_ERR_ARG, "batch too large (max 2^32-1 allele slots, signatures and k-mers per call)");
+  mh::SignatureCsr &p = c->ascii_batch;
+  p.clear();
+  p.var_allele_off.assign(in->var_allele_off, in->var_allele_off + nv + 1);  // (u64 -> u32)
+  p.allele_sig_off.assign(in->allele_sig_off, in->allele_sig_off + na + 1);
+  p.sig_kmer_off.assign(in->sig_kmer_off, in->sig_kmer_off + ns + 1);
+  for (uint64_t i = 0; i < nk; ++i)
+    p.add_kmer(in->pool + in->kmer_off[i], in->kmer_off[i + 1] - in->kmer_off[i], c->k, false);
+  for (uint64_t v = 0; v < nv; ++v) {
+    const uint64_t a0 = in->var_allele_off[v];
+    if (in->var_allele_off[v + 1] == a0) continue;
+    for (uint64_t q = in->sig_kmer_off[in->allele_sig_off[a0]]; q < in->sig_kmer_off[in->allele_sig_off[a0 + 1]]; ++q)
+      p.kmers[2 * q + 1] |= mh::SIG_REF_ALLELE;
+  }
+  const mg_packed_batch pb = {nv, p.var_allele_off.data(), p.allele_sig_off.data(), p.sig_kmer_off.data(), p.kmers.data(),
+                              in->freq, p.n_irregular(), p.irr_off.data(), p.irr_pool.data(), p.irr_kmer.data()};
+  return mg_genotype_packed(c, &pb, out, error_rate, max_coverage, haploid);
 }
 
 extern "C" int mg_bf_popcount(mg_ctx *c, int which, uint64_t *ones) {
@@ -2020,15 +1921,6 @@ extern "C" uint64_t mg_selftest_hash_packed_k43(uint64_t lo, uint64_t hi) {
 }
 extern "C" uint64_t mg_selftest_hash_ascii(const char *s, int len) {
   return mg::hash_ascii(reinterpret_cast<const uint8_t *>(s), len);
-}
-extern "C" int mg_selftest_pack35(const char *s35, uint64_t *lo, uint64_t *hi) {
-  uint32_t t[9] = {0};
-  memcpy(t, s35, 35);
-  u128 x;
-  uint32_t bad = mg::pack_words<35>(t, &x);
-  if (lo) *lo = x.lo;
-  if (hi) *hi = x.hi;
-  return bad ? 0 : 1;
 }
 extern "C" float mg_selftest_logf(float x) { return mg::glibc_logf(x); }
 extern "C" int mg_selftest_genotype(const uint32_t *cov, const float *freq, int n_alleles, float error_rate,

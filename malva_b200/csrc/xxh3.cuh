@@ -353,42 +353,4 @@ MG_HD bool pack_ascii(const uint8_t *s, int len, int k, u128 *out) {
   return true;
 }
 
-// Pack a K-byte ASCII k-mer given as little-endian 32-bit words (first base in the low byte of t[0]) and
-// validate it at the same time: returns 0 iff every one of the K bytes is one of A, C, G, T.
-//   code of an ASCII base: ((c >> 1) ^ (c >> 2)) & 3  ->  A=0 C=1 G=2 T=3; re-expanding the codes through the
-//   byte table "ACGT" and comparing with the input catches every other byte value.
-template <int K>
-MG_HD uint32_t pack_words(const uint32_t *t, u128 *out) {
-  constexpr int NW = (K + 3) / 4;
-  constexpr int REM = K - 4 * (NW - 1);  // bases in the last group
-  u128 x;
-  x.lo = 0;
-  x.hi = 0;
-  uint32_t bad = 0;
-#pragma unroll
-  for (int j = 0; j < NW; ++j) {
-    const uint32_t c = ((t[j] >> 1) ^ (t[j] >> 2)) & 0x03030303u;
-    const uint32_t sel = (c & 0x3u) | ((c >> 4) & 0x30u) | ((c >> 8) & 0x300u) | ((c >> 12) & 0x3000u);
-#if defined(__CUDA_ARCH__)
-    const uint32_t back = __byte_perm(0x54474341u, 0u, sel);
-#else
-    uint32_t back = 0;
-    for (int q = 0; q < 4; ++q) back |= ((0x54474341u >> (8 * ((sel >> (4 * q)) & 3))) & 0xFFu) << (8 * q);
-#endif
-    const uint32_t m = (j == NW - 1 && REM < 4) ? ((1u << (8 * (REM & 3))) - 1u) : 0xFFFFFFFFu;
-    bad |= (back ^ t[j]) & m;
-    uint32_t x8 = (c * 0x40100401u) >> 24;  // b0<<6 | b1<<4 | b2<<2 | b3
-    if (j == NW - 1 && REM < 4) {
-      x8 >>= 2 * (4 - REM);
-      x.hi = (x.hi << (2 * REM)) | (x.lo >> (64 - 2 * REM));
-      x.lo = (x.lo << (2 * REM)) | x8;
-    } else {
-      x.hi = (x.hi << 8) | (x.lo >> 56);
-      x.lo = (x.lo << 8) | x8;
-    }
-  }
-  *out = x;
-  return bad;
-}
-
 }  // namespace mg

@@ -138,22 +138,3 @@ def test_genotype_zero_alleles_writes_nothing(L):
                                 lik.ctypes.data_as(C.POINTER(C.c_double)), C.byref(st), C.byref(bg), C.byref(gq))
     assert (ng, st.value, bg.value, gq.value) == (0, 2, 0, 0)
     assert (lik == 7.0).all()
-
-
-def test_wordwise_packer_of_the_lookup_kernel(L):
-    """pack_words<35> (xxh3.cuh, used by k_lookup_fast): packs ACGT 35-mers exactly like kmc.pack_kmer and rejects
-    every other byte value at every position."""
-    rng = random.Random(5)
-    lo, hi = C.c_uint64(0), C.c_uint64(0)
-    for _ in range(2000):
-        s = "".join(rng.choice("ACGT") for _ in range(35))
-        assert L.mg_selftest_pack35(s.encode(), C.byref(lo), C.byref(hi)) == 1
-        assert (hi.value << 64) | lo.value == kmc.pack_kmer(s)
-    base = "ACGTTGCAACGTACGTTTGACCAGTACGATCGATCGA"[:35]
-    for pos in range(35):
-        for byte in range(1, 256):
-            if chr(byte) in "ACGT":
-                continue
-            b = bytearray(base.encode())
-            b[pos] = byte
-            assert L.mg_selftest_pack35(bytes(b) + b"\0", C.byref(lo), C.byref(hi)) == 0, (pos, byte)

@@ -175,8 +175,9 @@ def test_empty_and_ragged_inputs(oracle_lib):
 
 @pytest.mark.parametrize("haploid", [False, True])
 @pytest.mark.parametrize("err", [0.001, 0.05])
-def test_coverage_and_genotype(oracle_lib, haploid, err):
-    g, o, genome, nested, freqs, ks, fl, words = _run_pair(oracle_lib, 35, 43, 1 << 22, seed=42, n_var=600,
+@pytest.mark.parametrize("k,ref_k", [(35, 43), (31, 39), (63, 64)])  # k_lookup_packed<35>, <0>, wide keys (k >= 48)
+def test_coverage_and_genotype(oracle_lib, k, ref_k, haploid, err):
+    g, o, genome, nested, freqs, ks, fl, words = _run_pair(oracle_lib, k, ref_k, 1 << 22, seed=42, n_var=600,
                                                           n_sample=20000)
     try:
         batch = SignatureBatch.from_nested(nested, freqs)
@@ -196,8 +197,8 @@ def test_coverage_and_genotype(oracle_lib, haploid, err):
             assert np.array_equal(got == 0, e["probs"] == 0)
             seen.add(e["status"])
         assert seen == {0, 1, 2}, seen
-        # the packed batch form (what the C++ host sends) is the same computation: identical bits out
-        pb = PackedSignatureBatch.from_batch(batch, 35)
+        # mg_genotype packs the batch on the host: the Python packer of the same batch gives identical bits out
+        pb = PackedSignatureBatch.from_batch(batch, k)
         assert len(pb.irr_kmer) > 0, "the synthetic signatures should include irregular k-mers"
         rp = g.genotype_packed(pb, err, max_cov, haploid)
         for name in ("cov", "status", "n_gts", "best_gt", "gq"):
