@@ -178,6 +178,24 @@ class OracleRun:
         return cov[:na], res
 
 
+class _DevArray:
+    def __init__(self, ptr, n):
+        self.__cuda_array_interface__ = {"shape": (n,), "typestr": "<u4", "data": (ptr, False), "version": 2}
+
+
+def counter_arrays(g) -> list:
+    """the three u32 counter arrays of a context (what a multi-GPU run sum-reduces), gathered, as host arrays:
+    bf counters (rank order), key counts of the probe lines (line order), overflow counts"""
+    import torch
+
+    g.sync()
+    out = []
+    for ptr, n in g.counter_buffers(gather=True):
+        out.append(torch.as_tensor(_DevArray(ptr, n), device=f"cuda:{g.device}").cpu().numpy().copy() if n
+                   else np.zeros(0, np.uint32))
+    return out
+
+
 def synth_signatures(rng: random.Random, genome: str, k: int, n_var: int, irregular: bool = True):
     """Simple per-variant signatures: the reference window (allele 0) and 1-3 mutated windows (alts).
     Returns nested[v][allele][signature] = [k-mers], freqs[v][allele]."""

@@ -304,22 +304,6 @@ def test_kmc_records_decoded_on_device(oracle_lib, tmp_path, version, p, k, ref_
         o.close()
 
 
-class _DevArray:
-    def __init__(self, ptr, n):
-        self.__cuda_array_interface__ = {"shape": (n,), "typestr": "<u4", "data": (ptr, False), "version": 2}
-
-
-def _counter_arrays(g):
-    """the three u32 counter arrays of a context (what a multi-GPU run sum-reduces), as host arrays"""
-    import torch
-
-    g.sync()
-    out = []
-    for ptr, n in g.counter_buffers(gather=True):
-        out.append(torch.as_tensor(_DevArray(ptr, n), device="cuda:0").cpu().numpy().copy() if n else np.zeros(0, np.uint32))
-    return out
-
-
 @pytest.mark.parametrize("bf_bits", [1 << 13, 1 << 22])
 def test_replicas_built_in_any_order_have_one_image_and_their_counters_add_up(oracle_lib, bf_bits):
     """Multi-GPU contract (DESIGN 7): every replica builds the index on its own, scans a share of the stream, and the
@@ -354,7 +338,7 @@ def test_replicas_built_in_any_order_have_one_image_and_their_counters_add_up(or
         b.scan_sample_kmers(packed[half:], counts[half:])
         whole.scan_sample_kmers(packed, counts)
         o.scan_sample_kmers(packed, counts)
-        ca, cb, cw = _counter_arrays(a), _counter_arrays(b), _counter_arrays(whole)
+        ca, cb, cw = util.counter_arrays(a), util.counter_arrays(b), util.counter_arrays(whole)
         for i, name in enumerate(("bf counters", "line key counts", "overflow counts")):
             assert len(ca[i]) == len(cb[i]) == len(cw[i]), name
             assert np.array_equal(ca[i] + cb[i], cw[i]), name
