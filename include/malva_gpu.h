@@ -216,6 +216,36 @@ int mg_counters_scatter(mg_ctx *ctx);
  * mg_get_counts for the whole stream. */
 int mg_reduce_counts(mg_ctx **ctx, int n);
 
+/* Sample sets: several samples genotyped against one index, each from its own counters.  Every counter a signature
+ * k-mer can read has a ROW fixed by the index: rows [0, bf_ones) are the set bits of bf in rank order, the next
+ * (ref keys - overflow keys) rows the ref keys held by the probe lines in line order, the last (overflow capacity)
+ * rows the slots of the overflow table (mg_index_stats).  A set keeps one u32 COLUMN per sample over those rows,
+ * row-major (the counts of one row for all samples are adjacent): 4 bytes x rows of device memory per sample.
+ *   mg_samples_begin   allocates a set of n_samples (1..MG_SAMPLE_SET_MAX) zeroed columns; a column never taken
+ *                      reads as zero.  Calling it again replaces the set; needs mg_finalize_alt.
+ *   mg_samples_take    waits for the scans enqueued so far, then copies every live counter into column s (the
+ *                      inline alt counters, bf_counts, the key counts, the overflow counts) and ZEROES the live
+ *                      counters: column s holds exactly what the live counters held at the call, and the live
+ *                      counters are zero after it, so the next sample scans into a clean index.  Nothing else in the
+ *                      index changes.  mg_get_counts, mg_genotype_packed and mg_counters_* keep reading the live
+ *                      counters (a gathered dense image is zeroed with them).
+ *   mg_genotype_samples_packed   mg_genotype_packed (HOST buffers) for every sample of the set at once: out[s] gets
+ *                      exactly what mg_genotype_packed returns on a context whose live counters equal column s.  One
+ *                      look-up for the set, then coverage and likelihoods per sample; n_samples must equal the size
+ *                      of the set (MG_ERR_ARG), and a set must exist (MG_ERR_STATE).  out[s].lik are all NULL or all
+ *                      set; the likelihood slots are those of out[0].lik_off for every sample.
+ *                      mg_genotype_kernel_ms reports its look-up, the coverage of all samples and their likelihoods.
+ *   mg_samples_end     frees the set (mg_destroy does too). */
+#define MG_SAMPLE_SET_MAX 32
+int mg_samples_begin(mg_ctx *ctx, int n_samples);
+/* the largest set that fits: MG_SAMPLE_SET_MAX at most, and columns in at most 3/4 of the free device memory (the
+ * current set counted as free); 0 when not even one column fits */
+int mg_samples_capacity(mg_ctx *ctx, int *n);
+int mg_samples_take(mg_ctx *ctx, int s);
+int mg_genotype_samples_packed(mg_ctx *ctx, const mg_packed_batch *in, const mg_genotype_out *out, int n_samples,
+                               float error_rate, int max_coverage, int haploid);
+int mg_samples_end(mg_ctx *ctx);
+
 /* index image for the index file (BF::operator>> / KMAP::operator>>, main.cpp:406-412; loading :455-461).
  * Filters travel as sorted lists of set-bit indices (the reference writes the raw 2 x bf_bits/8 bytes), ref_bf
  * as its packed canonical keys.  Call with out == NULL to get the count first.  Import the bits of bf (which=0)

@@ -118,6 +118,12 @@ SYMBOLS = {
     "mg_counters_scatter": (C.c_int, [C.c_void_p]),
     "mg_counter_buffers": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), u64p]),
     "mg_reduce_counts": (C.c_int, [C.POINTER(C.c_void_p), C.c_int]),
+    "mg_samples_begin": (C.c_int, [C.c_void_p, C.c_int]),
+    "mg_samples_capacity": (C.c_int, [C.c_void_p, C.POINTER(C.c_int)]),
+    "mg_samples_take": (C.c_int, [C.c_void_p, C.c_int]),
+    "mg_genotype_samples_packed": (C.c_int, [C.c_void_p, C.POINTER(PackedBatch), C.POINTER(GenotypeOut), C.c_int,
+                                             C.c_float, C.c_int, C.c_int]),
+    "mg_samples_end": (C.c_int, [C.c_void_p]),
     "mg_export_set_bits": (C.c_int, [C.c_void_p, C.c_int, u64p, C.c_uint64, u64p]),
     "mg_import_set_bits": (C.c_int, [C.c_void_p, C.c_int, u64p, C.c_uint64]),
     "mg_export_ref_keys": (C.c_int, [C.c_void_p, u64p, C.c_uint64, u64p]),

@@ -13,6 +13,7 @@ reference's names where a 1:1 method exists:
     context_bf.switch_mode()            main:404   MalvaGpu.finalize_context()
     KMC loop: increment / test_key      main:487   MalvaGpu.scan_sample_kmers(packed, counts)
     set_coverages + VB::genotype        main:151   MalvaGpu.genotype(batch, ...)
+    (one run per sample)                           MalvaGpu.samples_begin / samples_take / genotype_samples_packed
     BF::test_key / KMAP::test_key                  MalvaGpu.bf.test_key(...) etc. (views)
     BF::get_count / KMAP::get_count                MalvaGpu.bf.get_count(...)
 
@@ -183,6 +184,7 @@ class MalvaGpu:
         self._L = _lib.load()
         self._h = C.c_void_p()
         self.k, self.ref_k, self.bf_bits, self.device = k, ref_k, bf_bits, device
+        self._n_samples = 0
         check(self._L.mg_create(C.byref(self._h), device, k, ref_k, bf_bits))
         self.bf = _View(self, BF_ALT)
         self.context_bf = _View(self, BF_CONTEXT)
@@ -349,32 +351,62 @@ class MalvaGpu:
     def genotype_packed(self, batch: "PackedSignatureBatch", error_rate: float = 0.001, max_coverage: int = 200,
                         haploid: bool = False, want_lik: bool = True) -> GenotypeResult:
         """mg_genotype_packed: the batch form the C++ host sends (2-bit k-mer words, u32 offsets)."""
+        return self._genotype_packed_sets(batch, 1, False, error_rate, max_coverage, haploid, want_lik)[0]
+
+    def genotype_samples_packed(self, batch: "PackedSignatureBatch", error_rate: float = 0.001, max_coverage: int = 200,
+                                haploid: bool = False, want_lik: bool = True,
+                                n_samples: int | None = None) -> List[GenotypeResult]:
+        """mg_genotype_samples_packed: genotype_packed for every sample of the set (samples_begin), one result per
+        column; n_samples defaults to the size of the set."""
+        n = self._n_samples if n_samples is None else n_samples
+        return self._genotype_packed_sets(batch, n, True, error_rate, max_coverage, haploid, want_lik)
+
+    def _genotype_packed_sets(self, batch, n_sets, samples, error_rate, max_coverage, haploid, want_lik):
         nv = batch.n_variants
         na = int(batch.var_allele_off[-1]) if nv else 0
         nall = np.diff(batch.var_allele_off.astype(np.int64))
         slots = np.maximum(nall if haploid else nall * (nall + 1) // 2, nall)
         lik_off = np.zeros(nv + 1, dtype=np.uint64)
         lik_off[1:] = np.cumsum(slots, dtype=np.uint64)
-        res = GenotypeResult(np.zeros(max(na, 1), np.uint32), np.zeros(nv, np.int32), np.zeros(nv, np.int32),
-                             np.zeros(nv, np.int32), np.zeros(nv, np.int32), lik_off,
-                             np.zeros(int(lik_off[-1]) if want_lik else 0, np.float64))
-        if nv == 0:
-            res.cov = res.cov[:0]
+        res = [GenotypeResult(np.zeros(max(na, 1), np.uint32), np.zeros(nv, np.int32), np.zeros(nv, np.int32),
+                              np.zeros(nv, np.int32), np.zeros(nv, np.int32), lik_off,
+                              np.zeros(int(lik_off[-1]) if want_lik else 0, np.float64)) for _ in range(max(n_sets, 1))]
+        if nv == 0 and not samples:
+            res[0].cov = res[0].cov[:0]
             return res
         pb = _lib.PackedBatch(nv, _p(batch.var_allele_off, _lib.u32p), _p(batch.allele_sig_off, _lib.u32p),
                               _p(batch.sig_kmer_off, _lib.u32p), batch.kmers.ctypes.data, _p(batch.freq, _lib.f32p),
                               len(batch.irr_kmer), _p(batch.irr_off, _lib.u64p),
                               C.cast(C.c_char_p(batch.irr_pool), C.c_void_p), _p(batch.irr_kmer, _lib.u32p))
-        out = _lib.GenotypeOut(_p(res.cov, _lib.u32p), _p(res.n_gts, _lib.i32p), _p(res.status, _lib.i32p),
-                               _p(res.best_gt, _lib.i32p), _p(res.gq, _lib.i32p),
-                               _p(lik_off, _lib.u64p) if want_lik else None,
-                               _p(res.lik, _lib.f64p) if want_lik and len(res.lik) else None)
-        if want_lik and not len(res.lik):
-            out.lik_off = None
-        check(self._L.mg_genotype_packed(self._h, C.byref(pb), C.byref(out), C.c_float(error_rate), int(max_coverage),
-                                         int(bool(haploid))))
-        res.cov = res.cov[:na]
-        return res
+        outs = (_lib.GenotypeOut * len(res))()
+        for o, r in zip(outs, res):
+            o.cov, o.n_gts, o.status = _p(r.cov, _lib.u32p), _p(r.n_gts, _lib.i32p), _p(r.status, _lib.i32p)
+            o.best_gt, o.gq = _p(r.best_gt, _lib.i32p), _p(r.gq, _lib.i32p)
+            o.lik_off = _p(lik_off, _lib.u64p) if want_lik and len(r.lik) else None
+            o.lik = _p(r.lik, _lib.f64p) if want_lik and len(r.lik) else None
+        if samples:
+            check(self._L.mg_genotype_samples_packed(self._h, C.byref(pb), outs, n_sets, C.c_float(error_rate),
+                                                     int(max_coverage), int(bool(haploid))))
+        else:
+            check(self._L.mg_genotype_packed(self._h, C.byref(pb), outs, C.c_float(error_rate), int(max_coverage),
+                                             int(bool(haploid))))
+        for r in res:
+            r.cov = r.cov[:na]
+        return res[:n_sets]
+
+    # ---- sample sets: several samples genotyped against this index (include/malva_gpu.h) ------------------------
+    def samples_begin(self, n: int) -> None:
+        """a set of n (1..32) zeroed sample columns; replaces the previous set"""
+        check(self._L.mg_samples_begin(self._h, int(n)))
+        self._n_samples = int(n)
+
+    def samples_take(self, s: int) -> None:
+        """the live counters (everything scanned since the last take) into column s; the live counters are zeroed"""
+        check(self._L.mg_samples_take(self._h, int(s)))
+
+    def samples_end(self) -> None:
+        check(self._L.mg_samples_end(self._h))
+        self._n_samples = 0
 
     def genotype_packed_device(self, ptrs: dict, dims: tuple, error_rate: float, max_coverage: int, haploid: bool) -> None:
         """ptrs: device addresses keyed like mg_packed_batch / mg_genotype_out fields ("lik"/"lik_off" may be 0);

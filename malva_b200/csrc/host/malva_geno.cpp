@@ -2,6 +2,7 @@
 //
 //   malva-geno index [flags] <reference.fa> <variants.vcf> <kmc_output_prefix>
 //   malva-geno call  [flags] <reference.fa> <variants.vcf> <kmc_output_prefix>   > out.vcf
+//   malva-geno call  [flags] <reference.fa> <variants.vcf> <db1> <db2> .. --out-dir DIR   (DIR/<basename>.vcf each)
 //
 // Same sub-commands, flags (-k -r -e -s -f -c -b -p -u -v -1), index file name, stderr phase lines and VCF
 // output as the reference (main.cpp:226-594, argument_parser.hpp:51-159).  The host keeps VCF/FASTA reading and
@@ -29,6 +30,7 @@
 //   malva-geno container-selftest                           InlineVec / Chain against std::vector (CPU tests)
 #include <getopt.h>
 #include <sys/resource.h>
+#include <sys/stat.h>
 #include <unistd.h>
 
 #include <algorithm>
@@ -37,6 +39,7 @@
 #include <condition_variable>
 #include <deque>
 #include <mutex>
+#include <cerrno>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -79,6 +82,8 @@ const char *USAGE =
     "          --device N                    CUDA device (default: 0)\n"
     "          --devices A,B,..              call: replicate the index on these devices, deal the KMC records\n"
     "                                        round-robin, add the counters up on the first one\n"
+    "          --out-dir DIR                 call with several KMC databases (call [opts] ref.fa vars.vcf DB1 DB2 ..):\n"
+    "                                        genotype every sample against one index, sample DB to DIR/basename(DB).vcf\n"
     "\n";
 
 struct Options {
@@ -92,10 +97,13 @@ struct Options {
   bool trace = false;  // --trace: per-batch host/device timings on stderr
   std::vector<int> devices;  // --devices a,b,..: `call` replicates the index and deals the KMC records round-robin
   std::string fasta_path, vcf_path, kmc_path;
+  std::vector<std::string> kmc_paths;  // call: one or more KMC databases (kmc_path = the first)
+  std::string out_dir;                 // call with several databases: sample P is written to out_dir/basename(P).vcf
 };
 
 // argument_parser.hpp:86-159; values are read like `istringstream >> x` reads them
-bool parse_arguments(int argc, char **argv, Options &o, int n_positional) {
+// more_dbs: `call` takes one or more KMC databases after the VCF
+bool parse_arguments(int argc, char **argv, Options &o, int n_positional, bool more_dbs = false) {
   static const option longopts[] = {{"kmer-size", required_argument, nullptr, 'k'},
                                     {"ref-kmer-size", required_argument, nullptr, 'r'},
                                     {"error-rate", required_argument, nullptr, 'e'},
@@ -115,6 +123,7 @@ bool parse_arguments(int argc, char **argv, Options &o, int n_positional) {
                                     {"index-blocks", no_argument, nullptr, 1002},
                                     {"trace", no_argument, nullptr, 1003},
                                     {"devices", required_argument, nullptr, 1004},
+                                    {"out-dir", required_argument, nullptr, 1005},
                                     {nullptr, 0, nullptr, 0}};
   bool die = false;
   optind = 1;
@@ -145,6 +154,7 @@ bool parse_arguments(int argc, char **argv, Options &o, int n_positional) {
           if (!tok.empty()) o.devices.push_back(atoi(tok.c_str()));
         break;
       }
+      case 1005: o.out_dir = optarg ? optarg : ""; break;
       case '?': die = true; break;
       case 'h':
         std::cout << USAGE;
@@ -154,7 +164,7 @@ bool parse_arguments(int argc, char **argv, Options &o, int n_positional) {
   if (argc - optind < n_positional) {
     std::cerr << "malva : missing arguments\n";
     die = true;
-  } else if (argc - optind > n_positional) {
+  } else if (argc - optind > n_positional && !more_dbs) {
     std::cerr << "malva : too many arguments\n";
     die = true;
   }
@@ -164,7 +174,8 @@ bool parse_arguments(int argc, char **argv, Options &o, int n_positional) {
   }
   o.fasta_path = argv[optind++];
   o.vcf_path = argv[optind++];
-  if (n_positional > 2) o.kmc_path = argv[optind++];
+  if (n_positional > 2) o.kmc_path = argv[optind];
+  while (n_positional > 2 && optind < argc) o.kmc_paths.push_back(argv[optind++]);
   if (o.threads <= 0) o.threads = (int)std::max(1u, std::thread::hardware_concurrency());
   mh::io_threads() = o.threads;
   if (o.devices.empty()) o.devices.push_back(o.device);
@@ -882,25 +893,216 @@ int container_selftest_main() {
   return bad ? 1 : 0;
 }
 
+// STEP 2: the sample k-mer scan (main.cpp:482-500) of one database.  Raw suffix records go through rings of pinned
+// buffers, one ring per device, chunks dealt round-robin; the library copies and scans them asynchronously
+// (double-buffered on its side), a buffer is refilled only after the event recorded behind its scan has completed.
+// With several devices the counters are then added up on the first one (all updates are commutative adds,
+// main.cpp:495-499) and the replicas are destroyed.
+void scan_kmc(const Options &o, std::vector<Ctx> &gs, mh::KmcDb &db, const std::string &path) {
+  const int n_dev = (int)gs.size();
+  constexpr int RING = 4;
+  constexpr uint64_t CHUNK = 1ull << 22;  // records per buffer
+  std::vector<uint8_t *> buf((size_t)(n_dev * RING), nullptr);
+  std::vector<char> used((size_t)(n_dev * RING), 0);
+  Stopwatch sw;
+  for (int d = 0; d < n_dev; ++d) {
+    gpu(mg_kmc_open(gs[(size_t)d].c, db.lut.data(), db.lut.size(), db.lut_prefix_len, db.kmer_len, db.counter_size,
+                    db.min_count, db.max_count),
+        "mg_kmc_open");
+    for (int s = 0; s < RING; ++s) gpu(mg_host_alloc((void **)&buf[(size_t)(d * RING + s)], CHUNK * db.record_bytes + 64), "mg_host_alloc");
+  }
+  uint64_t first = 0;
+  double t_alloc = sw.lap(), t_wait = 0, t_read = 0, t_submit = 0;
+  for (uint64_t chunk = 0;; ++chunk) {
+    const int d = (int)(chunk % (uint64_t)n_dev), slot = d * RING + (int)((chunk / (uint64_t)n_dev) % RING);
+    mg_ctx *c = gs[(size_t)d].c;
+    if (used[(size_t)slot]) gpu(mg_event_sync(c, 32 + slot % RING), "mg_event_sync");
+    t_wait += sw.lap();
+    uint64_t n = db.read_records(buf[(size_t)slot], first, CHUNK);
+    t_read += sw.lap();
+    if (n == 0) break;
+    gpu(mg_scan_kmc_records(c, buf[(size_t)slot], first, n), "mg_scan_kmc_records");
+    gpu(mg_event_record(c, 32 + slot % RING), "mg_event_record");
+    t_submit += sw.lap();
+    used[(size_t)slot] = 1;
+    first += n;
+  }
+  for (auto &x : gs) gpu(mg_sync(x.c), "mg_sync");
+  const double t_drain = sw.lap();
+  for (auto &b : buf) mg_host_free(b);
+  if (o.trace)
+    fprintf(stderr, "[trace] KMC scan: %llu records; pinned buffers %.1f ms, file reads %.1f ms, waiting for a free buffer "
+                    "%.1f ms, submitting %.1f ms, draining %.1f ms, freeing %.1f ms\n",
+            (unsigned long long)first, t_alloc, t_read, t_wait, t_submit, t_drain, sw.lap());
+  if (first != db.total_kmers) throw std::runtime_error(path + ".kmc_suf is shorter than its header says");
+  if (n_dev > 1) {
+    std::vector<mg_ctx *> all;
+    for (auto &x : gs) all.push_back(x.c);
+    gpu(mg_reduce_counts(all.data(), n_dev), "mg_reduce_counts");
+    for (size_t d = 1; d < gs.size(); ++d) {  // the replicas are no longer needed
+      mg_destroy(gs[d].c);
+      gs[d].c = nullptr;
+    }
+  }
+}
+
+// STEP 3: genotype (main.cpp:504-581), one pass over the VCF.  outs[s] receives the VCF body of output s: the live
+// counters of g (mg_genotype_packed, one output), or with sample_set every sample of g's sample set
+// (mg_genotype_samples_packed, sample s into outs[s]).  Three stages on three threads: enumerate
+// (EnumeratedBatches) | device (below) | format + write (this thread).
+void genotype_pass(const Options &o, mg_ctx *g, bool sample_set, EnumeratedBatches &batches,
+                   const std::vector<FILE *> &outs) {
+  const size_t n_out = outs.size();
+  Channel<std::unique_ptr<Batch>> done(2);
+  std::exception_ptr dev_err;
+  std::thread device([&] {
+    try {
+      std::unique_ptr<Batch> b;
+      std::vector<mg_genotype_out> res(n_out);
+      while (batches.next(b)) {
+        Stopwatch sw;
+        const mh::SignatureCsr &sg = b->sigs;
+        const uint64_t nv = sg.n_variants(), na = sg.n_alleles();
+        if (nv) {
+          if (o.verbose) {
+            b->lik_off.assign(nv + 1, 0);
+            for (uint64_t i = 0; i < nv; ++i) {
+              uint64_t n = sg.var_allele_off[i + 1] - sg.var_allele_off[i];
+              b->lik_off[i + 1] = b->lik_off[i] + std::max<uint64_t>(n, o.haploid ? n : n * (n + 1) / 2);
+            }
+            b->lik.assign(b->lik_off[nv] * n_out, 0.0);
+          }
+          // (a recycled batch: nothing of its previous results may show through)
+          b->cov.assign(na * n_out, 0);
+          b->n_gts.assign(nv * n_out, 0), b->status.assign(nv * n_out, 0), b->best.assign(nv * n_out, 0);
+          b->gq.assign(nv * n_out, 0);
+          mg_packed_batch in = {nv,
+                                sg.var_allele_off.data(),
+                                sg.allele_sig_off.data(),
+                                sg.sig_kmer_off.data(),
+                                sg.kmers.data(),
+                                sg.freq.data(),
+                                sg.n_irregular(),
+                                sg.irr_off.data(),
+                                sg.irr_pool.data(),
+                                sg.irr_kmer.data()};
+          for (size_t s = 0; s < n_out; ++s)
+            res[s] = {b->cov.data() + s * na, b->n_gts.data() + s * nv, b->status.data() + s * nv,
+                      b->best.data() + s * nv, b->gq.data() + s * nv, o.verbose ? b->lik_off.data() : nullptr,
+                      o.verbose ? b->lik.data() + s * b->lik_off[nv] : nullptr};
+          if (!sample_set)
+            gpu(mg_genotype_packed(g, &in, res.data(), o.error_rate, (int)o.max_coverage, o.haploid ? 1 : 0),
+                "mg_genotype_packed");
+          else
+            gpu(mg_genotype_samples_packed(g, &in, res.data(), (int)n_out, o.error_rate, (int)o.max_coverage,
+                                           o.haploid ? 1 : 0),
+                "mg_genotype_samples_packed");
+        }
+        b->t_dev = sw.lap();
+        done.push(std::move(b));
+      }
+    } catch (...) {
+      dev_err = std::current_exception();
+    }
+    done.close();
+  });
+  struct Joiner {  // (an exception below must not leave the thread running)
+    std::thread &t;
+    Channel<std::unique_ptr<Batch>> &c;
+    ~Joiner() {
+      c.close();
+      if (t.joinable()) t.join();
+    }
+  } joiner{device, done};
+  std::vector<const mh::Variant *> order;
+  std::vector<std::string> text;
+  std::unique_ptr<Batch> b;
+  Stopwatch sw;
+  while (done.pop(b)) {
+    sw.lap();
+    const mh::SignatureCsr &sg = b->sigs;
+    const uint64_t nv = sg.n_variants(), na = sg.n_alleles();
+    if (nv == 0) {
+      batches.recycle(std::move(b));
+      continue;
+    }
+    order.clear();
+    for (const auto &blk : b->vb.blocks)
+      for (size_t i = 0; i < blk.size(); ++i) order.push_back(&blk[i]);
+    const size_t chunk = 4096, n_chunks = (nv + chunk - 1) / chunk;
+    if (text.size() < n_chunks * n_out) text.resize(n_chunks * n_out);
+    for (size_t c = 0; c < n_chunks * n_out; ++c) text[c].clear();  // (capacity kept from batch to batch)
+    parallel_for(n_chunks * n_out, o.threads, [&](size_t t) {
+      const size_t s = t / n_chunks, c = t % n_chunks;
+      const uint32_t *cov = b->cov.data() + s * na;
+      const int32_t *n_gts = b->n_gts.data() + s * nv, *status = b->status.data() + s * nv,
+                    *best = b->best.data() + s * nv, *gq = b->gq.data() + s * nv;
+      const double *lik = o.verbose ? b->lik.data() + s * b->lik_off[nv] : nullptr;
+      for (size_t i = c * chunk; i < std::min<size_t>(nv, (c + 1) * chunk); ++i)
+        format_variant(*order[i], cov + sg.var_allele_off[i], n_gts[i], status[i], best[i], gq[i],
+                       o.verbose ? lik + b->lik_off[i] : nullptr, o, text[t]);
+    });
+    for (size_t s = 0; s < n_out; ++s)
+      for (size_t c = 0; c < n_chunks; ++c) fwrite(text[s * n_chunks + c].data(), 1, text[s * n_chunks + c].size(), outs[s]);
+    if (o.trace)
+      fprintf(stderr, "[trace] call batch: %llu variants, %llu k-mers: read+decode wait %.1f ms, enumerate %.1f ms, device %.1f ms, print %.1f ms\n",
+              (unsigned long long)nv, (unsigned long long)sg.n_kmers(), b->t_parse, b->t_enum, b->t_dev, sw.lap());
+    batches.recycle(std::move(b));
+  }
+  device.join();
+  if (dev_err) std::rethrow_exception(dev_err);
+  batches.join();
+}
+
+std::string base_name(const std::string &path) {
+  const size_t p = path.find_last_of('/');
+  return p == std::string::npos ? path : path.substr(p + 1);
+}
+
 int call_main(int argc, char **argv) {
   Options o;
-  if (!parse_arguments(argc, argv, o, 3)) return EXIT_FAILURE;
-  std::vector<std::future<int>> cuda_up;  // CUDA start-up on every device, overlapped with the file reading
-  for (int d : o.devices) cuda_up.push_back(std::async(std::launch::async, [d] { return mg_warmup(d); }));
-  BlockStream stream(o, false);
-  if (stream.samples_code != 0) {
-    std::cerr << "ERROR: VCF samples subset (code: " << stream.samples_code << ")" << std::endl;
+  if (!parse_arguments(argc, argv, o, 3, true)) return EXIT_FAILURE;
+  const size_t n_db = o.kmc_paths.size();
+  if (n_db > 1 && o.out_dir.empty()) {
+    std::cerr << "ERROR: several KMC databases need --out-dir DIR (sample P is written to DIR/basename(P).vcf)"
+              << std::endl;
     return 1;
   }
-  mh::KmcDb db;
-  {
+  if (n_db == 1 && !o.out_dir.empty()) {
+    std::cerr << "ERROR: --out-dir is for several KMC databases; with one the VCF goes to stdout" << std::endl;
+    return 1;
+  }
+  if (n_db > 1 && o.devices.size() > 1) {
+    std::cerr << "ERROR: --devices takes one KMC database; several databases run on one device (--device N)"
+              << std::endl;
+    return 1;
+  }
+  for (size_t i = 0; i < n_db; ++i)
+    for (size_t j = 0; j < i; ++j)
+      if (base_name(o.kmc_paths[i]) == base_name(o.kmc_paths[j])) {
+        std::cerr << "ERROR: two KMC databases are named " << base_name(o.kmc_paths[i])
+                  << ": both would be written to " << o.out_dir << "/" << base_name(o.kmc_paths[i]) << ".vcf (given twice)"
+                  << std::endl;
+        return 1;
+      }
+  std::vector<std::future<int>> cuda_up;  // CUDA start-up on every device, overlapped with the file reading
+  for (int d : o.devices) cuda_up.push_back(std::async(std::launch::async, [d] { return mg_warmup(d); }));
+  auto stream = std::make_unique<BlockStream>(o, false);
+  if (stream->samples_code != 0) {
+    std::cerr << "ERROR: VCF samples subset (code: " << stream->samples_code << ")" << std::endl;
+    return 1;
+  }
+  std::vector<std::unique_ptr<mh::KmcDb>> dbs;  // every database is opened before any work
+  for (const std::string &path : o.kmc_paths) {
+    dbs.push_back(std::make_unique<mh::KmcDb>());
     std::string why;
-    if (!db.open(o.kmc_path, why)) {
-      std::cerr << "ERROR: cannot open " << o.kmc_path << std::endl;
+    if (!dbs.back()->open(path, why)) {
+      std::cerr << "ERROR: cannot open " << path << std::endl;
       return 1;
     }
   }
-  BatchPrefetcher call_batches(stream, LINES_PER_BATCH);  // first VCF batch decoded while the index loads and the scan runs
+  // first VCF batch decoded while the index loads and the scan runs
+  auto call_batches = std::make_unique<BatchPrefetcher>(*stream, LINES_PER_BATCH);
   // the reference FASTA is read while CUDA starts and the index loads (host-only work, 1.4 s for 250 Mbp)
   std::future<std::map<std::string, std::string>> refs_ready =
       std::async(std::launch::async, [&o] { return mh::read_fasta(o.fasta_path, o.strip_chr); });
@@ -928,150 +1130,64 @@ int call_main(int argc, char **argv) {
   std::map<std::string, std::string> refs = refs_ready.get();
   pelapsed("Reference processed");
   // (host only: the first batches are decoded and enumerated while the KMC records stream through the device)
-  EnumeratedBatches batches(call_batches, refs, o);
+  auto batches = std::make_unique<EnumeratedBatches>(*call_batches, refs, o);
 
-  // STEP 2: the sample k-mer scan (main.cpp:482-500).  Raw suffix records go through rings of pinned buffers, one
-  // ring per device, chunks dealt round-robin; the library copies and scans them asynchronously (double-buffered on
-  // its side), a buffer is refilled only after the event recorded behind its scan has completed.  With several
-  // devices the counters are then added up on the first one (all updates are commutative adds, main.cpp:495-499).
-  pelapsed("KMC output processing");
-  {
-    constexpr int RING = 4;
-    constexpr uint64_t CHUNK = 1ull << 22;  // records per buffer
-    std::vector<uint8_t *> buf((size_t)(n_dev * RING), nullptr);
-    std::vector<char> used((size_t)(n_dev * RING), 0);
-    Stopwatch sw;
-    for (int d = 0; d < n_dev; ++d) {
-      gpu(mg_kmc_open(gs[(size_t)d].c, db.lut.data(), db.lut.size(), db.lut_prefix_len, db.kmer_len, db.counter_size,
-                      db.min_count, db.max_count),
-          "mg_kmc_open");
-      for (int s = 0; s < RING; ++s) gpu(mg_host_alloc((void **)&buf[(size_t)(d * RING + s)], CHUNK * db.record_bytes + 64), "mg_host_alloc");
-    }
-    uint64_t first = 0;
-    double t_alloc = sw.lap(), t_wait = 0, t_read = 0, t_submit = 0;
-    for (uint64_t chunk = 0;; ++chunk) {
-      const int d = (int)(chunk % (uint64_t)n_dev), slot = d * RING + (int)((chunk / (uint64_t)n_dev) % RING);
-      mg_ctx *c = gs[(size_t)d].c;
-      if (used[(size_t)slot]) gpu(mg_event_sync(c, 32 + slot % RING), "mg_event_sync");
-      t_wait += sw.lap();
-      uint64_t n = db.read_records(buf[(size_t)slot], first, CHUNK);
-      t_read += sw.lap();
-      if (n == 0) break;
-      gpu(mg_scan_kmc_records(c, buf[(size_t)slot], first, n), "mg_scan_kmc_records");
-      gpu(mg_event_record(c, 32 + slot % RING), "mg_event_record");
-      t_submit += sw.lap();
-      used[(size_t)slot] = 1;
+  if (n_db == 1) {
+    pelapsed("KMC output processing");
+    scan_kmc(o, gs, *dbs[0], o.kmc_path);
+    pelapsed("BF weights created");
+    std::cout << stream->header().cleaned(o.verbose);
+    pelapsed("VCF parsing and genotyping");
+    genotype_pass(o, g.c, false, *batches, {stdout});
+  } else {
+    // several samples: groups of up to MG_SAMPLE_SET_MAX (as many as device memory holds) share one VCF pass -- each
+    // sample of a group is scanned into the live counters and moved into its column of the sample set, then one
+    // pass genotypes the whole set.  The index, the FASTA and the CUDA context serve every group.
+    if (mkdir(o.out_dir.c_str(), 0777) != 0 && errno != EEXIST)
+      throw std::runtime_error("cannot create " + o.out_dir + ": " + strerror(errno));
+    const std::string header = stream->header().cleaned(o.verbose);
+    for (size_t first = 0; first < n_db;) {
+      int fit = 0;
+      gpu(mg_samples_capacity(g.c, &fit), "mg_samples_capacity");
+      if (fit < 1) throw std::runtime_error("not even one sample column fits in device memory next to the index");
+      const size_t n = std::min<size_t>((size_t)fit, n_db - first);
+      if (first > 0) {  // a fresh VCF pass (the previous group's has ended)
+        batches.reset();
+        call_batches.reset();
+        stream = std::make_unique<BlockStream>(o, false);
+        call_batches = std::make_unique<BatchPrefetcher>(*stream, LINES_PER_BATCH);
+        batches = std::make_unique<EnumeratedBatches>(*call_batches, refs, o);
+      }
+      gpu(mg_samples_begin(g.c, (int)n), "mg_samples_begin");
+      pelapsed("KMC output processing");
+      for (size_t s = 0; s < n; ++s) {
+        scan_kmc(o, gs, *dbs[first + s], o.kmc_paths[first + s]);
+        gpu(mg_samples_take(g.c, (int)s), "mg_samples_take");
+      }
+      pelapsed("BF weights created");
+      std::vector<FILE *> outs;
+      struct Files {  // (closed on every way out)
+        std::vector<FILE *> &f;
+        ~Files() {
+          for (FILE *x : f) fclose(x);
+        }
+      } files{outs};
+      for (size_t s = 0; s < n; ++s) {
+        const std::string path = o.out_dir + "/" + base_name(o.kmc_paths[first + s]) + ".vcf";
+        FILE *f = fopen(path.c_str(), "wb");
+        if (!f) throw std::runtime_error("cannot write " + path + ": " + strerror(errno));
+        outs.push_back(f);
+        fwrite(header.data(), 1, header.size(), f);
+      }
+      pelapsed("VCF parsing and genotyping");
+      genotype_pass(o, g.c, true, *batches, outs);
+      for (FILE *f : outs)
+        if (fflush(f) != 0) throw std::runtime_error("cannot write to " + o.out_dir + ": " + strerror(errno));
+      gpu(mg_samples_end(g.c), "mg_samples_end");
       first += n;
     }
-    for (auto &x : gs) gpu(mg_sync(x.c), "mg_sync");
-    const double t_drain = sw.lap();
-    for (auto &b : buf) mg_host_free(b);
-    if (o.trace)
-      fprintf(stderr, "[trace] KMC scan: %llu records; pinned buffers %.1f ms, file reads %.1f ms, waiting for a free buffer "
-                      "%.1f ms, submitting %.1f ms, draining %.1f ms, freeing %.1f ms\n",
-              (unsigned long long)first, t_alloc, t_read, t_wait, t_submit, t_drain, sw.lap());
-    if (first != db.total_kmers)
-      throw std::runtime_error(o.kmc_path + ".kmc_suf is shorter than its header says");
-    if (n_dev > 1) {
-      std::vector<mg_ctx *> all;
-      for (auto &x : gs) all.push_back(x.c);
-      gpu(mg_reduce_counts(all.data(), n_dev), "mg_reduce_counts");
-      for (size_t d = 1; d < gs.size(); ++d) {  // the replicas are no longer needed
-        mg_destroy(gs[d].c);
-        gs[d].c = nullptr;
-      }
-    }
   }
-  pelapsed("BF weights created");
-
-  // STEP 3: genotype (main.cpp:504-581)
-  std::cout << stream.header().cleaned(o.verbose);
-  pelapsed("VCF parsing and genotyping");
-  // three stages on three threads: enumerate (EnumeratedBatches) | device (below) | format + write (this thread)
-  Channel<std::unique_ptr<Batch>> done(2);
-  std::exception_ptr dev_err;
-  std::thread device([&] {
-    try {
-      std::unique_ptr<Batch> b;
-      while (batches.next(b)) {
-        Stopwatch sw;
-        const mh::SignatureCsr &sg = b->sigs;
-        const uint64_t nv = sg.n_variants();
-        if (nv) {
-          if (o.verbose) {
-            b->lik_off.assign(nv + 1, 0);
-            for (uint64_t i = 0; i < nv; ++i) {
-              uint64_t n = sg.var_allele_off[i + 1] - sg.var_allele_off[i];
-              b->lik_off[i + 1] = b->lik_off[i] + std::max<uint64_t>(n, o.haploid ? n : n * (n + 1) / 2);
-            }
-            b->lik.assign(b->lik_off[nv], 0.0);
-          }
-          b->cov.assign(sg.n_alleles(), 0);  // (a recycled batch: nothing of its previous results may show through)
-          b->n_gts.assign(nv, 0), b->status.assign(nv, 0), b->best.assign(nv, 0), b->gq.assign(nv, 0);
-          mg_packed_batch in = {nv,
-                                sg.var_allele_off.data(),
-                                sg.allele_sig_off.data(),
-                                sg.sig_kmer_off.data(),
-                                sg.kmers.data(),
-                                sg.freq.data(),
-                                sg.n_irregular(),
-                                sg.irr_off.data(),
-                                sg.irr_pool.data(),
-                                sg.irr_kmer.data()};
-          mg_genotype_out res = {b->cov.data(),  b->n_gts.data(), b->status.data(),
-                                 b->best.data(), b->gq.data(),    o.verbose ? b->lik_off.data() : nullptr,
-                                 o.verbose ? b->lik.data() : nullptr};
-          gpu(mg_genotype_packed(g.c, &in, &res, o.error_rate, (int)o.max_coverage, o.haploid ? 1 : 0), "mg_genotype_packed");
-        }
-        b->t_dev = sw.lap();
-        done.push(std::move(b));
-      }
-    } catch (...) {
-      dev_err = std::current_exception();
-    }
-    done.close();
-  });
-  struct Joiner {  // (an exception below must not leave the thread running)
-    std::thread &t;
-    Channel<std::unique_ptr<Batch>> &c;
-    ~Joiner() {
-      c.close();
-      if (t.joinable()) t.join();
-    }
-  } joiner{device, done};
-  std::vector<const mh::Variant *> order;
-  std::vector<std::string> text;
-  std::unique_ptr<Batch> b;
-  Stopwatch sw;
-  while (done.pop(b)) {
-    sw.lap();
-    const mh::SignatureCsr &sg = b->sigs;
-    const uint64_t nv = sg.n_variants();
-    if (nv == 0) {
-      batches.recycle(std::move(b));
-      continue;
-    }
-    order.clear();
-    for (const auto &blk : b->vb.blocks)
-      for (size_t i = 0; i < blk.size(); ++i) order.push_back(&blk[i]);
-    const size_t chunk = 4096, n_chunks = (nv + chunk - 1) / chunk;
-    if (text.size() < n_chunks) text.resize(n_chunks);
-    for (size_t c = 0; c < n_chunks; ++c) text[c].clear();  // (capacity kept from batch to batch)
-    parallel_for(n_chunks, o.threads, [&](size_t c) {
-      for (size_t i = c * chunk; i < std::min<size_t>(nv, (c + 1) * chunk); ++i)
-        format_variant(*order[i], b->cov.data() + sg.var_allele_off[i], b->n_gts[i], b->status[i], b->best[i], b->gq[i],
-                       o.verbose ? b->lik.data() + b->lik_off[i] : nullptr, o, text[c]);
-    });
-    for (size_t c = 0; c < n_chunks; ++c) fwrite(text[c].data(), 1, text[c].size(), stdout);
-    if (o.trace)
-      fprintf(stderr, "[trace] call batch: %llu variants, %llu k-mers: read+decode wait %.1f ms, enumerate %.1f ms, device %.1f ms, print %.1f ms\n",
-              (unsigned long long)nv, (unsigned long long)sg.n_kmers(), b->t_parse, b->t_enum, b->t_dev, sw.lap());
-    batches.recycle(std::move(b));
-  }
-  device.join();
-  if (dev_err) std::rethrow_exception(dev_err);
-  batches.join();
-  pelapsed("Processed " + std::to_string(stream.n_records) + " variants");
+  pelapsed("Processed " + std::to_string(stream->n_records) + " variants");
   fflush(stdout);
   pelapsed("Execution completed");
   finish(0);

@@ -5,6 +5,7 @@
 //   K4  k_lookup_packed / k_lookup / k_coverage                        coverage read-back
 //   K5  k_genotype                                                     likelihoods + posterior arg-max
 //       k_counters_xfer / k_sum_peers                                  dense counter image for the multi-GPU reduce
+//       k_samples_take_* / k_lookup_samples / k_lookup_samples_irr     sample sets: several samples on one index
 #pragma once
 #include <cuda_runtime.h>
 
@@ -1071,6 +1072,223 @@ __global__ void __launch_bounds__(LOOKUP_THREADS) k_lookup_packed(const uint4 *_
     out[i] = res;
   }
 }
+// ---------------------------------------------------------------------------
+// Sample sets (include/malva_gpu.h, mg_samples_*): the counters of up to 32 samples side by side.  Every counter a
+// signature k-mer can read has a ROW that depends on the index only:
+//   [0, bf_ones)                    a set bit of bf: its rank + j                     (BF::get_count)
+//   [key_base, key_base + keys)     a ref key held by a probe line: key_rank[L] + slot (KMAP::get_count)
+//   [ovf_base, ovf_base + ovf cap)  a slot of the overflow table
+// and a sample is a column of u32 counts over those rows.  The set is row-major, mat[row * g + s]: the g counts of
+// a row share one 128-byte line, so a signature k-mer costs one probe line and one count line for all samples.
+// ---------------------------------------------------------------------------
+constexpr uint32_t NO_ROW = 0xFFFFFFFFu;
+constexpr int SAMPLE_SET_MAX = 32;
+struct SampleView {
+  uint32_t *mat;
+  const uint32_t *key_rank;  // keys held by the lines before line L
+  uint64_t key_base, ovf_base;
+  int g;
+};
+__device__ __forceinline__ uint32_t *sample_cell(const SampleView &sv, uint64_t row, int col) {
+  return sv.mat + row * (uint64_t)sv.g + (uint64_t)col;
+}
+
+// mg_samples_take, dense part: src[i] (bf_counts, ovf_counts) -> row row0 + i of column col; src is zeroed
+__global__ void __launch_bounds__(256) k_samples_take_dense(uint32_t *__restrict__ src, uint64_t n, uint64_t row0,
+                                                           SampleView sv, int col) {
+  const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+  for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+    const uint32_t c = src[i];
+    *sample_cell(sv, row0 + i, col) = c;
+    if (c) src[i] = 0;
+  }
+}
+// mg_samples_take, the counters inside the probe lines (k_counters_xfer's walk: eight lanes per line, one uint4
+// each): the inline counters of set bits 0..2 and the key counts go to column col and are zeroed in place.  Runs
+// after k_samples_take_dense of bf_counts, whose entries for set bits 0..2 of a line are not live counters.
+__global__ void __launch_bounds__(256) k_samples_take_lines(DevView v, SampleView sv, int col) {
+  const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const uint64_t line = t >> 3;
+  const int sub = (int)(t & 7);
+  const bool ok = line < v.n_lines;
+  const uint4 q = ok ? v.lines[line * LINE_U4 + (uint64_t)sub] : make_uint4(0, 0, 0, 0);
+  const uint32_t pc = sub < 2 ? (uint32_t)(__popc(q.x) + __popc(q.y) + __popc(q.z) + __popc(q.w)) : 0u;
+  const int g0 = (int)(threadIdx.x & 24);
+  const uint32_t n_alt = __shfl_sync(0xffffffffu, pc, g0) + __shfl_sync(0xffffffffu, pc, g0 + 1);
+  if (!ok) return;
+  uint32_t *w = line_words(v, line);
+  if (sub == 7) {
+    const uint32_t c[3] = {q.y, q.z, q.w};
+#pragma unroll
+    for (int j = 0; j < LINE_INLINE_ALT; ++j)
+      if ((uint32_t)j < n_alt) *sample_cell(sv, (uint64_t)q.x + (uint64_t)j, col) = c[j];
+    if (q.y | q.z | q.w) v.lines[line * LINE_U4 + 7] = make_uint4(q.x, 0u, 0u, 0u);
+  } else if (sub >= 2) {
+    const int s = sub - 2;
+    if (key_empty(v, key_of(v, q))) return;
+    const uint64_t row = sv.key_base + (uint64_t)sv.key_rank[line] + (uint64_t)s;
+    uint32_t *cp = v.inline_counts ? w + 8 + 4 * s + 3 : v.key_counts + line * LINE_KEYS + (uint64_t)s;
+    const uint32_t c = v.inline_counts ? q.w : *cp;
+    *sample_cell(sv, row, col) = c;
+    if (c) *cp = 0;
+  }
+}
+
+// row of a set bit of bf (bf index idx), or NO_ROW when the bit is clear
+__device__ __forceinline__ uint32_t alt_row(const DevView &v, uint64_t idx) {
+  const uint4 *p = v.lines + (idx >> 8) * LINE_U4;
+  const uint4 a = __ldg(p), b = __ldg(p + 1), m = __ldg(p + 7);
+  const uint32_t w[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
+  const uint32_t ws = (uint32_t)((idx & 255) >> 5), below = (1u << (idx & 31)) - 1u;
+  uint32_t mine = 0, j = 0;
+#pragma unroll
+  for (uint32_t x = 0; x < 8; ++x) {
+    mine = x == ws ? w[x] : mine;
+    j += (uint32_t)__popc(w[x] & (x < ws ? 0xFFFFFFFFu : (x == ws ? below : 0u)));
+  }
+  return ((mine >> (idx & 31)) & 1u) ? m.x + j : NO_ROW;
+}
+// row of ref key `canon` (bf index idx), or NO_ROW when the key is absent
+__device__ __forceinline__ uint32_t key_row(const DevView &v, const SampleView &sv, uint64_t idx, u128 canon) {
+  const uint64_t line = idx >> 8;
+  const uint4 *p = v.lines + line * LINE_U4 + 2;
+  uint4 q[LINE_KEYS];
+#pragma unroll
+  for (int s = 0; s < LINE_KEYS; ++s) q[s] = __ldg(p + s);
+#pragma unroll
+  for (int s = 0; s < LINE_KEYS; ++s)
+    if (key_eq(key_of(v, q[s]), canon)) return (uint32_t)(sv.key_base + __ldg(sv.key_rank + line) + (uint64_t)s);
+  if (!(u128_of(q[LINE_KEYS - 1]).hi & v.ovf_flag_hi)) return NO_ROW;
+  const int64_t slot = ovf_find(v, canon);
+  return slot < 0 ? NO_ROW : (uint32_t)(sv.ovf_base + (uint64_t)slot);
+}
+
+// The look-up of k_lookup_packed for a whole sample set: every lane resolves the ROW of its k-mer from the probe line
+// (same tile, same gather), then the warp reads the 32 rows one after the other with the lanes on the samples (one
+// coalesced line per k-mer), transposes them through shared memory and writes the weights sample-major,
+// out[s * n + i], 128 bytes per store.  bf weights are BF::get_count's uint16_t, ref weights KMAP::get_count's int.
+// Irregular k-mers get 0 here; k_lookup_samples_irr writes them afterwards.
+constexpr int LOOKUP_SAMPLES_SMEM = LOOKUP_SMEM + (LOOKUP_THREADS / 32) * 32 * 33 * 4;
+template <int K>
+__global__ void __launch_bounds__(LOOKUP_THREADS) k_lookup_samples(const uint4 *__restrict__ kmers, uint64_t n, DevView v,
+                                                                  SampleView sv, int32_t *__restrict__ out) {
+  extern __shared__ uint4 lk_sm[];
+  const int lane = threadIdx.x & 31, sub = lane & 7, grp = lane >> 3, wid = threadIdx.x >> 5;
+  uint4 *tile = lk_sm + wid * 256;
+  uint32_t *tr = reinterpret_cast<uint32_t *>(lk_sm + (LOOKUP_THREADS / 32) * 256) + wid * 32 * 33;
+  const uint32_t tile_addr = (uint32_t)__cvta_generic_to_shared(tile);
+  const uint32_t d_even = tile_addr + (uint32_t)(grp * 128 + ((sub ^ grp) * 16));
+  const uint32_t d_odd = tile_addr + (uint32_t)(grp * 128 + ((sub ^ (grp + 4)) * 16));
+  const char *line_src = reinterpret_cast<const char *>(v.lines) + sub * 16;
+  const int k = K > 0 ? K : v.k;
+  const bool inl = K > 0 ? (K <= INLINE_MAX_K) : (v.inline_counts != 0);
+  const uint32_t mz = inl ? 0x7FFFFFFFu : 0xFFFFFFFFu, mw = inl ? 0u : 0x3FFFFFFFu;
+  const int g = sv.g;
+  const uint64_t warp0 = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = ((uint64_t)gridDim.x * blockDim.x) >> 5;
+  for (uint64_t base = warp0 * 32; base < n; base += n_warps * 32) {
+    const uint64_t i = base + (uint64_t)lane;
+    const uint4 q = i < n ? __ldg(kmers + i) : make_uint4(0, 0, 0, 0x80000000u);
+    const bool active = !(q.w >> 31);
+    const bool is_ref = (q.w >> 30) & 1u;
+    u128 canon;
+    const uint64_t h = canon_hash_k<K>(mask128(u128_of(q), 2 * k), k, &canon);
+    const uint64_t idx = bf_index(v, h);
+    const uint32_t line = (uint32_t)(idx >> 8), bit = (uint32_t)(idx & 255);
+    const uint32_t act = __ballot_sync(0xffffffffu, active), refs = __ballot_sync(0xffffffffu, is_ref);
+    __syncwarp();  // the previous batch's reads of the tile and of the transposition buffer are done
+#pragma unroll
+    for (int r = 0; r < 8; ++r) {
+      const uint32_t lid = __shfl_sync(0xffffffffu, line, 4 * r + grp);
+      if ((act >> (4 * r + grp)) & 1u)
+        cp_async16(((r & 1) ? d_odd : d_even) + (uint32_t)(r * 512), line_src + ((uint64_t)lid << 7));
+    }
+    asm volatile("cp.async.commit_group;\ncp.async.wait_group 0;\n" ::: "memory");
+    __syncwarp();
+    uint32_t row = NO_ROW;
+    if (active) {
+      const uint4 *mine = tile + lane * 8;
+      const int sw = lane & 7;
+      if (is_ref) {
+        const uint32_t c0 = (uint32_t)canon.lo, c1 = (uint32_t)(canon.lo >> 32), c2 = (uint32_t)canon.hi,
+                       c3 = (uint32_t)(canon.hi >> 32);
+        int slot = -1;
+        uint32_t flag_w = 0;
+#pragma unroll
+        for (int s = 0; s < LINE_KEYS; ++s) {
+          const uint4 p = mine[(2 + s) ^ sw];
+          if (((p.x ^ c0) | (p.y ^ c1) | ((p.z ^ c2) & mz) | ((p.w ^ c3) & mw)) == 0) slot = s;
+          if (s == LINE_KEYS - 1) flag_w = inl ? p.z : p.w;
+        }
+        if (slot >= 0) {
+          row = (uint32_t)(sv.key_base + __ldg(sv.key_rank + line) + (uint32_t)slot);
+        } else if (flag_w >> 31) {
+          const int64_t os = ovf_find(v, canon);
+          if (os >= 0) row = (uint32_t)(sv.ovf_base + (uint64_t)os);
+        }
+      } else {
+        const uint32_t ws = bit >> 5, below = (1u << (bit & 31u)) - 1u;
+        const uint4 b0 = mine[0 ^ sw], b1 = mine[1 ^ sw], m = mine[7 ^ sw];
+        const uint32_t wx[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
+        uint32_t hit_w = 0, j = 0;
+#pragma unroll
+        for (uint32_t x = 0; x < 8; ++x) {
+          hit_w = x == ws ? wx[x] : hit_w;
+          j += (uint32_t)__popc(wx[x] & (x < ws ? 0xFFFFFFFFu : (x == ws ? below : 0u)));
+        }
+        if ((hit_w >> (bit & 31u)) & 1u) row = m.x + j;
+      }
+    }
+    // the counts of the 32 rows, lanes = samples
+#pragma unroll 8
+    for (int r = 0; r < 32; ++r) {
+      const uint32_t rr = __shfl_sync(0xffffffffu, row, r);
+      uint32_t c = 0;
+      if (rr != NO_ROW && lane < g) c = __ldg(sv.mat + (uint64_t)rr * (uint64_t)g + (uint64_t)lane);
+      tr[r * 33 + lane] = ((refs >> r) & 1u) ? c : (c & 0xFFFFu);
+    }
+    __syncwarp();
+    if (i < n)
+      for (int s = 0; s < g; ++s) out[(uint64_t)s * n + i] = (int32_t)tr[lane * 33 + s];
+  }
+}
+// the irregular k-mers of a sample-set look-up (not k symbols of ACGT): k_lookup's byte-exact ASCII path, resolved to
+// a row instead of a count -- an irregular alt k-mer can hit a set bit of bf; an irregular ref key is never in the
+// device map and counts 0.  out[s * n + irr_kmer[j]] for every sample s.
+__global__ void __launch_bounds__(128) k_lookup_samples_irr(const uint8_t *__restrict__ pool, const uint64_t *__restrict__ off,
+                                                           const uint32_t *__restrict__ irr_kmer, uint64_t n_irr,
+                                                           const uint4 *__restrict__ packed, uint64_t n, DevView v,
+                                                           SampleView sv, int32_t *__restrict__ out,
+                                                           unsigned long long *scalars) {
+  const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n_irr) return;
+  const uint64_t o = irr_kmer[i];
+  const uint64_t b = off[i];
+  const int len = (int)(off[i + 1] - b);
+  const bool ref_flag = ((packed[o].w >> 30) & 1u) != 0;
+  uint32_t row = NO_ROW;
+  if (len > 128) {
+    atomicExch(&scalars[3], 1ull);
+  } else {
+    uint8_t s[128];
+    for (int j = 0; j < len; ++j) s[j] = pool[b + j];
+    u128 x, canon;
+    if (ref_flag) {
+      if (pack_ascii(s, len, v.k, &x)) {
+        const uint64_t h = canon_hash_rt(x, v.k, &canon);
+        row = key_row(v, sv, bf_index(v, h), canon);
+      }
+    } else {
+      const bool regular = len >= 1 && len <= 64 && pack_ascii(s, len, len, &x);
+      const uint64_t h = regular ? canon_hash_rt(x, len, &canon) : hash_ascii(s, len);
+      row = alt_row(v, bf_index(v, h));
+    }
+  }
+  for (int c = 0; c < sv.g; ++c) {
+    const uint32_t cnt = row == NO_ROW ? 0u : __ldg(sv.mat + (uint64_t)row * (uint64_t)sv.g + (uint64_t)c);
+    out[(uint64_t)c * n + o] = (int32_t)(ref_flag ? cnt : (cnt & 0xFFFFu));
+  }
+}
+
 // BF::get_count's uint16_t of summed raw bf counters (the k-mers that are not flagged as ref-allele k-mers)
 __global__ void __launch_bounds__(256) k_mask_alt(const uint4 *__restrict__ kmers, uint64_t n, int32_t *__restrict__ w) {
   uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;

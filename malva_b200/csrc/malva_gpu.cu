@@ -82,8 +82,8 @@ struct mg_ctx {
   int occ_shift = 0;
   uint32_t *bf_counts = nullptr;   // one per set bit of bf (dense image; live for set bits 3.. of a line)
   uint32_t *key_counts = nullptr;  // n_lines x 5, wide layout (k >= 48) only
-  uint32_t *key_rank = nullptr;    // keys held by the lines before line L (built by the first mg_counters_gather)
-  uint32_t *key_dense = nullptr;   // dense image of the in-line key counts (n_keys - ovf_n entries)
+  uint32_t *key_rank = nullptr;    // keys held by the lines before line L (built on first use: ensure_key_rank)
+  uint32_t *key_dense = nullptr;   // dense image of the in-line key counts (n_keys - ovf_n entries; first mg_counters_gather)
   u128 *ovf_keys = nullptr;
   uint32_t *ovf_counts = nullptr;
   int ovf_log2 = 0;
@@ -124,6 +124,9 @@ struct mg_ctx {
   uint64_t geno_arena_bytes = 0;
   mh::SignatureCsr ascii_batch;  // mg_genotype's batch packed on the host (grow-only)
   cudaEvent_t evs[64] = {};
+  uint32_t *samples = nullptr;  // sample set of mg_samples_begin: rows x samples_g u32 (kernels.cuh SampleView)
+  uint64_t sample_rows = 0;
+  int samples_g = 0;
 
   DevView view() const {
     DevView v;
@@ -294,6 +297,7 @@ extern "C" void mg_destroy(mg_ctx *c) {
   cudaFree(c->geno_arena);
   cudaFree(c->log_table);
   cudaFree(c->kmc_lut);
+  cudaFree(c->samples);
   for (int i = 0; i < 2; ++i) {
     cudaFree(c->hit_buf[i]);
     cudaFree(c->hit_counts[i]);
@@ -633,17 +637,22 @@ extern "C" int mg_finalize_alt(mg_ctx *c) {
 }
 
 // ---- dense counter image (index.cuh): gather before a reduce / download, scatter after a reduce ----
+// keys held by the lines before each line: built once, on first use (the key slots are final after mg_finalize_alt)
+static int ensure_key_rank(mg_ctx *c) {
+  if (c->key_rank) return MG_OK;
+  DevFree cnt;
+  CU(cudaMalloc(&cnt.p, (c->n_lines + 1) * 4));
+  CU(cudaMalloc(&c->key_rank, (c->n_lines + 1) * 4));
+  CU(cudaMemsetAsync((uint32_t *)cnt.p + c->n_lines, 0, 4, c->stream[0]));
+  c->launches++;
+  mg::k_line_keycount<<<grid_for(c->n_lines, 256), 256, 0, c->stream[0]>>>(c->view(), (uint32_t *)cnt.p);
+  CU(cudaGetLastError());
+  return line_scan(c, (uint32_t *)cnt.p, c->key_rank);
+}
 static int counters_xfer(mg_ctx *c, bool scatter) {
   const uint64_t n_line_keys = c->n_keys - c->ovf_n;
-  if (!c->key_rank) {  // keys held by the lines before each line: built once, on first use
-    DevFree cnt;
-    CU(cudaMalloc(&cnt.p, (c->n_lines + 1) * 4));
-    CU(cudaMalloc(&c->key_rank, (c->n_lines + 1) * 4));
-    CU(cudaMemsetAsync((uint32_t *)cnt.p + c->n_lines, 0, 4, c->stream[0]));
-    c->launches++;
-    mg::k_line_keycount<<<grid_for(c->n_lines, 256), 256, 0, c->stream[0]>>>(c->view(), (uint32_t *)cnt.p);
-    CU(cudaGetLastError());
-    int rc = line_scan(c, (uint32_t *)cnt.p, c->key_rank);
+  if (!c->key_dense) {
+    int rc = ensure_key_rank(c);
     if (rc) return rc;
     CU(cudaMalloc(&c->key_dense, (n_line_keys ? n_line_keys : 1) * 4));
     CU(cudaMemsetAsync(c->key_dense, 0, (n_line_keys ? n_line_keys : 1) * 4, c->stream[0]));
@@ -670,11 +679,117 @@ extern "C" int mg_counters_gather(mg_ctx *c) {
 }
 extern "C" int mg_counters_scatter(mg_ctx *c) {
   if (!c) return set_err(MG_ERR_ARG, "NULL ctx");
-  if (!c->key_rank) return set_err(MG_ERR_STATE, "mg_counters_scatter before mg_counters_gather");
+  if (!c->key_dense) return set_err(MG_ERR_STATE, "mg_counters_scatter before mg_counters_gather");
   CU(cudaSetDevice(c->device));
   int rc = counters_xfer(c, true);
   if (rc) return rc;
   CU(cudaStreamSynchronize(c->stream[0]));
+  return MG_OK;
+}
+
+// ---- sample sets (kernels.cuh SampleView): the counters of several samples side by side on one index ----
+static mg::SampleView sample_view(const mg_ctx *c) {
+  mg::SampleView sv;
+  sv.mat = c->samples;
+  sv.key_rank = c->key_rank;
+  sv.key_base = c->bf_ones;
+  sv.ovf_base = c->bf_ones + (c->n_keys - c->ovf_n);
+  sv.g = c->samples_g;
+  return sv;
+}
+extern "C" int mg_samples_end(mg_ctx *c) {
+  if (!c) return set_err(MG_ERR_ARG, "NULL ctx");
+  CU(cudaSetDevice(c->device));
+  if (c->samples) {
+    int rc = mg_sync(c);
+    if (rc) return rc;
+    CU(cudaFree(c->samples));
+  }
+  c->samples = nullptr;
+  c->sample_rows = 0;
+  c->samples_g = 0;
+  return MG_OK;
+}
+extern "C" int mg_samples_begin(mg_ctx *c, int n_samples) {
+  if (!c) return set_err(MG_ERR_ARG, "NULL ctx");
+  if (!c->alt_final) return set_err(MG_ERR_STATE, "mg_samples_begin before mg_finalize_alt");
+  if (n_samples < 1 || n_samples > MG_SAMPLE_SET_MAX)
+    return set_err(MG_ERR_ARG, "a sample set holds 1 to %d samples, not %d", MG_SAMPLE_SET_MAX, n_samples);
+  int rc = mg_samples_end(c);
+  if (rc) return rc;
+  const uint64_t rows = c->bf_ones + (c->n_keys - c->ovf_n) + (1ull << c->ovf_log2);
+  if (rows >= mg::NO_ROW) return set_err(MG_ERR_ARG, "the index has %llu counter rows; a sample set takes < 2^32",
+                                         (unsigned long long)rows);
+  rc = ensure_key_rank(c);
+  if (rc) return rc;
+  const size_t bytes = rows * (uint64_t)n_samples * 4;
+  CU(cudaMalloc(&c->samples, bytes));
+  CU(cudaMemsetAsync(c->samples, 0, bytes, c->stream[0]));
+  CU(cudaStreamSynchronize(c->stream[0]));
+  c->sample_rows = rows;
+  c->samples_g = n_samples;
+  return MG_OK;
+}
+// how many sample columns fit: MG_SAMPLE_SET_MAX at most, and no more than three quarters of the free device memory
+// (the rest is left to the genotyping batches, whose weights grow with the set)
+extern "C" int mg_samples_capacity(mg_ctx *c, int *n) {
+  if (!c || !n) return set_err(MG_ERR_ARG, "NULL argument");
+  if (!c->alt_final) return set_err(MG_ERR_STATE, "mg_samples_capacity before mg_finalize_alt");
+  CU(cudaSetDevice(c->device));
+  size_t free_b = 0, total_b = 0;
+  CU(cudaMemGetInfo(&free_b, &total_b));
+  const uint64_t column = 4 * (c->bf_ones + (c->n_keys - c->ovf_n) + (1ull << c->ovf_log2));
+  const uint64_t fit = (uint64_t)free_b / 4 * 3 / column + (c->samples ? (uint64_t)c->samples_g : 0);
+  *n = (int)std::min<uint64_t>(fit, MG_SAMPLE_SET_MAX);
+  return MG_OK;
+}
+extern "C" int mg_samples_take(mg_ctx *c, int s) {
+  if (!c) return set_err(MG_ERR_ARG, "NULL ctx");
+  if (!c->samples) return set_err(MG_ERR_STATE, "mg_samples_take before mg_samples_begin");
+  if (s < 0 || s >= c->samples_g) return set_err(MG_ERR_ARG, "sample %d outside the set of %d", s, c->samples_g);
+  int rc = mg_sync(c);  // the sample's scans (both streams, deferred filter hits included) are complete
+  if (rc) return rc;
+  cudaStream_t st = c->stream[0];
+  const mg::SampleView sv = sample_view(c);
+  const uint64_t ovf_cap = 1ull << c->ovf_log2;
+  const int dense_grid = c->sms * 8;
+  if (c->bf_ones) {  // first: the entries of set bits 0..2 of a line are overwritten by the line pass
+    c->launches++;
+    mg::k_samples_take_dense<<<dense_grid, 256, 0, st>>>(c->bf_counts, c->bf_ones, 0, sv, s);
+    CU(cudaGetLastError());
+  }
+  c->launches++;
+  mg::k_samples_take_lines<<<grid_for(c->n_lines * 8, 256), 256, 0, st>>>(c->view(), sv, s);
+  CU(cudaGetLastError());
+  c->launches++;
+  mg::k_samples_take_dense<<<dense_grid, 256, 0, st>>>(c->ovf_counts, ovf_cap, sv.ovf_base, sv, s);
+  CU(cudaGetLastError());
+  CU(cudaStreamSynchronize(st));
+  return MG_OK;
+}
+// K4 for a sample set: the weights of every sample, sample-major, into d_w [samples_g][n_kmers] (DEVICE batch)
+static int lookup_samples_on_device(mg_ctx *c, const mg_packed_batch *in, const mg_packed_dims *dm, int32_t *d_w) {
+  cudaStream_t st = c->stream[0];
+  const uint64_t nk = dm->n_kmers;
+  if (!nk) return MG_OK;
+  const mg::SampleView sv = sample_view(c);
+  const uint4 *km = (const uint4 *)in->kmers;
+  {
+    const uint64_t want = (nk + mg::LOOKUP_THREADS - 1) / mg::LOOKUP_THREADS, cap = (uint64_t)c->sms * 32;
+    const int grid = (int)(want < cap ? want : cap);
+    auto kernel = c->k == 35 ? mg::k_lookup_samples<35> : mg::k_lookup_samples<0>;
+    CU(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, mg::LOOKUP_SAMPLES_SMEM));
+    c->launches++;
+    kernel<<<grid, mg::LOOKUP_THREADS, mg::LOOKUP_SAMPLES_SMEM, st>>>(km, nk, c->view(), sv, d_w);
+    CU(cudaGetLastError());
+  }
+  if (in->n_irregular) {
+    c->launches++;
+    mg::k_lookup_samples_irr<<<grid_for(in->n_irregular, 128), 128, 0, st>>>(
+        (const uint8_t *)in->irr_pool, in->irr_off, in->irr_kmer, in->n_irregular, km, nk, c->view(), sv, d_w,
+        c->d_scalars);
+    CU(cudaGetLastError());
+  }
   return MG_OK;
 }
 
@@ -1085,22 +1200,30 @@ static int lookup_packed_on_device(mg_ctx *c, const mg_packed_batch *in, const m
   }
   return MG_OK;
 }
-// set_coverages + VB::genotype from the weights in d_w; out->lik == NULL: the likelihoods stay in library scratch
-static int genotype_from_weights(mg_ctx *c, const mg_packed_batch *in, const mg_genotype_out *out, const mg_packed_dims *dm,
-                                 const int32_t *d_w, double *d_lik, float error_rate, int max_coverage, int haploid) {
+// set_coverages + VB::genotype from the weights in d_w, for n_out output sets: set s reads the weights at d_w + s * n_kmers
+// (a sample set; the single-sample calls pass one).  A set whose lik is NULL has its likelihoods in scratch_lik.
+static int genotype_from_weights(mg_ctx *c, const mg_packed_batch *in, const mg_genotype_out *out, int n_out,
+                                 const mg_packed_dims *dm, const int32_t *d_w, double *scratch_lik, float error_rate,
+                                 int max_coverage, int haploid) {
   cudaStream_t st = c->stream[0];
   const uint64_t nv = dm->n_variants, na = dm->n_alleles;
-  const bool own_lik = out->lik == nullptr;
-  c->launches++;
-  mg::k_coverage<<<grid_for(na, 128), 128, 0, st>>>(d_w, in->sig_kmer_off, in->allele_sig_off, na, out->cov);
-  CU(cudaGetLastError());
+  for (int s = 0; s < n_out; ++s) {
+    c->launches++;
+    mg::k_coverage<<<grid_for(na, 128), 128, 0, st>>>(d_w + (uint64_t)s * dm->n_kmers, in->sig_kmer_off,
+                                                      in->allele_sig_off, na, out[s].cov);
+    CU(cudaGetLastError());
+  }
   CU(cudaEventRecord(c->ge[2], st));
-  if (own_lik) CU(cudaMemsetAsync(c->d_scalars + 5, 0, 8, st));
-  c->launches++;
-  mg::k_genotype<<<grid_for(nv, 128), 128, 0, st>>>(out->cov, in->freq, in->var_allele_off, own_lik ? nullptr : out->lik_off,
-                                                    c->d_scalars + 5, nv, error_rate, max_coverage, haploid, c->log_table,
-                                                    d_lik, out->n_gts, out->status, out->best_gt, out->gq);
-  CU(cudaGetLastError());
+  for (int s = 0; s < n_out; ++s) {
+    const bool own_lik = out[s].lik == nullptr;
+    if (own_lik) CU(cudaMemsetAsync(c->d_scalars + 5, 0, 8, st));
+    c->launches++;
+    mg::k_genotype<<<grid_for(nv, 128), 128, 0, st>>>(
+        out[s].cov, in->freq, in->var_allele_off, own_lik ? nullptr : out[s].lik_off, c->d_scalars + 5, nv, error_rate,
+        max_coverage, haploid, c->log_table, own_lik ? scratch_lik : out[s].lik, out[s].n_gts, out[s].status,
+        out[s].best_gt, out[s].gq);
+    CU(cudaGetLastError());
+  }
   CU(cudaEventRecord(c->ge[3], st));
   return MG_OK;
 }
@@ -1123,7 +1246,7 @@ static int genotype_packed_on_device(mg_ctx *c, const mg_packed_batch *in, const
   if (rc) return rc;
   CU(cudaEventRecord(c->ge[1], st));
   CU(cudaEventRecord(c->ge[4], st));
-  return genotype_from_weights(c, in, out, dm, d_w, d_lik, error_rate, max_coverage, haploid);
+  return genotype_from_weights(c, in, out, 1, dm, d_w, d_lik, error_rate, max_coverage, haploid);
 }
 
 // ---- the two halves on their own: replicas sum the LOOK-UP RESULTS of a batch instead of their counters ----
@@ -1168,7 +1291,7 @@ extern "C" int mg_genotype_weights_device(mg_ctx *c, const mg_packed_batch *in, 
                                                                             reinterpret_cast<int32_t *>(d_weights));
     CU(cudaGetLastError());
   }
-  return genotype_from_weights(c, in, out, dims, reinterpret_cast<const int32_t *>(d_weights),
+  return genotype_from_weights(c, in, out, 1, dims, reinterpret_cast<const int32_t *>(d_weights),
                                own_lik ? reinterpret_cast<double *>(c->geno_scratch) : out->lik, error_rate, max_coverage,
                                haploid);
 }
@@ -1207,16 +1330,22 @@ extern "C" int mg_genotype_packed_device(mg_ctx *c, const mg_packed_batch *in, c
   return genotype_packed_on_device(c, in, out, dims, error_rate, max_coverage, haploid);
 }
 
-extern "C" int mg_genotype_packed(mg_ctx *c, const mg_packed_batch *in, const mg_genotype_out *out, float error_rate,
-                                  int max_coverage, int haploid) {
-  if (!c || !in || !out) return set_err(MG_ERR_ARG, "NULL argument");
-  if (!c->alt_final) return set_err(MG_ERR_STATE, "mg_genotype_packed before mg_finalize_alt");
+static int lookup_samples_on_device(mg_ctx *c, const mg_packed_batch *in, const mg_packed_dims *dm, int32_t *d_w);
+
+// mg_genotype_packed and mg_genotype_samples_packed: the HOST batch goes into the grow-only device arena, is genotyped
+// for n_out output sets (one, or one per sample of the set: samples), and the results come back.  The likelihood
+// slots (out[0].lik_off) are the same for every set.
+static int genotype_packed_host(mg_ctx *c, const mg_packed_batch *in, const mg_genotype_out *out, int n_out,
+                                bool samples, float error_rate, int max_coverage, int haploid) {
   const uint64_t nv = in->n_variants;
   if (nv == 0) return MG_OK;
-  if (!in->var_allele_off || !in->allele_sig_off || !in->sig_kmer_off || !in->freq || !out->cov || !out->n_gts ||
-      !out->status || !out->best_gt || !out->gq || (out->lik && !out->lik_off) ||
+  if (!in->var_allele_off || !in->allele_sig_off || !in->sig_kmer_off || !in->freq ||
       (in->n_irregular && (!in->irr_off || !in->irr_pool || !in->irr_kmer)))
     return set_err(MG_ERR_ARG, "NULL array in batch");
+  for (int s = 0; s < n_out; ++s)
+    if (!out[s].cov || !out[s].n_gts || !out[s].status || !out[s].best_gt || !out[s].gq ||
+        (out[s].lik && !out[s].lik_off) || (out[s].lik == nullptr) != (out[0].lik == nullptr))
+      return set_err(MG_ERR_ARG, "NULL array in batch");
   CU(cudaSetDevice(c->device));
   mg_packed_dims dm;
   dm.n_variants = nv;
@@ -1227,13 +1356,14 @@ extern "C" int mg_genotype_packed(mg_ctx *c, const mg_packed_batch *in, const mg
   dm.lik_slots = out->lik ? out->lik_off[nv] : lik_slots_of(in->var_allele_off, nv, haploid);
   if (dm.n_kmers && !in->kmers) return set_err(MG_ERR_ARG, "NULL array in batch");
   const uint64_t na = dm.n_alleles, ns = dm.n_sigs, nk = dm.n_kmers, ni = in->n_irregular, nl = out->lik ? dm.lik_slots : 0;
+  const uint64_t g = (uint64_t)n_out;
   cudaStream_t st = c->stream[0];
   auto al = [](uint64_t x) { return (x + 255) & ~255ull; };
   const uint64_t o_vao = 0, o_aso = o_vao + al((nv + 1) * 4), o_sko = o_aso + al((na + 1) * 4),
                  o_km = o_sko + al((ns + 1) * 4), o_freq = o_km + al(nk * 16), o_io = o_freq + al(na * 4),
                  o_ip = o_io + al((ni + 1) * 8), o_ik = o_ip + al(dm.irr_pool_bytes), o_lo = o_ik + al(ni * 4),
-                 o_cov = o_lo + al(nl ? (nv + 1) * 8 : 0), o_i32 = o_cov + al(na * 4), o_lik = o_i32 + al(nv * 16),
-                 total = o_lik + al(nl * 8) + 256;
+                 o_cov = o_lo + al(nl ? (nv + 1) * 8 : 0), o_i32 = o_cov + g * al(na * 4), o_lik = o_i32 + g * al(nv * 16),
+                 total = o_lik + g * al(nl * 8) + 256;
   if (c->geno_arena_bytes < total) {  // grow-only device arena, reused across calls
     CU(cudaStreamSynchronize(st));
     cudaFree(c->geno_arena);
@@ -1265,25 +1395,63 @@ extern "C" int mg_genotype_packed(mg_ctx *c, const mg_packed_batch *in, const mg
   din.irr_off = reinterpret_cast<uint64_t *>(d + o_io);
   din.irr_pool = reinterpret_cast<const char *>(d + o_ip);
   din.irr_kmer = reinterpret_cast<uint32_t *>(d + o_ik);
-  mg_genotype_out dout;
-  int32_t *i32 = reinterpret_cast<int32_t *>(d + o_i32);
-  dout.cov = reinterpret_cast<uint32_t *>(d + o_cov);
-  dout.n_gts = i32;
-  dout.status = i32 + nv;
-  dout.best_gt = i32 + 2 * nv;
-  dout.gq = i32 + 3 * nv;
-  dout.lik_off = nl ? reinterpret_cast<uint64_t *>(d + o_lo) : nullptr;
-  dout.lik = nl ? reinterpret_cast<double *>(d + o_lik) : nullptr;
-  int rc = genotype_packed_on_device(c, &din, &dout, &dm, error_rate, max_coverage, haploid);
+  std::vector<mg_genotype_out> dout(n_out);
+  for (uint64_t s = 0; s < g; ++s) {
+    int32_t *i32 = reinterpret_cast<int32_t *>(d + o_i32 + s * al(nv * 16));
+    dout[s].cov = reinterpret_cast<uint32_t *>(d + o_cov + s * al(na * 4));
+    dout[s].n_gts = i32;
+    dout[s].status = i32 + nv;
+    dout[s].best_gt = i32 + 2 * nv;
+    dout[s].gq = i32 + 3 * nv;
+    dout[s].lik_off = nl ? reinterpret_cast<uint64_t *>(d + o_lo) : nullptr;
+    dout[s].lik = nl ? reinterpret_cast<double *>(d + o_lik + s * al(nl * 8)) : nullptr;
+  }
+  int rc;
+  if (!samples) {
+    rc = genotype_packed_on_device(c, &din, dout.data(), &dm, error_rate, max_coverage, haploid);
+  } else {  // one look-up for the whole set, then coverage + likelihoods per sample on its column of the weights
+    const uint64_t w_bytes = al((nk ? nk : 1) * 4 * g);
+    rc = geno_scratch(c, w_bytes + (nl ? 0 : dm.lik_slots * 8 + 256));
+    if (!rc) rc = join_streams(c);
+    if (!rc) rc = geno_events(c);
+    if (rc) return rc;
+    int32_t *d_w = reinterpret_cast<int32_t *>(c->geno_scratch);
+    CU(cudaEventRecord(c->ge[0], st));
+    rc = lookup_samples_on_device(c, &din, &dm, d_w);
+    if (rc) return rc;
+    CU(cudaEventRecord(c->ge[1], st));
+    CU(cudaEventRecord(c->ge[4], st));
+    rc = genotype_from_weights(c, &din, dout.data(), n_out, &dm, d_w,
+                               reinterpret_cast<double *>(reinterpret_cast<uint8_t *>(c->geno_scratch) + w_bytes),
+                               error_rate, max_coverage, haploid);
+  }
   if (rc) return rc;
-  CU(cudaMemcpyAsync(out->cov, dout.cov, na * 4, cudaMemcpyDeviceToHost, st));
-  CU(cudaMemcpyAsync(out->n_gts, dout.n_gts, nv * 4, cudaMemcpyDeviceToHost, st));
-  CU(cudaMemcpyAsync(out->status, dout.status, nv * 4, cudaMemcpyDeviceToHost, st));
-  CU(cudaMemcpyAsync(out->best_gt, dout.best_gt, nv * 4, cudaMemcpyDeviceToHost, st));
-  CU(cudaMemcpyAsync(out->gq, dout.gq, nv * 4, cudaMemcpyDeviceToHost, st));
-  if (nl) CU(cudaMemcpyAsync(out->lik, dout.lik, nl * 8, cudaMemcpyDeviceToHost, st));
+  for (int s = 0; s < n_out; ++s) {
+    CU(cudaMemcpyAsync(out[s].cov, dout[s].cov, na * 4, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(out[s].n_gts, dout[s].n_gts, nv * 4, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(out[s].status, dout[s].status, nv * 4, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(out[s].best_gt, dout[s].best_gt, nv * 4, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(out[s].gq, dout[s].gq, nv * 4, cudaMemcpyDeviceToHost, st));
+    if (nl) CU(cudaMemcpyAsync(out[s].lik, dout[s].lik, nl * 8, cudaMemcpyDeviceToHost, st));
+  }
   CU(cudaStreamSynchronize(st));
   return check_too_long(c);
+}
+
+extern "C" int mg_genotype_packed(mg_ctx *c, const mg_packed_batch *in, const mg_genotype_out *out, float error_rate,
+                                  int max_coverage, int haploid) {
+  if (!c || !in || !out) return set_err(MG_ERR_ARG, "NULL argument");
+  if (!c->alt_final) return set_err(MG_ERR_STATE, "mg_genotype_packed before mg_finalize_alt");
+  return genotype_packed_host(c, in, out, 1, false, error_rate, max_coverage, haploid);
+}
+
+extern "C" int mg_genotype_samples_packed(mg_ctx *c, const mg_packed_batch *in, const mg_genotype_out *out, int n_samples,
+                                          float error_rate, int max_coverage, int haploid) {
+  if (!c || !in || !out) return set_err(MG_ERR_ARG, "NULL argument");
+  if (!c->samples) return set_err(MG_ERR_STATE, "mg_genotype_samples_packed before mg_samples_begin");
+  if (n_samples != c->samples_g)
+    return set_err(MG_ERR_ARG, "%d output sets for a sample set of %d", n_samples, c->samples_g);
+  return genotype_packed_host(c, in, out, n_samples, true, error_rate, max_coverage, haploid);
 }
 
 // The reference-shaped batch (ASCII k-mers, u64 offsets), packed on the host into the batch of mg_genotype_packed by
@@ -1389,7 +1557,7 @@ extern "C" int mg_index_stats(mg_ctx *c, uint64_t *stats, int n) {
 extern "C" int mg_counter_buffers(mg_ctx *c, void **d_ptr, uint64_t *n) {
   if (!c || !d_ptr || !n) return set_err(MG_ERR_ARG, "NULL argument");
   if (!c->alt_final) return set_err(MG_ERR_STATE, "no counters before mg_finalize_alt");
-  if (!c->key_rank) return set_err(MG_ERR_STATE, "mg_counter_buffers before mg_counters_gather");
+  if (!c->key_dense) return set_err(MG_ERR_STATE, "mg_counter_buffers before mg_counters_gather");
   d_ptr[0] = c->bf_counts;
   n[0] = c->bf_ones;
   d_ptr[1] = c->key_dense;
