@@ -160,21 +160,58 @@ __device__ __forceinline__ int64_t ovf_find(const DevView &v, u128 canon) {
   }
 }
 
-// Where the count of canonical key `canon` (bf index idx) lives, or nullptr when the key is absent.
-__device__ __forceinline__ uint32_t *key_count_ptr(const DevView &v, uint64_t idx, u128 canon) {
-  const uint64_t line = idx >> 8;
-  const uint4 *p = v.lines + line * LINE_U4 + 2;
-  uint4 q[LINE_KEYS];
+// ---- What a probe line says about one k-mer: the decoder of every signature look-up.  `at(u)` returns uint4 u
+// (0..7) of the line: a row of a look-up's swizzled shared-memory tile, or the line in global memory (line_at). ----
+__device__ __forceinline__ auto line_at(const DevView &v, uint64_t line) {
+  const uint4 *p = v.lines + line * LINE_U4;
+  return [p](int u) { return __ldg(p + u); };
+}
+// Alt bit `bit` (0..255 inside the line): whether it is set.  *j = set bits below it in the line, *m = uint4 7 (the
+// rank and the counters of set bits 0..2).
+template <class At>
+__device__ __forceinline__ bool line_alt(At at, uint32_t bit, int *j, uint4 *m) {
+  const uint32_t ws = bit >> 5, below = (1u << (bit & 31u)) - 1u;
+  const uint4 b0 = at(0), b1 = at(1);
+  *m = at(7);
+  const uint32_t wx[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
+  uint32_t hit_w = 0;
+  int n = 0;
 #pragma unroll
-  for (int s = 0; s < LINE_KEYS; ++s) q[s] = __ldg(p + s);
+  for (uint32_t x = 0; x < 8; ++x) {
+    hit_w = x == ws ? wx[x] : hit_w;
+    n += __popc(wx[x] & (x < ws ? 0xFFFFFFFFu : (x == ws ? below : 0u)));
+  }
+  *j = n;
+  return (hit_w >> (bit & 31u)) & 1u;
+}
+// the inline key layout, for a look-up specialised for k = K (0: k of the view)
+template <int K>
+__device__ __forceinline__ bool inline_keys(const DevView &v) {
+  return K > 0 ? (K <= INLINE_MAX_K) : (v.inline_counts != 0);
+}
+// Ref key `canon`: the slot that holds it, or -1.  *w3 = word 3 of that slot (the count in the inline layout), *ovf =
+// the line's OVERFLOW flag.  One masked compare serves both layouts: mz / mw are key_of's key_hi_mask, constants when
+// K > 0.
+template <int K, class At>
+__device__ __forceinline__ int line_key(const DevView &v, At at, u128 canon, uint32_t *w3, bool *ovf) {
+  const bool inl = inline_keys<K>(v);
+  const uint32_t mz = inl ? 0x7FFFFFFFu : 0xFFFFFFFFu, mw = inl ? 0u : 0x3FFFFFFFu;
+  const uint32_t c0 = (uint32_t)canon.lo, c1 = (uint32_t)(canon.lo >> 32), c2 = (uint32_t)canon.hi,
+                 c3 = (uint32_t)(canon.hi >> 32);
+  int slot = -1;
+  uint32_t cnt_w = 0, flag_w = 0;
 #pragma unroll
-  for (int s = 0; s < LINE_KEYS; ++s)
-    if (key_eq(key_of(v, q[s]), canon))
-      return v.inline_counts ? line_words(v, line) + 8 + 4 * s + 3 : v.key_counts + line * LINE_KEYS + (uint64_t)s;
-  const uint64_t hi4 = (uint64_t)q[LINE_KEYS - 1].z | ((uint64_t)q[LINE_KEYS - 1].w << 32);
-  if (!(hi4 & v.ovf_flag_hi)) return nullptr;
-  const int64_t slot = ovf_find(v, canon);
-  return slot < 0 ? nullptr : v.ovf_counts + slot;
+  for (int s = 0; s < LINE_KEYS; ++s) {
+    const uint4 p = at(2 + s);
+    if (((p.x ^ c0) | (p.y ^ c1) | ((p.z ^ c2) & mz) | ((p.w ^ c3) & mw)) == 0) {
+      slot = s;
+      cnt_w = p.w;
+    }
+    if (s == LINE_KEYS - 1) flag_w = inl ? p.z : p.w;
+  }
+  *w3 = cnt_w;
+  *ovf = (flag_w >> 31) != 0;
+  return slot;
 }
 
 // insert into the five slots of a line; returns 1 = newly inserted, 0 = already present, -1 = line full

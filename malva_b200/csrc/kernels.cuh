@@ -2,10 +2,10 @@
 //   K3  k_add_signatures / k_add_packed / k_add_spill / k_line_popc    index-time inserts + switch_mode
 //   K2  k_refpass / k_refpass_short                                    reference rolling pass
 //   K1  k_scan / k_scan_hits                                           sample k-mer scan
-//   K4  k_lookup_packed / k_lookup / k_coverage                        coverage read-back
+//   K4  k_lookup_packed / k_lookup_irr / k_lookup / k_coverage         coverage read-back (one sample, or a sample set)
 //   K5  k_genotype                                                     likelihoods + posterior arg-max
 //       k_counters_xfer / k_sum_peers                                  dense counter image for the multi-GPU reduce
-//       k_samples_take_* / k_lookup_samples / k_lookup_samples_irr     sample sets: several samples on one index
+//       k_samples_take_*                                               sample sets: several samples on one index
 #pragma once
 #include <cuda_runtime.h>
 
@@ -899,180 +899,6 @@ __global__ void __launch_bounds__(256) k_scan_hits(const uint4 *__restrict__ hit
 }
 
 // ---------------------------------------------------------------------------
-// K4: signature look-ups (BF::get_count / KMAP::get_count) + coverage.  One probe line per look-up: the count of a
-// ref key is in its slot, the counter of an alt bit in words 29..31 of the line (index.cuh).
-// ---------------------------------------------------------------------------
-// Both read everything they may need from the probe line in ONE round of independent loads (the filter words, the
-// rank + inline counters; the five slots with their counts): a look-up is one memory round trip, not two.
-__device__ __forceinline__ int32_t alt_get_count(const DevView &v, uint64_t idx, bool raw = false) {  // BF::get_count (u16)
-  if (!v.bf_counts) return 0;  // write mode: no counters yet (bloom_filter.hpp:115-125)
-  const uint4 *p = v.lines + (idx >> 8) * LINE_U4;
-  const uint4 a = __ldg(p), b = __ldg(p + 1), m = __ldg(p + 7);
-  const uint32_t w[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
-  const uint32_t ws = (uint32_t)((idx & 255) >> 5), below = (1u << (idx & 31)) - 1u;
-  uint32_t mine = 0;
-  int j = 0;
-#pragma unroll
-  for (uint32_t x = 0; x < 8; ++x) {
-    mine = x == ws ? w[x] : mine;
-    j += __popc(w[x] & (x < ws ? 0xFFFFFFFFu : (x == ws ? below : 0u)));
-  }
-  if (!((mine >> (idx & 31)) & 1u)) return 0;
-  const uint32_t c = j == 0 ? m.y : (j == 1 ? m.z : (j == 2 ? m.w : __ldg(v.bf_counts + (uint64_t)m.x + (uint64_t)j)));
-  return raw ? (int32_t)c : (int32_t)(c & 0xFFFFu);
-}
-__device__ __forceinline__ int32_t ref_get_count(const DevView &v, uint64_t idx, u128 canon) {  // KMAP::get_count
-  const uint64_t line = idx >> 8;
-  const uint4 *p = v.lines + line * LINE_U4 + 2;
-  uint4 q[LINE_KEYS];
-#pragma unroll
-  for (int s = 0; s < LINE_KEYS; ++s) q[s] = __ldg(p + s);
-#pragma unroll
-  for (int s = 0; s < LINE_KEYS; ++s)
-    if (key_eq(key_of(v, q[s]), canon))
-      return v.inline_counts ? (int32_t)q[s].w : (int32_t)__ldg(v.key_counts + line * LINE_KEYS + (uint64_t)s);
-  if (!(u128_of(q[LINE_KEYS - 1]).hi & v.ovf_flag_hi)) return 0;
-  const int64_t slot = ovf_find(v, canon);
-  return slot < 0 ? 0 : (int32_t)__ldg(v.ovf_counts + slot);
-}
-
-// mode 0: get_count  (is_ref selects KMAP/BF, out = int32 count)
-// mode 1: test_key on filter/table `which` (0 bf, 1 context_bf, 2 ref_bf; out = 0/1, -1 = irregular KMAP key)
-// out_pos != nullptr: k-mer i is written to out[out_pos[i]] and its is_ref flag is bit 62 of packed[out_pos[i]].hi
-// (the irregular k-mers of a packed batch)
-__global__ void __launch_bounds__(128) k_lookup(const uint8_t *__restrict__ pool, const uint64_t *__restrict__ off,
-                                               const uint8_t *__restrict__ is_ref, uint64_t n, DevView v, int mode,
-                                               int which, int32_t *__restrict__ out, unsigned long long *scalars,
-                                               const uint32_t *__restrict__ out_pos, const uint4 *__restrict__ packed,
-                                               bool raw = false) {
-  uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  const uint64_t o = out_pos ? (uint64_t)out_pos[i] : i;
-  uint64_t b = off[i], e = off[i + 1];
-  int len = (int)(e - b);
-  if (len > 128) {
-    atomicExch(&scalars[3], 1ull);
-    out[o] = 0;
-    return;
-  }
-  uint8_t s[128];
-  for (int j = 0; j < len; ++j) s[j] = pool[b + j];
-  const bool ref_flag = out_pos ? ((packed[o].w >> 30) & 1u) != 0 : (is_ref && is_ref[i] != 0);
-  bool use_table = mode == 0 ? ref_flag : (which == 2);
-  u128 x, canon;
-  if (use_table) {
-    if (!pack_ascii(s, len, v.k, &x)) {
-      out[o] = (mode == 1) ? -1 : 0;  // irregular keys are resolved on the host (always count 0)
-      return;
-    }
-    uint64_t h = canon_hash_rt(x, v.k, &canon);
-    const uint32_t *cp = key_count_ptr(v, bf_index(v, h), canon);
-    if (mode == 1)
-      out[o] = cp != nullptr;
-    else
-      out[o] = cp ? (int32_t)*cp : 0;
-    return;
-  }
-  // a Bloom filter: hash the canonical ASCII bytes of whatever length was given
-  bool regular = len >= 1 && len <= 64 && pack_ascii(s, len, len, &x);
-  uint64_t h = regular ? canon_hash_rt(x, len, &canon) : hash_ascii(s, len);
-  uint64_t idx = bf_index(v, h);
-  if (mode == 1)
-    out[o] = which == 1 ? ctx_test(v, idx) : bf_test(v, idx);
-  else
-    out[o] = alt_get_count(v, idx, raw);
-}
-
-// Packed signature k-mers (exactly k symbols of ACGT, the form the host enumerator emits): {lo, hi} words;
-// hi bit 62 = k-mer of allele slot 0 (looked up in ref_bf), hi bit 63 = irregular (not k x ACGT: resolved by k_lookup
-// from the side pool).  16 bytes in, 4 bytes out, one probe line per k-mer.
-// A warp takes 32 k-mers at a time: every lane hashes one, then the 32 probe lines are gathered into the warp's
-// 4 KB shared-memory tile exactly like a round of the sample scan (eight LDGSTS rounds, four whole lines each, the
-// line of row L announced by a shuffle), and every lane reads its own row.  One thread fetching its line by itself
-// -- five 16-byte loads for a ref key, three for an alt bit -- cost five (three) L1 tag look-ups per line and ran at
-// 45 % of the device's random-line rate with the load queues full (ncu, profiles/round2_k4.md).
-constexpr int LOOKUP_THREADS = 256;
-constexpr int LOOKUP_SMEM = (LOOKUP_THREADS / 32) * 4096;
-
-// RAW: bf counters are returned as the u32 accumulators they are (partial results of replicas are summed first, the
-// u16 wrap of int_vector<16> is applied to the sum: k_mask_alt)
-template <int K, bool RAW>
-__global__ void __launch_bounds__(LOOKUP_THREADS) k_lookup_packed(const uint4 *__restrict__ kmers, uint64_t n, DevView v,
-                                                                 int32_t *__restrict__ out) {
-  extern __shared__ uint4 lk_sm[];
-  const int lane = threadIdx.x & 31, sub = lane & 7, grp = lane >> 3;
-  uint4 *tile = lk_sm + (threadIdx.x >> 5) * 256;
-  const uint32_t tile_addr = (uint32_t)__cvta_generic_to_shared(tile);
-  const uint32_t d_even = tile_addr + (uint32_t)(grp * 128 + ((sub ^ grp) * 16));
-  const uint32_t d_odd = tile_addr + (uint32_t)(grp * 128 + ((sub ^ (grp + 4)) * 16));
-  const char *line_src = reinterpret_cast<const char *>(v.lines) + sub * 16;
-  const int k = K > 0 ? K : v.k;
-  const bool inl = K > 0 ? (K <= INLINE_MAX_K) : (v.inline_counts != 0);
-  const uint32_t mz = inl ? 0x7FFFFFFFu : 0xFFFFFFFFu, mw = inl ? 0u : 0x3FFFFFFFu;
-  const uint64_t warp0 = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = ((uint64_t)gridDim.x * blockDim.x) >> 5;
-  for (uint64_t base = warp0 * 32; base < n; base += n_warps * 32) {
-    const uint64_t i = base + (uint64_t)lane;
-    const uint4 q = i < n ? __ldg(kmers + i) : make_uint4(0, 0, 0, 0x80000000u);
-    const bool active = !(q.w >> 31);  // (past the end, or irregular: nothing to fetch)
-    const bool is_ref = (q.w >> 30) & 1u;
-    u128 canon;
-    const uint64_t h = canon_hash_k<K>(mask128(u128_of(q), 2 * k), k, &canon);
-    const uint64_t idx = bf_index(v, h);
-    const uint32_t line = (uint32_t)(idx >> 8), bit = (uint32_t)(idx & 255);
-    const uint32_t act = __ballot_sync(0xffffffffu, active);
-    __syncwarp();  // the previous batch's reads of the tile are done
-#pragma unroll
-    for (int r = 0; r < 8; ++r) {
-      const uint32_t lid = __shfl_sync(0xffffffffu, line, 4 * r + grp);
-      if ((act >> (4 * r + grp)) & 1u)
-        cp_async16(((r & 1) ? d_odd : d_even) + (uint32_t)(r * 512), line_src + ((uint64_t)lid << 7));
-    }
-    asm volatile("cp.async.commit_group;\ncp.async.wait_group 0;\n" ::: "memory");
-    __syncwarp();
-    if (!active) continue;
-    const uint4 *mine = tile + lane * 8;
-    const int sw = lane & 7;
-    int32_t res = 0;
-    if (is_ref) {  // KMAP::get_count: the count sits in the slot that holds the key
-      const uint32_t c0 = (uint32_t)canon.lo, c1 = (uint32_t)(canon.lo >> 32), c2 = (uint32_t)canon.hi,
-                     c3 = (uint32_t)(canon.hi >> 32);
-      int slot = -1;
-      uint32_t cnt_w = 0, flag_w = 0;
-#pragma unroll
-      for (int s = 0; s < LINE_KEYS; ++s) {
-        const uint4 p = mine[(2 + s) ^ sw];
-        if (((p.x ^ c0) | (p.y ^ c1) | ((p.z ^ c2) & mz) | ((p.w ^ c3) & mw)) == 0) {
-          slot = s;
-          cnt_w = p.w;
-        }
-        if (s == LINE_KEYS - 1) flag_w = inl ? p.z : p.w;
-      }
-      if (slot >= 0) {
-        res = inl ? (int32_t)cnt_w : (int32_t)__ldg(v.key_counts + (uint64_t)line * LINE_KEYS + (uint32_t)slot);
-      } else if (flag_w >> 31) {
-        const int64_t os = ovf_find(v, canon);
-        if (os >= 0) res = (int32_t)__ldg(v.ovf_counts + os);
-      }
-    } else if (v.bf_counts) {  // BF::get_count (u16); no counters before switch_mode
-      const uint32_t ws = bit >> 5, below = (1u << (bit & 31u)) - 1u;
-      const uint4 b0 = mine[0 ^ sw], b1 = mine[1 ^ sw], m = mine[7 ^ sw];
-      const uint32_t wx[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
-      uint32_t hit_w = 0;
-      int j = 0;
-#pragma unroll
-      for (uint32_t x = 0; x < 8; ++x) {
-        hit_w = x == ws ? wx[x] : hit_w;
-        j += __popc(wx[x] & (x < ws ? 0xFFFFFFFFu : (x == ws ? below : 0u)));
-      }
-      if ((hit_w >> (bit & 31u)) & 1u) {
-        const uint32_t c = j == 0 ? m.y : (j == 1 ? m.z : (j == 2 ? m.w : __ldg(v.bf_counts + (uint64_t)m.x + (uint64_t)j)));
-        res = RAW ? (int32_t)c : (int32_t)(c & 0xFFFFu);
-      }
-    }
-    out[i] = res;
-  }
-}
-// ---------------------------------------------------------------------------
 // Sample sets (include/malva_gpu.h, mg_samples_*): the counters of up to 32 samples side by side.  Every counter a
 // signature k-mer can read has a ROW that depends on the index only:
 //   [0, bf_ones)                    a set bit of bf: its rank + j                     (BF::get_count)
@@ -1134,68 +960,162 @@ __global__ void __launch_bounds__(256) k_samples_take_lines(DevView v, SampleVie
   }
 }
 
-// row of a set bit of bf (bf index idx), or NO_ROW when the bit is clear
-__device__ __forceinline__ uint32_t alt_row(const DevView &v, uint64_t idx) {
-  const uint4 *p = v.lines + (idx >> 8) * LINE_U4;
-  const uint4 a = __ldg(p), b = __ldg(p + 1), m = __ldg(p + 7);
-  const uint32_t w[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
-  const uint32_t ws = (uint32_t)((idx & 255) >> 5), below = (1u << (idx & 31)) - 1u;
-  uint32_t mine = 0, j = 0;
-#pragma unroll
-  for (uint32_t x = 0; x < 8; ++x) {
-    mine = x == ws ? w[x] : mine;
-    j += (uint32_t)__popc(w[x] & (x < ws ? 0xFFFFFFFFu : (x == ws ? below : 0u)));
-  }
-  return ((mine >> (idx & 31)) & 1u) ? m.x + j : NO_ROW;
+// ---------------------------------------------------------------------------
+// K4: signature look-ups (BF::get_count / KMAP::get_count) + coverage.  One probe line per look-up: the count of a
+// ref key is in its slot, the counter of an alt bit in words 29..31 of the line (index.cuh).  Every look-up decodes
+// the line with line_alt / line_key (index.cuh) and ends in one of the four readers below: a count, or a ROW of a
+// sample set.
+// ---------------------------------------------------------------------------
+// BF::get_count (u16; RAW: the u32 accumulator, for replicas that sum their look-ups first)
+template <bool RAW, class At>
+__device__ __forceinline__ int32_t alt_count(const DevView &v, At at, uint32_t bit) {
+  if (!v.bf_counts) return 0;  // write mode: no counters yet (bloom_filter.hpp:115-125)
+  int j;
+  uint4 m;
+  if (!line_alt(at, bit, &j, &m)) return 0;
+  const uint32_t c = j == 0 ? m.y : (j == 1 ? m.z : (j == 2 ? m.w : __ldg(v.bf_counts + (uint64_t)m.x + (uint64_t)j)));
+  return RAW ? (int32_t)c : (int32_t)(c & 0xFFFFu);
 }
-// row of ref key `canon` (bf index idx), or NO_ROW when the key is absent
-__device__ __forceinline__ uint32_t key_row(const DevView &v, const SampleView &sv, uint64_t idx, u128 canon) {
-  const uint64_t line = idx >> 8;
-  const uint4 *p = v.lines + line * LINE_U4 + 2;
-  uint4 q[LINE_KEYS];
-#pragma unroll
-  for (int s = 0; s < LINE_KEYS; ++s) q[s] = __ldg(p + s);
-#pragma unroll
-  for (int s = 0; s < LINE_KEYS; ++s)
-    if (key_eq(key_of(v, q[s]), canon)) return (uint32_t)(sv.key_base + __ldg(sv.key_rank + line) + (uint64_t)s);
-  if (!(u128_of(q[LINE_KEYS - 1]).hi & v.ovf_flag_hi)) return NO_ROW;
-  const int64_t slot = ovf_find(v, canon);
-  return slot < 0 ? NO_ROW : (uint32_t)(sv.ovf_base + (uint64_t)slot);
+template <class At>
+__device__ __forceinline__ uint32_t alt_row(At at, uint32_t bit) {
+  int j;
+  uint4 m;
+  return line_alt(at, bit, &j, &m) ? m.x + (uint32_t)j : NO_ROW;
+}
+// KMAP::get_count of ref key `canon`, whose bf index lies in probe line `line`
+template <int K, class At>
+__device__ __forceinline__ int32_t key_count(const DevView &v, At at, uint64_t line, u128 canon) {
+  uint32_t w3;
+  bool ovf;
+  const int slot = line_key<K>(v, at, canon, &w3, &ovf);
+  if (slot >= 0) return inline_keys<K>(v) ? (int32_t)w3 : (int32_t)__ldg(v.key_counts + line * LINE_KEYS + (uint32_t)slot);
+  if (!ovf) return 0;
+  const int64_t os = ovf_find(v, canon);
+  return os < 0 ? 0 : (int32_t)__ldg(v.ovf_counts + os);
+}
+template <int K, class At>
+__device__ __forceinline__ uint32_t key_row(const DevView &v, const SampleView &sv, At at, uint64_t line, u128 canon) {
+  uint32_t w3;
+  bool ovf;
+  const int slot = line_key<K>(v, at, canon, &w3, &ovf);
+  if (slot >= 0) return (uint32_t)(sv.key_base + __ldg(sv.key_rank + line) + (uint32_t)slot);
+  if (!ovf) return NO_ROW;
+  const int64_t os = ovf_find(v, canon);
+  return os < 0 ? NO_ROW : (uint32_t)(sv.ovf_base + (uint64_t)os);
+}
+// the weight of sample s at counter row `row` (NO_ROW, or s past the set: 0): KMAP::get_count's int for a ref key,
+// BF::get_count's uint16_t otherwise
+__device__ __forceinline__ int32_t sample_weight(const SampleView &sv, uint32_t row, int s, bool ref) {
+  const uint32_t c = row != NO_ROW && s < sv.g ? __ldg(sv.mat + (uint64_t)row * (uint64_t)sv.g + (uint64_t)s) : 0u;
+  return (int32_t)(ref ? c : (c & 0xFFFFu));
 }
 
-// The look-up of k_lookup_packed for a whole sample set: every lane resolves the ROW of its k-mer from the probe line
-// (same tile, same gather), then the warp reads the 32 rows one after the other with the lanes on the samples (one
-// coalesced line per k-mer), transposes them through shared memory and writes the weights sample-major,
-// out[s * n + i], 128 bytes per store.  bf weights are BF::get_count's uint16_t, ref weights KMAP::get_count's int.
-// Irregular k-mers get 0 here; k_lookup_samples_irr writes them afterwards.
-constexpr int LOOKUP_SAMPLES_SMEM = LOOKUP_SMEM + (LOOKUP_THREADS / 32) * 32 * 33 * 4;
-template <int K>
-__global__ void __launch_bounds__(LOOKUP_THREADS) k_lookup_samples(const uint4 *__restrict__ kmers, uint64_t n, DevView v,
-                                                                  SampleView sv, int32_t *__restrict__ out) {
+// k-mer i of an ASCII pool (any length, any symbols), resolved byte-exactly as the reference does: a ref key (KMAP)
+// must be exactly k symbols of ACGT; the Bloom filters hash the canonical ASCII bytes of whatever length was given
+// (BF::_get_hash).  Returns 1 with *idx = the bf index (and *canon = the canonical key of a ref key), -1 for a ref key
+// that is not k x ACGT (never in the device map: the host keeps those), 0 for a k-mer longer than 128 bytes (flagged
+// in scalars[3]).
+__device__ __forceinline__ int ascii_kmer(const uint8_t *__restrict__ pool, const uint64_t *__restrict__ off, uint64_t i,
+                                          bool ref, const DevView &v, unsigned long long *scalars, uint64_t *idx,
+                                          u128 *canon) {
+  const uint64_t b = off[i];
+  const int len = (int)(off[i + 1] - b);
+  if (len > 128) {
+    atomicExch(&scalars[3], 1ull);
+    return 0;
+  }
+  uint8_t s[128];
+  for (int j = 0; j < len; ++j) s[j] = pool[b + j];
+  u128 x;
+  uint64_t h;
+  if (ref) {
+    if (!pack_ascii(s, len, v.k, &x)) return -1;
+    h = canon_hash_rt(x, v.k, canon);
+  } else {
+    const bool regular = len >= 1 && len <= 64 && pack_ascii(s, len, len, &x);
+    h = regular ? canon_hash_rt(x, len, canon) : hash_ascii(s, len);
+  }
+  *idx = bf_index(v, h);
+  return 1;
+}
+
+// The ASCII look-ups of mg_get_counts and mg_test_keys:
+// mode 0: get_count  (is_ref selects KMAP/BF, out = int32 count)
+// mode 1: test_key on filter/table `which` (0 bf, 1 context_bf, 2 ref_bf; out = 0/1, -1 = irregular KMAP key)
+__global__ void __launch_bounds__(128) k_lookup(const uint8_t *__restrict__ pool, const uint64_t *__restrict__ off,
+                                               const uint8_t *__restrict__ is_ref, uint64_t n, DevView v, int mode,
+                                               int which, int32_t *__restrict__ out, unsigned long long *scalars) {
+  uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const bool use_table = mode == 0 ? (is_ref && is_ref[i] != 0) : (which == 2);
+  uint64_t idx = 0;
+  u128 canon;
+  const int r = ascii_kmer(pool, off, i, use_table, v, scalars, &idx, &canon);
+  if (r <= 0) {
+    out[i] = (mode == 1 && r < 0) ? -1 : 0;  // irregular keys are resolved on the host (always count 0)
+    return;
+  }
+  const uint64_t line = idx >> 8;
+  const auto at = line_at(v, line);
+  if (use_table && mode == 0) {
+    out[i] = key_count<0>(v, at, line, canon);
+  } else if (use_table) {
+    uint32_t w3;
+    bool ovf;
+    out[i] = line_key<0>(v, at, canon, &w3, &ovf) >= 0 || (ovf && ovf_find(v, canon) >= 0);
+  } else if (mode == 1) {
+    out[i] = which == 1 ? ctx_test(v, idx) : bf_test(v, idx);
+  } else {
+    out[i] = alt_count<false>(v, at, (uint32_t)(idx & 255));
+  }
+}
+
+// What a look-up of a packed batch writes per k-mer: BF::get_count / KMAP::get_count (COUNT); the same with the bf
+// counters as the u32 accumulators they are (RAW: partial results of replicas are summed first, the u16 wrap of
+// int_vector<16> is applied to the sum: k_mask_alt); or the weights of every sample of the sample set, sample-major,
+// out[s * n + i] (SAMPLES).
+enum LookupOut { OUT_COUNT, OUT_RAW, OUT_SAMPLES };
+
+// Packed signature k-mers (exactly k symbols of ACGT, the form the host enumerator emits): {lo, hi} words;
+// hi bit 62 = k-mer of allele slot 0 (looked up in ref_bf), hi bit 63 = irregular (not k x ACGT: resolved by
+// k_lookup_irr from the side pool).  16 bytes in, 4 bytes out, one probe line per k-mer.
+// A warp takes 32 k-mers at a time: every lane hashes one, then the 32 probe lines are gathered into the warp's
+// 4 KB shared-memory tile exactly like a round of the sample scan (eight LDGSTS rounds, four whole lines each, the
+// line of row L announced by a shuffle), and every lane reads its own row.  One thread fetching its line by itself
+// -- five 16-byte loads for a ref key, three for an alt bit -- cost five (three) L1 tag look-ups per line and ran at
+// 45 % of the device's random-line rate with the load queues full (ncu, profiles/round2_k4.md).
+// SAMPLES: every lane resolves the ROW of its k-mer instead, then the warp reads the 32 rows one after the other with
+// the lanes on the samples (one coalesced line per k-mer), transposes them through shared memory and writes 128 bytes
+// per store.
+constexpr int LOOKUP_THREADS = 256;
+constexpr int LOOKUP_SMEM = (LOOKUP_THREADS / 32) * 4096;
+__host__ __device__ constexpr int lookup_smem(int out) {  // + the 32 x 33 transposition buffer of every warp
+  return LOOKUP_SMEM + (out == OUT_SAMPLES ? (LOOKUP_THREADS / 32) * 32 * 33 * 4 : 0);
+}
+
+template <int K, int OUT>
+__global__ void __launch_bounds__(LOOKUP_THREADS) k_lookup_packed(const uint4 *__restrict__ kmers, uint64_t n, DevView v,
+                                                                 int32_t *__restrict__ out, SampleView sv) {
   extern __shared__ uint4 lk_sm[];
-  const int lane = threadIdx.x & 31, sub = lane & 7, grp = lane >> 3, wid = threadIdx.x >> 5;
-  uint4 *tile = lk_sm + wid * 256;
-  uint32_t *tr = reinterpret_cast<uint32_t *>(lk_sm + (LOOKUP_THREADS / 32) * 256) + wid * 32 * 33;
+  const int lane = threadIdx.x & 31, sub = lane & 7, grp = lane >> 3;
+  uint4 *tile = lk_sm + (threadIdx.x >> 5) * 256;
   const uint32_t tile_addr = (uint32_t)__cvta_generic_to_shared(tile);
   const uint32_t d_even = tile_addr + (uint32_t)(grp * 128 + ((sub ^ grp) * 16));
   const uint32_t d_odd = tile_addr + (uint32_t)(grp * 128 + ((sub ^ (grp + 4)) * 16));
   const char *line_src = reinterpret_cast<const char *>(v.lines) + sub * 16;
   const int k = K > 0 ? K : v.k;
-  const bool inl = K > 0 ? (K <= INLINE_MAX_K) : (v.inline_counts != 0);
-  const uint32_t mz = inl ? 0x7FFFFFFFu : 0xFFFFFFFFu, mw = inl ? 0u : 0x3FFFFFFFu;
-  const int g = sv.g;
   const uint64_t warp0 = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = ((uint64_t)gridDim.x * blockDim.x) >> 5;
   for (uint64_t base = warp0 * 32; base < n; base += n_warps * 32) {
     const uint64_t i = base + (uint64_t)lane;
     const uint4 q = i < n ? __ldg(kmers + i) : make_uint4(0, 0, 0, 0x80000000u);
-    const bool active = !(q.w >> 31);
+    const bool active = !(q.w >> 31);  // (past the end, or irregular: nothing to fetch)
     const bool is_ref = (q.w >> 30) & 1u;
     u128 canon;
     const uint64_t h = canon_hash_k<K>(mask128(u128_of(q), 2 * k), k, &canon);
     const uint64_t idx = bf_index(v, h);
     const uint32_t line = (uint32_t)(idx >> 8), bit = (uint32_t)(idx & 255);
-    const uint32_t act = __ballot_sync(0xffffffffu, active), refs = __ballot_sync(0xffffffffu, is_ref);
-    __syncwarp();  // the previous batch's reads of the tile and of the transposition buffer are done
+    const uint32_t act = __ballot_sync(0xffffffffu, active);
+    __syncwarp();  // the previous batch's reads of the tile (and of the transposition buffer) are done
 #pragma unroll
     for (int r = 0; r < 8; ++r) {
       const uint32_t lid = __shfl_sync(0xffffffffu, line, 4 * r + grp);
@@ -1204,88 +1124,49 @@ __global__ void __launch_bounds__(LOOKUP_THREADS) k_lookup_samples(const uint4 *
     }
     asm volatile("cp.async.commit_group;\ncp.async.wait_group 0;\n" ::: "memory");
     __syncwarp();
-    uint32_t row = NO_ROW;
-    if (active) {
-      const uint4 *mine = tile + lane * 8;
-      const int sw = lane & 7;
-      if (is_ref) {
-        const uint32_t c0 = (uint32_t)canon.lo, c1 = (uint32_t)(canon.lo >> 32), c2 = (uint32_t)canon.hi,
-                       c3 = (uint32_t)(canon.hi >> 32);
-        int slot = -1;
-        uint32_t flag_w = 0;
-#pragma unroll
-        for (int s = 0; s < LINE_KEYS; ++s) {
-          const uint4 p = mine[(2 + s) ^ sw];
-          if (((p.x ^ c0) | (p.y ^ c1) | ((p.z ^ c2) & mz) | ((p.w ^ c3) & mw)) == 0) slot = s;
-          if (s == LINE_KEYS - 1) flag_w = inl ? p.z : p.w;
-        }
-        if (slot >= 0) {
-          row = (uint32_t)(sv.key_base + __ldg(sv.key_rank + line) + (uint32_t)slot);
-        } else if (flag_w >> 31) {
-          const int64_t os = ovf_find(v, canon);
-          if (os >= 0) row = (uint32_t)(sv.ovf_base + (uint64_t)os);
-        }
-      } else {
-        const uint32_t ws = bit >> 5, below = (1u << (bit & 31u)) - 1u;
-        const uint4 b0 = mine[0 ^ sw], b1 = mine[1 ^ sw], m = mine[7 ^ sw];
-        const uint32_t wx[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
-        uint32_t hit_w = 0, j = 0;
-#pragma unroll
-        for (uint32_t x = 0; x < 8; ++x) {
-          hit_w = x == ws ? wx[x] : hit_w;
-          j += (uint32_t)__popc(wx[x] & (x < ws ? 0xFFFFFFFFu : (x == ws ? below : 0u)));
-        }
-        if ((hit_w >> (bit & 31u)) & 1u) row = m.x + j;
-      }
-    }
-    // the counts of the 32 rows, lanes = samples
+    const uint4 *mine = tile + lane * 8;
+    const int sw = lane & 7;
+    const auto at = [mine, sw](int u) { return mine[u ^ sw]; };
+    if constexpr (OUT != OUT_SAMPLES) {
+      if (!active) continue;
+      out[i] = is_ref ? key_count<K>(v, at, line, canon) : alt_count<OUT == OUT_RAW>(v, at, bit);
+    } else {
+      const uint32_t row = !active ? NO_ROW : (is_ref ? key_row<K>(v, sv, at, line, canon) : alt_row(at, bit));
+      const uint32_t refs = __ballot_sync(0xffffffffu, is_ref);
+      uint32_t *tr = reinterpret_cast<uint32_t *>(lk_sm + (LOOKUP_THREADS / 32) * 256) + (threadIdx.x >> 5) * 32 * 33;
 #pragma unroll 8
-    for (int r = 0; r < 32; ++r) {
-      const uint32_t rr = __shfl_sync(0xffffffffu, row, r);
-      uint32_t c = 0;
-      if (rr != NO_ROW && lane < g) c = __ldg(sv.mat + (uint64_t)rr * (uint64_t)g + (uint64_t)lane);
-      tr[r * 33 + lane] = ((refs >> r) & 1u) ? c : (c & 0xFFFFu);
+      for (int r = 0; r < 32; ++r)  // the counts of the 32 rows, lanes = samples
+        tr[r * 33 + lane] = (uint32_t)sample_weight(sv, __shfl_sync(0xffffffffu, row, r), lane, (refs >> r) & 1u);
+      __syncwarp();
+      if (i < n)
+        for (int s = 0; s < sv.g; ++s) out[(uint64_t)s * n + i] = (int32_t)tr[lane * 33 + s];
     }
-    __syncwarp();
-    if (i < n)
-      for (int s = 0; s < g; ++s) out[(uint64_t)s * n + i] = (int32_t)tr[lane * 33 + s];
   }
 }
-// the irregular k-mers of a sample-set look-up (not k symbols of ACGT): k_lookup's byte-exact ASCII path, resolved to
-// a row instead of a count -- an irregular alt k-mer can hit a set bit of bf; an irregular ref key is never in the
-// device map and counts 0.  out[s * n + irr_kmer[j]] for every sample s.
-__global__ void __launch_bounds__(128) k_lookup_samples_irr(const uint8_t *__restrict__ pool, const uint64_t *__restrict__ off,
-                                                           const uint32_t *__restrict__ irr_kmer, uint64_t n_irr,
-                                                           const uint4 *__restrict__ packed, uint64_t n, DevView v,
-                                                           SampleView sv, int32_t *__restrict__ out,
-                                                           unsigned long long *scalars) {
-  const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n_irr) return;
-  const uint64_t o = irr_kmer[i];
-  const uint64_t b = off[i];
-  const int len = (int)(off[i + 1] - b);
-  const bool ref_flag = ((packed[o].w >> 30) & 1u) != 0;
-  uint32_t row = NO_ROW;
-  if (len > 128) {
-    atomicExch(&scalars[3], 1ull);
+
+// The irregular k-mers of a packed batch: k-mer j of the side pool is k-mer irr_kmer[j] of the batch (whose bit 62
+// says ref or alt), resolved byte-exactly; written where k_lookup_packed, with the same OUT, writes that k-mer.  An
+// irregular alt k-mer can hit a set bit of bf; an irregular ref key is never in the device map and counts 0.
+template <int OUT>
+__global__ void __launch_bounds__(128) k_lookup_irr(const uint8_t *__restrict__ pool, const uint64_t *__restrict__ off,
+                                                   const uint32_t *__restrict__ irr_kmer, uint64_t n_irr,
+                                                   const uint4 *__restrict__ kmers, uint64_t n, DevView v,
+                                                   int32_t *__restrict__ out, SampleView sv, unsigned long long *scalars) {
+  const uint64_t j = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= n_irr) return;
+  const uint64_t i = irr_kmer[j];
+  const bool ref = ((kmers[i].w >> 30) & 1u) != 0;
+  uint64_t idx = 0;
+  u128 canon;
+  const bool found = ascii_kmer(pool, off, j, ref, v, scalars, &idx, &canon) > 0;
+  const uint64_t line = idx >> 8;
+  const uint32_t bit = (uint32_t)(idx & 255);
+  const auto at = line_at(v, line);
+  if constexpr (OUT != OUT_SAMPLES) {
+    out[i] = !found ? 0 : (ref ? key_count<0>(v, at, line, canon) : alt_count<OUT == OUT_RAW>(v, at, bit));
   } else {
-    uint8_t s[128];
-    for (int j = 0; j < len; ++j) s[j] = pool[b + j];
-    u128 x, canon;
-    if (ref_flag) {
-      if (pack_ascii(s, len, v.k, &x)) {
-        const uint64_t h = canon_hash_rt(x, v.k, &canon);
-        row = key_row(v, sv, bf_index(v, h), canon);
-      }
-    } else {
-      const bool regular = len >= 1 && len <= 64 && pack_ascii(s, len, len, &x);
-      const uint64_t h = regular ? canon_hash_rt(x, len, &canon) : hash_ascii(s, len);
-      row = alt_row(v, bf_index(v, h));
-    }
-  }
-  for (int c = 0; c < sv.g; ++c) {
-    const uint32_t cnt = row == NO_ROW ? 0u : __ldg(sv.mat + (uint64_t)row * (uint64_t)sv.g + (uint64_t)c);
-    out[(uint64_t)c * n + o] = (int32_t)(ref_flag ? cnt : (cnt & 0xFFFFu));
+    const uint32_t row = !found ? NO_ROW : (ref ? key_row<0>(v, sv, at, line, canon) : alt_row(at, bit));
+    for (int s = 0; s < sv.g; ++s) out[(uint64_t)s * n + i] = sample_weight(sv, row, s, ref);
   }
 }
 

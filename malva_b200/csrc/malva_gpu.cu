@@ -124,8 +124,7 @@ struct mg_ctx {
   uint64_t geno_arena_bytes = 0;
   mh::SignatureCsr ascii_batch;  // mg_genotype's batch packed on the host (grow-only)
   cudaEvent_t evs[64] = {};
-  uint32_t *samples = nullptr;  // sample set of mg_samples_begin: rows x samples_g u32 (kernels.cuh SampleView)
-  uint64_t sample_rows = 0;
+  uint32_t *samples = nullptr;  // sample set of mg_samples_begin: sample_rows x samples_g u32 (kernels.cuh SampleView)
   int samples_g = 0;
 
   DevView view() const {
@@ -688,6 +687,8 @@ extern "C" int mg_counters_scatter(mg_ctx *c) {
 }
 
 // ---- sample sets (kernels.cuh SampleView): the counters of several samples side by side on one index ----
+// rows of a sample column: the set bits of bf, the ref keys held by probe lines, the slots of the overflow table
+static uint64_t sample_rows(const mg_ctx *c) { return c->bf_ones + (c->n_keys - c->ovf_n) + (1ull << c->ovf_log2); }
 static mg::SampleView sample_view(const mg_ctx *c) {
   mg::SampleView sv;
   sv.mat = c->samples;
@@ -706,7 +707,6 @@ extern "C" int mg_samples_end(mg_ctx *c) {
     CU(cudaFree(c->samples));
   }
   c->samples = nullptr;
-  c->sample_rows = 0;
   c->samples_g = 0;
   return MG_OK;
 }
@@ -717,7 +717,7 @@ extern "C" int mg_samples_begin(mg_ctx *c, int n_samples) {
     return set_err(MG_ERR_ARG, "a sample set holds 1 to %d samples, not %d", MG_SAMPLE_SET_MAX, n_samples);
   int rc = mg_samples_end(c);
   if (rc) return rc;
-  const uint64_t rows = c->bf_ones + (c->n_keys - c->ovf_n) + (1ull << c->ovf_log2);
+  const uint64_t rows = sample_rows(c);
   if (rows >= mg::NO_ROW) return set_err(MG_ERR_ARG, "the index has %llu counter rows; a sample set takes < 2^32",
                                          (unsigned long long)rows);
   rc = ensure_key_rank(c);
@@ -726,7 +726,6 @@ extern "C" int mg_samples_begin(mg_ctx *c, int n_samples) {
   CU(cudaMalloc(&c->samples, bytes));
   CU(cudaMemsetAsync(c->samples, 0, bytes, c->stream[0]));
   CU(cudaStreamSynchronize(c->stream[0]));
-  c->sample_rows = rows;
   c->samples_g = n_samples;
   return MG_OK;
 }
@@ -738,7 +737,7 @@ extern "C" int mg_samples_capacity(mg_ctx *c, int *n) {
   CU(cudaSetDevice(c->device));
   size_t free_b = 0, total_b = 0;
   CU(cudaMemGetInfo(&free_b, &total_b));
-  const uint64_t column = 4 * (c->bf_ones + (c->n_keys - c->ovf_n) + (1ull << c->ovf_log2));
+  const uint64_t column = 4 * sample_rows(c);
   const uint64_t fit = (uint64_t)free_b / 4 * 3 / column + (c->samples ? (uint64_t)c->samples_g : 0);
   *n = (int)std::min<uint64_t>(fit, MG_SAMPLE_SET_MAX);
   return MG_OK;
@@ -767,32 +766,6 @@ extern "C" int mg_samples_take(mg_ctx *c, int s) {
   CU(cudaStreamSynchronize(st));
   return MG_OK;
 }
-// K4 for a sample set: the weights of every sample, sample-major, into d_w [samples_g][n_kmers] (DEVICE batch)
-static int lookup_samples_on_device(mg_ctx *c, const mg_packed_batch *in, const mg_packed_dims *dm, int32_t *d_w) {
-  cudaStream_t st = c->stream[0];
-  const uint64_t nk = dm->n_kmers;
-  if (!nk) return MG_OK;
-  const mg::SampleView sv = sample_view(c);
-  const uint4 *km = (const uint4 *)in->kmers;
-  {
-    const uint64_t want = (nk + mg::LOOKUP_THREADS - 1) / mg::LOOKUP_THREADS, cap = (uint64_t)c->sms * 32;
-    const int grid = (int)(want < cap ? want : cap);
-    auto kernel = c->k == 35 ? mg::k_lookup_samples<35> : mg::k_lookup_samples<0>;
-    CU(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, mg::LOOKUP_SAMPLES_SMEM));
-    c->launches++;
-    kernel<<<grid, mg::LOOKUP_THREADS, mg::LOOKUP_SAMPLES_SMEM, st>>>(km, nk, c->view(), sv, d_w);
-    CU(cudaGetLastError());
-  }
-  if (in->n_irregular) {
-    c->launches++;
-    mg::k_lookup_samples_irr<<<grid_for(in->n_irregular, 128), 128, 0, st>>>(
-        (const uint8_t *)in->irr_pool, in->irr_off, in->irr_kmer, in->n_irregular, km, nk, c->view(), sv, d_w,
-        c->d_scalars);
-    CU(cudaGetLastError());
-  }
-  return MG_OK;
-}
-
 template <int K, int REFK>
 static cudaError_t launch_refpass(mg_ctx *c, const uint8_t *d_chunk, uint64_t chunk_base, uint64_t p_begin, uint64_t p_end) {
   int grid = (int)((p_end - p_begin + mg::RP_TILE - 1) / mg::RP_TILE);
@@ -1110,7 +1083,7 @@ static int lookup_common(mg_ctx *c, const char *pool, const uint64_t *off, const
   CU(cudaMalloc(&d_out.p, (n ? n : 1) * 4));
   c->launches++;
   mg::k_lookup<<<grid_for(n, 128), 128, 0, c->stream[0]>>>(b.pool, b.off, b.flags, n, c->view(), mode, which,
-                                                           (int32_t *)d_out.p, c->d_scalars, nullptr, nullptr);
+                                                           (int32_t *)d_out.p, c->d_scalars);
   CU(cudaGetLastError());
   CU(cudaMemcpyAsync(out_host, d_out.p, n * 4, cudaMemcpyDeviceToHost, c->stream[0]));
   CU(cudaStreamSynchronize(c->stream[0]));
@@ -1171,31 +1144,35 @@ static int geno_events(mg_ctx *c) {
   return MG_OK;
 }
 // all pointers of in/out are DEVICE pointers
-// K4 alone: the count of every signature k-mer of the batch into d_w (raw: bf counters unmasked)
-static int lookup_packed_on_device(mg_ctx *c, const mg_packed_batch *in, const mg_packed_dims *dm, int32_t *d_w, bool raw) {
+// K4 alone: the weights of every signature k-mer of the batch into d_w, as mg::LookupOut `o` says (OUT_SAMPLES:
+// [samples_g][n_kmers], sample-major)
+static int lookup_on_device(mg_ctx *c, const mg_packed_batch *in, const mg_packed_dims *dm, int32_t *d_w,
+                            mg::LookupOut o) {
+  using namespace mg;
+  using Packed = void (*)(const uint4 *, uint64_t, DevView, int32_t *, SampleView);
+  static const Packed packed[2][3] = {
+      {k_lookup_packed<35, OUT_COUNT>, k_lookup_packed<35, OUT_RAW>, k_lookup_packed<35, OUT_SAMPLES>},
+      {k_lookup_packed<0, OUT_COUNT>, k_lookup_packed<0, OUT_RAW>, k_lookup_packed<0, OUT_SAMPLES>}};
+  using Irr = void (*)(const uint8_t *, const uint64_t *, const uint32_t *, uint64_t, const uint4 *, uint64_t, DevView,
+                       int32_t *, SampleView, unsigned long long *);
+  static const Irr irr[3] = {k_lookup_irr<OUT_COUNT>, k_lookup_irr<OUT_RAW>, k_lookup_irr<OUT_SAMPLES>};
   cudaStream_t st = c->stream[0];
   const uint64_t nk = dm->n_kmers;
   if (!nk) return MG_OK;
+  const mg::SampleView sv = o == mg::OUT_SAMPLES ? sample_view(c) : mg::SampleView{};
+  const uint4 *km = (const uint4 *)in->kmers;
+  const uint64_t want = (nk + mg::LOOKUP_THREADS - 1) / mg::LOOKUP_THREADS, cap = (uint64_t)c->sms * 32;
+  const int grid = (int)(want < cap ? want : cap);
+  const Packed kernel = packed[c->k == 35 ? 0 : 1][o];
+  const int smem = mg::lookup_smem(o);
+  if (smem > 48 * 1024) CU(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
   c->launches++;
-  {
-    const uint64_t want = (nk + mg::LOOKUP_THREADS - 1) / mg::LOOKUP_THREADS, cap = (uint64_t)c->sms * 32;
-    const int grid = (int)(want < cap ? want : cap);
-    const uint4 *km = (const uint4 *)in->kmers;
-    if (c->k == 35 && !raw)
-      mg::k_lookup_packed<35, false><<<grid, mg::LOOKUP_THREADS, mg::LOOKUP_SMEM, st>>>(km, nk, c->view(), d_w);
-    else if (c->k == 35)
-      mg::k_lookup_packed<35, true><<<grid, mg::LOOKUP_THREADS, mg::LOOKUP_SMEM, st>>>(km, nk, c->view(), d_w);
-    else if (!raw)
-      mg::k_lookup_packed<0, false><<<grid, mg::LOOKUP_THREADS, mg::LOOKUP_SMEM, st>>>(km, nk, c->view(), d_w);
-    else
-      mg::k_lookup_packed<0, true><<<grid, mg::LOOKUP_THREADS, mg::LOOKUP_SMEM, st>>>(km, nk, c->view(), d_w);
-  }
+  kernel<<<grid, mg::LOOKUP_THREADS, smem, st>>>(km, nk, c->view(), d_w, sv);
   CU(cudaGetLastError());
   if (in->n_irregular) {  // not k symbols of ACGT: the byte-exact path, written to their places in the weight array
     c->launches++;
-    mg::k_lookup<<<grid_for(in->n_irregular, 128), 128, 0, st>>>(
-        (const uint8_t *)in->irr_pool, in->irr_off, nullptr, in->n_irregular, c->view(), 0, 0, d_w, c->d_scalars,
-        in->irr_kmer, (const uint4 *)in->kmers, raw);
+    irr[o]<<<grid_for(in->n_irregular, 128), 128, 0, st>>>((const uint8_t *)in->irr_pool, in->irr_off, in->irr_kmer,
+                                                          in->n_irregular, km, nk, c->view(), d_w, sv, c->d_scalars);
     CU(cudaGetLastError());
   }
   return MG_OK;
@@ -1227,12 +1204,15 @@ static int genotype_from_weights(mg_ctx *c, const mg_packed_batch *in, const mg_
   CU(cudaEventRecord(c->ge[3], st));
   return MG_OK;
 }
-static int genotype_packed_on_device(mg_ctx *c, const mg_packed_batch *in, const mg_genotype_out *out,
-                                     const mg_packed_dims *dm, float error_rate, int max_coverage, int haploid) {
+// the look-up (OUT_COUNT for one output set, OUT_SAMPLES for one per sample of the set), then coverage + likelihoods
+// for each of the n_out output sets on its column of the weights
+static int genotype_packed_on_device(mg_ctx *c, const mg_packed_batch *in, const mg_genotype_out *out, int n_out,
+                                     mg::LookupOut o, const mg_packed_dims *dm, float error_rate, int max_coverage,
+                                     int haploid) {
   cudaStream_t st = c->stream[0];
   const uint64_t nk = dm->n_kmers;
   const bool own_lik = out->lik == nullptr;
-  const uint64_t w_bytes = ((nk ? nk : 1) * 4 + 255) & ~255ull;
+  const uint64_t w_bytes = ((nk ? nk : 1) * 4 * (uint64_t)n_out + 255) & ~255ull;
   int rc = geno_scratch(c, w_bytes + (own_lik ? dm->lik_slots * 8 + 256 : 0));
   if (rc) return rc;
   rc = join_streams(c);
@@ -1242,11 +1222,16 @@ static int genotype_packed_on_device(mg_ctx *c, const mg_packed_batch *in, const
   rc = geno_events(c);
   if (rc) return rc;
   CU(cudaEventRecord(c->ge[0], st));
-  rc = lookup_packed_on_device(c, in, dm, d_w, false);
+  rc = lookup_on_device(c, in, dm, d_w, o);
   if (rc) return rc;
   CU(cudaEventRecord(c->ge[1], st));
   CU(cudaEventRecord(c->ge[4], st));
-  return genotype_from_weights(c, in, out, 1, dm, d_w, d_lik, error_rate, max_coverage, haploid);
+  return genotype_from_weights(c, in, out, n_out, dm, d_w, d_lik, error_rate, max_coverage, haploid);
+}
+
+// the arrays a genotyping call writes for one output set (lik is optional, but needs its offsets)
+static bool out_arrays_ok(const mg_genotype_out &o) {
+  return o.cov && o.n_gts && o.status && o.best_gt && o.gq && (!o.lik || o.lik_off);
 }
 
 // ---- the two halves on their own: replicas sum the LOOK-UP RESULTS of a batch instead of their counters ----
@@ -1265,7 +1250,7 @@ extern "C" int mg_lookup_packed_device(mg_ctx *c, const mg_packed_batch *in, con
   rc = geno_events(c);
   if (rc) return rc;
   CU(cudaEventRecord(c->ge[0], c->stream[0]));
-  rc = lookup_packed_on_device(c, in, dims, reinterpret_cast<int32_t *>(d_weights), true);
+  rc = lookup_on_device(c, in, dims, reinterpret_cast<int32_t *>(d_weights), mg::OUT_RAW);
   if (rc) return rc;
   CU(cudaEventRecord(c->ge[1], c->stream[0]));
   return MG_OK;
@@ -1276,7 +1261,7 @@ extern "C" int mg_genotype_weights_device(mg_ctx *c, const mg_packed_batch *in, 
   if (!c || !in || !out || !dims || (!d_weights && dims->n_kmers)) return set_err(MG_ERR_ARG, "NULL argument");
   if (dims->n_variants == 0) return MG_OK;
   if (!in->var_allele_off || !in->allele_sig_off || !in->sig_kmer_off || (!in->kmers && dims->n_kmers) || !in->freq ||
-      !out->cov || !out->n_gts || !out->status || !out->best_gt || !out->gq || (out->lik && !out->lik_off))
+      !out_arrays_ok(*out))
     return set_err(MG_ERR_ARG, "NULL array in batch");
   CU(cudaSetDevice(c->device));
   const bool own_lik = out->lik == nullptr;
@@ -1323,14 +1308,11 @@ extern "C" int mg_genotype_packed_device(mg_ctx *c, const mg_packed_batch *in, c
   if (!c->alt_final) return set_err(MG_ERR_STATE, "mg_genotype_packed_device before mg_finalize_alt");
   if (dims->n_variants == 0) return MG_OK;
   if (!in->var_allele_off || !in->allele_sig_off || !in->sig_kmer_off || (!in->kmers && dims->n_kmers) || !in->freq ||
-      !out->cov || !out->n_gts || !out->status || !out->best_gt || !out->gq || (out->lik && !out->lik_off) ||
-      (in->n_irregular && (!in->irr_off || !in->irr_pool || !in->irr_kmer)))
+      !out_arrays_ok(*out) || (in->n_irregular && (!in->irr_off || !in->irr_pool || !in->irr_kmer)))
     return set_err(MG_ERR_ARG, "NULL array in batch");
   CU(cudaSetDevice(c->device));
-  return genotype_packed_on_device(c, in, out, dims, error_rate, max_coverage, haploid);
+  return genotype_packed_on_device(c, in, out, 1, mg::OUT_COUNT, dims, error_rate, max_coverage, haploid);
 }
-
-static int lookup_samples_on_device(mg_ctx *c, const mg_packed_batch *in, const mg_packed_dims *dm, int32_t *d_w);
 
 // mg_genotype_packed and mg_genotype_samples_packed: the HOST batch goes into the grow-only device arena, is genotyped
 // for n_out output sets (one, or one per sample of the set: samples), and the results come back.  The likelihood
@@ -1343,8 +1325,7 @@ static int genotype_packed_host(mg_ctx *c, const mg_packed_batch *in, const mg_g
       (in->n_irregular && (!in->irr_off || !in->irr_pool || !in->irr_kmer)))
     return set_err(MG_ERR_ARG, "NULL array in batch");
   for (int s = 0; s < n_out; ++s)
-    if (!out[s].cov || !out[s].n_gts || !out[s].status || !out[s].best_gt || !out[s].gq ||
-        (out[s].lik && !out[s].lik_off) || (out[s].lik == nullptr) != (out[0].lik == nullptr))
+    if (!out_arrays_ok(out[s]) || (out[s].lik == nullptr) != (out[0].lik == nullptr))
       return set_err(MG_ERR_ARG, "NULL array in batch");
   CU(cudaSetDevice(c->device));
   mg_packed_dims dm;
@@ -1406,25 +1387,8 @@ static int genotype_packed_host(mg_ctx *c, const mg_packed_batch *in, const mg_g
     dout[s].lik_off = nl ? reinterpret_cast<uint64_t *>(d + o_lo) : nullptr;
     dout[s].lik = nl ? reinterpret_cast<double *>(d + o_lik + s * al(nl * 8)) : nullptr;
   }
-  int rc;
-  if (!samples) {
-    rc = genotype_packed_on_device(c, &din, dout.data(), &dm, error_rate, max_coverage, haploid);
-  } else {  // one look-up for the whole set, then coverage + likelihoods per sample on its column of the weights
-    const uint64_t w_bytes = al((nk ? nk : 1) * 4 * g);
-    rc = geno_scratch(c, w_bytes + (nl ? 0 : dm.lik_slots * 8 + 256));
-    if (!rc) rc = join_streams(c);
-    if (!rc) rc = geno_events(c);
-    if (rc) return rc;
-    int32_t *d_w = reinterpret_cast<int32_t *>(c->geno_scratch);
-    CU(cudaEventRecord(c->ge[0], st));
-    rc = lookup_samples_on_device(c, &din, &dm, d_w);
-    if (rc) return rc;
-    CU(cudaEventRecord(c->ge[1], st));
-    CU(cudaEventRecord(c->ge[4], st));
-    rc = genotype_from_weights(c, &din, dout.data(), n_out, &dm, d_w,
-                               reinterpret_cast<double *>(reinterpret_cast<uint8_t *>(c->geno_scratch) + w_bytes),
-                               error_rate, max_coverage, haploid);
-  }
+  int rc = genotype_packed_on_device(c, &din, dout.data(), n_out, samples ? mg::OUT_SAMPLES : mg::OUT_COUNT, &dm,
+                                     error_rate, max_coverage, haploid);
   if (rc) return rc;
   for (int s = 0; s < n_out; ++s) {
     CU(cudaMemcpyAsync(out[s].cov, dout[s].cov, na * 4, cudaMemcpyDeviceToHost, st));

@@ -5,7 +5,8 @@
 
   take          mg_samples_take per sample at the `wg` workload's index (bench.py's build: 2^35-bit filters, 1e8 alt
                 + 1e8 ref signature k-mers), after a scan of one bench.py sample batch (2^27 43-mers)
-  lookups       k_lookup_samples for sets of 1, 8 and 32 samples against one k_lookup_packed on the same batch
+  lookups       k_lookup_packed<K,OUT_SAMPLES> for sets of 1, 8 and 32 samples against one single-sample look-up on the
+                same batch
                 (bench.py's 2.85e6-variant batch; device time of the look-up phase, mg_genotype_kernel_ms[0])
   whole_program tests/bench_cli_e2e.py's 5 Mbp shape: `malva-geno call` with N donor databases against N single
                 calls on the same index; the outputs must be byte-identical
@@ -109,7 +110,7 @@ def device_part():
             res = g.genotype_samples_packed(pb, want_lik=False)
             ms.append(g.genotype_kernel_ms())
         same = same and all(np.array_equal(r.gq, ref_res.gq) and np.array_equal(r.cov, ref_res.cov) for r in res)
-        lookups[f"k_lookup_samples_G{n}"] = {
+        lookups[f"samples_G{n}"] = {
             "lookup_ms": round(statistics.median(x[0] for x in ms), 3),
             "coverage_all_samples_ms": round(statistics.median(x[1] for x in ms), 3),
             "likelihoods_all_samples_ms": round(statistics.median(x[2] for x in ms), 3)}

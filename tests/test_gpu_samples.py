@@ -2,8 +2,8 @@
 with several KMC databases.
 
 A sample set keeps one u32 column per sample over the counter rows of the index; mg_samples_take moves the live
-counters into a column and zeroes them, k_lookup_samples reads the rows of a batch for every column at once.  Column
-s must genotype exactly like a fresh context that scanned sample s alone, at every probe-line key layout and at the
+counters into a column and zeroes them, the sample-set look-up reads the rows of a batch for every column at once.
+Column s must genotype exactly like a fresh context that scanned sample s alone, at every probe-line key layout and at the
 filter sizes where counters live in different places (overflowed keys, set bits past the three inline counters of a
 line, the partial last line), and a CLI run over N databases must write, per database, the bytes a single-database
 run prints."""
