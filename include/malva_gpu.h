@@ -216,6 +216,15 @@ int mg_counters_scatter(mg_ctx *ctx);
  * mg_get_counts for the whole stream. */
 int mg_reduce_counts(mg_ctx **ctx, int n);
 
+/* A new context on `device` holding exactly src's index and live counters: both filters, the ref keys, the rank
+ * directory, the overflow table, every counter, the irregular ref keys and the finalize state.  Device-to-device
+ * copies (cudaMemcpyPeerAsync; the same device works too) instead of a second load: the index image is canonical.
+ * Waits for src's enqueued work first and returns after the copies completed.  Not copied: a sample set, the KMC
+ * parameters of mg_kmc_open, a caller stream of mg_set_stream.  The two contexts are independent afterwards (either
+ * may be destroyed first).  src must be past mg_finalize_alt (MG_ERR_STATE); a device that is not visible fails
+ * like mg_create. */
+int mg_replicate(mg_ctx **out, mg_ctx *src, int device);
+
 /* Sample sets: several samples genotyped against one index, each from its own counters.  Every counter a signature
  * k-mer can read has a ROW fixed by the index: rows [0, bf_ones) are the set bits of bf in rank order, the next
  * (ref keys - overflow keys) rows the ref keys held by the probe lines in line order, the last (overflow capacity)

@@ -118,6 +118,7 @@ SYMBOLS = {
     "mg_counters_scatter": (C.c_int, [C.c_void_p]),
     "mg_counter_buffers": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), u64p]),
     "mg_reduce_counts": (C.c_int, [C.POINTER(C.c_void_p), C.c_int]),
+    "mg_replicate": (C.c_int, [C.POINTER(C.c_void_p), C.c_void_p, C.c_int]),
     "mg_samples_begin": (C.c_int, [C.c_void_p, C.c_int]),
     "mg_samples_capacity": (C.c_int, [C.c_void_p, C.POINTER(C.c_int)]),
     "mg_samples_take": (C.c_int, [C.c_void_p, C.c_int]),

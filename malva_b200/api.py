@@ -181,14 +181,25 @@ class MalvaGpu:
     """Device-resident bf / context_bf / ref_bf of one malva-geno run (main.cpp:300-302)."""
 
     def __init__(self, k: int = 35, ref_k: int = 43, bf_bits: int = 1 << 35, device: int = 0):
+        self._attach(k, ref_k, bf_bits, device)
+        check(self._L.mg_create(C.byref(self._h), device, k, ref_k, bf_bits))
+
+    def _attach(self, k: int, ref_k: int, bf_bits: int, device: int) -> None:
         self._L = _lib.load()
         self._h = C.c_void_p()
         self.k, self.ref_k, self.bf_bits, self.device = k, ref_k, bf_bits, device
         self._n_samples = 0
-        check(self._L.mg_create(C.byref(self._h), device, k, ref_k, bf_bits))
         self.bf = _View(self, BF_ALT)
         self.context_bf = _View(self, BF_CONTEXT)
         self.ref_bf = _View(self, KMAP_REF)
+
+    def replicate(self, device: int) -> "MalvaGpu":
+        """a new context on `device` (this one's included) holding exactly this index and its live counters
+        (mg_replicate: device-to-device copies, no reload); needs finalize_alt.  A sample set is not copied."""
+        r = MalvaGpu.__new__(MalvaGpu)
+        r._attach(self.k, self.ref_k, self.bf_bits, device)
+        check(self._L.mg_replicate(C.byref(r._h), self._h, device))
+        return r
 
     def close(self) -> None:
         if self._h:

@@ -84,6 +84,9 @@ const char *USAGE =
     "                                        round-robin, add the counters up on the first one\n"
     "          --out-dir DIR                 call with several KMC databases (call [opts] ref.fa vars.vcf DB1 DB2 ..):\n"
     "                                        genotype every sample against one index, sample DB to DIR/basename(DB).vcf\n"
+    "          --sample-devices A,B,..       call with --out-dir: replicate the index on these devices (a device may\n"
+    "                                        repeat) and scan and genotype a share of every round's samples on each\n"
+    "                                        (instead of --device / --devices)\n"
     "\n";
 
 struct Options {
@@ -96,6 +99,8 @@ struct Options {
   int threads = 0, device = 0;
   bool trace = false;  // --trace: per-batch host/device timings on stderr
   std::vector<int> devices;  // --devices a,b,..: `call` replicates the index and deals the KMC records round-robin
+  bool devices_given = false;  // --device or --devices was given
+  std::vector<int> sample_devices;  // --sample-devices a,b,..: `call --out-dir` spreads the samples over replicas
   std::string fasta_path, vcf_path, kmc_path;
   std::vector<std::string> kmc_paths;  // call: one or more KMC databases (kmc_path = the first)
   std::string out_dir;                 // call with several databases: sample P is written to out_dir/basename(P).vcf
@@ -124,6 +129,7 @@ bool parse_arguments(int argc, char **argv, Options &o, int n_positional, bool m
                                     {"trace", no_argument, nullptr, 1003},
                                     {"devices", required_argument, nullptr, 1004},
                                     {"out-dir", required_argument, nullptr, 1005},
+                                    {"sample-devices", required_argument, nullptr, 1006},
                                     {nullptr, 0, nullptr, 0}};
   bool die = false;
   optind = 1;
@@ -145,13 +151,19 @@ bool parse_arguments(int argc, char **argv, Options &o, int n_positional, bool m
       case 'v': o.verbose = true; break;
       case '1': o.haploid = true; break;
       case 1000: arg >> o.threads; break;
-      case 1001: arg >> o.device; break;
+      case 1001:
+        arg >> o.device;
+        o.devices_given = true;
+        break;
       case 1002: o.index_blocks = true; break;
       case 1003: o.trace = true; break;
-      case 1004: {
+      case 1004:
+      case 1006: {
+        std::vector<int> &list = c == 1004 ? o.devices : o.sample_devices;
         std::string tok;
         while (std::getline(arg, tok, ','))
-          if (!tok.empty()) o.devices.push_back(atoi(tok.c_str()));
+          if (!tok.empty()) list.push_back(atoi(tok.c_str()));
+        o.devices_given = o.devices_given || c == 1004;
         break;
       }
       case 1005: o.out_dir = optarg ? optarg : ""; break;
@@ -896,9 +908,9 @@ int container_selftest_main() {
 // STEP 2: the sample k-mer scan (main.cpp:482-500) of one database.  Raw suffix records go through rings of pinned
 // buffers, one ring per device, chunks dealt round-robin; the library copies and scans them asynchronously
 // (double-buffered on its side), a buffer is refilled only after the event recorded behind its scan has completed.
-// With several devices the counters are then added up on the first one (all updates are commutative adds,
-// main.cpp:495-499) and the replicas are destroyed.
-void scan_kmc(const Options &o, std::vector<Ctx> &gs, mh::KmcDb &db, const std::string &path) {
+// With several contexts the counters are then added up on the first one (all updates are commutative adds,
+// main.cpp:495-499).
+void scan_kmc(const Options &o, std::vector<mg_ctx *> gs, mh::KmcDb &db, const std::string &path) {
   const int n_dev = (int)gs.size();
   constexpr int RING = 4;
   constexpr uint64_t CHUNK = 1ull << 22;  // records per buffer
@@ -906,7 +918,7 @@ void scan_kmc(const Options &o, std::vector<Ctx> &gs, mh::KmcDb &db, const std::
   std::vector<char> used((size_t)(n_dev * RING), 0);
   Stopwatch sw;
   for (int d = 0; d < n_dev; ++d) {
-    gpu(mg_kmc_open(gs[(size_t)d].c, db.lut.data(), db.lut.size(), db.lut_prefix_len, db.kmer_len, db.counter_size,
+    gpu(mg_kmc_open(gs[(size_t)d], db.lut.data(), db.lut.size(), db.lut_prefix_len, db.kmer_len, db.counter_size,
                     db.min_count, db.max_count),
         "mg_kmc_open");
     for (int s = 0; s < RING; ++s) gpu(mg_host_alloc((void **)&buf[(size_t)(d * RING + s)], CHUNK * db.record_bytes + 64), "mg_host_alloc");
@@ -915,7 +927,7 @@ void scan_kmc(const Options &o, std::vector<Ctx> &gs, mh::KmcDb &db, const std::
   double t_alloc = sw.lap(), t_wait = 0, t_read = 0, t_submit = 0;
   for (uint64_t chunk = 0;; ++chunk) {
     const int d = (int)(chunk % (uint64_t)n_dev), slot = d * RING + (int)((chunk / (uint64_t)n_dev) % RING);
-    mg_ctx *c = gs[(size_t)d].c;
+    mg_ctx *c = gs[(size_t)d];
     if (used[(size_t)slot]) gpu(mg_event_sync(c, 32 + slot % RING), "mg_event_sync");
     t_wait += sw.lap();
     uint64_t n = db.read_records(buf[(size_t)slot], first, CHUNK);
@@ -927,7 +939,7 @@ void scan_kmc(const Options &o, std::vector<Ctx> &gs, mh::KmcDb &db, const std::
     used[(size_t)slot] = 1;
     first += n;
   }
-  for (auto &x : gs) gpu(mg_sync(x.c), "mg_sync");
+  for (mg_ctx *x : gs) gpu(mg_sync(x), "mg_sync");
   const double t_drain = sw.lap();
   for (auto &b : buf) mg_host_free(b);
   if (o.trace)
@@ -935,24 +947,19 @@ void scan_kmc(const Options &o, std::vector<Ctx> &gs, mh::KmcDb &db, const std::
                     "%.1f ms, submitting %.1f ms, draining %.1f ms, freeing %.1f ms\n",
             (unsigned long long)first, t_alloc, t_read, t_wait, t_submit, t_drain, sw.lap());
   if (first != db.total_kmers) throw std::runtime_error(path + ".kmc_suf is shorter than its header says");
-  if (n_dev > 1) {
-    std::vector<mg_ctx *> all;
-    for (auto &x : gs) all.push_back(x.c);
-    gpu(mg_reduce_counts(all.data(), n_dev), "mg_reduce_counts");
-    for (size_t d = 1; d < gs.size(); ++d) {  // the replicas are no longer needed
-      mg_destroy(gs[d].c);
-      gs[d].c = nullptr;
-    }
-  }
+  if (n_dev > 1) gpu(mg_reduce_counts(gs.data(), n_dev), "mg_reduce_counts");
 }
 
-// STEP 3: genotype (main.cpp:504-581), one pass over the VCF.  outs[s] receives the VCF body of output s: the live
-// counters of g (mg_genotype_packed, one output), or with sample_set every sample of g's sample set
-// (mg_genotype_samples_packed, sample s into outs[s]).  Three stages on three threads: enumerate
+// STEP 3: genotype (main.cpp:504-581), one pass over the VCF.  outs[s] receives the VCF body of output s.  Without
+// sets: the live counters of gs[0] (mg_genotype_packed, one output).  With sets: context i holds a sample set of
+// sets[i] samples, and they are the next sets[i] outputs after those of contexts 0..i-1 (mg_genotype_samples_packed,
+// every context on its own worker, all on the same read-only batch).  Three stages on three threads: enumerate
 // (EnumeratedBatches) | device (below) | format + write (this thread).
-void genotype_pass(const Options &o, mg_ctx *g, bool sample_set, EnumeratedBatches &batches,
-                   const std::vector<FILE *> &outs) {
+void genotype_pass(const Options &o, const std::vector<mg_ctx *> &gs, const std::vector<int> &sets,
+                   EnumeratedBatches &batches, const std::vector<FILE *> &outs) {
   const size_t n_out = outs.size();
+  std::vector<size_t> set_first(sets.size(), 0);
+  for (size_t i = 1; i < sets.size(); ++i) set_first[i] = set_first[i - 1] + (size_t)sets[i - 1];
   Channel<std::unique_ptr<Batch>> done(2);
   std::exception_ptr dev_err;
   std::thread device([&] {
@@ -990,13 +997,15 @@ void genotype_pass(const Options &o, mg_ctx *g, bool sample_set, EnumeratedBatch
             res[s] = {b->cov.data() + s * na, b->n_gts.data() + s * nv, b->status.data() + s * nv,
                       b->best.data() + s * nv, b->gq.data() + s * nv, o.verbose ? b->lik_off.data() : nullptr,
                       o.verbose ? b->lik.data() + s * b->lik_off[nv] : nullptr};
-          if (!sample_set)
-            gpu(mg_genotype_packed(g, &in, res.data(), o.error_rate, (int)o.max_coverage, o.haploid ? 1 : 0),
+          if (sets.empty())
+            gpu(mg_genotype_packed(gs[0], &in, res.data(), o.error_rate, (int)o.max_coverage, o.haploid ? 1 : 0),
                 "mg_genotype_packed");
           else
-            gpu(mg_genotype_samples_packed(g, &in, res.data(), (int)n_out, o.error_rate, (int)o.max_coverage,
-                                           o.haploid ? 1 : 0),
-                "mg_genotype_samples_packed");
+            parallel_for(gs.size(), (int)gs.size(), [&](size_t i) {
+              gpu(mg_genotype_samples_packed(gs[i], &in, res.data() + set_first[i], sets[i], o.error_rate,
+                                             (int)o.max_coverage, o.haploid ? 1 : 0),
+                  "mg_genotype_samples_packed");
+            });
         }
         b->t_dev = sw.lap();
         done.push(std::move(b));
@@ -1063,6 +1072,19 @@ int call_main(int argc, char **argv) {
   Options o;
   if (!parse_arguments(argc, argv, o, 3, true)) return EXIT_FAILURE;
   const size_t n_db = o.kmc_paths.size();
+  if (!o.sample_devices.empty() && o.devices_given) {
+    std::cerr << "ERROR: --sample-devices goes with neither --devices nor --device (--devices deals the records of one "
+                 "KMC database over devices, --device picks the one device of a run, --sample-devices lists the "
+                 "devices of several databases)"
+              << std::endl;
+    return 1;
+  }
+  if (!o.sample_devices.empty() && n_db == 1) {
+    std::cerr << "ERROR: --sample-devices is for several KMC databases (call [opts] ref.fa vars.vcf DB1 DB2 .. --out-dir "
+                 "DIR); one database goes over several devices with --devices"
+              << std::endl;
+    return 1;
+  }
   if (n_db > 1 && o.out_dir.empty()) {
     std::cerr << "ERROR: several KMC databases need --out-dir DIR (sample P is written to DIR/basename(P).vcf)"
               << std::endl;
@@ -1073,7 +1095,8 @@ int call_main(int argc, char **argv) {
     return 1;
   }
   if (n_db > 1 && o.devices.size() > 1) {
-    std::cerr << "ERROR: --devices takes one KMC database; several databases run on one device (--device N)"
+    std::cerr << "ERROR: --devices takes one KMC database; several databases run on one device (--device N) or are "
+                 "spread over devices with --sample-devices A,B,.."
               << std::endl;
     return 1;
   }
@@ -1085,8 +1108,19 @@ int call_main(int argc, char **argv) {
                   << std::endl;
         return 1;
       }
+  if (!o.sample_devices.empty()) {  // (before any file is read; without a usable driver mg_create fails as for --devices)
+    const int visible = mg_device_count();
+    for (int d : o.sample_devices)
+      if (visible >= 0 && (d < 0 || d >= visible)) {
+        std::cerr << "ERROR: --sample-devices: device " << d << " is not visible (" << visible << " visible)" << std::endl;
+        return 1;
+      }
+  }
+  // the contexts: one database is dealt over the --devices replicas, several databases over the --sample-devices ones
+  // (a device may be listed more than once: one context each)
+  const std::vector<int> &ctx_devices = o.sample_devices.empty() ? o.devices : o.sample_devices;
   std::vector<std::future<int>> cuda_up;  // CUDA start-up on every device, overlapped with the file reading
-  for (int d : o.devices) cuda_up.push_back(std::async(std::launch::async, [d] { return mg_warmup(d); }));
+  for (int d : ctx_devices) cuda_up.push_back(std::async(std::launch::async, [d] { return mg_warmup(d); }));
   auto stream = std::make_unique<BlockStream>(o, false);
   if (stream->samples_code != 0) {
     std::cerr << "ERROR: VCF samples subset (code: " << stream->samples_code << ")" << std::endl;
@@ -1106,26 +1140,27 @@ int call_main(int argc, char **argv) {
   // the reference FASTA is read while CUDA starts and the index loads (host-only work, 1.4 s for 250 Mbp)
   std::future<std::map<std::string, std::string>> refs_ready =
       std::async(std::launch::async, [&o] { return mh::read_fasta(o.fasta_path, o.strip_chr); });
-  const int n_dev = (int)o.devices.size();
-  std::vector<Ctx> gs((size_t)n_dev);
+  const int n_ctx = (int)ctx_devices.size();
+  std::vector<Ctx> gs((size_t)n_ctx);
   Ctx &g = gs[0];  // the context that answers after the reduce
-  {  // load the index: context_bf, bf, ref_bf (main.cpp:455-461) -- once from the file, then onto every device
+  {  // load the index: context_bf, bf, ref_bf (main.cpp:455-461) -- from the file onto the first context, then
+     // device-to-device copies of its image onto the others
     mh::IndexReader r(o.vcf_path + ".c" + std::to_string(o.ref_k) + ".k" + std::to_string(o.k) + ".malvax.zst");
     if (r.k != o.k || r.ref_k != o.ref_k)
       throw std::runtime_error("the index was built with -k " + std::to_string(r.k) + " -r " + std::to_string(r.ref_k));
     std::vector<uint64_t> ctx_bits = r.read_bits(), bf_bits = r.read_bits(), keys = r.read_keys();
     std::vector<uint8_t> flags(keys.size() / 2, 1);
-    for (int d = 0; d < n_dev; ++d) {
-      // the filter size travels with the index, like the reference's serialised bit vectors (-b matters at index time)
-      gpu(mg_create(&gs[(size_t)d].c, o.devices[(size_t)d], (int)o.k, (int)o.ref_k, r.bf_bits), "mg_create");
-      mg_ctx *c = gs[(size_t)d].c;
-      gpu(mg_import_set_bits(c, 0, bf_bits.data(), bf_bits.size()), "mg_import_set_bits");
-      gpu(mg_add_signatures_packed(c, keys.data(), flags.data(), flags.size()), "mg_add_signatures_packed");
-      gpu(mg_finalize_alt(c), "mg_finalize_alt");
-      gpu(mg_import_set_bits(c, 1, ctx_bits.data(), ctx_bits.size()), "mg_import_set_bits");
-      gpu(mg_finalize_context(c), "mg_finalize_context");
-    }
+    // the filter size travels with the index, like the reference's serialised bit vectors (-b matters at index time)
+    gpu(mg_create(&g.c, ctx_devices[0], (int)o.k, (int)o.ref_k, r.bf_bits), "mg_create");
+    gpu(mg_import_set_bits(g.c, 0, bf_bits.data(), bf_bits.size()), "mg_import_set_bits");
+    gpu(mg_add_signatures_packed(g.c, keys.data(), flags.data(), flags.size()), "mg_add_signatures_packed");
+    gpu(mg_finalize_alt(g.c), "mg_finalize_alt");
+    gpu(mg_import_set_bits(g.c, 1, ctx_bits.data(), ctx_bits.size()), "mg_import_set_bits");
+    gpu(mg_finalize_context(g.c), "mg_finalize_context");
+    for (int i = 1; i < n_ctx; ++i) gpu(mg_replicate(&gs[(size_t)i].c, g.c, ctx_devices[(size_t)i]), "mg_replicate");
   }
+  std::vector<mg_ctx *> cs;
+  for (Ctx &x : gs) cs.push_back(x.c);
   pelapsed("Reference parsing");
   std::map<std::string, std::string> refs = refs_ready.get();
   pelapsed("Reference processed");
@@ -1134,23 +1169,46 @@ int call_main(int argc, char **argv) {
 
   if (n_db == 1) {
     pelapsed("KMC output processing");
-    scan_kmc(o, gs, *dbs[0], o.kmc_path);
+    scan_kmc(o, cs, *dbs[0], o.kmc_path);
+    for (size_t d = 1; d < gs.size(); ++d) {  // the replicas are no longer needed
+      mg_destroy(gs[d].c);
+      gs[d].c = nullptr;
+    }
     pelapsed("BF weights created");
     std::cout << stream->header().cleaned(o.verbose);
     pelapsed("VCF parsing and genotyping");
-    genotype_pass(o, g.c, false, *batches, {stdout});
+    genotype_pass(o, {g.c}, {}, *batches, {stdout});
   } else {
-    // several samples: groups of up to MG_SAMPLE_SET_MAX (as many as device memory holds) share one VCF pass -- each
-    // sample of a group is scanned into the live counters and moved into its column of the sample set, then one
-    // pass genotypes the whole set.  The index, the FASTA and the CUDA context serve every group.
+    // several samples, in rounds: every context takes a sample set of up to MG_SAMPLE_SET_MAX (as many as device
+    // memory holds), and a round's sets share one VCF pass.  Each context scans its samples one after the other into
+    // its live counters and moves each into its column; the contexts scan at the same time, each on its own thread.
+    // The index, the FASTA and the CUDA contexts serve every round.
     if (mkdir(o.out_dir.c_str(), 0777) != 0 && errno != EEXIST)
       throw std::runtime_error("cannot create " + o.out_dir + ": " + strerror(errno));
     const std::string header = stream->header().cleaned(o.verbose);
     for (size_t first = 0; first < n_db;) {
-      int fit = 0;
-      gpu(mg_samples_capacity(g.c, &fit), "mg_samples_capacity");
-      if (fit < 1) throw std::runtime_error("not even one sample column fits in device memory next to the index");
-      const size_t n = std::min<size_t>((size_t)fit, n_db - first);
+      // a round takes the next samples in command-line order: ceil(remaining / contexts) each, as far as they fit.
+      // Planned one context after the other: contexts on one device share its memory.
+      const size_t per_ctx = (n_db - first + (size_t)n_ctx - 1) / (size_t)n_ctx;
+      std::vector<int> sets((size_t)n_ctx, 0);
+      size_t n = 0;
+      for (size_t i = 0; i < (size_t)n_ctx; ++i) {
+        int fit = 0;
+        gpu(mg_samples_capacity(cs[i], &fit), "mg_samples_capacity");
+        sets[i] = (int)std::min({per_ctx, (size_t)fit, n_db - first - n});
+        if (sets[i] > 0) gpu(mg_samples_begin(cs[i], sets[i]), "mg_samples_begin");
+        n += (size_t)sets[i];
+      }
+      if (n == 0) throw std::runtime_error("not even one sample column fits in device memory next to the index");
+      if (o.trace) {
+        std::string plan;
+        for (int x : sets) plan += " " + std::to_string(x);
+        fprintf(stderr, "[trace] round of %zu samples, sets per context:%s\n", n, plan.c_str());
+      }
+      std::vector<mg_ctx *> set_ctx;  // the contexts with a set this round, and their sets
+      std::vector<int> set_n;
+      for (size_t i = 0; i < (size_t)n_ctx; ++i)
+        if (sets[i] > 0) set_ctx.push_back(cs[i]), set_n.push_back(sets[i]);
       if (first > 0) {  // a fresh VCF pass (the previous group's has ended)
         batches.reset();
         call_batches.reset();
@@ -1158,12 +1216,16 @@ int call_main(int argc, char **argv) {
         call_batches = std::make_unique<BatchPrefetcher>(*stream, LINES_PER_BATCH);
         batches = std::make_unique<EnumeratedBatches>(*call_batches, refs, o);
       }
-      gpu(mg_samples_begin(g.c, (int)n), "mg_samples_begin");
       pelapsed("KMC output processing");
-      for (size_t s = 0; s < n; ++s) {
-        scan_kmc(o, gs, *dbs[first + s], o.kmc_paths[first + s]);
-        gpu(mg_samples_take(g.c, (int)s), "mg_samples_take");
-      }
+      std::vector<size_t> set_first(set_n.size(), first);
+      for (size_t i = 1; i < set_n.size(); ++i) set_first[i] = set_first[i - 1] + (size_t)set_n[i - 1];
+      parallel_for(set_ctx.size(), (int)set_ctx.size(), [&](size_t i) {
+        for (int s = 0; s < set_n[i]; ++s) {
+          const size_t db = set_first[i] + (size_t)s;
+          scan_kmc(o, {set_ctx[i]}, *dbs[db], o.kmc_paths[db]);
+          gpu(mg_samples_take(set_ctx[i], s), "mg_samples_take");
+        }
+      });
       pelapsed("BF weights created");
       std::vector<FILE *> outs;
       struct Files {  // (closed on every way out)
@@ -1180,10 +1242,10 @@ int call_main(int argc, char **argv) {
         fwrite(header.data(), 1, header.size(), f);
       }
       pelapsed("VCF parsing and genotyping");
-      genotype_pass(o, g.c, true, *batches, outs);
+      genotype_pass(o, set_ctx, set_n, *batches, outs);
       for (FILE *f : outs)
         if (fflush(f) != 0) throw std::runtime_error("cannot write to " + o.out_dir + ": " + strerror(errno));
-      gpu(mg_samples_end(g.c), "mg_samples_end");
+      for (mg_ctx *c : set_ctx) gpu(mg_samples_end(c), "mg_samples_end");
       first += n;
     }
   }

@@ -46,7 +46,7 @@ static int set_err(int code, const char *fmt, ...) {
   } while (0)
 
 extern "C" const char *mg_last_error(void) { return g_err; }
-extern "C" int mg_version(void) { return 201; }
+extern "C" int mg_version(void) { return 202; }
 extern "C" int mg_device_count(void) {
   int n = 0;
   cudaError_t e = cudaGetDeviceCount(&n);
@@ -192,6 +192,21 @@ static int ovf_reserve(mg_ctx *c, uint64_t extra) {
 }
 
 static int ctx_init(mg_ctx *c);
+// mg_destroy of a context whose set-up failed (e.g. out of device memory for a large -b): nothing is left behind, and
+// the error text of the failure stays
+static void destroy_keep_error(mg_ctx *c) {
+  char msg[sizeof(g_err)];
+  memcpy(msg, g_err, sizeof(msg));
+  mg_destroy(c);
+  memcpy(g_err, msg, sizeof(msg));
+}
+static int check_device(int device) {
+  int ndev = 0;
+  CU(cudaGetDeviceCount(&ndev));
+  if (device < 0 || device >= ndev) return set_err(MG_ERR_CUDA, "device %d not available (%d visible)", device, ndev);
+  CU(cudaSetDevice(device));
+  return MG_OK;
+}
 extern "C" int mg_create(mg_ctx **out, int device, int k, int ref_k, uint64_t bf_bits) {
   if (!out) return set_err(MG_ERR_ARG, "out is NULL");
   *out = nullptr;
@@ -199,48 +214,51 @@ extern "C" int mg_create(mg_ctx **out, int device, int k, int ref_k, uint64_t bf
     return set_err(MG_ERR_ARG, "unsupported k=%d ref_k=%d (need 1 <= k <= 63, k <= ref_k <= 64)", k, ref_k);
   if (bf_bits == 0) return set_err(MG_ERR_ARG, "bf_bits must be > 0 (the reference divides by it)");
   if (bf_bits >= (1ull << 40)) return set_err(MG_ERR_ARG, "bf_bits must be < 2^40");
-  int ndev = 0;
-  CU(cudaGetDeviceCount(&ndev));
-  if (device < 0 || device >= ndev) return set_err(MG_ERR_CUDA, "device %d not available (%d visible)", device, ndev);
-  CU(cudaSetDevice(device));
+  int rc = check_device(device);
+  if (rc) return rc;
   mg_ctx *c = new mg_ctx();
   c->device = device;
   c->k = k;
   c->ref_k = ref_k;
   c->bf_bits = bf_bits;
-  int rc = ctx_init(c);
-  if (rc) {  // (e.g. out of device memory for a large -b): nothing is left behind
-    char msg[sizeof(g_err)];
-    memcpy(msg, g_err, sizeof(msg));
-    mg_destroy(c);
-    memcpy(g_err, msg, sizeof(msg));
+  rc = ctx_init(c);
+  if (rc) {
+    destroy_keep_error(c);
     return rc;
   }
   *out = c;
   return MG_OK;
 }
 
-static int ctx_init(mg_ctx *c) {
-  const int device = c->device;
-  const uint64_t bf_bits = c->bf_bits;
-  c->n_lines = (bf_bits + 255) / 256;
-  c->n_ctx_words = c->n_lines * 8;
+// The arrays every context owns from its creation: streams, probe lines, context filter, the key counts of the wide
+// layout and the occupancy pre-filter (n_lines, n_ctx_words and n_occ_words set by the caller).  Only the tables no
+// index image carries are filled here; the caller clears the rest (mg_create) or overwrites it (mg_replicate).
+static int ctx_alloc(mg_ctx *c) {
   cudaDeviceProp prop;
-  CU(cudaGetDeviceProperties(&prop, device));
+  CU(cudaGetDeviceProperties(&prop, c->device));
   c->sms = prop.multiProcessorCount;
   if (const char *e = getenv("MG_SCAN_DEFER_HITS")) c->defer_hits = atoi(e) != 0;
   for (int i = 0; i < 2; ++i) CU(cudaStreamCreateWithFlags(&c->stream[i], cudaStreamNonBlocking));
   CU(cudaMalloc(&c->lines, c->n_lines * 128));
   CU(cudaMalloc(&c->ctx_words, c->n_ctx_words * 4));
-  c->launches++;
-  mg::k_init_lines<<<grid_for(c->n_lines * mg::LINE_U4, 256), 256, 0, c->stream[0]>>>(c->lines, c->n_lines,
-                                                                                      mg::key_hi_mask_for(c->k));
-  CU(cudaGetLastError());
-  CU(cudaMemsetAsync(c->ctx_words, 0, c->n_ctx_words * 4, c->stream[0]));
-  if (c->k > mg::INLINE_MAX_K) {  // wide keys leave no room for the count inside the slot
+  if (c->k > mg::INLINE_MAX_K)  // wide keys leave no room for the count inside the slot
     CU(cudaMalloc(&c->key_counts, c->n_lines * mg::LINE_KEYS * 4));
-    CU(cudaMemsetAsync(c->key_counts, 0, c->n_lines * mg::LINE_KEYS * 4, c->stream[0]));
+  if (c->n_occ_words) CU(cudaMalloc(&c->occ, c->n_occ_words * 4));
+  {  // log_binomial's logs of small integers from the reference's libm: GT of exact ties comes from their last bits
+    std::vector<double> tab(mg::LOG_TABLE_N, 0.0);
+    for (int i = 1; i < mg::LOG_TABLE_N; ++i) tab[i] = log((double)i);
+    CU(cudaMalloc(&c->log_table, tab.size() * sizeof(double)));
+    CU(cudaMemcpy(c->log_table, tab.data(), tab.size() * sizeof(double), cudaMemcpyHostToDevice));
   }
+  CU(cudaMalloc(&c->d_scalars, 8 * sizeof(unsigned long long)));
+  CU(cudaMemsetAsync(c->d_scalars, 0, 8 * sizeof(unsigned long long), c->stream[0]));
+  return MG_OK;
+}
+
+static int ctx_init(mg_ctx *c) {
+  const uint64_t bf_bits = c->bf_bits;
+  c->n_lines = (bf_bits + 255) / 256;
+  c->n_ctx_words = c->n_lines * 8;
   // occupancy pre-filter: at most 2^MG_OCC_LOG2_BITS bits (default 2^29 = 64 MB: half of the 126 MB L2, the measured optimum)
   {
     int cap_log2 = 29;
@@ -251,20 +269,19 @@ static int ctx_init(mg_ctx *c) {
       while (((bf_bits - 1) >> c->occ_shift) + 1 > (1ull << cap_log2)) ++c->occ_shift;
       c->n_occ_words = ((((bf_bits - 1) >> c->occ_shift) + 1) + 31) / 32;
       c->n_occ_words = (c->n_occ_words + 3) & ~3ull;  // whole 16-byte pieces (the scan copies them with cp.async)
-      CU(cudaMalloc(&c->occ, c->n_occ_words * 4));
-      CU(cudaMemsetAsync(c->occ, 0, c->n_occ_words * 4, c->stream[0]));
     }
   }
-  {  // log_binomial's logs of small integers from the reference's libm: GT of exact ties comes from their last bits
-    std::vector<double> tab(mg::LOG_TABLE_N, 0.0);
-    for (int i = 1; i < mg::LOG_TABLE_N; ++i) tab[i] = log((double)i);
-    CU(cudaMalloc(&c->log_table, tab.size() * sizeof(double)));
-    CU(cudaMemcpy(c->log_table, tab.data(), tab.size() * sizeof(double), cudaMemcpyHostToDevice));
-  }
-  CU(cudaMalloc(&c->d_scalars, 8 * sizeof(unsigned long long)));
-  CU(cudaMemsetAsync(c->d_scalars, 0, 8 * sizeof(unsigned long long), c->stream[0]));
+  int rc = ctx_alloc(c);
+  if (rc) return rc;
+  c->launches++;
+  mg::k_init_lines<<<grid_for(c->n_lines * mg::LINE_U4, 256), 256, 0, c->stream[0]>>>(c->lines, c->n_lines,
+                                                                                      mg::key_hi_mask_for(c->k));
+  CU(cudaGetLastError());
+  CU(cudaMemsetAsync(c->ctx_words, 0, c->n_ctx_words * 4, c->stream[0]));
+  if (c->key_counts) CU(cudaMemsetAsync(c->key_counts, 0, c->n_lines * mg::LINE_KEYS * 4, c->stream[0]));
+  if (c->occ) CU(cudaMemsetAsync(c->occ, 0, c->n_occ_words * 4, c->stream[0]));
   c->ovf_log2 = 10;
-  int rc = ovf_alloc(c, c->ovf_log2, &c->ovf_keys, &c->ovf_counts);
+  rc = ovf_alloc(c, c->ovf_log2, &c->ovf_keys, &c->ovf_counts);
   if (rc) return rc;
   CU(cudaStreamSynchronize(c->stream[0]));
   return MG_OK;
@@ -633,6 +650,76 @@ extern "C" int mg_finalize_alt(mg_ctx *c) {
   if (rc) return rc;
   c->alt_final = true;
   return pin_occ_in_l2(c);
+}
+
+// The index image is canonical (canonicalize_keys), so a replica is a copy of the device arrays: no inserts, no
+// rank pass, no canonicalisation.  cudaMemcpyPeerAsync serves every pair of contexts -- two devices, with or without
+// peer access, and two contexts on one device.
+static int replicate_into(mg_ctx *c, const mg_ctx *src) {
+  c->k = src->k;
+  c->ref_k = src->ref_k;
+  c->bf_bits = src->bf_bits;
+  c->n_lines = src->n_lines;
+  c->n_ctx_words = src->n_ctx_words;
+  c->occ_shift = src->occ_shift;
+  c->n_occ_words = src->n_occ_words;
+  int rc = ctx_alloc(c);
+  if (rc) return rc;
+  c->bf_ones = src->bf_ones;
+  c->n_keys = src->n_keys;
+  c->ovf_n = src->ovf_n;
+  c->ovf_log2 = src->ovf_log2;
+  c->alt_final = src->alt_final;
+  c->ctx_final = src->ctx_final;
+  c->irregular_ref = src->irregular_ref;
+  const uint64_t bf_count_bytes = (c->bf_ones ? c->bf_ones : 1) * 4, ovf_cap = 1ull << c->ovf_log2;
+  CU(cudaMalloc(&c->bf_counts, bf_count_bytes));
+  CU(cudaMalloc(&c->ovf_keys, ovf_cap * sizeof(u128)));
+  CU(cudaMalloc(&c->ovf_counts, ovf_cap * sizeof(uint32_t)));
+  if (c->device != src->device) {  // (a direct copy over NVLink where the devices allow it; staged otherwise)
+    int can = 0;
+    CU(cudaDeviceCanAccessPeer(&can, c->device, src->device));
+    if (can) {
+      cudaError_t e = cudaDeviceEnablePeerAccess(src->device, 0);
+      if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled)
+        return set_err(MG_ERR_CUDA, "cudaDeviceEnablePeerAccess(%d) -> %s", src->device, cudaGetErrorString(e));
+      cudaGetLastError();
+    }
+  }
+  const struct {
+    void *dst;
+    const void *from;
+    uint64_t bytes;
+  } arrays[] = {{c->lines, src->lines, c->n_lines * 128},  // (the live alt and inline key counters included)
+                {c->ctx_words, src->ctx_words, c->n_ctx_words * 4},
+                {c->occ, src->occ, c->n_occ_words * 4},
+                {c->bf_counts, src->bf_counts, bf_count_bytes},
+                {c->key_counts, src->key_counts, c->key_counts ? c->n_lines * mg::LINE_KEYS * 4 : 0},
+                {c->ovf_keys, src->ovf_keys, ovf_cap * sizeof(u128)},
+                {c->ovf_counts, src->ovf_counts, ovf_cap * sizeof(uint32_t)}};
+  for (const auto &a : arrays)
+    if (a.bytes) CU(cudaMemcpyPeerAsync(a.dst, c->device, a.from, src->device, a.bytes, c->stream[0]));
+  CU(cudaStreamSynchronize(c->stream[0]));
+  return pin_occ_in_l2(c);
+}
+
+extern "C" int mg_replicate(mg_ctx **out, mg_ctx *src, int device) {
+  if (!out || !src) return set_err(MG_ERR_ARG, "NULL argument");
+  *out = nullptr;
+  if (!src->alt_final) return set_err(MG_ERR_STATE, "mg_replicate before mg_finalize_alt");
+  int rc = mg_sync(src);  // (the scans enqueued so far are in the copied counters)
+  if (rc) return rc;
+  rc = check_device(device);
+  if (rc) return rc;
+  mg_ctx *c = new mg_ctx();
+  c->device = device;
+  rc = replicate_into(c, src);
+  if (rc) {
+    destroy_keep_error(c);
+    return rc;
+  }
+  *out = c;
+  return MG_OK;
 }
 
 // ---- dense counter image (index.cuh): gather before a reduce / download, scatter after a reduce ----
