@@ -173,10 +173,21 @@ void mg_count_destroy(mg_counter *c);
 int mg_count_set_partition(mg_counter *c, int part_bits, uint32_t part_lo, uint32_t part_hi);
 int mg_count_reset(mg_counter *c);
 int mg_count_add(mg_counter *c, const char *bases, uint64_t n);
+/* Counting restricted to what ctx's index can use: from then on mg_count_add inserts only the ref_k-mers whose
+ * central k-mer (taken as the sample scan takes it from a record) sets a bit of ctx's bf or is a key of its ref_bf.
+ * Every other ref_k-mer changes no counter in mg_scan_counted, and every occurrence of a ref_k-mer gets the same
+ * answer, so restricted counting + mg_scan_counted leaves exactly the counters of unrestricted counting; the table
+ * only holds the ref_k-mers that matter.  A partition still applies on top.  Needs c and ctx on one device,
+ * c's k == ctx's ref_k (MG_ERR_ARG), ctx past mg_finalize_alt and an empty counter -- fresh or just reset
+ * (MG_ERR_STATE).  The counter keeps the pointer and reads ctx's index at every mg_count_add: ctx must outlive the
+ * restricted adds.  ctx == NULL lifts the restriction (also on an empty counter only). */
+int mg_count_restrict(mg_counter *c, mg_ctx *ctx);
 int mg_count_finish(mg_counter *c, uint32_t min_count, uint32_t counter_max, uint64_t max_count, uint64_t *n_kmers);
 int mg_count_download(mg_counter *c, uint64_t *lohi, uint32_t *counts, uint64_t cap);
 /* {distinct k-mers in the table, k-mer instances counted, table capacity, kernels launched[, device time of the
- * counting kernels in microseconds]}; n >= 4 */
+ * counting kernels in microseconds[, valid windows examined]]}; n >= 4.  Windows are counted before the partition and
+ * index tests of a restricted counter; an unrestricted counter reports its instances there (without a partition
+ * it inserts every valid window). */
 int mg_count_stats(mg_counter *c, uint64_t *stats, int n);
 /* the counted k-mers straight into the sample scan (same device): no database file, no host round trip */
 int mg_scan_counted(mg_ctx *ctx, mg_counter *c);

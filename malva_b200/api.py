@@ -554,6 +554,13 @@ class KmerCounter:
     def reset(self):
         check(self._L.mg_count_reset(self._h))
 
+    def restrict(self, g: "MalvaGpu | None") -> None:
+        """Count from now on only the ref_k-mers that ``g``'s index can use (``mg_count_restrict``): their central
+        k-mer sets a bit of bf or is a ref key.  ``scan_counted`` then gives ``g`` the counters an unrestricted count
+        would.  Needs an empty counter (fresh or just reset) and ``g`` past ``finalize_alt``; ``g`` must stay open
+        while restricted adds run.  ``None`` lifts the restriction."""
+        check(self._L.mg_count_restrict(self._h, g._h if g is not None else None))
+
     def add(self, reads) -> None:
         b = reads if isinstance(reads, (bytes, bytearray)) else "\n".join(reads).encode()
         check(self._L.mg_count_add(self._h, bytes(b), len(b)))
@@ -568,9 +575,9 @@ class KmerCounter:
         return keys, counts
 
     def stats(self) -> dict:
-        s = (C.c_uint64 * 5)()
-        check(self._L.mg_count_stats(self._h, s, 5))
-        return dict(zip(("distinct", "instances", "capacity", "launches", "kernel_us"), [int(x) for x in s]))
+        s = (C.c_uint64 * 6)()
+        check(self._L.mg_count_stats(self._h, s, 6))
+        return dict(zip(("distinct", "instances", "capacity", "launches", "kernel_us", "windows"), [int(x) for x in s]))
 
 
 def diag_bandwidth(device: int, mode: int, nbytes: int, reps: int = 3) -> float:

@@ -9,6 +9,7 @@
 //                   complement shifting right) and a run length of valid symbols, and inserts the canonical word of
 //                   every valid window into an open-addressing table of 32-byte slots {key 16 B, count 4 B}: one
 //                   16-byte read of the home slot, a 128-bit CAS only when the slot is empty, one atomicAdd.
+//                   Restricted builds (mg_count_restrict) insert only the windows the index can use (index_hit).
 //   k_count_rehash  table growth (load factor <= 0.5)
 //   k_count_emit    kept entries (count >= min_count, saturated) appended to dense arrays; a radix sort by key then
 //                   gives KMC's listing order.
@@ -64,15 +65,39 @@ __device__ __forceinline__ void count_insert(CountSlot *table, uint64_t mask, u1
   }
 }
 
+// Restricted counting (mg_count_restrict): whether the sample scan can do anything with the canonical ref_k-mer
+// `canon` -- its central kc-mer, taken as k_scan takes it from a KMC record, sets a bit of bf or is a ref key of
+// ref_bf.  Decided from the filter bits and the keys of the probe line only (immutable after mg_finalize_alt), so
+// every occurrence of a ref_k-mer gets the same answer.  KC: kc specialised (K = 0: v.k).
+template <int KC>
+__device__ __forceinline__ bool index_hit(const DevView &v, u128 canon, int ref_k) {
+  const int kc = KC > 0 ? KC : v.k;
+  const int tail = ref_k - kc - (ref_k - kc) / 2;  // (as k_scan: bases of the context after the k-mer)
+  u128 c;
+  const uint64_t idx = bf_index(v, canon_hash_k<KC>(mask128(shr128(canon, 2 * tail), 2 * kc), kc, &c));
+  if (!occ_test(v, idx)) return false;  // (L2: the probe line holds nothing for this k-mer)
+  const auto at = line_at(v, idx >> 8);
+  int j;
+  uint4 m;
+  if (line_alt(at, (uint32_t)(idx & 255), &j, &m)) return true;
+  uint32_t w3;
+  bool ovf;
+  if (line_key<KC>(v, at, c, &w3, &ovf) >= 0) return true;
+  return ovf && ovf_find(v, c) >= 0;
+}
+
 // seq: read bytes, records separated by any non-ACGT byte (the host puts '\n' between reads).  Window end
 // positions [k-1, len).  Only canonical k-mers whose top `part_bits` bits fall in [part_lo, part_hi) are counted
 // (prefix-partitioned passes for inputs whose distinct k-mers do not fit the table at once; part_bits = 0: all).
-template <int K>
+// KC < 0: every k-mer.  KC >= 0 (restricted, k = v.ref_k): only the k-mers index_hit<KC> keeps; *n_windows then
+// counts the valid windows, before the partition and index tests.
+template <int K, int KC>
 __global__ void __launch_bounds__(CNT_THREADS) k_count_kmers(const uint8_t *__restrict__ seq, uint64_t len, int k_rt,
                                                             CountSlot *table, uint64_t mask, int part_bits,
                                                             uint32_t part_lo, uint32_t part_hi,
                                                             unsigned long long *n_distinct,
-                                                            unsigned long long *n_instances) {
+                                                            unsigned long long *n_instances, DevView v,
+                                                            unsigned long long *n_windows) {
   extern __shared__ uint8_t cnt_sm[];
   const int k = K > 0 ? K : k_rt;
   uint64_t p0 = (uint64_t)(k - 1) + (uint64_t)blockIdx.x * CNT_TILE;
@@ -110,19 +135,24 @@ __global__ void __launch_bounds__(CNT_THREADS) k_count_kmers(const uint8_t *__re
   };
   int o = (int)(q0 - base) - (k - 1);
   for (int j = 0; j < k - 1; ++j) push(cnt_sm[o + j]);
-  uint32_t mine = 0;
+  uint32_t mine = 0, seen = 0;
   for (uint64_t p = q0; p < q1; ++p) {
     push(cnt_sm[(int)(p - base)]);
     if (run < k) continue;
     u128 canon = less128(r, f) ? r : f;  // (ties: the two strands are the same word)
+    if constexpr (KC >= 0) ++seen;
     if (part_bits) {
       uint32_t part = (uint32_t)(shr128(canon, 2 * k - part_bits).lo);
       if (part < part_lo || part >= part_hi) continue;
     }
+    if constexpr (KC >= 0)
+      if (!index_hit<KC>(v, canon, k)) continue;
     count_insert(table, mask, canon, 1u, n_distinct);
     ++mine;
   }
   if (mine) atomicAdd(n_instances, (unsigned long long)mine);
+  if constexpr (KC >= 0)
+    if (seen) atomicAdd(n_windows, (unsigned long long)seen);
 }
 
 __global__ void k_count_clear(CountSlot *table, uint64_t cap) {

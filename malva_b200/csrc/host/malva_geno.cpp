@@ -3,6 +3,9 @@
 //   malva-geno index [flags] <reference.fa> <variants.vcf> <kmc_output_prefix>
 //   malva-geno call  [flags] <reference.fa> <variants.vcf> <kmc_output_prefix>   > out.vcf
 //   malva-geno call  [flags] <reference.fa> <variants.vcf> <db1> <db2> .. --out-dir DIR   (DIR/<basename>.vcf each)
+//   malva-geno call  [flags] <reference.fa> <variants.vcf> <reads.fq|fa[.gz]> [<reads2> .. --out-dir DIR] --reads
+//        genotype straight from reads: each sample is counted on the device, only the ref_k-mers the index can use
+//        (mg_count_restrict), and scanned from the count table -- the VCFs of `count` + `call DB`, no database on disk
 //
 // Same sub-commands, flags (-k -r -e -s -f -c -b -p -u -v -1), index file name, stderr phase lines and VCF
 // output as the reference (main.cpp:226-594, argument_parser.hpp:51-159).  The host keeps VCF/FASTA reading and
@@ -18,9 +21,11 @@
 //     thread, and a batch the last stage is done with goes back to the first (its buffers keep their pages);
 //   * the KMC database is not decoded on the host: raw suffix records stream through pinned buffers into
 //     mg_scan_kmc_records;
+//   * with --reads there is no database: the reads are counted on the device and scanned from the count table;
 //   * the index file holds sparse lists (index_file.hpp).
 //
-// Extra (non-reference) flags: --threads N, --device N, --trace.  Extra sub-commands:
+// Extra (non-reference) flags: --threads N, --device N, --devices, --out-dir, --sample-devices, --reads, --trace.
+// Extra sub-commands:
 //   malva-geno count [-k43 -ci2 -cs255 ...] <reads.fq|fa[.gz]> <kmc_output_prefix> [tmp_dir]
 //        the `kmc` step of the MALVA wrapper (MALVA:107) on the GPU: same command-line shape as kmc, writes a KMC
 //        database that `index` / `call` (and the reference) read
@@ -87,6 +92,9 @@ const char *USAGE =
     "          --sample-devices A,B,..       call with --out-dir: replicate the index on these devices (a device may\n"
     "                                        repeat) and scan and genotype a share of every round's samples on each\n"
     "                                        (instead of --device / --devices)\n"
+    "          --reads                       call: the samples are FASTA/FASTQ read files (plain or gz), not KMC\n"
+    "                                        databases; each is counted on the device (as `count` -k<ref_k> -ci2\n"
+    "                                        -cs255 would) and genotyped, no database is written (not with --devices)\n"
     "\n";
 
 struct Options {
@@ -104,6 +112,7 @@ struct Options {
   std::string fasta_path, vcf_path, kmc_path;
   std::vector<std::string> kmc_paths;  // call: one or more KMC databases (kmc_path = the first)
   std::string out_dir;                 // call with several databases: sample P is written to out_dir/basename(P).vcf
+  bool reads = false;                  // --reads: call's samples (kmc_paths) are read files, counted on the device
 };
 
 // argument_parser.hpp:86-159; values are read like `istringstream >> x` reads them
@@ -130,6 +139,7 @@ bool parse_arguments(int argc, char **argv, Options &o, int n_positional, bool m
                                     {"devices", required_argument, nullptr, 1004},
                                     {"out-dir", required_argument, nullptr, 1005},
                                     {"sample-devices", required_argument, nullptr, 1006},
+                                    {"reads", no_argument, nullptr, 1007},
                                     {nullptr, 0, nullptr, 0}};
   bool die = false;
   optind = 1;
@@ -167,6 +177,7 @@ bool parse_arguments(int argc, char **argv, Options &o, int n_positional, bool m
         break;
       }
       case 1005: o.out_dir = optarg ? optarg : ""; break;
+      case 1007: o.reads = true; break;
       case '?': die = true; break;
       case 'h':
         std::cout << USAGE;
@@ -905,6 +916,138 @@ int container_selftest_main() {
   return bad ? 1 : 0;
 }
 
+struct ReadFeeder {
+  // sequences of a FASTA / FASTQ file (plain or gz), upper-cased, '\n' between records, in chunks of whole records.
+  // Lines are taken block-wise as views (no per-line allocation); FASTQ records are four lines (header, sequence,
+  // '+', qualities), FASTA sequences may span lines.
+  explicit ReadFeeder(const std::string &path) : in_(path) {}
+  bool next_chunk(std::string &out, size_t target) {
+    out.clear();
+    while (out.size() < target) {
+      if (li_ == lines_.size()) {
+        if (done_) break;
+        li_ = 0;
+        if (!in_.next_block(store_, lines_, 1u << 20, 32u << 20, true)) done_ = true;
+        if (lines_.empty()) continue;
+      }
+      for (; li_ < lines_.size() && out.size() < target; ++li_) {
+        const char *b = lines_[li_].b, *e = lines_[li_].e;
+        if (format_ == 0) {
+          if (b == e) continue;                   // blank lines before the first record
+          format_ = *b == '>' ? 1 : 2;            // by the first byte of the file, whatever -f says
+        }
+        if (format_ == 1 && b == e) continue;     // blank line inside a FASTA file
+        if (format_ == 2) {  // FASTQ
+          if (phase_ == 1) {
+            append_upper(out, b, e);
+            out.push_back('\n');
+          }
+          phase_ = (phase_ + 1) & 3;
+        } else if (*b == '>') {  // FASTA header: the previous record ends here
+          if (open_) out.push_back('\n');
+          open_ = true;
+        } else {
+          append_upper(out, b, e);
+        }
+      }
+      if (format_ == 1 && open_ && out.size() >= target) {  // a FASTA record larger than a chunk is cut with k-mers
+        // lost at the seam only if a chunk ends inside it: keep going to the end of the record instead
+        while (true) {
+          if (li_ == lines_.size()) {
+            if (done_) break;
+            li_ = 0;
+            if (!in_.next_block(store_, lines_, 1u << 20, 32u << 20, true)) done_ = true;
+            if (lines_.empty()) continue;
+          }
+          if (lines_[li_].b != lines_[li_].e && *lines_[li_].b == '>') break;
+          append_upper(out, lines_[li_].b, lines_[li_].e);
+          ++li_;
+        }
+      }
+    }
+    if (done_ && li_ == lines_.size() && open_) {
+      out.push_back('\n');
+      open_ = false;
+    }
+    return !out.empty();
+  }
+
+ private:
+  static void append_upper(std::string &out, const char *b, const char *e) {
+    const size_t o = out.size();
+    out.resize(o + (size_t)(e - b));
+    char *d = &out[o];
+    for (const char *p = b; p < e; ++p) *d++ = (char)(*p & 0xDF);  // a-z -> A-Z; nothing else can become A, C, G or T
+  }
+  mh::BlockLineReader in_;
+  mh::TextBuf store_;
+  std::vector<mh::BlockLineReader::View> lines_;
+  size_t li_ = 0;
+  int format_ = 0, phase_ = 0;
+  bool done_ = false, open_ = false;
+};
+
+struct Counter {
+  mg_counter *c = nullptr;
+  ~Counter() { mg_count_destroy(c); }
+};
+
+constexpr size_t READ_CHUNK = 64u << 20;  // read bytes per mg_count_add (count and call --reads)
+
+// STEP 2 with --reads: the sample's reads counted on the device, restricted to the ref_k-mers the index of c can use,
+// then scanned from there (mg_scan_counted).  The counters end up as they would after `count` (-ci2 -cs255 -cx1e9,
+// its defaults and the MALVA wrapper's) and the scan of that database, with no database written.  A thread parses
+// the next chunk of reads while the device counts this one.
+void scan_reads(const Options &o, mg_ctx *c, mg_counter *cn, const std::string &path) {
+  Stopwatch sw;
+  uint64_t st0[6] = {}, st[6] = {};  // (the device time of the counting kernels adds up over the counter's life)
+  if (o.trace) gpu(mg_count_stats(cn, st0, 6), "mg_count_stats");
+  gpu(mg_count_reset(cn), "mg_count_reset");
+  gpu(mg_count_restrict(cn, c), "mg_count_restrict");
+  ReadFeeder feed(path);
+  std::string cur, next;
+  uint64_t bytes = 0;
+  double t_read = 0, t_wait = 0, t_count = 0;
+  bool more = feed.next_chunk(cur, READ_CHUNK);
+  t_read += sw.lap();
+  while (more) {
+    std::future<bool> ahead = std::async(std::launch::async, [&] {
+      Stopwatch r;
+      const bool m = feed.next_chunk(next, READ_CHUNK);
+      t_read += r.lap();
+      return m;
+    });
+    bytes += cur.size();
+    gpu(mg_count_add(cn, cur.data(), cur.size()), "mg_count_add");
+    t_count += sw.lap();
+    more = ahead.get();
+    t_wait += sw.lap();
+    std::swap(cur, next);
+  }
+  uint64_t n = 0;
+  gpu(mg_count_finish(cn, 2, 255, 1000000000ull, &n), "mg_count_finish");
+  gpu(mg_scan_counted(c, cn), "mg_scan_counted");
+  t_count += sw.lap();
+  if (o.trace) {
+    gpu(mg_count_stats(cn, st, 6), "mg_count_stats");
+    fprintf(stderr, "[trace] reads %s: %llu read bytes, %llu windows examined, %llu distinct kept (%llu seen twice or "
+                    "more), table capacity %llu slots; reading %.1f ms (%.1f ms waited for), counting + scan %.1f ms "
+                    "(counting kernels %.1f ms)\n",
+            path.c_str(), (unsigned long long)bytes, (unsigned long long)st[5], (unsigned long long)st[0],
+            (unsigned long long)n, (unsigned long long)st[2], t_read, t_wait, t_count, (double)(st[4] - st0[4]) * 1e-3);
+  }
+}
+
+// Before every chunk, a counter's table grows to 2 x (distinct + chunk) slots, so that an insert never meets a full
+// table: from the second 64 MB chunk of a sample on, 2^28 slots (8.6 GB).  Sample sets take the device memory left
+// free, so a cohort grows its counters to that size before it plans them: one poly-A read and 128 MB of record
+// separators.
+void grow_counter(mg_counter *cn, unsigned k) {
+  std::string warm(2 * READ_CHUNK, '\n');
+  std::fill_n(warm.begin(), k, 'A');
+  gpu(mg_count_add(cn, warm.data(), warm.size()), "mg_count_add");
+}
+
 // STEP 2: the sample k-mer scan (main.cpp:482-500) of one database.  Raw suffix records go through rings of pinned
 // buffers, one ring per device, chunks dealt round-robin; the library copies and scans them asynchronously
 // (double-buffered on its side), a buffer is refilled only after the event recorded behind its scan has completed.
@@ -1108,6 +1251,28 @@ int call_main(int argc, char **argv) {
                   << std::endl;
         return 1;
       }
+  if (o.reads) {
+    if (o.devices.size() > 1) {
+      std::cerr << "ERROR: --reads takes no --devices: the counts of one sample are complete only after all its reads "
+                   "(k-mers seen once are dropped), so its reads cannot be dealt over devices; several read files go "
+                   "over devices with --sample-devices A,B,.."
+                << std::endl;
+      return 1;
+    }
+    if (o.ref_k > 63) {
+      std::cerr << "ERROR: --reads counts the ref k-mers on the device, which counts k <= 63 (-r " << o.ref_k << ")"
+                << std::endl;
+      return 1;
+    }
+    for (const std::string &path : o.kmc_paths) {
+      FILE *f = fopen(path.c_str(), "rb");
+      if (!f) {
+        std::cerr << "ERROR: cannot open " << path << std::endl;
+        return 1;
+      }
+      fclose(f);
+    }
+  }
   if (!o.sample_devices.empty()) {  // (before any file is read; without a usable driver mg_create fails as for --devices)
     const int visible = mg_device_count();
     for (int d : o.sample_devices)
@@ -1127,7 +1292,7 @@ int call_main(int argc, char **argv) {
     return 1;
   }
   std::vector<std::unique_ptr<mh::KmcDb>> dbs;  // every database is opened before any work
-  for (const std::string &path : o.kmc_paths) {
+  for (const std::string &path : o.reads ? std::vector<std::string>() : o.kmc_paths) {
     dbs.push_back(std::make_unique<mh::KmcDb>());
     std::string why;
     if (!dbs.back()->open(path, why)) {
@@ -1161,6 +1326,12 @@ int call_main(int argc, char **argv) {
   }
   std::vector<mg_ctx *> cs;
   for (Ctx &x : gs) cs.push_back(x.c);
+  // --reads: one counter per context, reset between its samples (its table keeps the size it grew to)
+  std::vector<Counter> counters(o.reads ? (size_t)n_ctx : 0);
+  for (size_t i = 0; i < counters.size(); ++i) {
+    gpu(mg_count_create(&counters[i].c, ctx_devices[i], (int)o.ref_k), "mg_count_create");
+    if (n_db > 1) grow_counter(counters[i].c, o.ref_k);
+  }
   pelapsed("Reference parsing");
   std::map<std::string, std::string> refs = refs_ready.get();
   pelapsed("Reference processed");
@@ -1169,7 +1340,10 @@ int call_main(int argc, char **argv) {
 
   if (n_db == 1) {
     pelapsed("KMC output processing");
-    scan_kmc(o, cs, *dbs[0], o.kmc_path);
+    if (o.reads)
+      scan_reads(o, g.c, counters[0].c, o.kmc_path);
+    else
+      scan_kmc(o, cs, *dbs[0], o.kmc_path);
     for (size_t d = 1; d < gs.size(); ++d) {  // the replicas are no longer needed
       mg_destroy(gs[d].c);
       gs[d].c = nullptr;
@@ -1220,9 +1394,15 @@ int call_main(int argc, char **argv) {
       std::vector<size_t> set_first(set_n.size(), first);
       for (size_t i = 1; i < set_n.size(); ++i) set_first[i] = set_first[i - 1] + (size_t)set_n[i - 1];
       parallel_for(set_ctx.size(), (int)set_ctx.size(), [&](size_t i) {
+        mg_counter *cn = nullptr;
+        for (size_t j = 0; j < (size_t)n_ctx && o.reads; ++j)
+          if (cs[j] == set_ctx[i]) cn = counters[j].c;
         for (int s = 0; s < set_n[i]; ++s) {
           const size_t db = set_first[i] + (size_t)s;
-          scan_kmc(o, {set_ctx[i]}, *dbs[db], o.kmc_paths[db]);
+          if (o.reads)
+            scan_reads(o, set_ctx[i], cn, o.kmc_paths[db]);
+          else
+            scan_kmc(o, {set_ctx[i]}, *dbs[db], o.kmc_paths[db]);
           gpu(mg_samples_take(set_ctx[i], s), "mg_samples_take");
         }
       });
@@ -1320,82 +1500,6 @@ int signatures_main(int argc, char **argv) {
 // value like kmc's (-k43) or separated (-k 43); -m / -t / -f* / the tmp directory are accepted and ignored (the file
 // format is detected from its first byte).  --passes N counts in N prefix-partitioned passes over the reads for
 // inputs whose distinct k-mers do not fit device memory at once.
-struct ReadFeeder {
-  // sequences of a FASTA / FASTQ file (plain or gz), upper-cased, '\n' between records, in chunks of whole records.
-  // Lines are taken block-wise as views (no per-line allocation); FASTQ records are four lines (header, sequence,
-  // '+', qualities), FASTA sequences may span lines.
-  explicit ReadFeeder(const std::string &path) : in_(path) {}
-  bool next_chunk(std::string &out, size_t target) {
-    out.clear();
-    while (out.size() < target) {
-      if (li_ == lines_.size()) {
-        if (done_) break;
-        li_ = 0;
-        if (!in_.next_block(store_, lines_, 1u << 20, 32u << 20, true)) done_ = true;
-        if (lines_.empty()) continue;
-      }
-      for (; li_ < lines_.size() && out.size() < target; ++li_) {
-        const char *b = lines_[li_].b, *e = lines_[li_].e;
-        if (format_ == 0) {
-          if (b == e) continue;                   // blank lines before the first record
-          format_ = *b == '>' ? 1 : 2;            // by the first byte of the file, whatever -f says
-        }
-        if (format_ == 1 && b == e) continue;     // blank line inside a FASTA file
-        if (format_ == 2) {  // FASTQ
-          if (phase_ == 1) {
-            append_upper(out, b, e);
-            out.push_back('\n');
-          }
-          phase_ = (phase_ + 1) & 3;
-        } else if (*b == '>') {  // FASTA header: the previous record ends here
-          if (open_) out.push_back('\n');
-          open_ = true;
-        } else {
-          append_upper(out, b, e);
-        }
-      }
-      if (format_ == 1 && open_ && out.size() >= target) {  // a FASTA record larger than a chunk is cut with k-mers
-        // lost at the seam only if a chunk ends inside it: keep going to the end of the record instead
-        while (true) {
-          if (li_ == lines_.size()) {
-            if (done_) break;
-            li_ = 0;
-            if (!in_.next_block(store_, lines_, 1u << 20, 32u << 20, true)) done_ = true;
-            if (lines_.empty()) continue;
-          }
-          if (lines_[li_].b != lines_[li_].e && *lines_[li_].b == '>') break;
-          append_upper(out, lines_[li_].b, lines_[li_].e);
-          ++li_;
-        }
-      }
-    }
-    if (done_ && li_ == lines_.size() && open_) {
-      out.push_back('\n');
-      open_ = false;
-    }
-    return !out.empty();
-  }
-
- private:
-  static void append_upper(std::string &out, const char *b, const char *e) {
-    const size_t o = out.size();
-    out.resize(o + (size_t)(e - b));
-    char *d = &out[o];
-    for (const char *p = b; p < e; ++p) *d++ = (char)(*p & 0xDF);  // a-z -> A-Z; nothing else can become A, C, G or T
-  }
-  mh::BlockLineReader in_;
-  mh::TextBuf store_;
-  std::vector<mh::BlockLineReader::View> lines_;
-  size_t li_ = 0;
-  int format_ = 0, phase_ = 0;
-  bool done_ = false, open_ = false;
-};
-
-struct Counter {
-  mg_counter *c = nullptr;
-  ~Counter() { mg_count_destroy(c); }
-};
-
 int count_main(int argc, char **argv) {
   unsigned k = 43, ci = 2, cs = 255, passes = 1;
   unsigned long long cx = 1000000000ull;
@@ -1441,7 +1545,7 @@ int count_main(int argc, char **argv) {
     }
     ReadFeeder feed(pos[0]);
     std::string chunk;
-    while (feed.next_chunk(chunk, 64u << 20)) {
+    while (feed.next_chunk(chunk, READ_CHUNK)) {
       if (p == 0) total_bases += chunk.size();
       gpu(mg_count_add(cn.c, chunk.data(), chunk.size()), "mg_count_add");
     }

@@ -17,14 +17,6 @@
 
 namespace mg {
 
-template <int K>
-__device__ __forceinline__ uint64_t canon_hash_k(u128 x, int k, u128 *canon) {
-  if constexpr (K > 0) {
-    return canon_hash<K>(x, canon);
-  } else {
-    return canon_hash_rt(x, k, canon);
-  }
-}
 __device__ __forceinline__ u128 u128_of(uint4 q) {
   u128 r;
   r.lo = (uint64_t)q.x | ((uint64_t)q.y << 32);

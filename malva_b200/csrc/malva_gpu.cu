@@ -46,7 +46,7 @@ static int set_err(int code, const char *fmt, ...) {
   } while (0)
 
 extern "C" const char *mg_last_error(void) { return g_err; }
-extern "C" int mg_version(void) { return 202; }
+extern "C" int mg_version(void) { return 203; }
 extern "C" int mg_device_count(void) {
   int n = 0;
   cudaError_t e = cudaGetDeviceCount(&n);
@@ -1760,12 +1760,15 @@ struct mg_counter {
   uint32_t part_lo = 0, part_hi = 0;
   cudaStream_t st = nullptr;
   mg::CountSlot *table = nullptr;
-  unsigned long long *d_scalars = nullptr;  // [0] distinct keys in the table [1] instances counted [2] emit cursor
+  // [0] distinct keys in the table [1] instances counted [2] emit cursor [3] windows examined (restricted)
+  unsigned long long *d_scalars = nullptr;
   uint8_t *d_seq = nullptr;
   uint64_t seq_cap = 0, n_out = 0, launches = 0;
   u128 *out_keys = nullptr;
   uint32_t *out_counts = nullptr;
   bool finished = false;
+  bool empty = true;  // nothing added since mg_count_create / mg_count_reset
+  mg_ctx *restrict_to = nullptr;  // mg_count_restrict: insert only what this context's index can use
   cudaEvent_t ev[2] = {nullptr, nullptr};
   double kernel_ms = 0;  // device time of the counting kernels so far
 };
@@ -1773,7 +1776,12 @@ constexpr uint64_t COUNT_CHUNK = 1ull << 26;  // read bytes per kernel launch
 
 static int counter_alloc_table(mg_counter *c, int log2cap, mg::CountSlot **t) {
   uint64_t cap = 1ull << log2cap;
-  CU(cudaMalloc(t, cap * sizeof(mg::CountSlot)));
+  if (cudaMalloc(t, cap * sizeof(mg::CountSlot)) == cudaErrorMemoryAllocation) {
+    cudaGetLastError();
+    return set_err(MG_ERR_NOMEM, "the k-mer table of %llu slots (%.1f GB) does not fit in device memory",
+                   (unsigned long long)cap, cap * sizeof(mg::CountSlot) / 1e9);
+  }
+  CU(cudaGetLastError());
   c->launches++;
   mg::k_count_clear<<<grid_for(cap, 256), 256, 0, c->st>>>(*t, cap);
   CU(cudaGetLastError());
@@ -1848,6 +1856,19 @@ extern "C" int mg_count_reset(mg_counter *c) {
   CU(cudaMemsetAsync(c->d_scalars, 0, 4 * sizeof(unsigned long long), c->st));
   CU(cudaStreamSynchronize(c->st));
   c->finished = false;
+  c->empty = true;
+  return MG_OK;
+}
+
+extern "C" int mg_count_restrict(mg_counter *c, mg_ctx *ctx) {
+  if (!c) return set_err(MG_ERR_ARG, "NULL counter");
+  if (ctx) {
+    if (c->device != ctx->device) return set_err(MG_ERR_ARG, "counter and context live on different devices");
+    if (c->k != ctx->ref_k) return set_err(MG_ERR_ARG, "counter holds %d-mers but ref_k is %d", c->k, ctx->ref_k);
+    if (!ctx->alt_final) return set_err(MG_ERR_STATE, "mg_count_restrict before mg_finalize_alt");
+  }
+  if (!c->empty) return set_err(MG_ERR_STATE, "mg_count_restrict on a counter that is not empty (call mg_count_reset)");
+  c->restrict_to = ctx;
   return MG_OK;
 }
 
@@ -1878,8 +1899,11 @@ extern "C" int mg_count_add(mg_counter *c, const char *bases, uint64_t n) {
   if (!c || (!bases && n)) return set_err(MG_ERR_ARG, "NULL argument");
   if (c->finished) return set_err(MG_ERR_STATE, "mg_count_add after mg_count_finish (call mg_count_reset)");
   CU(cudaSetDevice(c->device));
+  c->empty = false;
   const uint64_t halo = (uint64_t)(c->k - 1);
   if (n <= halo) return MG_OK;
+  const mg_ctx *x = c->restrict_to;
+  const DevView v = x ? x->view() : DevView{};
   if (!c->d_seq) {
     uint64_t cap = COUNT_CHUNK;
     if (const char *e = getenv("MG_COUNT_CHUNK"))  // (tests shrink it to exercise the sub-chunk seams)
@@ -1901,12 +1925,11 @@ extern "C" int mg_count_add(mg_counter *c, const char *bases, uint64_t n) {
     for (int i = 0; i < 2; ++i)
       if (!c->ev[i]) CU(cudaEventCreate(&c->ev[i]));
     CU(cudaEventRecord(c->ev[0], c->st));
-    if (c->k == 43)
-      mg::k_count_kmers<43><<<grid, mg::CNT_THREADS, smem, c->st>>>(c->d_seq, len, c->k, c->table, mask, c->part_bits,
-                                                                    c->part_lo, c->part_hi, c->d_scalars, c->d_scalars + 1);
-    else
-      mg::k_count_kmers<0><<<grid, mg::CNT_THREADS, smem, c->st>>>(c->d_seq, len, c->k, c->table, mask, c->part_bits,
-                                                                   c->part_lo, c->part_hi, c->d_scalars, c->d_scalars + 1);
+    // (43, 35) is the specialised build, as for the scan; the restricted builds see the index through v
+    auto kern = !x ? (c->k == 43 ? mg::k_count_kmers<43, -1> : mg::k_count_kmers<0, -1>)
+                   : (x->ref_k == 43 && x->k == 35 ? mg::k_count_kmers<43, 35> : mg::k_count_kmers<0, 0>);
+    kern<<<grid, mg::CNT_THREADS, smem, c->st>>>(c->d_seq, len, c->k, c->table, mask, c->part_bits, c->part_lo, c->part_hi,
+                                                 c->d_scalars, c->d_scalars + 1, v, c->d_scalars + 3);
     CU(cudaGetLastError());
     CU(cudaEventRecord(c->ev[1], c->st));
     CU(cudaStreamSynchronize(c->st));  // d_seq is reused by the next sub-chunk
@@ -1960,6 +1983,7 @@ extern "C" int mg_count_finish(mg_counter *c, uint32_t min_count, uint32_t count
   }
   c->n_out = n;
   c->finished = true;
+  c->empty = false;
   if (n_kmers) *n_kmers = n;
   return MG_OK;
 }
@@ -1978,13 +2002,15 @@ extern "C" int mg_count_download(mg_counter *c, uint64_t *lohi, uint32_t *counts
 extern "C" int mg_count_stats(mg_counter *c, uint64_t *stats, int n) {
   if (!c || !stats || n < 4) return set_err(MG_ERR_ARG, "bad argument");
   CU(cudaSetDevice(c->device));
-  unsigned long long sc[2];
-  CU(cudaMemcpy(sc, c->d_scalars, 16, cudaMemcpyDeviceToHost));
+  unsigned long long sc[4];
+  CU(cudaMemcpy(sc, c->d_scalars, 32, cudaMemcpyDeviceToHost));
   stats[0] = sc[0];
   stats[1] = sc[1];
   stats[2] = 1ull << c->log2cap;
   stats[3] = c->launches;
   if (n >= 5) stats[4] = (uint64_t)(c->kernel_ms * 1e3);
+  // (the unrestricted builds do not count windows: without a partition every window they examine is inserted)
+  if (n >= 6) stats[5] = c->restrict_to ? sc[3] : sc[1];
   return MG_OK;
 }
 

@@ -282,6 +282,16 @@ MG_HD uint64_t canon_hash_rt(u128 x, int k, u128 *canon) {
   return xxh3_64_words(w, k);
 }
 
+// canon_hash<K> for a build specialised for k = K, canon_hash_rt for K = 0
+template <int K>
+MG_HD uint64_t canon_hash_k(u128 x, int k, u128 *canon) {
+  if constexpr (K > 0) {
+    return canon_hash<K>(x, canon);
+  } else {
+    return canon_hash_rt(x, k, canon);
+  }
+}
+
 // ---------------------------------------------------------------------------
 // ASCII k-mers (signature side): arbitrary bytes, length <= 128.
 // ---------------------------------------------------------------------------
