@@ -182,12 +182,31 @@ int mg_count_add(mg_counter *c, const char *bases, uint64_t n);
  * (MG_ERR_STATE).  The counter keeps the pointer and reads ctx's index at every mg_count_add: ctx must outlive the
  * restricted adds.  ctx == NULL lifts the restriction (also on an empty counter only). */
 int mg_count_restrict(mg_counter *c, mg_ctx *ctx);
+/* Counting inputs larger than the table can hold, with one read of the input.
+ * mg_count_set_limit caps the table at max_slots slots (0, the default: only device memory limits it; a non-zero cap
+ * is at least 65536).  A growth past the cap fails as one that does not fit the device does: MG_ERR_NOMEM, the table
+ * left as it was.  The environment variable MG_COUNT_MAX_SLOTS sets the same cap at mg_count_create.
+ * mg_count_add_keep counts as mg_count_add does and also returns the 2-bit copy of what it counted: every maximal run
+ * of A/C/G/T bytes at least k long, 2 bits a base (A0 C1 G2 T3), 4 to a byte, first base in the high bits, each run
+ * from a byte boundary, appended to packed (*n_bytes) with its length in run_len (*n_runs).  Capacities of
+ * n / 2 + 1 bytes and n / (k + 1) + 2 runs always suffice (MG_ERR_ARG when they do not).  When the table
+ * meets its limit (or device memory) the counter is OVERFLOWED: counting stops, packing goes on for this and later
+ * calls, mg_count_stats reports it and mg_count_finish refuses it (MG_ERR_STATE) until mg_count_reset.
+ * mg_count_add_packed counts such a copy from host memory (the caller's runs, concatenated), staged through pinned
+ * buffers; the partition and the limit apply: it fails with MG_ERR_NOMEM once the table nears its limit, for the
+ * caller to reset and count a narrower prefix range.  Both refuse a restricted counter (MG_ERR_STATE). */
+int mg_count_set_limit(mg_counter *c, uint64_t max_slots);
+int mg_count_add_keep(mg_counter *c, const char *bases, uint64_t n, uint8_t *packed, uint64_t packed_cap,
+                      uint32_t *run_len, uint64_t len_cap, uint64_t *n_bytes, uint64_t *n_runs);
+int mg_count_add_packed(mg_counter *c, const uint8_t *packed, uint64_t n_bytes, const uint32_t *run_len,
+                        uint64_t n_runs);
 int mg_count_finish(mg_counter *c, uint32_t min_count, uint32_t counter_max, uint64_t max_count, uint64_t *n_kmers);
 int mg_count_download(mg_counter *c, uint64_t *lohi, uint32_t *counts, uint64_t cap);
 /* {distinct k-mers in the table, k-mer instances counted, table capacity, kernels launched[, device time of the
- * counting kernels in microseconds[, valid windows examined]]}; n >= 4.  Windows are counted before the partition and
- * index tests of a restricted counter; an unrestricted counter reports its instances there (without a partition
- * it inserts every valid window). */
+ * counting kernels in microseconds[, valid windows examined[, overflowed (0/1)[, device time of the host-to-device
+ * copies of mg_count_add_packed in microseconds[, device time of packing in microseconds]]]]]}; n >= 4.  Windows are
+ * counted before the partition and index tests of a restricted counter; an unrestricted counter reports its
+ * instances there (without a partition it inserts every valid window). */
 int mg_count_stats(mg_counter *c, uint64_t *stats, int n);
 /* the counted k-mers straight into the sample scan (same device): no database file, no host round trip */
 int mg_scan_counted(mg_ctx *ctx, mg_counter *c);

@@ -104,6 +104,9 @@ SYMBOLS = {
     "mg_count_reset": (C.c_int, [C.c_void_p]),
     "mg_count_add": (C.c_int, [C.c_void_p, C.c_char_p, C.c_uint64]),
     "mg_count_restrict": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "mg_count_set_limit": (C.c_int, [C.c_void_p, C.c_uint64]),
+    "mg_count_add_keep": (C.c_int, [C.c_void_p, C.c_char_p, C.c_uint64, u8p, C.c_uint64, u32p, C.c_uint64, u64p, u64p]),
+    "mg_count_add_packed": (C.c_int, [C.c_void_p, u8p, C.c_uint64, u32p, C.c_uint64]),
     "mg_count_finish": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint64, u64p]),
     "mg_count_download": (C.c_int, [C.c_void_p, u64p, u32p, C.c_uint64]),
     "mg_count_stats": (C.c_int, [C.c_void_p, u64p, C.c_int]),

@@ -565,6 +565,29 @@ class KmerCounter:
         b = reads if isinstance(reads, (bytes, bytearray)) else "\n".join(reads).encode()
         check(self._L.mg_count_add(self._h, bytes(b), len(b)))
 
+    def set_limit(self, max_slots: int) -> None:
+        """Cap the table at ``max_slots`` slots (0: device memory only; ``mg_count_set_limit``)."""
+        check(self._L.mg_count_set_limit(self._h, max_slots))
+
+    def add_keep(self, reads):
+        """``add`` that also returns the 2-bit copy of what it counted (``mg_count_add_keep``): (uint8 packed bytes,
+        uint32 run lengths) of every maximal A/C/G/T run at least k long.  Past the table limit the counter is
+        overflowed (``stats()["overflowed"]``): counting stops, packing goes on."""
+        b = bytes(reads if isinstance(reads, (bytes, bytearray)) else "\n".join(reads).encode())
+        packed = np.zeros(len(b) // 2 + 1, dtype=np.uint8)
+        run_len = np.zeros(len(b) // (self.k + 1) + 2, dtype=np.uint32)
+        nb, nr = C.c_uint64(0), C.c_uint64(0)
+        check(self._L.mg_count_add_keep(self._h, b, len(b), _p(packed, _lib.u8p), len(packed), _p(run_len, _lib.u32p),
+                                        len(run_len), C.byref(nb), C.byref(nr)))
+        return packed[:nb.value].copy(), run_len[:nr.value].copy()
+
+    def add_packed(self, packed, run_len) -> None:
+        """count a copy from ``add_keep`` (runs of several calls concatenated; ``mg_count_add_packed``)"""
+        packed = np.ascontiguousarray(packed, dtype=np.uint8)
+        run_len = np.ascontiguousarray(run_len, dtype=np.uint32)
+        check(self._L.mg_count_add_packed(self._h, _p(packed, _lib.u8p), len(packed), _p(run_len, _lib.u32p),
+                                          len(run_len)))
+
     def finish(self, min_count: int = 2, counter_max: int = 255, max_count: int = 10 ** 9):
         """-> (packed k-mers in ascending order, u32 counts)"""
         n = C.c_uint64(0)
@@ -575,9 +598,10 @@ class KmerCounter:
         return keys, counts
 
     def stats(self) -> dict:
-        s = (C.c_uint64 * 6)()
-        check(self._L.mg_count_stats(self._h, s, 6))
-        return dict(zip(("distinct", "instances", "capacity", "launches", "kernel_us", "windows"), [int(x) for x in s]))
+        s = (C.c_uint64 * 9)()
+        check(self._L.mg_count_stats(self._h, s, 9))
+        return dict(zip(("distinct", "instances", "capacity", "launches", "kernel_us", "windows", "overflowed",
+                         "transfer_us", "pack_us"), [int(x) for x in s]))
 
 
 def diag_bandwidth(device: int, mode: int, nbytes: int, reps: int = 3) -> float:

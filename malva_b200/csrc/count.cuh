@@ -10,6 +10,9 @@
 //                   every valid window into an open-addressing table of 32-byte slots {key 16 B, count 4 B}: one
 //                   16-byte read of the home slot, a 128-bit CAS only when the slot is empty, one atomicAdd.
 //                   Restricted builds (mg_count_restrict) insert only the windows the index can use (index_hit).
+//   k_pack_*        the 2-bit copy of the runs of >= k bases (mg_count_add_keep): a stream compaction per sub-chunk
+//   k_count_packed  the same windows counted from that copy (mg_count_add_packed); both counting kernels hand each
+//                   window to count_window
 //   k_count_rehash  table growth (load factor <= 0.5)
 //   k_count_emit    kept entries (count >= min_count, saturated) appended to dense arrays; a radix sort by key then
 //                   gives KMC's listing order.
@@ -17,6 +20,7 @@
 #include <cuda_runtime.h>
 
 #include <cstdint>
+#include <cub/block/block_scan.cuh>
 
 #include "index.cuh"
 #include "xxh3.cuh"
@@ -86,6 +90,23 @@ __device__ __forceinline__ bool index_hit(const DevView &v, u128 canon, int ref_
   return ovf && ovf_find(v, c) >= 0;
 }
 
+// One valid window of either counting kernel, from its forward and reverse-complement words: the canonical form, the
+// prefix-partition test, the index test of a restricted build (KC >= 0), the insert; ++*mine when inserted.
+template <int KC>
+__device__ __forceinline__ void count_window(const u128 &f, const u128 &r, int k, int part_bits, uint32_t part_lo, uint32_t part_hi,
+                                             const DevView &v, CountSlot *table, uint64_t mask,
+                                             unsigned long long *n_distinct, uint32_t &mine) {
+  u128 canon = less128(r, f) ? r : f;  // (ties: the two strands are the same word)
+  if (part_bits) {
+    uint32_t part = (uint32_t)(shr128(canon, 2 * k - part_bits).lo);
+    if (part < part_lo || part >= part_hi) return;
+  }
+  if constexpr (KC >= 0)
+    if (!index_hit<KC>(v, canon, k)) return;
+  count_insert(table, mask, canon, 1u, n_distinct);
+  ++mine;
+}
+
 // seq: read bytes, records separated by any non-ACGT byte (the host puts '\n' between reads).  Window end
 // positions [k-1, len).  Only canonical k-mers whose top `part_bits` bits fall in [part_lo, part_hi) are counted
 // (prefix-partitioned passes for inputs whose distinct k-mers do not fit the table at once; part_bits = 0: all).
@@ -139,20 +160,179 @@ __global__ void __launch_bounds__(CNT_THREADS) k_count_kmers(const uint8_t *__re
   for (uint64_t p = q0; p < q1; ++p) {
     push(cnt_sm[(int)(p - base)]);
     if (run < k) continue;
-    u128 canon = less128(r, f) ? r : f;  // (ties: the two strands are the same word)
     if constexpr (KC >= 0) ++seen;
-    if (part_bits) {
-      uint32_t part = (uint32_t)(shr128(canon, 2 * k - part_bits).lo);
-      if (part < part_lo || part >= part_hi) continue;
-    }
-    if constexpr (KC >= 0)
-      if (!index_hit<KC>(v, canon, k)) continue;
-    count_insert(table, mask, canon, 1u, n_distinct);
-    ++mine;
+    count_window<KC>(f, r, k, part_bits, part_lo, part_hi, v, table, mask, n_distinct, mine);
   }
   if (mine) atomicAdd(n_instances, (unsigned long long)mine);
   if constexpr (KC >= 0)
     if (seen) atomicAdd(n_windows, (unsigned long long)seen);
+}
+
+// ---- the device-packed copy of the reads (mg_count_add_keep) and counting from it (mg_count_add_packed) ----
+// A run is a maximal stretch of A/C/G/T bytes of one mg_count_add_keep call, kept when it is at least k long (the
+// window rule of k_count_kmers: shorter runs hold no window).  Runs are stored 2 bits a base (A0 C1 G2 T3), 4 to a
+// byte, first base in the high bits, each run from a byte boundary; a length entry per run.
+//
+// Per device sub-chunk, over its own bytes [own, len) (a later sub-chunk's first k-1 bytes are the halo it shares
+// with the previous one): a piece is a maximal ACGT stretch there.  A piece that starts at `own` while the previous
+// sub-chunk ended inside a run (`carry` bases of it so far) continues that run: its bases go on at 2-bit phase
+// carry % 4, its first byte re-written from `carry_byte`.  A piece that reaches the end of the sub-chunk while more
+// follow (`more`) is kept whatever its length; the host drops it later if the run ends shorter than k.
+constexpr int PACK_THREADS = 256;
+constexpr int PACK_RUN = 16;
+constexpr int PACK_TILE = PACK_THREADS * PACK_RUN;
+
+__device__ __forceinline__ bool is_acgt(uint8_t ch) { return ch == 'A' || ch == 'C' || ch == 'G' || ch == 'T'; }
+
+// WRITE = false: the number of piece starts of each tile into tile_n.  WRITE = true (tile_n = their exclusive
+// prefix): the start and the end position of piece i into starts[i], ends[i].
+template <bool WRITE>
+__global__ void __launch_bounds__(PACK_THREADS) k_pack_pieces(const uint8_t *__restrict__ seq, uint32_t own, uint32_t len,
+                                                             uint32_t *tile_n, uint32_t *starts, uint32_t *ends) {
+  using Scan = cub::BlockScan<uint32_t, PACK_THREADS>;
+  __shared__ typename Scan::TempStorage tmp;
+  const uint64_t p0 = (uint64_t)own + (uint64_t)blockIdx.x * PACK_TILE + (uint64_t)threadIdx.x * PACK_RUN;
+  const uint64_t p1 = p0 + PACK_RUN < len ? p0 + PACK_RUN : len;
+  auto start_at = [&](uint64_t p) { return is_acgt(seq[p]) && (p == own || !is_acgt(seq[p - 1])); };
+  uint32_t n = 0;
+  for (uint64_t p = p0; p < p1; ++p) n += start_at(p);
+  uint32_t before, total;
+  Scan(tmp).ExclusiveSum(n, before, total);
+  if (!WRITE) {
+    if (threadIdx.x == 0) tile_n[blockIdx.x] = total;
+    return;
+  }
+  uint32_t rank = tile_n[blockIdx.x] + before;  // starts at positions < p
+  for (uint64_t p = p0; p < p1; ++p) {
+    if (!is_acgt(seq[p])) continue;
+    if (start_at(p)) starts[rank++] = (uint32_t)p;
+    if (p + 1 == len || !is_acgt(seq[p + 1])) ends[rank - 1] = (uint32_t)p;
+  }
+}
+
+struct PackPiece {
+  uint32_t start, len, phase;
+  uint64_t total;  // bases of the run so far (the carried ones included)
+  bool kept;
+};
+__device__ __forceinline__ PackPiece pack_piece(const uint32_t *starts, const uint32_t *ends, uint32_t i, uint32_t own,
+                                                uint32_t len, uint32_t carry, bool more, int k) {
+  PackPiece q;
+  q.start = starts[i];
+  q.len = ends[i] - q.start + 1;
+  const bool cont = i == 0 && carry && q.start == own;
+  q.phase = cont ? carry & 3u : 0u;
+  q.total = (uint64_t)q.len + (cont ? carry : 0u);
+  q.kept = q.total >= (uint64_t)k || (more && ends[i] + 1 == len);
+  return q;
+}
+
+// per piece: (output bytes << 32) | kept, for an exclusive scan that gives output byte offsets and run ranks;
+// val[n] = 0 so that the scan's last entry holds the totals.  flags: bit 0 piece 0 continues the carried run, bit 1
+// it is kept.
+__global__ void k_pack_plan(const uint32_t *starts, const uint32_t *ends, uint32_t n, uint32_t own, uint32_t len,
+                            uint32_t carry, int more, int k, unsigned long long *val, unsigned long long *flags) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i > n) return;
+  if (i == n) {
+    val[n] = 0;
+    return;
+  }
+  const PackPiece q = pack_piece(starts, ends, i, own, len, carry, more, k);
+  val[i] = q.kept ? ((unsigned long long)((q.phase + q.len + 3) / 4) << 32) | 1ull : 0ull;
+  if (i == 0) *flags = (carry && q.start == own ? 1ull : 0ull) | (q.kept ? 2ull : 0ull);
+}
+
+// one thread per output byte: its piece by binary search over the scanned offsets, 4 bases (or the carried byte's
+// bases before the phase of a continued run); the thread of a piece's first byte writes the run's length.
+__global__ void k_pack_write(const uint8_t *__restrict__ seq, const uint32_t *starts, const uint32_t *ends, uint32_t n,
+                             const unsigned long long *off, uint32_t own, uint32_t len, uint32_t carry,
+                             uint8_t carry_byte, int more, int k, uint8_t *out, uint32_t *run_len) {
+  const uint64_t j = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= (off[n] >> 32)) return;
+  uint32_t lo = 0, hi = n;  // the last piece i with off_bytes[i] <= j (a kept one: a dropped piece has no bytes)
+  while (hi - lo > 1) {
+    uint32_t mid = (lo + hi) / 2;
+    if ((off[mid] >> 32) <= j) lo = mid;
+    else hi = mid;
+  }
+  const PackPiece q = pack_piece(starts, ends, lo, own, len, carry, more, k);
+  const uint64_t bj = j - (off[lo] >> 32);
+  uint32_t b = 0;
+  for (int s = 0; s < 4; ++s) {
+    const int64_t x = (int64_t)(4 * bj + s) - (int64_t)q.phase;  // base of the piece in this slot
+    uint32_t c = 0;
+    if (x < 0) c = (carry_byte >> (6 - 2 * s)) & 3u;
+    else if (x < (int64_t)q.len) {
+      const uint8_t ch = seq[q.start + x];
+      c = ch == 'A' ? 0u : ch == 'C' ? 1u : ch == 'G' ? 2u : 3u;
+    }
+    b |= c << (6 - 2 * s);
+  }
+  out[j] = (uint8_t)b;
+  if (bj == 0) run_len[off[lo] & 0xffffffffull] = (uint32_t)q.total;
+}
+
+// Counting from the packed copy: a staged chunk of runs, run i from byte run_off[i], run_len[i] bases; the chunk's
+// base positions are tiled as k_count_kmers tiles the read bytes, and a thread finds the run of its first position by
+// a binary search inside the range of runs its tile spans.  Run 0 may be the later part of a run split over two
+// chunks: its first skip0 windows were counted with the earlier part.
+template <int K>
+__global__ void __launch_bounds__(CNT_THREADS) k_count_packed(const uint8_t *__restrict__ packed,
+                                                             const uint32_t *__restrict__ run_off,
+                                                             const uint32_t *__restrict__ run_len, uint32_t n_runs,
+                                                             uint64_t n_pos, uint32_t skip0, int k_rt, CountSlot *table,
+                                                             uint64_t mask, int part_bits, uint32_t part_lo,
+                                                             uint32_t part_hi, unsigned long long *n_distinct,
+                                                             unsigned long long *n_instances) {
+  __shared__ uint32_t span[2];
+  const int k = K > 0 ? K : k_rt;
+  const uint64_t t0 = (uint64_t)blockIdx.x * CNT_TILE, t1 = t0 + CNT_TILE < n_pos ? t0 + CNT_TILE : n_pos;
+  auto find = [&](uint64_t pos, uint32_t lo, uint32_t hi) {  // the last run in [lo, hi] starting at or before pos
+    while (lo < hi) {
+      uint32_t mid = (lo + hi + 1) / 2;
+      if (4ull * run_off[mid] <= pos) lo = mid;
+      else hi = mid - 1;
+    }
+    return lo;
+  };
+  if (threadIdx.x < 2) span[threadIdx.x] = find(threadIdx.x ? t1 - 1 : t0, 0, n_runs - 1);
+  __syncthreads();
+  const uint64_t q0 = t0 + (uint64_t)threadIdx.x * CNT_RUN;
+  if (q0 >= t1) return;
+  const uint64_t q1 = q0 + CNT_RUN < t1 ? q0 + CNT_RUN : t1;
+  const u128 m = mask128(u128{~0ull, ~0ull}, 2 * k);
+  const int top = 2 * (k - 1);
+  const DevView none{};
+  u128 f = {0, 0}, r = {0, 0};
+  auto push = [&](uint64_t j) {
+    const uint32_t c = (packed[j >> 2] >> (6 - 2 * (int)(j & 3))) & 3u;
+    f.hi = ((f.hi << 2) | (f.lo >> 62)) & m.hi;
+    f.lo = ((f.lo << 2) | c) & m.lo;
+    r.lo = (r.lo >> 2) | (r.hi << 62);
+    r.hi >>= 2;
+    const uint64_t cc = 3u - c;
+    if (top >= 64)
+      r.hi |= cc << (top - 64);
+    else
+      r.lo |= cc << (top & 63);
+  };
+  uint32_t mine = 0;
+  for (uint32_t i = find(q0, span[0], span[1]); i < n_runs; ++i) {
+    const uint64_t rs = 4ull * run_off[i];
+    if (rs >= q1) break;
+    const uint64_t re = rs + run_len[i];
+    const uint64_t first = rs + (uint64_t)(k - 1) + (i == 0 ? skip0 : 0u);  // first window end counted
+    const uint64_t a = q0 > first ? q0 : first, b = re < q1 ? re : q1;
+    if (a >= b) continue;
+    f = r = u128{0, 0};
+    for (uint64_t j = a - (uint64_t)(k - 1); j < a; ++j) push(j);
+    for (uint64_t p = a; p < b; ++p) {
+      push(p);
+      count_window<-1>(f, r, k, part_bits, part_lo, part_hi, none, table, mask, n_distinct, mine);
+    }
+  }
+  if (mine) atomicAdd(n_instances, (unsigned long long)mine);
 }
 
 __global__ void k_count_clear(CountSlot *table, uint64_t cap) {

@@ -1495,15 +1495,118 @@ int signatures_main(int argc, char **argv) {
   return 0;
 }
 
+// The 2-bit copy of the reads that `count` keeps while it counts (mg_count_add_keep): segments in host memory up to
+// a budget, the rest in one spill file.  The file is unlinked as soon as it is created, so that it goes away with
+// the process on every exit path.
+class PackedStore {
+ public:
+  PackedStore(uint64_t budget, std::string dir) : budget_(budget), dir_(std::move(dir)) {}
+  ~PackedStore() {
+    if (fp_) fclose(fp_);
+  }
+  PackedStore(const PackedStore &) = delete;
+  PackedStore &operator=(const PackedStore &) = delete;
+
+  void add(const uint8_t *b, uint64_t nb, const uint32_t *l, uint64_t nr) {
+    if (!nr) return;
+    Seg g{nb, nr, -1, {}, {}};
+    if (in_mem_ + nb + 4 * nr <= budget_) {
+      g.bytes.assign(b, b + nb);
+      g.lens.assign(l, l + nr);
+      in_mem_ += nb + 4 * nr;
+    } else {
+      if (!fp_) open_spill();
+      g.at = (int64_t)spilled_;
+      if (fwrite(b, 1, nb, fp_) != nb || fwrite(l, 4, nr, fp_) != nr)
+        throw std::runtime_error("short write on the spill file in " + dir_);
+      spilled_ += nb + 4 * nr;
+    }
+    bytes_ += nb;
+    runs_ += nr;
+    segs_.push_back(std::move(g));
+  }
+  // f(packed, n_bytes, run_len, n_runs) over every segment, in the order they were added
+  void each(const std::function<void(const uint8_t *, uint64_t, const uint32_t *, uint64_t)> &f) {
+    if (fp_ && fflush(fp_) != 0) throw std::runtime_error("cannot flush the spill file in " + dir_);
+    std::vector<uint8_t> buf;
+    for (const Seg &g : segs_) {
+      if (g.at < 0) {
+        f(g.bytes.data(), g.nb, g.lens.data(), g.nr);
+        continue;
+      }
+      buf.resize(g.nb + 4 * g.nr + 4);
+      uint8_t *lens = buf.data() + ((g.nb + 3) & ~3ull);
+      if (fseeko(fp_, (off_t)g.at, SEEK_SET) != 0 || fread(buf.data(), 1, g.nb, fp_) != g.nb ||
+          fread(lens, 4, g.nr, fp_) != g.nr)
+        throw std::runtime_error("cannot read back the spill file in " + dir_);
+      f(buf.data(), g.nb, reinterpret_cast<const uint32_t *>(lens), g.nr);
+    }
+    if (fp_) fseeko(fp_, 0, SEEK_END);
+  }
+  uint64_t bytes() const { return bytes_; }
+  uint64_t runs() const { return runs_; }
+  uint64_t in_memory() const { return in_mem_; }
+  uint64_t spilled() const { return spilled_; }
+  const std::string &spill_path() const { return path_; }
+
+ private:
+  struct Seg {
+    uint64_t nb, nr;
+    int64_t at;  // offset in the spill file, -1: in memory
+    std::vector<uint8_t> bytes;
+    std::vector<uint32_t> lens;
+  };
+  void open_spill() {
+    std::string t = dir_ + "/malva-count-XXXXXX";
+    int fd = mkstemp(&t[0]);
+    if (fd < 0) throw std::runtime_error("cannot create a spill file in " + dir_ + ": " + strerror(errno));
+    unlink(t.c_str());
+    fp_ = fdopen(fd, "w+b");
+    if (!fp_) {
+      close(fd);
+      throw std::runtime_error("cannot open the spill file in " + dir_);
+    }
+    path_ = t;
+  }
+  uint64_t budget_, in_mem_ = 0, spilled_ = 0, bytes_ = 0, runs_ = 0;
+  std::string dir_, path_;
+  FILE *fp_ = nullptr;
+  std::vector<Seg> segs_;
+};
+
+// half of MemAvailable: the host memory the packed copy may take before it goes to the spill file
+uint64_t default_store_budget() {
+  if (const char *e = getenv("MG_COUNT_HOST_BUDGET")) return strtoull(e, nullptr, 10);  // (tests force the spill)
+  FILE *fp = fopen("/proc/meminfo", "r");
+  unsigned long long kb = 0;
+  if (fp) {
+    char line[256];
+    while (fgets(line, sizeof(line), fp))
+      if (sscanf(line, "MemAvailable: %llu kB", &kb) == 1) break;
+    fclose(fp);
+  }
+  return kb * 1024 / 2;
+}
+
+// a range of canonical k-mers: those whose top `bits` bits lie in [lo, hi) (bits = 0: all of them)
+struct PrefixRange {
+  int bits;
+  uint32_t lo, hi;
+};
+
 // ------------------------------------------------------------------------------------------------
 // `kmc -k43 -ci2 -cs255 -m4 -t1 -fm <sample> <out_prefix> <tmp>` (MALVA:107) on the GPU.  Flags come joined to their
-// value like kmc's (-k43) or separated (-k 43); -m / -t / -f* / the tmp directory are accepted and ignored (the file
-// format is detected from its first byte).  --passes N counts in N prefix-partitioned passes over the reads for
-// inputs whose distinct k-mers do not fit device memory at once.
+// value like kmc's (-k43) or separated (-k 43); -m / -t / -f* are accepted and ignored (the file format is detected
+// from its first byte).  The input is read once: while the device counts it, it also keeps a 2-bit copy of the
+// countable bases (host memory up to half of what is available, then a spill file in tmp_dir, by default the
+// directory of the output prefix).  When the k-mer table would outgrow the device, counting goes on in
+// prefix-partitioned passes over that copy, in ascending prefix order; a range that still does not fit is split in
+// two.  --passes N asks for N such passes from the start.
 int count_main(int argc, char **argv) {
   unsigned k = 43, ci = 2, cs = 255, passes = 1;
   unsigned long long cx = 1000000000ull;
   int device = 0;
+  bool trace = false;
   std::vector<std::string> pos;
   auto value = [&](const std::string &a, size_t skip, int &i) -> std::string {
     if (a.size() > skip) return a.substr(skip);
@@ -1514,6 +1617,7 @@ int count_main(int argc, char **argv) {
     std::string a = argv[i];
     if (a == "--passes") passes = (unsigned)atoi(value(a, a.size(), i).c_str());
     else if (a == "--device") device = atoi(value(a, a.size(), i).c_str());
+    else if (a == "--trace") trace = true;
     else if (a.compare(0, 3, "-ci") == 0) ci = (unsigned)atoi(value(a, 3, i).c_str());
     else if (a.compare(0, 3, "-cs") == 0) cs = (unsigned)atoi(value(a, 3, i).c_str());
     else if (a.compare(0, 3, "-cx") == 0) cx = strtoull(value(a, 3, i).c_str(), nullptr, 10);
@@ -1526,42 +1630,151 @@ int count_main(int argc, char **argv) {
     else pos.push_back(a);
   }
   if (pos.size() < 2 || passes < 1 || passes > 256) {
-    std::cerr << "Usage: malva-geno count [-k43] [-ci2] [-cs255] [-cx1000000000] [--passes N] [--device N] "
+    std::cerr << "Usage: malva-geno count [-k43] [-ci2] [-cs255] [-cx1000000000] [--passes N] [--device N] [--trace] "
                  "<reads.fq|fa[.gz]> <kmc_output_prefix> [tmp_dir]\n";
     return 1;
   }
   if (cs > 255) throw std::runtime_error("-cs above 255 is not supported (one counter byte per record)");
+  std::string spill_dir = pos.size() > 2 ? pos[2] : pos[1].substr(0, pos[1].find_last_of('/') + 1);
+  if (spill_dir.empty()) spill_dir = ".";
   pelapsed("k-mer counting");
   Counter cn;
   gpu(mg_count_create(&cn.c, device, (int)k), "mg_count_create");
+  std::deque<PrefixRange> plan;
+  for (unsigned p = 0; p < passes; ++p)
+    plan.push_back(passes > 1 ? PrefixRange{8, p * 256 / passes, (p + 1) * 256 / passes} : PrefixRange{0, 0, 0});
+  const PrefixRange first = plan.front();
+  gpu(mg_count_set_partition(cn.c, first.bits, first.lo, first.hi), "mg_count_set_partition");
+
+  // one read of the input: a thread parses the next chunk while the device counts and packs this one
+  PackedStore store(default_store_budget(), spill_dir);
+  ReadFeeder feed(pos[0]);
+  std::string cur, next;
+  std::vector<uint8_t> packed;
+  std::vector<uint32_t> run_len;
+  uint64_t total_bases = 0, st[9] = {}, at_overflow[9] = {};
+  bool overflowed = false;
+  Stopwatch sw;
+  double t_read = 0, t_count = 0, t_wait = 0, t_passes = 0;
+  bool more = feed.next_chunk(cur, READ_CHUNK);
+  t_read += sw.lap();
+  while (more) {
+    std::future<bool> ahead = std::async(std::launch::async, [&] {
+      Stopwatch r;
+      const bool m = feed.next_chunk(next, READ_CHUNK);
+      t_read += r.lap();
+      return m;
+    });
+    packed.resize(cur.size() / 2 + 1);
+    run_len.resize(cur.size() / (k + 1) + 2);
+    uint64_t nb = 0, nr = 0;
+    gpu(mg_count_add_keep(cn.c, cur.data(), cur.size(), packed.data(), packed.size(), run_len.data(), run_len.size(),
+                          &nb, &nr),
+        "mg_count_add_keep");
+    store.add(packed.data(), nb, run_len.data(), nr);
+    if (!overflowed) {
+      gpu(mg_count_stats(cn.c, st, 9), "mg_count_stats");
+      if (st[6]) {
+        overflowed = true;
+        memcpy(at_overflow, st, sizeof(st));
+      }
+    }
+    total_bases += cur.size();
+    t_count += sw.lap();
+    more = ahead.get();
+    t_wait += sw.lap();
+    std::swap(cur, next);
+  }
+  std::string().swap(cur);
+  std::string().swap(next);
+
   std::unique_ptr<mh::KmcWriter> w;
   std::vector<uint64_t> keys;
   std::vector<uint32_t> counts;
-  uint64_t instances = 0, distinct = 0, total_bases = 0;
-  for (unsigned p = 0; p < passes; ++p) {
-    if (passes > 1) {
-      gpu(mg_count_reset(cn.c), "mg_count_reset");
-      gpu(mg_count_set_partition(cn.c, 8, p * 256 / passes, (p + 1) * 256 / passes), "mg_count_set_partition");
-    }
-    ReadFeeder feed(pos[0]);
-    std::string chunk;
-    while (feed.next_chunk(chunk, READ_CHUNK)) {
-      if (p == 0) total_bases += chunk.size();
-      gpu(mg_count_add(cn.c, chunk.data(), chunk.size()), "mg_count_add");
-    }
-    uint64_t n = 0, st[4];
-    gpu(mg_count_finish(cn.c, ci, cs, cx, &n), "mg_count_finish");
-    gpu(mg_count_stats(cn.c, st, 4), "mg_count_stats");
-    distinct += st[0];
-    instances += st[1];
+  uint64_t instances = 0, distinct = 0, n_passes = 0, n_splits = 0;
+  auto write = [&](uint64_t n, uint64_t lut_n) {
+    uint64_t s[4];
+    gpu(mg_count_stats(cn.c, s, 4), "mg_count_stats");
+    distinct += s[0];
+    instances += s[1];
     keys.resize(2 * n);
     counts.resize(n);
     gpu(mg_count_download(cn.c, keys.data(), counts.data(), n), "mg_count_download");
-    if (!w) w.reset(new mh::KmcWriter(pos[1], k, passes == 1 ? mh::KmcWriter::choose_prefix_len(k, n)
-                                                             : mh::KmcWriter::choose_prefix_len(k, 1ull << 40), ci, cs));
+    if (!w) w.reset(new mh::KmcWriter(pos[1], k, mh::KmcWriter::choose_prefix_len(k, lut_n), ci, cs));
     w->append(keys.data(), counts.data(), n);
+  };
+  if (!overflowed) {  // the first range is counted
+    uint64_t n = 0;
+    gpu(mg_count_finish(cn.c, ci, cs, cx, &n), "mg_count_finish");
+    write(n, passes == 1 ? n : 1ull << 40);
+    plan.pop_front();
+  } else if (passes == 1) {
+    // the first plan: the distinct k-mers per counted window so far, over all the windows, in ranges a quarter of
+    // what the table held at the overflow; 4 ranges when it overflowed before it counted anything.  A range that
+    // still does not fit is split below.
+    const int bits = (int)std::min(30u, 2 * k);
+    uint64_t n = 4;
+    if (at_overflow[1]) {
+      const double est = (double)at_overflow[0] / (double)at_overflow[1] * (double)total_bases;
+      n = (uint64_t)std::ceil(est / (double)(at_overflow[2] / 4));
+    }
+    n = std::max<uint64_t>(4, std::min<uint64_t>(n, 1ull << bits));
+    plan.clear();
+    for (uint64_t p = 0; p < n; ++p)
+      plan.push_back(PrefixRange{bits, (uint32_t)((p << bits) / n), (uint32_t)(((p + 1) << bits) / n)});
   }
+  const uint64_t max_bits = std::min(30u, 2 * k);
+  // the remaining ranges over the packed copy, in ascending order
+  while (!plan.empty()) {
+    const PrefixRange r = plan.front();
+    plan.pop_front();
+    Stopwatch pw;
+    gpu(mg_count_reset(cn.c), "mg_count_reset");
+    gpu(mg_count_set_partition(cn.c, r.bits, r.lo, r.hi), "mg_count_set_partition");
+    int rc = MG_OK;
+    store.each([&](const uint8_t *b, uint64_t nb, const uint32_t *l, uint64_t nr) {
+      if (rc == MG_OK) rc = mg_count_add_packed(cn.c, b, nb, l, nr);
+    });
+    uint64_t n = 0;
+    if (rc == MG_OK) rc = mg_count_finish(cn.c, ci, cs, cx, &n);
+    t_passes += pw.lap();
+    if (rc == MG_ERR_NOMEM) {  // split the range in two and count both halves, in order
+      const std::string why = mg_last_error();
+      PrefixRange a = r, b = r;
+      if (r.hi - r.lo >= 2) {
+        a.hi = b.lo = r.lo + (r.hi - r.lo) / 2;
+      } else if ((uint64_t)r.bits < max_bits) {
+        a = {r.bits + 1, 2 * r.lo, 2 * r.lo + 1};
+        b = {r.bits + 1, 2 * r.lo + 1, 2 * r.lo + 2};
+      } else {
+        throw GpuError("the canonical k-mers of one " + std::to_string(r.bits) + "-bit prefix do not fit the k-mer "
+                       "table: " + why);
+      }
+      plan.push_front(b);
+      plan.push_front(a);
+      ++n_splits;
+      if (trace)
+        fprintf(stderr, "[trace] count: prefix range %u..%u of %d bits split (%s)\n", r.lo, r.hi, r.bits, why.c_str());
+      continue;
+    }
+    gpu(rc, "mg_count_add_packed / mg_count_finish");
+    write(n, 1ull << 40);
+    ++n_passes;
+  }
+  if (!w) w.reset(new mh::KmcWriter(pos[1], k, mh::KmcWriter::choose_prefix_len(k, 1ull << 40), ci, cs));
   w->close();
+  if (trace) {
+    gpu(mg_count_stats(cn.c, st, 9), "mg_count_stats");
+    fprintf(stderr, "[trace] count: %llu read bytes, one read of the input; %s; packed copy %llu bytes in %llu runs "
+                    "(%llu bytes in host memory, %llu bytes in %s); %llu passes over the copy, %llu splits; reading "
+                    "%.1f ms (%.1f ms waited for), counting + packing %.1f ms, passes %.1f ms; device time: counting "
+                    "kernels %.1f ms, host-to-device copies %.1f ms, packing %.1f ms\n",
+            (unsigned long long)total_bases, overflowed ? "the table met its limit while reading" : "no overflow",
+            (unsigned long long)store.bytes(), (unsigned long long)store.runs(), (unsigned long long)store.in_memory(),
+            (unsigned long long)store.spilled(), store.spilled() ? store.spill_path().c_str() : "no spill file",
+            (unsigned long long)n_passes, (unsigned long long)n_splits, t_read, t_wait, t_count, t_passes,
+            st[4] * 1e-3, st[7] * 1e-3, st[8] * 1e-3);
+  }
   std::cerr << "[malva-geno/count] " << total_bases << " read bytes, " << instances << " k-mer instances, " << distinct
             << " distinct, " << w->total() << " written (count >= " << ci << ", capped at " << cs << ")" << std::endl;
   pelapsed("k-mer counting complete");

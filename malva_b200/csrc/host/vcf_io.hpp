@@ -120,6 +120,8 @@ class BgzfSource {
  public:
   // true if the file starts with a BGZF member header
   static bool is_bgzf(const std::string &path) {
+    struct stat sb;  // (a pipe or FIFO is read once: no peeking at its first bytes)
+    if (stat(path.c_str(), &sb) != 0 || !S_ISREG(sb.st_mode)) return false;
     FILE *f = fopen(path.c_str(), "rb");
     if (!f) return false;
     unsigned char h[18];

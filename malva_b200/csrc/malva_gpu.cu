@@ -46,7 +46,7 @@ static int set_err(int code, const char *fmt, ...) {
   } while (0)
 
 extern "C" const char *mg_last_error(void) { return g_err; }
-extern "C" int mg_version(void) { return 203; }
+extern "C" int mg_version(void) { return 204; }
 extern "C" int mg_device_count(void) {
   int n = 0;
   cudaError_t e = cudaGetDeviceCount(&n);
@@ -1761,6 +1761,7 @@ struct mg_counter {
   cudaStream_t st = nullptr;
   mg::CountSlot *table = nullptr;
   // [0] distinct keys in the table [1] instances counted [2] emit cursor [3] windows examined (restricted)
+  // [4] flags of the last packed sub-chunk
   unsigned long long *d_scalars = nullptr;
   uint8_t *d_seq = nullptr;
   uint64_t seq_cap = 0, n_out = 0, launches = 0;
@@ -1771,8 +1772,34 @@ struct mg_counter {
   mg_ctx *restrict_to = nullptr;  // mg_count_restrict: insert only what this context's index can use
   cudaEvent_t ev[2] = {nullptr, nullptr};
   double kernel_ms = 0;  // device time of the counting kernels so far
+  uint64_t max_slots = 0;  // mg_count_set_limit: the table grows to at most this many slots (0: device memory only)
+  bool overflowed = false;  // mg_count_add_keep met the limit: counting stopped, packing goes on
+  // the packed copy (mg_count_add_keep): device buffers of one sub-chunk's stream compaction, in one allocation
+  uint8_t *pk_mem = nullptr;
+  uint32_t *pk_tiles = nullptr, *pk_tiles_x = nullptr, *pk_starts = nullptr, *pk_ends = nullptr, *pk_len = nullptr;
+  unsigned long long *pk_val = nullptr, *pk_off = nullptr;
+  uint8_t *pk_out = nullptr, *pk_scan_tmp = nullptr;
+  size_t pk_scan_bytes = 0;
+  double pack_ms = 0;  // device time of packing (kernels and the copies back) so far
+  // counting from a packed copy (mg_count_add_packed): two pinned host + device staging buffers
+  uint8_t *st_host[2] = {nullptr, nullptr}, *st_dev[2] = {nullptr, nullptr};
+  uint64_t st_bytes = 0, st_runs = 0;
+  cudaEvent_t st_ev[2][3] = {};
+  bool st_pending[2] = {false, false};
+  double xfer_ms = 0;  // device time of the host-to-device copies of mg_count_add_packed so far
 };
 constexpr uint64_t COUNT_CHUNK = 1ull << 26;  // read bytes per kernel launch
+
+// the device sub-chunk of the read bytes (tests shrink it with MG_COUNT_CHUNK to exercise the seams)
+static uint64_t count_chunk(const mg_counter *c) {
+  const uint64_t halo = (uint64_t)(c->k - 1);
+  uint64_t cap = COUNT_CHUNK;
+  if (const char *e = getenv("MG_COUNT_CHUNK"))
+    if (strtoull(e, nullptr, 10) > 2 * halo + 1 && strtoull(e, nullptr, 10) < (1ull << 31)) cap = strtoull(e, nullptr, 10);
+  return cap;
+}
+
+static bool mg_is_acgt(char ch) { return ch == 'A' || ch == 'C' || ch == 'G' || ch == 'T'; }
 
 static int counter_alloc_table(mg_counter *c, int log2cap, mg::CountSlot **t) {
   uint64_t cap = 1ull << log2cap;
@@ -1802,12 +1829,14 @@ extern "C" int mg_count_create(mg_counter **out, int device, int k) {
   c->k = k;
   auto init = [&]() -> int {
     CU(cudaStreamCreateWithFlags(&c->st, cudaStreamNonBlocking));
-    CU(cudaMalloc(&c->d_scalars, 4 * sizeof(unsigned long long)));
-    CU(cudaMemsetAsync(c->d_scalars, 0, 4 * sizeof(unsigned long long), c->st));
+    CU(cudaMalloc(&c->d_scalars, 5 * sizeof(unsigned long long)));
+    CU(cudaMemsetAsync(c->d_scalars, 0, 5 * sizeof(unsigned long long), c->st));
     c->log2cap = 16;
     int rc = counter_alloc_table(c, c->log2cap, &c->table);
     if (rc) return rc;
     CU(cudaStreamSynchronize(c->st));
+    if (const char *e = getenv("MG_COUNT_MAX_SLOTS"))  // (tests force the partitioned passes with it)
+      return mg_count_set_limit(c, strtoull(e, nullptr, 10));
     return MG_OK;
   };
   int rc = init();
@@ -1831,10 +1860,25 @@ extern "C" void mg_count_destroy(mg_counter *c) {
   cudaFree(c->d_seq);
   cudaFree(c->out_keys);
   cudaFree(c->out_counts);
-  for (int i = 0; i < 2; ++i)
+  cudaFree(c->pk_mem);
+  for (int i = 0; i < 2; ++i) {
     if (c->ev[i]) cudaEventDestroy(c->ev[i]);
+    cudaFreeHost(c->st_host[i]);
+    cudaFree(c->st_dev[i]);
+    for (cudaEvent_t e : c->st_ev[i])
+      if (e) cudaEventDestroy(e);
+  }
   if (c->st) cudaStreamDestroy(c->st);
   delete c;
+}
+
+extern "C" int mg_count_set_limit(mg_counter *c, uint64_t max_slots) {
+  if (!c) return set_err(MG_ERR_ARG, "NULL counter");
+  if (max_slots && max_slots < (1ull << 16))
+    return set_err(MG_ERR_ARG, "a table limit of %llu slots is below the initial table of 65536",
+                   (unsigned long long)max_slots);
+  c->max_slots = max_slots;
+  return MG_OK;
 }
 
 extern "C" int mg_count_set_partition(mg_counter *c, int part_bits, uint32_t part_lo, uint32_t part_hi) {
@@ -1857,6 +1901,7 @@ extern "C" int mg_count_reset(mg_counter *c) {
   CU(cudaStreamSynchronize(c->st));
   c->finished = false;
   c->empty = true;
+  c->overflowed = false;
   return MG_OK;
 }
 
@@ -1872,14 +1917,21 @@ extern "C" int mg_count_restrict(mg_counter *c, mg_ctx *ctx) {
   return MG_OK;
 }
 
-static int counter_reserve(mg_counter *c, uint64_t more) {
+// Before `more` more windows are inserted: the table grows to 2 x (distinct + more) slots, so that an insert never
+// meets a full table.  A growth past the limit fails as one that does not fit the device does (MG_ERR_NOMEM), and
+// leaves the table as it was.  *distinct: the distinct keys in the table before the growth.
+static int counter_reserve(mg_counter *c, uint64_t more, uint64_t *distinct = nullptr) {
   unsigned long long nd = 0;
   CU(cudaMemcpyAsync(&nd, c->d_scalars, 8, cudaMemcpyDeviceToHost, c->st));
   CU(cudaStreamSynchronize(c->st));
+  if (distinct) *distinct = nd;
   uint64_t need = (nd + more) * 2;
   if (need <= (1ull << c->log2cap)) return MG_OK;
   int nl = c->log2cap;
   while ((1ull << nl) < need) ++nl;
+  if (c->max_slots && (1ull << nl) > c->max_slots)
+    return set_err(MG_ERR_NOMEM, "the k-mer table of %llu slots would exceed its limit of %llu slots",
+                   (unsigned long long)(1ull << nl), (unsigned long long)c->max_slots);
   mg::CountSlot *nt = nullptr;
   int rc = counter_alloc_table(c, nl, &nt);
   if (rc) return rc;
@@ -1895,9 +1947,108 @@ static int counter_reserve(mg_counter *c, uint64_t more) {
   return MG_OK;
 }
 
-extern "C" int mg_count_add(mg_counter *c, const char *bases, uint64_t n) {
+// The packed copy of one mg_count_add_keep call, built sub-chunk by sub-chunk in the caller's buffers.  `carry`: the
+// bases so far of the run that reaches the end of the last sub-chunk (0: none).
+struct PackOut {
+  uint8_t *packed;
+  uint64_t packed_cap;
+  uint32_t *run_len;
+  uint64_t len_cap;
+  uint64_t n_bytes = 0, n_runs = 0, carry = 0;
+};
+
+static int pack_alloc(mg_counter *c) {
+  if (c->pk_mem) return MG_OK;
+  const uint64_t cap = c->seq_cap, tiles = cap / mg::PACK_TILE + 2, pieces = cap / 2 + 2;
+  size_t scan_a = 0, scan_b = 0;
+  CU(cub::DeviceScan::ExclusiveSum(nullptr, scan_a, (uint32_t *)nullptr, (uint32_t *)nullptr, (int64_t)tiles));
+  CU(cub::DeviceScan::ExclusiveSum(nullptr, scan_b, (unsigned long long *)nullptr, (unsigned long long *)nullptr,
+                                   (int64_t)pieces));
+  c->pk_scan_bytes = std::max(scan_a, scan_b);
+  auto up = [](uint64_t b) { return (b + 255) & ~255ull; };
+  const uint64_t sizes[] = {up(tiles * 4), up(tiles * 4), up(pieces * 4), up(pieces * 4), up(pieces * 4),
+                            up(pieces * 8), up(pieces * 8), up(cap / 2 + 64), up(c->pk_scan_bytes + 1)};
+  uint64_t total = 0;
+  for (uint64_t s : sizes) total += s;
+  if (cudaMalloc(&c->pk_mem, total) == cudaErrorMemoryAllocation) {
+    cudaGetLastError();
+    return set_err(MG_ERR_NOMEM, "the packing buffers (%.1f GB) do not fit in device memory", total / 1e9);
+  }
+  CU(cudaGetLastError());
+  uint8_t *p = c->pk_mem;
+  void **dst[] = {(void **)&c->pk_tiles, (void **)&c->pk_tiles_x, (void **)&c->pk_starts, (void **)&c->pk_ends,
+                  (void **)&c->pk_len, (void **)&c->pk_val, (void **)&c->pk_off, (void **)&c->pk_out,
+                  (void **)&c->pk_scan_tmp};
+  for (int i = 0; i < 9; ++i) {
+    *dst[i] = p;
+    p += sizes[i];
+  }
+  return MG_OK;
+}
+
+// the runs of the sub-chunk in d_seq (bytes [own, len) are its own, `more`: sub-chunks of the call follow) appended
+// to o; `host` is the sub-chunk's bytes in host memory
+static int pack_subchunk(mg_counter *c, const char *host, uint64_t own, uint64_t len, bool more, PackOut *o) {
+  const uint64_t n_tiles = (len - own + mg::PACK_TILE - 1) / mg::PACK_TILE;
+  if (o->carry + len > 0xffffffffull) return set_err(MG_ERR_ARG, "a run of more than 2^32-1 bases");
+  CU(cudaEventRecord(c->ev[0], c->st));
+  c->launches += 5;
+  mg::k_pack_pieces<false><<<(int)n_tiles, mg::PACK_THREADS, 0, c->st>>>(c->d_seq, (uint32_t)own, (uint32_t)len,
+                                                                          c->pk_tiles, nullptr, nullptr);
+  CU(cudaMemsetAsync(c->pk_tiles + n_tiles, 0, 4, c->st));
+  size_t tb = c->pk_scan_bytes;
+  CU(cub::DeviceScan::ExclusiveSum(c->pk_scan_tmp, tb, c->pk_tiles, c->pk_tiles_x, (int64_t)(n_tiles + 1), c->st));
+  mg::k_pack_pieces<true><<<(int)n_tiles, mg::PACK_THREADS, 0, c->st>>>(c->d_seq, (uint32_t)own, (uint32_t)len,
+                                                                         c->pk_tiles_x, c->pk_starts, c->pk_ends);
+  uint32_t n = 0;
+  CU(cudaMemcpyAsync(&n, c->pk_tiles_x + n_tiles, 4, cudaMemcpyDeviceToHost, c->st));
+  CU(cudaStreamSynchronize(c->st));
+  unsigned long long fl = 0, tot = 0;
+  CU(cudaMemsetAsync(c->d_scalars + 4, 0, 8, c->st));
+  mg::k_pack_plan<<<grid_for(n + 1, 256), 256, 0, c->st>>>(c->pk_starts, c->pk_ends, n, (uint32_t)own, (uint32_t)len,
+                                                          (uint32_t)o->carry, more, c->k, c->pk_val, c->d_scalars + 4);
+  tb = c->pk_scan_bytes;
+  CU(cub::DeviceScan::ExclusiveSum(c->pk_scan_tmp, tb, c->pk_val, c->pk_off, (int64_t)n + 1, c->st));
+  CU(cudaMemcpyAsync(&tot, c->pk_off + n, 8, cudaMemcpyDeviceToHost, c->st));
+  CU(cudaMemcpyAsync(&fl, c->d_scalars + 4, 8, cudaMemcpyDeviceToHost, c->st));
+  CU(cudaStreamSynchronize(c->st));
+  const bool cont = fl & 1, cont_kept = (fl & 3) == 3;
+  // the run carried from the previous sub-chunk ended at the seam or inside this one shorter than k: drop it
+  if (o->carry && !cont_kept && (cont || o->carry < (uint64_t)c->k)) {
+    o->n_bytes -= (o->carry + 3) / 4;
+    o->n_runs -= 1;
+  }
+  const uint64_t nb = tot >> 32, nr = tot & 0xffffffffull;
+  const uint64_t at_b = o->n_bytes - (cont_kept && (o->carry & 3) ? 1 : 0), at_r = o->n_runs - (cont_kept ? 1 : 0);
+  if (at_b + nb > o->packed_cap || at_r + nr > o->len_cap)
+    return set_err(MG_ERR_ARG, "packed output buffers too small (%llu bytes / %llu runs so far)",
+                   (unsigned long long)(at_b + nb), (unsigned long long)(at_r + nr));
+  if (nb) {
+    const uint8_t carry_byte = o->carry & 3 ? o->packed[o->n_bytes - 1] : 0;
+    mg::k_pack_write<<<grid_for(nb, 256), 256, 0, c->st>>>(c->d_seq, c->pk_starts, c->pk_ends, n, c->pk_off,
+                                                           (uint32_t)own, (uint32_t)len, (uint32_t)o->carry, carry_byte,
+                                                           more, c->k, c->pk_out, c->pk_len);
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(o->packed + at_b, c->pk_out, nb, cudaMemcpyDeviceToHost, c->st));
+    CU(cudaMemcpyAsync(o->run_len + at_r, c->pk_len, nr * 4, cudaMemcpyDeviceToHost, c->st));
+  }
+  CU(cudaEventRecord(c->ev[1], c->st));
+  CU(cudaStreamSynchronize(c->st));
+  o->n_bytes = at_b + nb;
+  o->n_runs = at_r + nr;
+  // a run that reaches the end of this sub-chunk goes on in the next (it was kept whatever its length)
+  o->carry = more && mg_is_acgt(host[len - 1]) ? o->run_len[o->n_runs - 1] : 0;
+  float ms = 0;
+  CU(cudaEventElapsedTime(&ms, c->ev[0], c->ev[1]));
+  c->pack_ms += ms;
+  return MG_OK;
+}
+
+// mg_count_add, and mg_count_add_keep when keep != nullptr
+static int count_add(mg_counter *c, const char *bases, uint64_t n, PackOut *keep) {
   if (!c || (!bases && n)) return set_err(MG_ERR_ARG, "NULL argument");
   if (c->finished) return set_err(MG_ERR_STATE, "mg_count_add after mg_count_finish (call mg_count_reset)");
+  if (c->overflowed && !keep) return set_err(MG_ERR_STATE, "mg_count_add on an overflowed counter (call mg_count_reset)");
   CU(cudaSetDevice(c->device));
   c->empty = false;
   const uint64_t halo = (uint64_t)(c->k - 1);
@@ -1905,39 +2056,182 @@ extern "C" int mg_count_add(mg_counter *c, const char *bases, uint64_t n) {
   const mg_ctx *x = c->restrict_to;
   const DevView v = x ? x->view() : DevView{};
   if (!c->d_seq) {
-    uint64_t cap = COUNT_CHUNK;
-    if (const char *e = getenv("MG_COUNT_CHUNK"))  // (tests shrink it to exercise the sub-chunk seams)
-      if (strtoull(e, nullptr, 10) > 2 * halo + 1) cap = strtoull(e, nullptr, 10);
+    const uint64_t cap = count_chunk(c);
     CU(cudaMalloc(&c->d_seq, cap + 64));
     c->seq_cap = cap;
+  }
+  for (int i = 0; i < 2; ++i)
+    if (!c->ev[i]) CU(cudaEventCreate(&c->ev[i]));
+  if (keep) {
+    int rc = pack_alloc(c);
+    if (rc) return rc;
   }
   // sub-chunks overlap by k-1 bytes: a launch counts the windows that END inside its own part
   for (uint64_t start = 0; start + halo < n;) {
     const uint64_t len = n - start < c->seq_cap ? n - start : c->seq_cap;
-    int rc = counter_reserve(c, len);
-    if (rc) return rc;
+    if (!c->overflowed) {
+      int rc = counter_reserve(c, len);
+      if (rc == MG_ERR_NOMEM && keep) c->overflowed = true;  // (counting stops here; packing goes on)
+      else if (rc) return rc;
+    }
     CU(cudaMemcpyAsync(c->d_seq, bases + start, len, cudaMemcpyHostToDevice, c->st));
-    const uint64_t n_pos = len - halo;
-    const int grid = (int)((n_pos + mg::CNT_TILE - 1) / mg::CNT_TILE);
-    const size_t smem = mg::CNT_TILE + 64;
-    const uint64_t mask = (1ull << c->log2cap) - 1;
-    c->launches++;
-    for (int i = 0; i < 2; ++i)
-      if (!c->ev[i]) CU(cudaEventCreate(&c->ev[i]));
-    CU(cudaEventRecord(c->ev[0], c->st));
-    // (43, 35) is the specialised build, as for the scan; the restricted builds see the index through v
-    auto kern = !x ? (c->k == 43 ? mg::k_count_kmers<43, -1> : mg::k_count_kmers<0, -1>)
-                   : (x->ref_k == 43 && x->k == 35 ? mg::k_count_kmers<43, 35> : mg::k_count_kmers<0, 0>);
-    kern<<<grid, mg::CNT_THREADS, smem, c->st>>>(c->d_seq, len, c->k, c->table, mask, c->part_bits, c->part_lo, c->part_hi,
-                                                 c->d_scalars, c->d_scalars + 1, v, c->d_scalars + 3);
-    CU(cudaGetLastError());
-    CU(cudaEventRecord(c->ev[1], c->st));
-    CU(cudaStreamSynchronize(c->st));  // d_seq is reused by the next sub-chunk
-    float ms = 0;
-    CU(cudaEventElapsedTime(&ms, c->ev[0], c->ev[1]));
-    c->kernel_ms += ms;
+    if (keep) {
+      int rc = pack_subchunk(c, bases + start, start ? halo : 0, len, start + len < n, keep);
+      if (rc) return rc;
+    }
+    if (!c->overflowed) {
+      const uint64_t n_pos = len - halo;
+      const int grid = (int)((n_pos + mg::CNT_TILE - 1) / mg::CNT_TILE);
+      const size_t smem = mg::CNT_TILE + 64;
+      const uint64_t mask = (1ull << c->log2cap) - 1;
+      c->launches++;
+      CU(cudaEventRecord(c->ev[0], c->st));
+      // (43, 35) is the specialised build, as for the scan; the restricted builds see the index through v
+      auto kern = !x ? (c->k == 43 ? mg::k_count_kmers<43, -1> : mg::k_count_kmers<0, -1>)
+                     : (x->ref_k == 43 && x->k == 35 ? mg::k_count_kmers<43, 35> : mg::k_count_kmers<0, 0>);
+      kern<<<grid, mg::CNT_THREADS, smem, c->st>>>(c->d_seq, len, c->k, c->table, mask, c->part_bits, c->part_lo,
+                                                   c->part_hi, c->d_scalars, c->d_scalars + 1, v, c->d_scalars + 3);
+      CU(cudaGetLastError());
+      CU(cudaEventRecord(c->ev[1], c->st));
+      CU(cudaStreamSynchronize(c->st));  // d_seq is reused by the next sub-chunk
+      float ms = 0;
+      CU(cudaEventElapsedTime(&ms, c->ev[0], c->ev[1]));
+      c->kernel_ms += ms;
+    }
     if (start + len >= n) break;
     start += len - halo;  // the next part re-sends the last k-1 bytes as its halo
+  }
+  return MG_OK;
+}
+
+extern "C" int mg_count_add(mg_counter *c, const char *bases, uint64_t n) { return count_add(c, bases, n, nullptr); }
+
+extern "C" int mg_count_add_keep(mg_counter *c, const char *bases, uint64_t n, uint8_t *packed, uint64_t packed_cap,
+                                 uint32_t *run_len, uint64_t len_cap, uint64_t *n_bytes, uint64_t *n_runs) {
+  if (!c || (!bases && n) || (!packed && packed_cap) || (!run_len && len_cap) || !n_bytes || !n_runs)
+    return set_err(MG_ERR_ARG, "NULL argument");
+  if (c->restrict_to) return set_err(MG_ERR_STATE, "mg_count_add_keep on a restricted counter");
+  PackOut o{packed, packed_cap, run_len, len_cap};
+  int rc = count_add(c, bases, n, &o);
+  *n_bytes = o.n_bytes;
+  *n_runs = o.n_runs;
+  return rc;
+}
+
+// Counting from a packed copy in host memory: whole runs (a run longer than a staged chunk in parts that overlap by
+// k-1 bases) are copied into one of two pinned buffers while the device counts the other.  Under a table limit a
+// chunk holds no more bases than the table has room for distinct keys; MG_ERR_NOMEM when that room is less than an
+// eighth of what the limit allows, or when a growth does not fit the device.
+extern "C" int mg_count_add_packed(mg_counter *c, const uint8_t *packed, uint64_t n_bytes, const uint32_t *run_len,
+                                   uint64_t n_runs) {
+  if (!c || (!packed && n_bytes) || (!run_len && n_runs)) return set_err(MG_ERR_ARG, "NULL argument");
+  if (c->restrict_to) return set_err(MG_ERR_STATE, "mg_count_add_packed on a restricted counter");
+  if (c->finished) return set_err(MG_ERR_STATE, "mg_count_add_packed after mg_count_finish (call mg_count_reset)");
+  if (c->overflowed) return set_err(MG_ERR_STATE, "mg_count_add_packed on an overflowed counter (call mg_count_reset)");
+  CU(cudaSetDevice(c->device));
+  c->empty = false;
+  const uint64_t k = (uint64_t)c->k;
+  if (!c->st_host[0]) {
+    c->st_bytes = std::max<uint64_t>(count_chunk(c) / 4, 64);
+    c->st_runs = c->st_bytes / 8 + 1;
+    const uint64_t sz = c->st_bytes + 64 + 8 * c->st_runs;
+    for (int s = 0; s < 2; ++s) {
+      CU(cudaHostAlloc(&c->st_host[s], sz, cudaHostAllocDefault));
+      CU(cudaMalloc(&c->st_dev[s], sz));
+      for (cudaEvent_t &e : c->st_ev[s]) CU(cudaEventCreate(&e));
+    }
+  }
+  auto settle = [&](int s) -> int {  // the launch of staging buffer s is done: account for its times
+    CU(cudaEventSynchronize(c->st_ev[s][2]));
+    if (c->st_pending[s]) {
+      float a = 0, b = 0;
+      CU(cudaEventElapsedTime(&a, c->st_ev[s][0], c->st_ev[s][1]));
+      CU(cudaEventElapsedTime(&b, c->st_ev[s][1], c->st_ev[s][2]));
+      c->xfer_ms += a;
+      c->kernel_ms += b;
+      c->st_pending[s] = false;
+    }
+    return MG_OK;
+  };
+  uint64_t i = 0, part = 0, byte = 0;  // next run, its next part's first base (a multiple of 4), its first byte
+  uint32_t skip = 0;                    // windows of that part counted with the previous one
+  uint64_t nd = 0, launched = 0;        // distinct keys at the last look, bases launched since
+  int s = 0;
+  int rc = counter_reserve(c, 0, &nd);
+  if (rc) return rc;
+  while (i < n_runs) {
+    uint64_t budget = c->st_bytes;
+    if (c->max_slots) {
+      uint64_t lim = 1;
+      while (lim * 2 <= c->max_slots) lim *= 2;
+      lim /= 2;  // distinct keys the largest table allowed holds
+      if (nd + launched + lim / 8 > lim) {  // the bound leaves too little: count the keys after the last launch
+        rc = counter_reserve(c, 0, &nd);
+        if (rc) return rc;
+        launched = 0;
+      }
+      const uint64_t ub = nd + launched, room = lim > ub ? lim - ub : 0;
+      if (room < lim / 8)
+        return set_err(MG_ERR_NOMEM, "the k-mer table limit of %llu slots is reached (%llu distinct k-mers)",
+                       (unsigned long long)c->max_slots, (unsigned long long)ub);
+      budget = std::min(budget, room / 4);
+    }
+    rc = settle(s);
+    if (rc) return rc;
+    uint8_t *hb = c->st_host[s];
+    uint32_t *h_off = reinterpret_cast<uint32_t *>(hb + c->st_bytes + 64), *h_len = h_off + c->st_runs;
+    uint64_t nb = 0, nr = 0;
+    const uint32_t skip0 = skip;
+    while (i < n_runs && nr < c->st_runs) {
+      const uint64_t len = run_len[i], rem = len - part, rem_b = (rem + 3) / 4;
+      if (nb + rem_b <= budget) {  // the rest of the run
+        memcpy(hb + nb, packed + byte + part / 4, rem_b);
+        h_off[nr] = (uint32_t)nb;
+        h_len[nr++] = (uint32_t)rem;
+        nb += rem_b;
+        byte += (len + 3) / 4;
+        part = 0;
+        skip = 0;
+        ++i;
+        continue;
+      }
+      if (nr) break;  // the run starts the next chunk
+      // a part of budget bytes; the next part starts k-1 bases before its end, rounded down to a byte
+      memcpy(hb, packed + byte + part / 4, budget);
+      h_off[0] = 0;
+      h_len[0] = (uint32_t)(4 * budget);
+      nb = budget;
+      nr = 1;
+      const uint64_t end = part + 4 * budget, next = (end - (k - 1)) & ~3ull;
+      skip = (uint32_t)(end - next - (k - 1));
+      part = next;
+      break;
+    }
+    rc = counter_reserve(c, 4 * nb, &nd);
+    if (rc) return rc;
+    launched = 4 * nb;
+    uint8_t *db = c->st_dev[s];
+    const uint32_t *d_off = reinterpret_cast<const uint32_t *>(db + c->st_bytes + 64), *d_len = d_off + c->st_runs;
+    CU(cudaEventRecord(c->st_ev[s][0], c->st));
+    CU(cudaMemcpyAsync(db, hb, nb, cudaMemcpyHostToDevice, c->st));
+    CU(cudaMemcpyAsync(db + c->st_bytes + 64, h_off, nr * 4, cudaMemcpyHostToDevice, c->st));
+    CU(cudaMemcpyAsync(db + c->st_bytes + 64 + c->st_runs * 4, h_len, nr * 4, cudaMemcpyHostToDevice, c->st));
+    CU(cudaEventRecord(c->st_ev[s][1], c->st));
+    const uint64_t n_pos = 4 * nb;
+    const int grid = (int)((n_pos + mg::CNT_TILE - 1) / mg::CNT_TILE);
+    c->launches++;
+    auto kern = c->k == 43 ? mg::k_count_packed<43> : mg::k_count_packed<0>;
+    kern<<<grid, mg::CNT_THREADS, 0, c->st>>>(db, d_off, d_len, (uint32_t)nr, n_pos, skip0, c->k, c->table,
+                                              (1ull << c->log2cap) - 1, c->part_bits, c->part_lo, c->part_hi,
+                                              c->d_scalars, c->d_scalars + 1);
+    CU(cudaGetLastError());
+    CU(cudaEventRecord(c->st_ev[s][2], c->st));
+    c->st_pending[s] = true;
+    s ^= 1;
+  }
+  for (int t = 0; t < 2; ++t) {
+    rc = settle(t);
+    if (rc) return rc;
   }
   return MG_OK;
 }
@@ -1945,6 +2239,9 @@ extern "C" int mg_count_add(mg_counter *c, const char *bases, uint64_t n) {
 extern "C" int mg_count_finish(mg_counter *c, uint32_t min_count, uint32_t counter_max, uint64_t max_count,
                                uint64_t *n_kmers) {
   if (!c) return set_err(MG_ERR_ARG, "NULL counter");
+  if (c->overflowed)
+    return set_err(MG_ERR_STATE, "mg_count_finish on an overflowed counter: its counts are incomplete (count the "
+                                 "packed copy in prefix-partitioned passes)");
   CU(cudaSetDevice(c->device));
   cudaFree(c->out_keys);
   cudaFree(c->out_counts);
@@ -1962,10 +2259,15 @@ extern "C" int mg_count_finish(mg_counter *c, uint32_t min_count, uint32_t count
   CU(cudaStreamSynchronize(c->st));
   if (n) {
     DevFree k0, v0, tmp;
-    CU(cudaMalloc(&k0.p, n * 16));
-    CU(cudaMalloc(&v0.p, n * 4));
-    CU(cudaMalloc(&c->out_keys, n * 16));
-    CU(cudaMalloc(&c->out_counts, n * 4));
+    // (device memory that runs out here is MG_ERR_NOMEM, as for the table: a narrower prefix range needs less)
+    for (auto a : {std::make_pair(&k0.p, n * 16), std::make_pair(&v0.p, n * 4),
+                   std::make_pair((void **)&c->out_keys, n * 16), std::make_pair((void **)&c->out_counts, n * 4)})
+      if (cudaMalloc(a.first, a.second) == cudaErrorMemoryAllocation) {
+        cudaGetLastError();
+        return set_err(MG_ERR_NOMEM, "the %llu counted k-mers do not fit in device memory next to the table",
+                       (unsigned long long)n);
+      }
+    CU(cudaGetLastError());
     CU(cudaMemsetAsync(c->d_scalars + 2, 0, 8, c->st));
     c->launches++;
     mg::k_count_emit<<<grid_for(cap, 256), 256, 0, c->st>>>(c->table, cap, min_count, counter_max, max_count,
@@ -1975,7 +2277,11 @@ extern "C" int mg_count_finish(mg_counter *c, uint32_t min_count, uint32_t count
     size_t tb = 0;
     CU(cub::DeviceRadixSort::SortPairs(nullptr, tb, (u128 *)k0.p, c->out_keys, (uint32_t *)v0.p, c->out_counts, (int64_t)n,
                                        mg::KmerDecomposer{}, 0, 2 * c->k, c->st));
-    CU(cudaMalloc(&tmp.p, tb ? tb : 1));
+    if (cudaMalloc(&tmp.p, tb ? tb : 1) == cudaErrorMemoryAllocation) {
+      cudaGetLastError();
+      return set_err(MG_ERR_NOMEM, "the sort of %llu counted k-mers does not fit in device memory next to the table",
+                     (unsigned long long)n);
+    }
     CU(cub::DeviceRadixSort::SortPairs(tmp.p, tb, (u128 *)k0.p, c->out_keys, (uint32_t *)v0.p, c->out_counts, (int64_t)n,
                                        mg::KmerDecomposer{}, 0, 2 * c->k, c->st));
     c->launches++;
@@ -2011,6 +2317,9 @@ extern "C" int mg_count_stats(mg_counter *c, uint64_t *stats, int n) {
   if (n >= 5) stats[4] = (uint64_t)(c->kernel_ms * 1e3);
   // (the unrestricted builds do not count windows: without a partition every window they examine is inserted)
   if (n >= 6) stats[5] = c->restrict_to ? sc[3] : sc[1];
+  if (n >= 7) stats[6] = c->overflowed ? 1 : 0;
+  if (n >= 8) stats[7] = (uint64_t)(c->xfer_ms * 1e3);
+  if (n >= 9) stats[8] = (uint64_t)(c->pack_ms * 1e3);
   return MG_OK;
 }
 
